@@ -10,11 +10,17 @@ A "step" is one fused step+obs pass over the whole resident batch (the synchrono
 5 agents, 4096 envs per GPU, uniform random actions, yaml-default extra_args.  Weak scaling: every rank owns 4096
 envs keyed by global env id; no collective on the step path.
 
-Timing: the K steps are captured as CUDA graphs (launch-bound inner loop), every graph is replayed once untimed (graph
-upload, TLB warm-up over the observation ring), then R >= 5 replays of the K-step schedule are timed one by one with CUDA
-events on the launch stream, bracketed by a barrier + synchronize; `ms_per_step` is the MEDIAN replay / K, MAX over ranks
-(min / median / max are all in the line).  Observations go round-robin into a ring of buffers larger than L2.
-Prints ONE JSON line on rank 0.
+Timing: exactly K = --steps steps are timed.  They are split into R replays of near-equal length (one per 1000 steps, at
+most 20; --replays overrides), each captured as CUDA graphs (launch-bound inner loop).  The same schedule is
+first run once untimed (graph upload, TLB warm-up over the observation ring), then the R replays are timed one by one with
+CUDA events on the launch stream, bracketed by a barrier + synchronize; `ms_per_step` is the MEDIAN over replays of replay
+time / replay steps, MAX over ranks (min / median / max replay times are all in the line).  Observations go round-robin
+into a ring of buffers larger than L2.  Prints ONE JSON line on rank 0.
+
+    python bench.py --steps 2000 --warmup 100 --dump-outputs DIR
+
+writes what the last timed step returned as DIR/<name>.npy (see dump_outputs); the inputs depend on the arguments only, so
+two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                                # the benchmark leaves the tree as it found it
 
 WORKLOADS = {
     # name: (env, map, num_agents, view_size, envs_per_gpu, BASELINE.json config it is)
@@ -51,12 +58,16 @@ METRIC = "agent-steps/sec (step+obs, device-timed)"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20000)
+    ap.add_argument("--steps", type=int, default=20000, help="number of timed steps K of the headline workload")
     ap.add_argument("--warmup", type=int, default=500)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="harvest5_b4096", choices=sorted(WORKLOADS))
     ap.add_argument("--envs", type=int, default=0, help="override envs per GPU")
-    ap.add_argument("--replays", type=int, default=0, help="timed replays of the K-step schedule (0 = auto, >= 5)")
+    ap.add_argument("--replays", type=int, default=0,
+                    help="the K timed steps are split into this many individually timed replays (0 = auto: one per 1000 steps, <= 20)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (obs, reward, clean, apple_cnt, done) as "
+                         "DIR/<name>.npy (float32; obs of a fixed sample of envs); rank 0's envs only")
     ap.add_argument("--groups", type=int, default=0,
                     help="step the batch as G independent env ranges on G streams (SSDBatchEnv.step_range, the asynchronous-sampler "
                          "API BatchedEpisodeRunner uses with args.env_groups); 0 = auto: 8 ranges for <= 4096 envs, 4 for <= 8192, else 1")
@@ -474,15 +485,24 @@ def auto_groups(B):
     return 1
 
 
+def replay_lengths(K, replays):
+    """K timed steps as `replays` replays of near-equal length (they sum to K)."""
+    R = max(1, min(replays, K))
+    q, r = divmod(K, R)
+    return [q + (i < r) for i in range(R)]
+
+
 def measure(cfg, a, dev, rank, world, K, warmup, replays, groups=1, clock=None, dist=None):
-    """Warm-up, one untimed pass over every graph of the schedule, then `replays` individually timed K-step replays."""
+    """Warm-up, one untimed pass over the schedule of the timed part, then exactly K timed steps as `replays` individually
+    timed replays."""
     import torch
     ro = DeviceRollout(cfg, a, dev, gid_base=rank * cfg["envs_per_gpu"] if "gid_base" not in cfg else cfg["gid_base"], groups=groups)
     ro.eager(max(warmup, 3))
-    ro.stream.synchronize()
-    cycle = LIMIT // math.gcd(K, LIMIT) if K <= 1000 else 1    # distinct schedule phases a K-step replay can start at
-    for _ in range(cycle):
-        ro.enqueue(K)                                          # untimed: captures + uploads every graph the timed part uses
+    lens = replay_lengths(K, replays)
+    s0 = ro.s
+    for k in lens:
+        ro.enqueue(k)                                          # untimed: captures + uploads every graph the timed part uses
+    ro.eager((s0 - ro.s) % LIMIT)                              # back to the same schedule phase, so the timed part reuses them
     ro.stream.synchronize()
 
     def barrier():
@@ -490,30 +510,56 @@ def measure(cfg, a, dev, rank, world, K, warmup, replays, groups=1, clock=None, 
             dist.barrier()
         torch.cuda.synchronize()
 
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(replays + 1)]
+    evs = [torch.cuda.Event(enable_timing=True) for _ in range(len(lens) + 1)]
     launches = 0
     barrier()
     ctx = clock if clock is not None else _Null()
     with ctx:
+        with torch.cuda.stream(ro.stream):
+            torch.cuda._sleep(2 * 10 ** 6)                    # ~1 ms spin: the first replay is queued before the clock starts
         evs[0].record(ro.stream)
-        for r in range(replays):
-            launches += ro.enqueue(K)
+        s_start = ro.s
+        for r, k in enumerate(lens):
+            launches += ro.enqueue(k)
             evs[r + 1].record(ro.stream)
+        timed_steps = ro.s - s_start
         if clock is not None:
             clock.sample()                                    # the GPU is still executing the enqueued replays here
         barrier()
-    per = np.array([evs[r].elapsed_time(evs[r + 1]) for r in range(replays)])      # ms per K-step replay
-    stats = torch.tensor([np.median(per), per.min(), per.max(), per.sum()], device=dev, dtype=torch.float64)
+    per = np.array([evs[r].elapsed_time(evs[r + 1]) for r in range(len(lens))])  # ms per replay
+    per_step = per / np.array(lens)
+    stats = torch.tensor([np.median(per_step), np.median(per), per.min(), per.max(), per.sum()], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(stats, op=dist.ReduceOp.MAX)
-    med, mn, mx, tot = (float(x) for x in stats)
+    ms_step, med, mn, mx, tot = (float(x) for x in stats)
     env = ro.env
     B, n = env.B, env.n
     alg = env.bytes_per_env_step() * B
-    res = dict(ms_per_step=med / K, value=B * n * world * K / (med * 1e-3), replay_ms={"min": mn, "median": med, "max": mx},
-               replays=replays, launches=launches, launches_per_replay=launches / replays, alg_bytes=alg,
+    res = dict(ms_per_step=ms_step, value=B * n * world / (ms_step * 1e-3), replay_ms={"min": mn, "median": med, "max": mx},
+               steps=K, timed_steps=timed_steps, env_steps=ro.s, replays=len(lens), launches=launches, alg_bytes=alg,
                bytes_per_env_step=env.bytes_per_env_step(), obs_bytes=ro.obs_bytes, ring_n=ro.ring_n, total_ms=tot)
     return res, ro
+
+
+def dump_outputs(ro, out_dir, obs_envs=256, envs=65536):
+    """Writes what the last timed step returned as float32 ``out_dir/<name>.npy``: ``reward`` / ``clean`` [E, n] and
+    ``apple_cnt`` / ``done`` [E] of the envs listed in ``envs`` (all of them up to 65 536), and ``obs`` [S, n, 3, N, N] (u8
+    pixel values) of the envs listed in ``obs_envs`` (a fixed sample of 256).  The samples depend on the batch size only;
+    at most ~60 MB in all."""
+    env = ro.env
+    B = env.B
+
+    def pick(cap):
+        return np.arange(B) if B <= cap else np.sort(np.random.RandomState(0).choice(B, cap, replace=False))
+    e_idx, o_idx = pick(envs), pick(obs_envs)
+    ei, oi = (ro.torch.as_tensor(i, device=env.device) for i in (e_idx, o_idx))
+    obs = env.obs_view(ro.ring[ro.s % ro.ring_n])             # step t wrote its observations to ring[(t + 1) % ring_n]
+    out = {"reward": env.reward[ei], "clean": env.clean[ei], "apple_cnt": env.apple_cnt[ei], "done": env.done[ei],
+           "obs": obs[oi], "envs": e_idx, "obs_envs": o_idx}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        v = v.cpu().numpy() if hasattr(v, "cpu") else v
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v, dtype=np.float32))
 
 
 class _Null:
@@ -532,7 +578,11 @@ def hbm_peak():
 
 
 def auto_replays(a, K):
-    return a.replays if a.replays > 0 else int(max(5, min(200, 60000 // max(K, 1))))
+    """Replays the K timed steps are split into: one per 1000 steps, 1 to 20 (--replays overrides).  A replay ends when
+    its slowest env range does, so shorter replays cost time per step: 100-step replays +0.7-0.9% over 1000-step ones at
+    4096 envs in 8 ranges (profiles/r3_replay_length.jsonl, B200 at a 1000 W power limit).  Below 2000 steps that leaves one
+    replay, which the line's `timing` says."""
+    return a.replays if a.replays > 0 else max(1, min(20, K // 1000))
 
 
 def run_b200(a):
@@ -556,7 +606,7 @@ def run_b200(a):
         a.groups = auto_groups(B)
     single = None
     if a.groups > 1:                                          # the same K steps as ONE launch per step, for the record
-        r1, ro1 = measure(cfg, a, dev, rank, world, K, a.warmup, max(5, R // 4), groups=1, dist=dist)
+        r1, ro1 = measure(cfg, a, dev, rank, world, K, a.warmup, max(1, R // 4), groups=1, dist=dist)
         single = {"us_per_step": r1["ms_per_step"] * 1e3, "value": r1["value"],
                   "frac": r1["alg_bytes"] / (r1["ms_per_step"] * 1e-3) / 1e9 / hbm_peak()[0],
                   "what": "same workload, one ssd_step launch per step over the whole batch (--groups 1)"}
@@ -564,6 +614,8 @@ def run_b200(a):
         del ro1
         torch.cuda.empty_cache()
     res, ro = measure(cfg, a, dev, rank, world, K, a.warmup, R, groups=a.groups, clock=clk, dist=dist)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(ro, a.dump_outputs)
     env = ro.env
     peak, peak_src = hbm_peak()
 
@@ -607,7 +659,7 @@ def run_b200(a):
                 c2["envs_per_gpu"], c2["global_envs"], c2["gid_base"] = hi - lo, WORKLOADS[name][4], lo
             try:
                 g2 = auto_groups(c2["envs_per_gpu"])
-                r2, ro2 = measure(c2, a, dev, rank, world, LIMIT, 5, 7, groups=g2, dist=dist)
+                r2, ro2 = measure(c2, a, dev, rank, world, 7 * LIMIT, 5, 7, groups=g2, dist=dist)
                 ro2.close()
                 del ro2
                 torch.cuda.empty_cache()
@@ -628,15 +680,17 @@ def run_b200(a):
             traffic = json.load(open(tpath)).get(a.workload, {}).get("dram_bytes_per_launch")
         d2h = B * (2 * n + 2 + 1) + obs_bytes
         line = {"metric": METRIC, "value": res["value"], "unit": "agent-steps/s", "n_gpus": world, "steps": K,
+                "timed_steps": res["timed_steps"], "env_steps": res["env_steps"],
                 "warmup": max(a.warmup, 3), "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "u8", "data": "synthetic", "config": cfg,
-                "replays": R, "replay_ms": res["replay_ms"],
-                "timing": "median of `replays` individually event-timed replays of the K-step CUDA-graph schedule, after one untimed "
-                          "replay of every graph; MAX over ranks",
+                "replays": res["replays"], "replay_ms": res["replay_ms"],
+                "timing": "the K timed steps as `replays` individually event-timed CUDA-graph replays, after one untimed pass over "
+                          "the same schedule; median over replays of time per step, MAX over ranks"
+                          + ("; ONE replay: a single sample, min = median = max, no spread" if res["replays"] == 1 else ""),
                 "l2": f"obs written round-robin into {res['ring_n']} buffers x {obs_bytes / 2**20:.1f} MiB (> {L2_BYTES >> 20} MiB L2), like an episode buffer",
                 "parallelism": f"env-sharded x{world} (no collective on the step path)" + (f", {a.groups} env ranges on {a.groups} streams" if a.groups > 1 else ""),
-                "clocks": clk.summary(), "gpu_launches": int(round(res["launches_per_replay"])),
-                "gpu_launches_how": "ssd_launch_count deltas recorded while each graph was captured, summed over the graphs of one K-step replay",
+                "clocks": clk.summary(), "gpu_launches": res["launches"],
+                "gpu_launches_how": "ssd_launch_count deltas recorded while each graph was captured, summed over the graphs of the K timed steps",
                 "launch_mode": "cuda-graph" if not a.no_graph else "python-loop",
                 "e2e": {"value": B * n * world * e2e_steps / (e2e_ms * 1e-3), "unit": "agent-steps/s",
                         "h2d_bytes_per_step": B * n, "d2h_bytes_per_step": d2h, "steps": e2e_steps,
@@ -685,4 +739,6 @@ def run_b200(a):
 
 if __name__ == "__main__":
     args = parse()
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs writes the outputs of the CUDA arm; it has no meaning with --impl reference")
     sys.exit(run_reference(args) if args.impl == "reference" else run_b200(args))

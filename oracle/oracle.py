@@ -6,9 +6,11 @@ legs only; never by ``homophily_marl_b200``.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -18,12 +20,21 @@ _lib = None
 
 
 def build(force: bool = False) -> str:
-    """Compile the C restatement with gcc (OpenMP when the toolchain has it)."""
+    """Compile the C restatement with gcc (OpenMP when the toolchain has it).  In a read-only tree the library is built
+    once per source version into a per-user cache in the temporary directory; returns the path of the library."""
     src = os.path.join(HERE, "ssd_oracle.c")
     hdr = os.path.join(HERE, "ssd_oracle.h")
     if not force and os.path.exists(LIB_PATH) and os.path.getmtime(LIB_PATH) >= max(os.path.getmtime(src), os.path.getmtime(hdr)):
         return LIB_PATH
-    base = ["-O2", "-ffp-contract=off", "-fPIC", "-std=c11", "-shared", "-o", LIB_PATH, src, "-lm"]
+    out = LIB_PATH
+    if not os.access(HERE, os.W_OK):                          # one cached library per source version and user
+        h = hashlib.sha256(b"".join(open(f, "rb").read() for f in (src, hdr))).hexdigest()[:16]
+        out = os.path.join(tempfile.gettempdir(), f"ssd_oracle_{os.getuid()}", f"libssd_oracle_{h}.so")
+        if os.path.exists(out) and not force:
+            return out
+        os.makedirs(os.path.dirname(out), exist_ok=True)
+    tmp = f"{out}.{os.getpid()}.tmp"
+    base = ["-O2", "-ffp-contract=off", "-fPIC", "-std=c11", "-shared", "-o", tmp, src, "-lm"]
     errors = []
     for cc in ("/usr/bin/gcc", shutil.which("gcc"), os.environ.get("CC"), shutil.which("cc")):
         if not cc or not os.path.exists(cc):
@@ -31,7 +42,8 @@ def build(force: bool = False) -> str:
         for omp in (["-fopenmp"], []):
             r = subprocess.run([cc] + omp + base, capture_output=True, text=True)
             if r.returncode == 0:
-                return LIB_PATH
+                os.replace(tmp, out)                          # atomic: concurrent processes never load a partial file
+                return out
             errors.append(r.stderr[-300:])
     raise RuntimeError("could not build the oracle: " + " | ".join(errors))
 
@@ -39,8 +51,7 @@ def build(force: bool = False) -> str:
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(LIB_PATH)
+        L = C.CDLL(build())
         L.ssdo_sizeof_map.restype = C.c_ulong
         L.ssdo_sizeof_env.restype = C.c_ulong
         L.ssdo_map_init.restype = C.c_int

@@ -11,6 +11,14 @@ BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_ste
              "vs_baseline", "dtype", "data", "config", "e2e", "cpu_baseline"}
 
 
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
 def _run(args, env=None):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True,
                        env={**os.environ, **(env or {})}, timeout=600)
@@ -50,12 +58,12 @@ def test_reference_arm_times_the_reference_training_loop():
 
 @pytest.mark.gpu
 def test_cuda_arm_line():
-    lines = _run(["--steps", "300", "--warmup", "20", "--envs", "512", "--e2e-steps", "5", "--no-extra", "--no-train"])
+    lines = _run(["--steps", "5000", "--warmup", "20", "--envs", "512", "--e2e-steps", "5", "--no-extra", "--no-train"])
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert BASE_KEYS | {"clocks", "gpu_launches", "roofline"} <= set(d)
-    assert d["n_gpus"] == 1 and d["steps"] == 300 and d["scaling"] == "weak" and d["dtype"] == "u8"
-    assert d["gpu_launches"] >= 300
+    assert d["n_gpus"] == 1 and d["steps"] == 5000 and d["scaling"] == "weak" and d["dtype"] == "u8"
+    assert d["gpu_launches"] >= 5000
     r = d["roofline"]
     assert r["bound"] == "hbm" and r["unit"] == "GB/s" and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9
     e = d["e2e"]
@@ -66,12 +74,66 @@ def test_cuda_arm_line():
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
 
 
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(tmp_path):
+    """--dump-outputs: what the last timed step returned, float32, identical in two runs with the same arguments and with
+    graphs + 8 env ranges or a Python loop + one launch per step, and equal to an oracle rollout of sampled envs with the
+    same seed and actions for the same number of steps.  The launch counter of the Python-loop run pins the timed steps."""
+    import numpy as np
+    import torch
+    from homophily_marl_b200 import mapspec
+    from oracle import oracle as O
+    B, K, W = 512, 250, 7
+    args = ["--steps", str(K), "--replays", "2", "--warmup", str(W), "--envs", str(B), "--e2e-steps", "1", "--no-extra",
+            "--no-train", "--no-cpu-baseline"]
+    lines, dumps = [], []
+    for k, more in enumerate(([], [], ["--no-graph", "--groups", "1"])):
+        out = tmp_path / str(k)
+        d = json.loads(_run(args + more + ["--dump-outputs", str(out)])[0])
+        assert d["steps"] == K and d["timed_steps"] == K and d["replays"] == 2
+        assert sum(f.stat().st_size for f in out.iterdir()) <= 64 * 10 ** 6
+        lines.append(d)
+        dumps.append({f.stem: np.load(f) for f in out.iterdir()})
+    a = dumps[0]
+    assert set(a) == {"reward", "clean", "apple_cnt", "done", "obs", "envs", "obs_envs"}
+    for b in dumps[1:]:
+        for k in a:
+            assert a[k].dtype == np.float32 and np.array_equal(a[k], b[k]), k
+    T = lines[0]["env_steps"]
+    assert T == lines[2]["env_steps"] and T >= W + K
+    assert lines[2]["gpu_launches"] == K + sum(t % 100 == 0 for t in range(T - K, T))       # one step launch + resets
+    assert a["reward"].shape == (B, 5) and a["done"].shape == (B,) and np.array_equal(a["envs"], np.arange(B))
+    assert a["obs"].shape == (256, 5, 3, 31, 31) and len(np.unique(a["obs_envs"])) == 256
+
+    spec = mapspec.compile_map("harvest", "default5", 5, 15, 100, obs_color="simplified")
+    g = torch.Generator(device="cuda").manual_seed(0)                                         # bench.py DeviceRollout, seed 0
+    acts = torch.randint(0, spec.n_actions, (100, B, 5), generator=g, device="cuda", dtype=torch.int32).to(torch.uint8).cpu().numpy()
+    for j in (0, 101, 255):
+        e = int(a["obs_envs"][j])
+        ob = O.OracleBatch.from_spec(spec, n_envs=1, seed=0, env_gid0=e, random_spawn_point=False, spawn_rotation=0)
+        for t in range(T):
+            if t % 100 == 0:
+                ob.reset()
+            o = ob.step(acts[t % 100, e:e + 1])
+        assert np.array_equal(a["obs"][j], o["obs"][0]), e
+        assert np.array_equal(a["reward"][e], o["reward"][0]) and np.array_equal(a["clean"][e], o["clean"][0]), e
+        assert a["apple_cnt"][e] == o["apple_cnt"][0] and a["done"][e] == o["done"][0], e
+
+
+def test_timed_steps_are_the_steps_argument():
+    """--steps K times exactly K steps, split into replays of near-equal length."""
+    bench = _bench_module()
+    for K in (1, 7, 99, 100, 250, 20000, 20001):
+        for R in (1, 3, 20, 200):
+            lens = bench.replay_lengths(K, R)
+            assert sum(lens) == K and len(lens) == min(R, K) and max(lens) - min(lens) <= 1
+    auto = lambda K: bench.auto_replays(type("A", (), {"replays": 0}), K)  # noqa: E731
+    assert [auto(K) for K in (1, 999, 2000, 5500, 20000, 50000)] == [1, 1, 2, 5, 20, 20]
+
+
 def test_env_range_rule():
     """Small batches are stepped as env ranges (profiles/r2_notes.md sections 2-3); every range size must divide the batch."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
-    bench = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(bench)
+    bench = _bench_module()
     assert [bench.auto_groups(b) for b in (512, 2048, 4096, 8192, 16384, 65536, 4095, 10000)] == [8, 8, 8, 4, 8, 1, 1, 1]
     for b in (512, 2048, 4096, 8192, 16384):
         assert b % bench.auto_groups(b) == 0

@@ -27,7 +27,7 @@ class SsdConfig(C.Structure):
                 ("height", C.c_int32), ("width", C.c_int32), ("view", C.c_int32),
                 ("episode_limit", C.c_int32), ("fire_cost", C.c_int32), ("hit_penalty", C.c_int32),
                 ("beam_len", C.c_int32), ("random_spawn_point", C.c_int32), ("spawn_rotation", C.c_int32),
-                ("device", C.c_int32), ("reserved0", C.c_int32),
+                ("device", C.c_int32), ("tag_timeout", C.c_int32),
                 ("seed", C.c_uint64), ("env_gid_base", C.c_uint32), ("n_waste_lut", C.c_uint32),
                 ("ascii_map", C.c_char_p), ("thr_apple", C.c_void_p), ("thr_waste", C.c_void_p),
                 ("thr_harvest", C.c_uint32 * 4), ("color_lut", (C.c_uint8 * 4) * 16)]

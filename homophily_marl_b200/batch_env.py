@@ -36,14 +36,16 @@ class SSDBatchEnv:
     def __init__(self, name, n_envs, num_agents, map="default", view_size=7, episode_limit=100,
                  extra_args=None, seed=0, device="cuda:0", env_gid_base=0, rows=None, params=None,
                  fire_cost=1, hit_penalty=0, want_state=False, check_actions=False):
+        # tag_timeout: steps an agent hit by a FIRE ray is out of play (off the map, action ignored, zero view); 0 = never
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
-                     disable_fire_action=True, obs_color="simplified")
+                     disable_fire_action=True, obs_color="simplified", tag_timeout=0)
         extra.update(extra_args or {})
         self.extra_args = extra
         self.name = name
         self.spec = mapspec.compile_map(name, map, num_agents, view_size, episode_limit,
                                         obs_color=extra["obs_color"], rows=rows, params=params,
-                                        fire_cost=fire_cost, hit_penalty=hit_penalty)
+                                        fire_cost=fire_cost, hit_penalty=hit_penalty,
+                                        tag_timeout=int(extra["tag_timeout"]))
         self.device = _require_cuda(device)
         # debug switch (one device sync per step): out-of-range action codes raise KeyError like the reference's action_map
         self.check_actions = bool(check_actions) or os.environ.get("SSD_B200_CHECK_ACTIONS") == "1"
@@ -57,6 +59,7 @@ class SSDBatchEnv:
         cfg.kind, cfg.n_envs, cfg.n_agents = s.kind, self.B, s.n_agents
         cfg.height, cfg.width, cfg.view, cfg.episode_limit = s.H, s.W, s.view, s.episode_limit
         cfg.fire_cost, cfg.hit_penalty, cfg.beam_len = s.fire_cost, s.hit_penalty, s.beam_len
+        cfg.tag_timeout = s.tag_timeout
         cfg.random_spawn_point = int(bool(extra["random_spawn_point"]))
         rot = extra["random_spawn_rotation"]
         cfg.spawn_rotation = -1 if rot is None else int(rot)
@@ -128,6 +131,11 @@ class SSDBatchEnv:
     def ep_ret(self):
         return self.ep_ret_buf[:, :self.n]
 
+    @property
+    def tag_out(self):
+        """[B, n] u8: steps each agent is still tagged out (off the map); 0 = in play."""
+        return ((self.agent_buf[:, :self.n] >> 24) & 0xFF).to(torch.uint8)
+
     def set_state(self, b, grid=None, pos_rc=None, orient=None):
         """Test/injection hook (SURVEY 5: get/set_state_tensors)."""
         if grid is not None:
@@ -140,7 +148,7 @@ class SSDBatchEnv:
                 pr = np.asarray(pos_rc, dtype=np.int64)
                 a = (a & ~0xFFFF) | pr[:, 0] | (pr[:, 1] << 8)
             if orient is not None:
-                a = (a & 0xFFFF) | (np.asarray(orient, dtype=np.int64) << 16)
+                a = (a & ~0xFF0000) | (np.asarray(orient, dtype=np.int64) << 16)
             self.agent_buf[b, :self.n] = torch.as_tensor(a.astype(np.int32), device=self.device)
 
     def _recount(self, sel):
@@ -148,20 +156,29 @@ class SSDBatchEnv:
         g = self.grid_buf[sel, :self.G]
         self.counts_buf[sel] = ((g == 2).sum(1) | ((g == 3).sum(1) << 16)).to(torch.int32)
 
-    def load_state(self, grid=None, pos_rc=None, orient=None, t=None):
-        """Batched variant of ``set_state``: NumPy arrays [B,H,W] / [B,n,2] / [B,n] / [B]."""
+    def load_state(self, grid=None, pos_rc=None, orient=None, t=None, tag_out=None):
+        """Batched variant of ``set_state``: NumPy arrays [B,H,W] / [B,n,2] / [B,n] / [B]; ``tag_out`` [B,n] sets the
+        tagging-out timers (non-zero only with ``tag_timeout`` > 0)."""
         if grid is not None:
             g = np.ascontiguousarray(grid, dtype=np.uint8).reshape(self.B, self.G)
             self.grid_buf[:, :self.G] = torch.as_tensor(g, device=self.device)
             self._recount(slice(None))
-        if pos_rc is not None or orient is not None:
+        if tag_out is not None:
+            tag_out = np.asarray(tag_out, dtype=np.int64)
+            if tag_out.any() and self.spec.tag_timeout == 0:
+                raise ValueError("tag_out needs tag_timeout > 0: with tag_timeout 0 the kernels ignore the timers")
+            if tag_out.min(initial=0) < 0 or tag_out.max(initial=0) > 255:
+                raise ValueError("tag_out must be in 0..255")
+        if pos_rc is not None or orient is not None or tag_out is not None:
             a = self.agent_buf[:, :self.n].cpu().numpy().astype(np.int64)
             if pos_rc is not None:
                 pr = np.asarray(pos_rc, dtype=np.int64)
                 a = (a & ~0xFFFF) | pr[..., 0] | (pr[..., 1] << 8)
             if orient is not None:
-                a = (a & 0xFFFF) | (np.asarray(orient, dtype=np.int64) << 16)
-            self.agent_buf[:, :self.n] = torch.as_tensor(a.astype(np.int32), device=self.device)
+                a = (a & ~0xFF0000) | (np.asarray(orient, dtype=np.int64) << 16)
+            if tag_out is not None:
+                a = (a & 0xFFFFFF) | (tag_out << 24)
+            self.agent_buf[:, :self.n] = torch.as_tensor((a & 0xFFFFFFFF).astype(np.uint32).view(np.int32), device=self.device)
         if t is not None:
             self.t_buf.copy_(torch.as_tensor(np.asarray(t, dtype=np.int32), device=self.device))
 

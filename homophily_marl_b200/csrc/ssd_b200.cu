@@ -86,6 +86,7 @@ struct KParams {
     int8_t* reward; uint8_t* clean; uint16_t* apple_cnt; uint8_t* done; uint8_t* obs; uint8_t* state_rgb;
     const uint32_t* d_prio; const uint32_t* d_uapple; const uint32_t* d_uwaste; const uint32_t* d_wkey;
     const uint32_t* d_spawnkey; const uint8_t* d_rot;
+    int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
 };
 
 
@@ -376,13 +377,14 @@ __device__ __forceinline__ void update_moves(const SW& w, const GEO& g, const KP
 constexpr uint8_t kOcc = 0x80;
 
 // ------------------------------------------------------------------ beams (map_env.py:663-769)
-template <class SW, class GEO>
+// TAG: every agent a FIRE ray hits (the one hit_penalty charges) sets `tagged`; it stays on the map until all beams are done.
+template <bool TAG, class SW, class GEO>
 __device__ __forceinline__ void beams(const SW& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent,
-                                      int act, int pos, int ori, int& reward, int& clean_num, int& waste) {
+                                      int act, int pos, int ori, int& reward, int& clean_num, int& waste, bool& tagged) {
     const bool fire = is_agent && act == 7;
     const bool clean = is_agent && act == 8 && g.kind() == SSD_KIND_CLEANUP;
     if (fire) reward -= p.fire_cost;                          // agent.py:188-190, 239-241
-    unsigned need = w.ballot(clean || (fire && p.hit_penalty != 0));
+    unsigned need = w.ballot(clean || (fire && (TAG || p.hit_penalty != 0)));
     while (need) {                                            // agent index order, map effects applied per agent (669-671)
         const int i = __ffs(need) - 1;
         need &= need - 1;
@@ -414,12 +416,15 @@ __device__ __forceinline__ void beams(const SW& w, const GEO& g, const KParams& 
         const unsigned um = w.ballot(upd >= 0);
         if (lane == i && is_clean) clean_num = __popc(um);    // 672-673
         waste -= __popc(um);                                  // only CLEAN produces updates: 'H' -> 'R'
-        if (p.hit_penalty != 0) {                             // hit(): the LAST index standing on the cell (agent.py:184-186)
+        if (TAG || p.hit_penalty != 0) {                      // hit(): the LAST index standing on the cell (agent.py:184-186)
 #pragma unroll
             for (int s = 0; s < 3; ++s) {
                 const int hq = w.shfl(hit, s);
                 const unsigned on = w.ballot(hq >= 0 && pos == hq);
-                if (on && lane == 31 - __clz(on)) reward -= p.hit_penalty;
+                if (on && lane == 31 - __clz(on)) {
+                    reward -= p.hit_penalty;
+                    if (TAG) tagged = true;
+                }
             }
         }
     }
@@ -515,6 +520,36 @@ __device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& 
     waste += wcell >= 0;
 }
 
+// ------------------------------------------------------------------ agent placement (map_env.py:771-793)
+// The agents in `who` take, in index order, the free spawn point with the largest (key, cell); lanes are spawn points.  At reset
+// every point is free; a respawn after tagging-out (RESPAWN) also skips the points in-play agents stand on (occupancy bits).
+template <bool RESPAWN, class SW, class GEO>
+__device__ __forceinline__ void place_agents(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, int lane, int env,
+                                             uint32_t gid, uint32_t tick, unsigned who, int& pos) {
+    const bool is_sp = lane < p.n_spawn;
+    const int mycell = is_sp ? (int)__ldg(&p.map->spawn_pts[lane]) : -1;
+    bool taken = RESPAWN && is_sp && (sg[mycell] & kOcc);
+    for (int i = 0; i < p.n; ++i) {
+        if (!((who >> i) & 1u)) continue;
+        uint32_t key = 0;
+        if (p.random_spawn && is_sp)
+            key = p.d_spawnkey ? p.d_spawnkey[((size_t)env * p.n + i) * g.G() + mycell]
+                               : philox_word(p, gid, tick, 3u, (uint32_t)(i * p.n_spawn + lane));
+        const bool cand = is_sp && !taken;
+        const uint32_t mk = w.rmax(cand ? key : 0u);
+        const unsigned eq = w.ballot(cand && key == mk);
+        const int win = 31 - __clz(eq);
+        const int cell = w.shfl(mycell, win);
+        if (lane == win) taken = true;
+        if (lane == i) pos = cell;
+    }
+}
+// spawn_rotation (map_env.py:786-793)
+__device__ __forceinline__ int spawn_orientation(const KParams& p, int env, uint32_t gid, uint32_t tick, int lane) {
+    if (p.spawn_rot >= 0) return p.spawn_rot;
+    return p.d_rot ? (int)(p.d_rot[(size_t)env * p.n + lane] & 3) : (int)(philox_word(p, gid, tick, 4u, (uint32_t)lane) >> 30);
+}
+
 // ------------------------------------------------------------------ render (map_env.py:360-379, 418-446, 795-815, 923-957)
 #ifndef SSD_ST_HINT
 #define SSD_ST_HINT ""                                        // cache operator of the observation stores (see profiles/r1_notes.md)
@@ -555,15 +590,17 @@ struct RowUnit {                                              // one (agent, y) 
     const uint32_t* w;
     uint8_t* dst;
     uint32_t sh, rev;
+    uint32_t keep;                                            // 0 for the rows of an agent that is out of play: written as zeros
     bool valid;
 };
 
 template <int OCT_T, class SW, class GEO>
 __device__ __forceinline__ void fetch_row(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane, int it, int units,
-                                          uint32_t abase_sh, int astep, RowUnit<OCT_T>& U) {
+                                          uint32_t abase_sh, int astep, unsigned outm, RowUnit<OCT_T>& U) {
     const int u = it * SW::kLanes + lane;
     U.valid = u < units;
     const int al = U.valid ? g.divN(u) : 0;
+    U.keep = ((outm >> al) & 1u) ? 0u : 0xffffffffu;
     const int y = u - al * g.N();
     const uint32_t ab = w.shfl(abase_sh, al);
     const int as = w.shfl(astep, al);
@@ -597,7 +634,7 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
         for (int k = 0; k < OCT_T; ++k) { v[2 * k] = __funnelshift_r(U.L[k], U.L[k + 1], sh); v[2 * k + 1] = v[2 * k] >> 16; }
 #pragma unroll
         for (int pl = 0; pl < 3; ++pl) {                      // one colour plane at a time: 2*OCT PRMTs, then one wide store
-            const uint32_t t0 = p.lut8[2 * pl], t1 = p.lut8[2 * pl + 1];
+            const uint32_t t0 = p.lut8[2 * pl] & U.keep, t1 = p.lut8[2 * pl + 1] & U.keep;
             uint32_t o[2 * OCT_T];
 #pragma unroll
             for (int k = 0; k < 2 * OCT_T; ++k) o[k] = prmt(t0, t1, v[k]);
@@ -618,7 +655,7 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
                 const uint32_t m = wd == WR - 1 ? lastmask : 0xffffffffu;
 #pragma unroll
                 for (int pl = 0; pl < 3; ++pl)
-                    *reinterpret_cast<uint32_t*>(U.dst + pl * g.PS() + 4 * wd) = prmt(p.lut8[2 * pl], p.lut8[2 * pl + 1], v) & m;
+                    *reinterpret_cast<uint32_t*>(U.dst + pl * g.PS() + 4 * wd) = prmt(p.lut8[2 * pl], p.lut8[2 * pl + 1], v) & m & U.keep;
             }
         }
     }
@@ -626,14 +663,14 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
 
 template <int OCT_T, class SW, class GEO>
 __device__ __forceinline__ void gather_rows(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane,
-                                            uint32_t abase_sh, int astep) {
+                                            uint32_t abase_sh, int astep, unsigned outm) {
     const int WR = g.RP() >> 2;
     const uint32_t lastmask = 0xffffffffu >> (8 * (4 * WR - g.N()));
     const int units = p.n * g.N(), iters = (units + SW::kLanes - 1) / SW::kLanes;
     RowUnit<OCT_T> cur, nxt;
-    fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, cur);
+    fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, outm, cur);
     for (int it = 0; it < iters; ++it) {                      // software pipeline: row it+1 is fetched while row it is emitted
-        if (it + 1 < iters) fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, it + 1, units, abase_sh, astep, nxt);
+        if (it + 1 < iters) fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, it + 1, units, abase_sh, astep, outm, nxt);
         emit_row<OCT_T>(g, p, cur, lastmask);
         cur = nxt;
     }
@@ -718,7 +755,7 @@ __device__ __forceinline__ void fill_outside(const SW& w, const GEO& g, const KP
 // written into the staged grid as index 7 by the caller.
 template <bool COLS, class SW, class GEO>
 __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, const uint8_t* rank2lane,
-                                             uint8_t* gobs, int lane, uint32_t apack, int n_in_class) {
+                                             uint8_t* gobs, int lane, uint32_t apack, int n_in_class, unsigned outm) {
     const int N = g.N(), V = g.V(), W = g.W(), units = n_in_class * N, WR = g.RP() >> 2;
     const uint32_t lastmask = 0xffffffffu >> (8 * (4 * WR - N));
     for (int u0 = 0; u0 < units; u0 += SW::kLanes) {
@@ -774,9 +811,10 @@ __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KP
         }
         const uint32_t v[4] = { n0, n0 >> 16, n1, n1 >> 16 };
         uint8_t* dst = gobs + al * g.AS() + y * g.RP();
+        const uint32_t keep = ((outm >> al) & 1u) ? 0u : 0xffffffffu;       // an agent out of play sees zeros
 #pragma unroll
         for (int pl = 0; pl < 3; ++pl) {
-            const uint32_t t0 = p.lut8[2 * pl], t1 = p.lut8[2 * pl + 1];
+            const uint32_t t0 = p.lut8[2 * pl] & keep, t1 = p.lut8[2 * pl + 1] & keep;
             uint32_t o4[4];
 #pragma unroll
             for (int k = 0; k < 4; ++k) o4[k] = prmt(t0, t1, v[k]);
@@ -795,7 +833,7 @@ __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KP
 // never touched by a gather load) maps (class, rank within class) -> agent lane.
 template <class SW, class GEO>
 __device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* tbl, uint8_t* gobs, int lane,
-                                              bool is_agent, int r0, int c0, int ori) {
+                                              bool is_agent, int r0, int c0, int ori, unsigned outm) {
     const uint32_t apack = (uint32_t)r0 | ((uint32_t)c0 << 8) | ((uint32_t)ori << 16);
     const unsigned m_rows = w.ballot(is_agent && ori >= 2), m_cols = w.ballot(is_agent && ori < 2);
     if (is_agent) {
@@ -803,16 +841,18 @@ __device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const K
         tbl[(cols ? 16 : 0) + __popc((cols ? m_cols : m_rows) & ((1u << lane) - 1u))] = (uint8_t)lane;
     }
     w.sync();
-    if (m_rows) gather_class<false>(w, g, p, sg, tbl, gobs, lane, apack, __popc(m_rows));
-    if (m_cols) gather_class<true>(w, g, p, sg, tbl + 16, gobs, lane, apack, __popc(m_cols));
+    if (m_rows) gather_class<false>(w, g, p, sg, tbl, gobs, lane, apack, __popc(m_rows), outm);
+    if (m_cols) gather_class<true>(w, g, p, sg, tbl + 16, gobs, lane, apack, __popc(m_cols), outm);
 }
 
+// live: the lane's agent is on the map; outm: agents out of play (tagged out), whose views are written as zeros.  Their rows go
+// through the same gather at cell (0, 0), masked, so that a warp trip never mixes two kinds of row.
 template <class SW, class GEO>
 __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
-                                       int lane, bool is_agent, int pos, int ori, int env, unsigned same) {
-    const bool top = is_agent && lane == 31 - __clz(same);   // later index overwrites (map_env.py:370); same = lanes on this lane's cell
+                                       int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm) {
+    const bool top = live && lane == 31 - __clz(same);       // later index overwrites (map_env.py:370); same = lanes on this lane's cell
     int r0 = 0, c0 = 0;
-    if (is_agent) { r0 = g.divW(pos); c0 = pos - r0 * g.W(); }
+    if (live) { r0 = g.divW(pos); c0 = pos - r0 * g.W(); }
 
     if (p.state_rgb) {                                        // get_state: unrotated full map (map_env.py:950-957)
         uint8_t* out = p.state_rgb + (size_t)env * 3 * g.G();
@@ -830,7 +870,7 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
     uint8_t* gobs = p.obs + (size_t)env * (p.n * g.AS());
 
     if (g.direct()) {
-        gather_direct(w, g, p, sg, const_cast<uint8_t*>(sg) - g.padF(), gobs, lane, is_agent, r0, c0, ori);
+        gather_direct(w, g, p, sg, const_cast<uint8_t*>(sg) - g.padF(), gobs, lane, is_agent, r0, c0, ori, outm);
     } else {
         // the maps were pre-filled with "outside the map" at kernel start (fill_outside); now the cells (agents are already in
         // the staged grid as index 7)
@@ -844,7 +884,7 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
         const uint32_t abase_sh = (uint32_t)(g.off_map(ori) + (rowc + (down ? 2 * g.V() : 0)) * pitch + ((s >> 3) << 2))
                                   | ((uint32_t)((rev ? 7 - (s & 7) : (s & 7)) * 4) << 16) | ((uint32_t)rev << 24);
         const int astep = down ? -pitch : pitch;
-        const bool needT = w.ballot(is_agent && ori < 2) != 0;
+        const bool needT = w.ballot(live && ori < 2) != 0;
         uint8_t* MT = pmap + g.off_map(0);
         uint8_t* M = pmap + g.off_map(2);
         build_rowmap(w, g, p, sg, M, lane);
@@ -853,8 +893,8 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
             build_colmap(w, g, p, M, MT, lane);
             w.sync();
         }
-        if (g.RP() == 32) gather_rows<4>(w, g, p, pmap, gobs, lane, abase_sh, astep);
-        else gather_rows<0>(w, g, p, pmap, gobs, lane, abase_sh, astep);
+        if (g.RP() == 32) gather_rows<4>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
+        else gather_rows<0>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
     }
     const int tail = g.AS() - 3 * g.PS();                         // pad bytes per agent block (0 for the shipped views)
     if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
@@ -870,7 +910,7 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
             const int al = valid ? q / p.n : 0, j = valid ? q - al * p.n : 0;
             const uint32_t api = w.shfl(apack, al), apj = w.shfl(apack, j);
             const bool topj = w.shfl((int)top, j);
-            if (!valid || !topj) continue;
+            if (!valid || !topj || ((outm >> al) & 1u)) continue;
             const int a = (int)(apj & 1023) - (int)(api & 1023) + g.V(), b = (int)((apj >> 10) & 1023) - (int)((api >> 10) & 1023) + g.V();
             if (a < 0 || a >= g.N() || b < 0 || b >= g.N()) continue;
             const int o = api >> 20;
@@ -885,7 +925,8 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
 }
 
 // ------------------------------------------------------------------ the kernel
-template <int MODE, class GEO, int LPE>
+// TAG: tagging-out timers are on (p.tag_timeout > 0; MODE_STEP and MODE_RENDER only, DESIGN.md §3 item 11).
+template <int MODE, class GEO, int LPE, bool TAG>
 __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const __grid_constant__ KParams p) {
     using SW = SubWarp<LPE>;
     const GEO g(p);
@@ -931,7 +972,7 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
         const uint32_t tick = __ldcg(p.tick + env);
         const int t_prev = MODE == MODE_STEP ? __ldcg(p.t + env) : 0;
         const uint32_t cnt = MODE == MODE_STEP ? __ldcg(p.counts + env) : 0u;
-        const int act = (MODE == MODE_STEP && is_agent) ? (int)__ldcg(p.actions + (size_t)env * p.n + lane) : 255;
+        int act = (MODE == MODE_STEP && is_agent) ? (int)__ldcg(p.actions + (size_t)env * p.n + lane) : 255;
         int pos = -1 - lane, ori = 0, ep_ret = 0;
         uint32_t a_rec = 0;
         if (MODE != MODE_RESET && is_agent) {
@@ -948,9 +989,18 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
             if (lane < n16) reinterpret_cast<uint4*>(sg)[lane] = g0;
             for (int i = lane + SW::kLanes; i < n16; i += SW::kLanes) reinterpret_cast<uint4*>(sg)[i] = __ldcg(src + i);
         }
+        // Tagging-out (TAG): an agent whose timer (bits 24..31 of its record) is non-zero is out of play for the whole step.  Its
+        // lane then acts like a lane without an agent (unique negative pos, no action), and `home` keeps the cell of its record.
+        bool live = is_agent;
+        int timer = 0, home = 0;
         if (MODE != MODE_RESET && is_agent) {
             pos = (int)(a_rec & 0xff) * g.W() + (int)((a_rec >> 8) & 0xff);
             ori = (int)((a_rec >> 16) & 3);
+            if (TAG) {
+                timer = (int)(a_rec >> 24);
+                home = pos;
+                if (timer) { live = false; pos = -1 - lane; act = 255; }
+            }
         }
         w.sync();
 
@@ -961,11 +1011,12 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
         if (MODE == MODE_RENDER) same = equal_lanes(w, pos, p.n);
         if (MODE == MODE_STEP) {
             int reward = 0, clean_num = 0;
-            update_moves(w, g, p, sg, lane, is_agent, act, pos, ori, env, gid, tick);                 // map_env.py:251
+            bool tagged = false;
+            update_moves(w, g, p, sg, lane, live, act, pos, ori, env, gid, tick);                     // map_env.py:251
             // consume in index order: the lowest index on a cell eats the apple (253-256); mark occupancy
-            same = surely_distinct(w, pos, is_agent, w.ballot(is_agent)) ? (1u << lane) : equal_lanes(w, pos, p.n);
-            const int here = is_agent ? sg[pos] : 0;
-            const bool first = is_agent && lane == __ffs(same) - 1;
+            same = surely_distinct(w, pos, live, w.ballot(live)) ? (1u << lane) : equal_lanes(w, pos, p.n);
+            const int here = live ? sg[pos] : 0;
+            const bool first = live && lane == __ffs(same) - 1;
             const unsigned ate = w.ballot(first && here == SSD_CELL_APPLE);
             w.sync();
             if (first) {
@@ -974,8 +1025,28 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
             }
             apples -= __popc(ate);
             w.sync();
-            beams(w, g, p, sg, lane, is_agent, act, pos, ori, reward, clean_num, waste);              // 259-260
+            beams<TAG>(w, g, p, sg, lane, live, act, pos, ori, reward, clean_num, waste, tagged);    // 259-260
+            unsigned gone = 0;
+            if (TAG) {                                 // the tagged leave the map; a cell stays occupied while an untagged agent is on it
+                gone = w.ballot(tagged);
+                if (gone) {
+                    if (live && lane == __ffs(same) - 1 && (same & ~gone) == 0) sg[pos] &= 0x7f;
+                    w.sync();
+                    if (tagged) { home = pos; pos = -1 - lane; live = false; }
+                }
+            }
             spawn(w, g, p, sg, lane, env, gid, tick, apples, waste);                                  // 263, 291-292
+            if (TAG) {                                 // the agents out during this step count down; those reaching 0 return
+                const bool back = timer == 1;
+                timer = tagged ? p.tag_timeout : (timer ? timer - 1 : 0);
+                const unsigned who = w.ballot(back);
+                if (who) {
+                    place_agents<true>(w, g, p, sg, lane, env, gid, tick, who, pos);
+                    if (back) { ori = spawn_orientation(p, env, gid, tick, lane); live = true; sg[pos] |= kOcc; }
+                    w.sync();
+                }
+                if (gone | who) same = equal_lanes(w, pos, p.n);
+            }
             const int t = t_prev + 1;
             if (is_agent) {
                 p.reward[(size_t)env * p.n + lane] = (int8_t)reward;
@@ -990,27 +1061,8 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
                 p.counts[env] = (uint32_t)apples | ((uint32_t)waste << 16);
             }
         } else if (MODE == MODE_RESET) {
-            // setup_agents: agent i takes the free spawn point with the largest (key, cell) (map_env.py:771-784)
-            const bool is_sp = lane < p.n_spawn;
-            const int mycell = is_sp ? (int)__ldg(&p.map->spawn_pts[lane]) : -1;
-            bool taken = false;
-            for (int i = 0; i < p.n; ++i) {
-                uint32_t key = 0;
-                if (p.random_spawn && is_sp)
-                    key = p.d_spawnkey ? p.d_spawnkey[((size_t)env * p.n + i) * g.G() + mycell]
-                                       : philox_word(p, gid, tick, 3u, (uint32_t)(i * p.n_spawn + lane));
-                const bool cand = is_sp && !taken;
-                const uint32_t mk = w.rmax(cand ? key : 0u);
-                const unsigned eq = w.ballot(cand && key == mk);
-                const int win = 31 - __clz(eq);
-                const int cell = w.shfl(mycell, win);
-                if (lane == win) taken = true;
-                if (lane == i) pos = cell;
-            }
-            if (is_agent) {                                                                     // spawn_rotation (786-793)
-                if (p.spawn_rot >= 0) ori = p.spawn_rot;
-                else ori = p.d_rot ? (int)(p.d_rot[(size_t)env * p.n + lane] & 3) : (int)(philox_word(p, gid, tick, 4u, (uint32_t)lane) >> 30);
-            }
+            place_agents<false>(w, g, p, sg, lane, env, gid, tick, ~0u, pos);                          // setup_agents (771-784)
+            if (is_agent) ori = spawn_orientation(p, env, gid, tick, lane);
             if (is_agent) sg[pos] |= kOcc;                         // distinct spawn points: no two lanes share a cell
             w.sync();
             apples = p.base_apples; waste = p.base_waste;
@@ -1023,13 +1075,15 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
         // for this whole grid before it reads any state)
         if (p.pdl) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
         if (MODE != MODE_RENDER) {                                 // strip the occupancy bits, write the state back
-            if (is_agent && lane == __ffs(same) - 1) sg[pos] &= 0x7f;
+            if (live && lane == __ffs(same) - 1) sg[pos] &= 0x7f;
             w.sync();
             uint4* dst = reinterpret_cast<uint4*>(p.grid + (size_t)env * g.GS());
             warp_for<SW::kLanes>(g.GS() >> 4, lane, [&](int i) { dst[i] = reinterpret_cast<const uint4*>(sg)[i]; });
-            if (is_agent) {
-                const int r = g.divW(pos);
-                p.agent[(size_t)env * p.NA + lane] = (uint32_t)r | ((uint32_t)(pos - r * g.W()) << 8) | ((uint32_t)ori << 16);
+            if (is_agent) {                                        // an agent out of play keeps the cell it left the map from
+                const int cell = (TAG && !live) ? home : pos;
+                const int r = g.divW(cell);
+                p.agent[(size_t)env * p.NA + lane] = (uint32_t)r | ((uint32_t)(cell - r * g.W()) << 8) | ((uint32_t)ori << 16)
+                                                     | (TAG ? (uint32_t)timer << 24 : 0u);
                 p.ep_ret[(size_t)env * p.NA + lane] = ep_ret;
             }
         }
@@ -1037,9 +1091,10 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
             // agent overlay: every occupied cell shows an agent (index 7; which agent only matters for the full-colour repaint and
             // the state image, both handled in render).  Same value from every lane on a shared cell: no race.
             w.sync();                                          // the write-back above has read the staged grid
-            if (is_agent) sg[pos] = 7;
+            if (live) sg[pos] = 7;
             w.sync();
-            render(w, g, p, sg, pmap, lut_s, lane, is_agent, pos, ori, env, same);
+            const unsigned outm = TAG ? w.ballot(is_agent && !live) : 0u;
+            render(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm);
         }
     }
 }
@@ -1121,7 +1176,7 @@ static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws
     return SSD_OK;
 }
 
-template <int MODE, class GEO, int LPE>
+template <int MODE, class GEO, int LPE, bool TAG>
 static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
@@ -1133,7 +1188,7 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         const int dev = h->device;
         if (dev < 0 || dev >= kMaxDevices) return SSD_ERR_INVALID;
         if ((int)h->smem_bytes > high_water[dev]) {
-            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, LPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, LPE, TAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
             high_water[dev] = (int)h->smem_bytes;
         }
     }
@@ -1149,9 +1204,9 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, LPE>, k));
+        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, LPE, TAG>, k));
     } else {
-        ssd_kernel<MODE, GEO, LPE><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
+        ssd_kernel<MODE, GEO, LPE, TAG><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
     }
     ++h->launches;
     SSD_CUDA(cudaGetLastError());
@@ -1168,10 +1223,13 @@ template <int MODE, class GEO>
 static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
     k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
+    if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation, one env per warp
+        if (k.tag_timeout != 0) return launch_lpe<MODE, GEO, 32, true>(h, k, stream);
+    }
 #ifdef SSD_ENABLE_LPE16                                        // experiment: two envs per warp (measured slower, profiles/r1_notes.md)
-    if (h->lanes_per_env == 16) return launch_lpe<MODE, GEO, 16>(h, k, stream);
+    if (h->lanes_per_env == 16) return launch_lpe<MODE, GEO, 16, false>(h, k, stream);
 #endif
-    return launch_lpe<MODE, GEO, 32>(h, k, stream);
+    return launch_lpe<MODE, GEO, 32, false>(h, k, stream);
 }
 
 // The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
@@ -1219,6 +1277,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     if (n < 1 || n > SSD_MAX_AGENTS || V < 1 || V > 31 || cfg->n_envs < 1) return SSD_ERR_INVALID;
     if (cfg->beam_len < 0 || cfg->episode_limit < 1 || cfg->spawn_rotation > 3) return SSD_ERR_INVALID;
     if (abs(cfg->fire_cost) + n * abs(cfg->hit_penalty) + 1 > 127) return SSD_ERR_INVALID;   // reward is int8
+    if (cfg->tag_timeout < 0 || cfg->tag_timeout > 255) return SSD_ERR_INVALID;              // 8-bit timer in the agent record
 
     MapDev* hm = new (std::nothrow) MapDev;
     if (!hm) return SSD_ERR_INVALID;
@@ -1266,6 +1325,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     k.direct = gv.direct; k.padF = gv.padF; k.padB = gv.padB;
     k.off_map[0] = gv.off0; k.off_map[1] = gv.off1; k.off_map[2] = gv.off2; k.off_map[3] = gv.off3;
     k.episode_limit = cfg->episode_limit; k.fire_cost = cfg->fire_cost; k.hit_penalty = cfg->hit_penalty;
+    k.tag_timeout = cfg->tag_timeout;
     k.beam_len = cfg->beam_len; k.n_actions = cfg->kind == SSD_KIND_CLEANUP ? 9 : 8;
     k.n_apple = na; k.n_waste = nw; k.n_spawn = ns; k.n_apple4 = (na + 3) / 4; k.n_waste2 = (nw + 1) / 2;
     k.base_apples = 0; k.base_waste = 0;
@@ -1292,7 +1352,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     // two envs per warp need the spawn points (reset) and the per-lane apple decision bits (64) to fit 16 lanes
     h->lanes_per_env = 32;
 #ifdef SSD_ENABLE_LPE16
-    if (ns <= 16 && k.n_apple4 <= 16 * 16) h->lanes_per_env = 16;
+    if (ns <= 16 && k.n_apple4 <= 16 * 16 && k.tag_timeout == 0) h->lanes_per_env = 16;
     { const char* e = getenv("SSD_B200_LPE"); if (e && atoi(e) == 32) h->lanes_per_env = 32; }
 #endif
     h->smem_bytes = (size_t)kWarps * (32 / h->lanes_per_env) * k.smem_per_warp;

@@ -147,6 +147,7 @@ class MapSpec:
     fire_cost: int = 1
     hit_penalty: int = 0
     beam_len: int = 5
+    tag_timeout: int = 0          # steps an agent hit by a FIRE ray stays off the map; 0 = never (the reference)
     base_grid: np.ndarray = field(default=None, repr=False)
     wall: np.ndarray = field(default=None, repr=False)
     apple_pts: np.ndarray = field(default=None, repr=False)
@@ -175,8 +176,10 @@ class MapSpec:
 
 def compile_map(name: str, map_name: str, n_agents: int, view: int, episode_limit: int,
                 obs_color: str = "simplified", rows=None, params: EnvParams | None = None,
-                fire_cost: int = 1, hit_penalty: int = 0) -> MapSpec:
+                fire_cost: int = 1, hit_penalty: int = 0, tag_timeout: int = 0) -> MapSpec:
     p = params if params is not None else params_for(name, map_name)
+    if not 0 <= int(tag_timeout) <= 255:
+        raise ValueError("tag_timeout must be in 0..255")
     rows = list(rows) if rows is not None else ascii_map(p.map_key)
     H, W = len(rows), len(rows[0])
     if H * W > MAX_CELLS:
@@ -221,7 +224,7 @@ def compile_map(name: str, map_name: str, n_agents: int, view: int, episode_limi
     thr_h = np.array([prob_to_threshold(x) for x in p.spawn_prob], dtype=np.uint32)
     return MapSpec(kind=p.kind, rows=rows, H=H, W=W, n_agents=n_agents, view=view,
                    episode_limit=episode_limit, obs_color=obs_color, params=p,
-                   fire_cost=fire_cost, hit_penalty=hit_penalty,
+                   fire_cost=fire_cost, hit_penalty=hit_penalty, tag_timeout=int(tag_timeout),
                    base_grid=base, wall=wall.astype(np.uint8), apple_pts=apple, waste_pts=waste,
                    spawn_pts=spawn, thr_apple=thr_a, thr_waste=thr_w, thr_harvest=thr_h,
                    lut=color_lut(p.kind, obs_color))

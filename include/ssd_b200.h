@@ -68,7 +68,9 @@ typedef struct ssd_config {
     int32_t random_spawn_point;   /* extra_args.random_spawn_point                      */
     int32_t spawn_rotation;       /* extra_args.random_spawn_rotation: 0..3, -1 = random */
     int32_t device;               /* CUDA device ordinal                                */
-    int32_t reserved0;
+    int32_t tag_timeout;          /* 0..255: steps an agent hit by a FIRE ray stays off the map (tagged out); 0 = never, as
+                                   * in the reference.  An agent out of play is not on the map, its action is ignored, its
+                                   * reward, clean count and observation are 0; it then respawns like at reset (DESIGN.md §3) */
     uint64_t seed;                /* Philox key                                         */
     uint32_t env_gid_base;        /* global id of env 0 (multi-GPU shards keep trajectories) */
     uint32_t n_waste_lut;         /* entries in thr_apple / thr_waste (= #waste points + 1)   */
@@ -96,7 +98,9 @@ typedef struct ssd_layout {
 /* Persistent per-env state (MapEnv.world_map, Agent.pos/orientation, _episode_steps, rewards). */
 typedef struct ssd_state {
     uint8_t*  grid;      /* [B][grid_stride]   cell codes, padding bytes stay 0           */
-    uint32_t* agent;     /* [B][agent_stride]  row | col<<8 | orientation<<16             */
+    uint32_t* agent;     /* [B][agent_stride]  row | col<<8 | orientation<<16 | tag_out<<24: tag_out = steps the agent is
+                          *                     still out of play (tagging-out), 0 = on the map; an agent out keeps the
+                          *                     row, col and orientation it had when it was tagged                          */
     int32_t*  ep_ret;    /* [B][agent_stride]  episode return per agent (map_env.py:885-888) */
     int32_t*  t;         /* [B]                _episode_steps                             */
     uint32_t* tick;      /* [B]                Philox step counter (never reset)          */
@@ -122,8 +126,9 @@ typedef struct ssd_draws {
     const uint32_t* u_apple;    /* [B][G]     np.random.rand per apple cell (cleanup.py:172, harvest.py:119)     */
     const uint32_t* u_waste;    /* [B][G]     np.random.rand per waste cell (cleanup.py:183)                      */
     const uint32_t* wkey;       /* [B][G]     random.shuffle(waste_points) (cleanup.py:178): ascending (key, cell) */
-    const uint32_t* spawn_key;  /* [B][n][G]  random.shuffle(spawn_points) (map_env.py:777): max (key, cell) wins  */
-    const uint8_t*  rot;        /* [B][n]     np.random.randint(4) (map_env.py:789)                               */
+    const uint32_t* spawn_key;  /* [B][n][G]  random.shuffle(spawn_points) (map_env.py:777): max (key, cell) wins;
+                                 *            read by reset, and by a step for the agents whose tagging-out ends   */
+    const uint8_t*  rot;        /* [B][n]     np.random.randint(4) (map_env.py:789); reset, and respawn in a step  */
 } ssd_draws;
 
 int ssd_abi_version(void);

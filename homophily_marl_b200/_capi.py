@@ -13,10 +13,12 @@ LIB_PATH = os.environ.get("SSD_B200_LIB") or os.path.join(
     PKG_DIR, "libssd_b200_check.so" if os.environ.get("SSD_B200_CHECKED") == "1" else "libssd_b200.so")
 
 SSD_OK, SSD_ERR_INVALID, SSD_ERR_CUDA, SSD_ERR_SPAWN, SSD_ERR_MAP = 0, -1, -2, -3, -4
+SSD_OBS_RGB, SSD_OBS_INDEX4 = 0, 1
 
 # every symbol include/ssd_b200.h declares (checked by tests/test_capi_symbols.py against the header text)
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
-           "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_reset", "ssd_step", "ssd_step_range", "ssd_render",
+           "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
+           "ssd_reset", "ssd_step", "ssd_step_range", "ssd_render",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_destroy", "ssd_frontend_last_cuda_error")
@@ -37,6 +39,10 @@ class SsdLayout(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("n_actions", "n_cells", "obs_n", "grid_stride", "agent_stride",
                                           "obs_plane_stride", "obs_agent_stride", "obs_env_stride",
                                           "n_apple_pts", "n_waste_pts", "n_spawn_pts", "obs_row_stride")]
+
+
+class SsdObsLayout(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("format", "row_stride", "plane_stride", "agent_stride", "env_stride")]
 
 
 class SsdState(C.Structure):
@@ -78,6 +84,9 @@ def load():
     L.ssd_create.argtypes = [C.POINTER(SsdConfig), C.POINTER(C.c_void_p)]
     L.ssd_destroy.argtypes = [C.c_void_p]
     L.ssd_get_layout.argtypes = [C.c_void_p, C.POINTER(SsdLayout)]
+    L.ssd_get_obs_layout.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdObsLayout)]
+    L.ssd_set_obs_format.argtypes = [C.c_void_p, C.c_int32]
+    L.ssd_expand_obs.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

@@ -28,6 +28,9 @@ def _require_cuda(device):
     return torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
 
 
+OBS_FORMATS = {"rgb": _capi.SSD_OBS_RGB, "index4": _capi.SSD_OBS_INDEX4}
+
+
 def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
@@ -37,9 +40,12 @@ class SSDBatchEnv:
                  extra_args=None, seed=0, device="cuda:0", env_gid_base=0, rows=None, params=None,
                  fire_cost=1, hit_penalty=0, want_state=False, check_actions=False):
         # tag_timeout: steps an agent hit by a FIRE ray is out of play (off the map, action ignored, zero view); 0 = never
+        # obs_format: "rgb" (u8 RGB planes, the reference's get_obs * 256) or "index4" (packed 4-bit colour indices)
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
-                     disable_fire_action=True, obs_color="simplified", tag_timeout=0)
+                     disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb")
         extra.update(extra_args or {})
+        if extra["obs_format"] not in OBS_FORMATS:
+            raise ValueError(f"obs_format must be one of {sorted(OBS_FORMATS)}, got {extra['obs_format']!r}")
         self.extra_args = extra
         self.name = name
         self.spec = mapspec.compile_map(name, map, num_agents, view_size, episode_limit,
@@ -82,6 +88,9 @@ class SSDBatchEnv:
         _capi.check(self.lib.ssd_get_layout(self._h, C.byref(lay)))
         self.layout = lay
         assert lay.n_actions == self.n_actions and lay.n_cells == self.G
+        self.obs_format, self.obs_layout = "rgb", self.get_obs_layout("rgb")
+        if extra["obs_format"] != "rgb":
+            self._set_format(extra["obs_format"])
 
         dev, B, n = self.device, self.B, self.n
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
@@ -101,17 +110,72 @@ class SSDBatchEnv:
                                                             self.t_buf, self.tick_buf, self.counts_buf)])
         self._keep = None
 
+    # ------------------------------------------------------------------ observation format
+    def get_obs_layout(self, fmt):
+        """``ssd_obs_layout`` (format, row_stride, plane_stride, agent_stride, env_stride) of "rgb" or "index4"."""
+        lay = _capi.SsdObsLayout()
+        _capi.check(self.lib.ssd_get_obs_layout(self._h, OBS_FORMATS[fmt], C.byref(lay)))
+        return lay
+
+    def _set_format(self, fmt):
+        _capi.check(self.lib.ssd_set_obs_format(self._h, OBS_FORMATS[fmt]))
+        self.obs_format, self.obs_layout = fmt, self.get_obs_layout(fmt)
+
+    def set_obs_format(self, fmt):
+        """Switches the format every later step / reset / render writes, and reallocates ``obs_buf`` for it.  Host-side: a
+        CUDA graph captured before keeps the format it was captured with."""
+        if fmt not in OBS_FORMATS:
+            raise ValueError(f"obs_format must be one of {sorted(OBS_FORMATS)}, got {fmt!r}")
+        self._set_format(fmt)
+        self.extra_args["obs_format"] = fmt
+        self.obs_buf = self.new_obs_buffer()
+
     # ------------------------------------------------------------------ buffers / views
     def new_obs_buffer(self):
-        """Flat u8 [B, obs_env_stride] buffer in the kernel's padded plane layout."""
-        return torch.zeros((self.B, self.layout.obs_env_stride), dtype=torch.uint8, device=self.device)
+        """Flat u8 [B, env_stride] buffer in the layout of the current observation format."""
+        return torch.zeros((self.B, self.obs_layout.env_stride), dtype=torch.uint8, device=self.device)
 
     def obs_view(self, buf=None):
-        """[B, n, 3, N, N] u8 view (no copy) of an obs buffer; ``view / 256`` equals get_obs()."""
+        """[B, n, 3, N, N] u8 view (no copy) of an RGB obs buffer; ``view / 256`` equals get_obs()."""
+        if self.obs_format != "rgb":
+            raise ValueError("obs_view() reads RGB planes; this env writes index4 observations (use obs_index / obs_float)")
         buf = self.obs_buf if buf is None else buf
         lay = self.layout
         return buf.as_strided((self.B, self.n, 3, self.N, self.N),
                               (lay.obs_env_stride, lay.obs_agent_stride, lay.obs_plane_stride, lay.obs_row_stride, 1))
+
+    def _index4(self, what):
+        if self.obs_format != "index4":
+            raise ValueError(f"{what} needs obs_format 'index4'")
+
+    def obs_packed(self, buf=None):
+        """[B, n, N, row_stride] u8 view (no copy) of an index4 buffer: pixel x of a row is byte x >> 1, low nibble when x is
+        even."""
+        self._index4("obs_packed()")
+        buf = self.obs_buf if buf is None else buf
+        lay = self.obs_layout
+        return buf.as_strided((self.B, self.n, self.N, lay.row_stride), (lay.env_stride, lay.agent_stride, lay.row_stride, 1))
+
+    def obs_index(self, buf=None):
+        """[B, n, N, N] u8 colour indices (unpacked copy): ``spec.lut[obs_index()]`` is the RGB observation."""
+        p = self.obs_packed(buf)
+        return torch.stack((p & 15, p >> 4), dim=-1).reshape(self.B, self.n, self.N, -1)[..., :self.N]
+
+    def obs_float(self, env_begin=0, env_count=None, buf=None, out=None):
+        """f32 [env_count, n, 3, N, N] of envs [env_begin, env_begin + env_count) of an index4 buffer, through one
+        ``ssd_expand_obs`` launch on the current stream: bit-identical to ``obs_view().float() / 256`` of an RGB env."""
+        self._index4("obs_float()")
+        buf = self.obs_buf if buf is None else buf
+        env_count = self.B - env_begin if env_count is None else int(env_count)
+        shape = (env_count, self.n, 3, self.N, self.N)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        elif out.dtype != torch.float32 or not out.is_cuda or not out.is_contiguous() or tuple(out.shape) != shape:
+            raise ValueError(f"out must be a contiguous float32 CUDA tensor of shape {shape}")
+        if buf.dtype != torch.uint8 or not buf.is_cuda or buf.numel() < self.B * self.obs_layout.env_stride:
+            raise ValueError("buf must be a uint8 CUDA index4 observation buffer of B * env_stride bytes")
+        _capi.check(self.lib.ssd_expand_obs(self._h, _ptr(buf), int(env_begin), env_count, _ptr(out), self._stream()))
+        return out
 
     @property
     def grid(self):
@@ -298,8 +362,10 @@ class SSDBatchEnv:
         return int(self.lib.ssd_launch_count(self._h))
 
     def bytes_per_env_step(self):
-        """ALGORITHMIC HBM bytes of one fused step+obs (SURVEY 8d): 2G + n(3N^2 + 11) + 3."""
-        return 2 * self.G + self.n * (3 * self.N * self.N + 11) + 3
+        """ALGORITHMIC HBM bytes of one fused step+obs (SURVEY 8d): 2G + n(3N^2 + 11) + 3 for RGB, 2G + n(N ceil(N/2) + 11) + 3
+        for index4."""
+        obs = 3 * self.N * self.N if self.obs_format == "rgb" else self.N * ((self.N + 1) // 2)
+        return 2 * self.G + self.n * (obs + 11) + 3
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:

@@ -73,6 +73,8 @@ class BatchedEpisodeRunner:
         # args.fused_frontend: during rollouts the MAC's rgb_preprocess (conv3x3 + FC on fp32 obs, homophily_controller.py:132-136)
         # is served by the fused u8 front-end kernel reading the env's observation buffer (frontend.MacFrontEnd)
         self.front = None
+        if getattr(self.args, "fused_frontend", False) and self.env.obs_format != "rgb":
+            raise ValueError("fused_frontend reads RGB observation planes; it cannot run with obs_format 'index4'")
         if getattr(self.args, "fused_frontend", False) and getattr(self.args, "rgb_input", False):
             from .frontend import MacFrontEnd
             self.front = MacFrontEnd(mac, self.env)
@@ -102,8 +104,13 @@ class BatchedEpisodeRunner:
     # ---- device-side views of what the reference env returns per step -------------------------------------
     def _pre_transition(self, sl=slice(None)):
         e = self.env                                          # obs AND state image were written by the last step / reset launch
+        if e.obs_format == "rgb":
+            obs = e.obs_view()[sl].float() / 256
+        else:                                                 # index4: expanded on the current (the range's) stream
+            lo, hi, _ = sl.indices(e.B)
+            obs = e.obs_float(lo, hi - lo)
         return {"state": e.state_rgb[sl].float() / 256, "avail_actions": self._avail[sl],
-                "obs": e.obs_view()[sl].float() / 256, "agent_pos": e.agent_pos[sl].float(),
+                "obs": obs, "agent_pos": e.agent_pos[sl].float(),
                 "agent_orientation": self._orient_vec[e.agent_orient[sl].long()]}
 
     def _range_step(self, r, t, last, homophily, test_mode, Bg):

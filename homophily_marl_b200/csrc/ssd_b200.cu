@@ -87,6 +87,7 @@ struct KParams {
     const uint32_t* d_prio; const uint32_t* d_uapple; const uint32_t* d_uwaste; const uint32_t* d_wkey;
     const uint32_t* d_spawnkey; const uint8_t* d_rot;
     int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
+    int RS4, AS4;                             // packed colour-index observations (SSD_OBS_INDEX4): row / agent strides
 };
 
 
@@ -99,6 +100,7 @@ struct GeoVals {
     int direct, padF, padB;                   // small views (RP <= 16) are gathered straight from the staged grid: no maps, but
                                               // V rows of slack before / after the grid so that column runs need no bounds test
     uint32_t maskM8, maskT8;
+    int RS4, AS4;                             // SSD_OBS_INDEX4: bytes per row (ceil(N/2) rounded to 4) and per agent (rounded to 16)
 };
 __host__ __device__ constexpr int cround_up(int v, int m) { return (v + m - 1) / m * m; }
 __host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V) {
@@ -119,6 +121,7 @@ __host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V) {
     g.padF = g.direct ? cround_up(V * W + 48, 16) : 16;      // + 32 bytes at the very front for the (class, rank) -> lane table
     g.padB = g.direct ? cround_up(V * W + 32, 16) : 32;
     if (g.direct) g.PMS = 0;
+    g.RS4 = cround_up((g.N + 1) / 2, 4); g.AS4 = cround_up(g.N * g.RS4, 16);
     return g;
 }
 
@@ -136,6 +139,8 @@ struct GeoS {                                                 // compile-time ge
     __device__ __forceinline__ int RP() const { return v.RP; }
     __device__ __forceinline__ int PS() const { return v.PS; }
     __device__ __forceinline__ int AS() const { return v.AS; }
+    __device__ __forceinline__ int RS4() const { return v.RS4; }
+    __device__ __forceinline__ int AS4() const { return v.AS4; }
     __device__ __forceinline__ int LPn() const { return v.LPn; }
     __device__ __forceinline__ int nw8M() const { return v.nw8M; }
     __device__ __forceinline__ int nw8T() const { return v.nw8T; }
@@ -165,6 +170,8 @@ struct GeoD {                                                 // runtime geometr
     __device__ __forceinline__ int RP() const { return p.RP; }
     __device__ __forceinline__ int PS() const { return p.PS; }
     __device__ __forceinline__ int AS() const { return p.AS; }
+    __device__ __forceinline__ int RS4() const { return p.RS4; }
+    __device__ __forceinline__ int AS4() const { return p.AS4; }
     __device__ __forceinline__ int LPn() const { return p.LPn; }
     __device__ __forceinline__ int nw8M() const { return p.nw8M; }
     __device__ __forceinline__ int nw8T() const { return p.nw8T; }
@@ -561,6 +568,9 @@ __device__ __forceinline__ void st_row32(uint8_t* dst, const uint32_t* w) {     
 __device__ __forceinline__ void st_row16(uint8_t* dst, const uint32_t* w) {
     asm volatile("st.global" SSD_ST_HINT ".v4.b32 [%0], {%1,%2,%3,%4};" :: "l"(dst), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
 }
+__device__ __forceinline__ void st_row8(uint8_t* dst, uint32_t w0, uint32_t w1) {
+    asm volatile("st.global" SSD_ST_HINT ".v2.b32 [%0], {%1,%2};" :: "l"(dst), "r"(w0), "r"(w1) : "memory");
+}
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {   // raw PRMT: no selector masking
     uint32_t d;
     asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(sel));
@@ -579,6 +589,9 @@ __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
 // of the result ARE the PRMT selector that looks 4 pixels up in the 8-entry colour LUT held in two registers
 // per plane.  The finished row leaves the SM as one 32-byte (st.global.v8.b32 -> STG.E.ENL2.256) or 16-byte
 // store per plane.  Indices: 0-5 cell codes, 6 outside, 7 agent.
+// IDX (SSD_OBS_INDEX4): the funnel-shifted words ARE the packed output row (pixel x = nibble x, little-endian), so they are
+// stored as they are, pad nibbles masked: one 16-byte store for N = 31, word stores otherwise; no PRMT.  In IDX kernels a
+// full-colour agent is staged as its own index 7..15 (the row maps and the direct gather carry any index below 16).
 __device__ __forceinline__ uint32_t nibble_reverse(uint32_t x) {
     const uint32_t y = prmt(x, 0u, 0x0123);
     return ((y << 4) & 0xf0f0f0f0u) | ((y >> 4) & 0x0f0f0f0fu);
@@ -594,7 +607,7 @@ struct RowUnit {                                              // one (agent, y) 
     bool valid;
 };
 
-template <int OCT_T, class SW, class GEO>
+template <int OCT_T, bool IDX, class SW, class GEO>
 __device__ __forceinline__ void fetch_row(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane, int it, int units,
                                           uint32_t abase_sh, int astep, unsigned outm, RowUnit<OCT_T>& U) {
     const int u = it * SW::kLanes + lane;
@@ -607,7 +620,7 @@ __device__ __forceinline__ void fetch_row(const SW& w, const GEO& g, const KPara
     U.w = reinterpret_cast<const uint32_t*>(pmap + (ab & 0xffffu) + (U.valid ? y * as : 0));
     U.sh = (ab >> 16) & 31u;
     U.rev = (ab >> 24) & 1u;
-    U.dst = gobs + al * g.AS() + y * g.RP();
+    U.dst = IDX ? gobs + al * g.AS4() + y * g.RS4() : gobs + al * g.AS() + y * g.RP();
     {   // the <= OCT+1 words of the run, ascending or descending, must lie inside this warp's map tile
         const int nwords = (OCT_T > 0 ? OCT_T : ((g.RP() >> 2) + 1) >> 1) + 1;
         const long off = reinterpret_cast<const uint8_t*>(U.w) - pmap;
@@ -624,11 +637,28 @@ __device__ __forceinline__ void fetch_row(const SW& w, const GEO& g, const KPara
     }
 }
 
-template <int OCT_T, class GEO>
+template <int OCT_T, bool IDX, class GEO>
 __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const RowUnit<OCT_T>& U, uint32_t lastmask) {
     if (!U.valid) return;
     const uint32_t sh = U.sh;
-    if constexpr (OCT_T > 0) {
+    if constexpr (IDX) {                                      // lastmask: valid nibbles of the row's last word
+        if constexpr (OCT_T > 0) {
+            uint32_t o[OCT_T];
+#pragma unroll
+            for (int k = 0; k < OCT_T; ++k) o[k] = __funnelshift_r(U.L[k], U.L[k + 1], sh) & U.keep;
+            o[OCT_T - 1] &= lastmask;
+            st_row16(U.dst, o);                               // OCT_T == 4: N = 29..31, 16 bytes a row
+        } else {
+            const int OCT = ((g.RP() >> 2) + 1) >> 1;         // == RS4 / 4 words of 8 pixels
+            uint32_t prev = U.rev ? nibble_reverse(U.w[0]) : U.w[0];
+            for (int k = 0; k < OCT; ++k) {
+                const uint32_t cur = U.rev ? nibble_reverse(*(U.w - (k + 1))) : U.w[k + 1];
+                const uint32_t m = k == OCT - 1 ? lastmask : 0xffffffffu;
+                *reinterpret_cast<uint32_t*>(U.dst + 4 * k) = __funnelshift_r(prev, cur, sh) & m & U.keep;
+                prev = cur;
+            }
+        }
+    } else if constexpr (OCT_T > 0) {
         uint32_t v[2 * OCT_T];
 #pragma unroll
         for (int k = 0; k < OCT_T; ++k) { v[2 * k] = __funnelshift_r(U.L[k], U.L[k + 1], sh); v[2 * k + 1] = v[2 * k] >> 16; }
@@ -661,17 +691,17 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
     }
 }
 
-template <int OCT_T, class SW, class GEO>
+template <int OCT_T, bool IDX, class SW, class GEO>
 __device__ __forceinline__ void gather_rows(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane,
                                             uint32_t abase_sh, int astep, unsigned outm) {
     const int WR = g.RP() >> 2;
-    const uint32_t lastmask = 0xffffffffu >> (8 * (4 * WR - g.N()));
+    const uint32_t lastmask = IDX ? 0xffffffffu >> (4 * (8 * ((WR + 1) >> 1) - g.N())) : 0xffffffffu >> (8 * (4 * WR - g.N()));
     const int units = p.n * g.N(), iters = (units + SW::kLanes - 1) / SW::kLanes;
     RowUnit<OCT_T> cur, nxt;
-    fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, outm, cur);
+    fetch_row<OCT_T, IDX>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, outm, cur);
     for (int it = 0; it < iters; ++it) {                      // software pipeline: row it+1 is fetched while row it is emitted
-        if (it + 1 < iters) fetch_row<OCT_T>(w, g, p, pmap, gobs, lane, it + 1, units, abase_sh, astep, outm, nxt);
-        emit_row<OCT_T>(g, p, cur, lastmask);
+        if (it + 1 < iters) fetch_row<OCT_T, IDX>(w, g, p, pmap, gobs, lane, it + 1, units, abase_sh, astep, outm, nxt);
+        emit_row<OCT_T, IDX>(g, p, cur, lastmask);
         cur = nxt;
     }
 }
@@ -753,7 +783,7 @@ __device__ __forceinline__ void fill_outside(const SW& w, const GEO& g, const KP
 // index 6, reverses the run for DOWN / RIGHT, and colours 4 pixels per PRMT as the map path does.  No padded maps are built.
 // The grid tile has V rows of slack on both sides (zeroed at kernel start), so no load needs a bounds test; agents were
 // written into the staged grid as index 7 by the caller.
-template <bool COLS, class SW, class GEO>
+template <bool COLS, bool IDX, class SW, class GEO>
 __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, const uint8_t* rank2lane,
                                              uint8_t* gobs, int lane, uint32_t apack, int n_in_class, unsigned outm) {
     const int N = g.N(), V = g.V(), W = g.W(), units = n_in_class * N, WR = g.RP() >> 2;
@@ -809,6 +839,13 @@ __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KP
             n0 = (uint32_t)rr;
             n1 = (uint32_t)(rr >> 32);
         }
+        if constexpr (IDX) {                                  // (n0, n1) is the packed row: keep its N nibbles
+            const uint32_t keep = ((outm >> al) & 1u) ? 0u : 0xffffffffu;
+            uint8_t* dst = gobs + al * g.AS4() + y * g.RS4();
+            if (g.RS4() == 8) st_row8(dst, n0 & keep, n1 & (0xffffffffu >> (4 * (16 - N))) & keep);
+            else *reinterpret_cast<uint32_t*>(dst) = n0 & (0xffffffffu >> (4 * (8 - N))) & keep;
+            continue;
+        }
         const uint32_t v[4] = { n0, n0 >> 16, n1, n1 >> 16 };
         uint8_t* dst = gobs + al * g.AS() + y * g.RP();
         const uint32_t keep = ((outm >> al) & 1u) ? 0u : 0xffffffffu;       // an agent out of play sees zeros
@@ -831,7 +868,7 @@ __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KP
 // The rows of UP / DOWN agents and of LEFT / RIGHT agents are gathered in two separate passes, so that a trip of the warp runs
 // ONE of the two load schemes instead of both under divergence.  `tbl` (32 bytes at the very start of the tile's front slack,
 // never touched by a gather load) maps (class, rank within class) -> agent lane.
-template <class SW, class GEO>
+template <bool IDX, class SW, class GEO>
 __device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* tbl, uint8_t* gobs, int lane,
                                               bool is_agent, int r0, int c0, int ori, unsigned outm) {
     const uint32_t apack = (uint32_t)r0 | ((uint32_t)c0 << 8) | ((uint32_t)ori << 16);
@@ -841,13 +878,13 @@ __device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const K
         tbl[(cols ? 16 : 0) + __popc((cols ? m_cols : m_rows) & ((1u << lane) - 1u))] = (uint8_t)lane;
     }
     w.sync();
-    if (m_rows) gather_class<false>(w, g, p, sg, tbl, gobs, lane, apack, __popc(m_rows), outm);
-    if (m_cols) gather_class<true>(w, g, p, sg, tbl + 16, gobs, lane, apack, __popc(m_cols), outm);
+    if (m_rows) gather_class<false, IDX>(w, g, p, sg, tbl, gobs, lane, apack, __popc(m_rows), outm);
+    if (m_cols) gather_class<true, IDX>(w, g, p, sg, tbl + 16, gobs, lane, apack, __popc(m_cols), outm);
 }
 
 // live: the lane's agent is on the map; outm: agents out of play (tagged out), whose views are written as zeros.  Their rows go
 // through the same gather at cell (0, 0), masked, so that a warp trip never mixes two kinds of row.
-template <class SW, class GEO>
+template <bool IDX, class SW, class GEO>
 __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
                                        int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm) {
     const bool top = live && lane == 31 - __clz(same);       // later index overwrites (map_env.py:370); same = lanes on this lane's cell
@@ -867,10 +904,10 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
         }
     }
     if (!p.obs) return;
-    uint8_t* gobs = p.obs + (size_t)env * (p.n * g.AS());
+    uint8_t* gobs = p.obs + (size_t)env * (p.n * (IDX ? g.AS4() : g.AS()));
 
     if (g.direct()) {
-        gather_direct(w, g, p, sg, const_cast<uint8_t*>(sg) - g.padF(), gobs, lane, is_agent, r0, c0, ori, outm);
+        gather_direct<IDX>(w, g, p, sg, const_cast<uint8_t*>(sg) - g.padF(), gobs, lane, is_agent, r0, c0, ori, outm);
     } else {
         // the maps were pre-filled with "outside the map" at kernel start (fill_outside); now the cells (agents are already in
         // the staged grid as index 7)
@@ -893,13 +930,19 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
             build_colmap(w, g, p, M, MT, lane);
             w.sync();
         }
-        if (g.RP() == 32) gather_rows<4>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
-        else gather_rows<0>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
+        if (g.RP() == 32) gather_rows<4, IDX>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
+        else gather_rows<0, IDX>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
     }
-    const int tail = g.AS() - 3 * g.PS();                         // pad bytes per agent block (0 for the shipped views)
-    if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
-        *reinterpret_cast<uint32_t*>(gobs + (i / (tail >> 2)) * g.AS() + 3 * g.PS() + 4 * (i % (tail >> 2))) = 0u;
-    if (!p.agents_uniform) {
+    if constexpr (IDX) {                                          // pad bytes per agent block (8 for N = 15)
+        const int body = g.N() * g.RS4(), tail = g.AS4() - body;
+        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
+            *reinterpret_cast<uint32_t*>(gobs + (i / (tail >> 2)) * g.AS4() + body + 4 * (i % (tail >> 2))) = 0u;
+    } else {
+        const int tail = g.AS() - 3 * g.PS();                     // pad bytes per agent block (0 for the shipped views)
+        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
+            *reinterpret_cast<uint32_t*>(gobs + (i / (tail >> 2)) * g.AS() + 3 * g.PS() + 4 * (i % (tail >> 2))) = 0u;
+    }
+    if (!IDX && !p.agents_uniform) {
         // full-colour scheme: every visible agent is re-painted with its own colour (after the row stores)
         w.sync();
         const uint32_t apack = (uint32_t)r0 | ((uint32_t)c0 << 10) | ((uint32_t)ori << 20);
@@ -926,7 +969,8 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
 
 // ------------------------------------------------------------------ the kernel
 // TAG: tagging-out timers are on (p.tag_timeout > 0; MODE_STEP and MODE_RENDER only, DESIGN.md §3 item 11).
-template <int MODE, class GEO, int LPE, bool TAG>
+// IDX: observations are written as packed colour indices (SSD_OBS_INDEX4, DESIGN.md §3 item 12) instead of RGB planes.
+template <int MODE, class GEO, int LPE, bool TAG, bool IDX>
 __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const __grid_constant__ KParams p) {
     using SW = SubWarp<LPE>;
     const GEO g(p);
@@ -1090,11 +1134,13 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
         if (p.obs || p.state_rgb) {
             // agent overlay: every occupied cell shows an agent (index 7; which agent only matters for the full-colour repaint and
             // the state image, both handled in render).  Same value from every lane on a shared cell: no race.
+            // IDX: the top agent of a cell is staged as its own colour index (7 in the simplified scheme), so no repaint follows.
             w.sync();                                          // the write-back above has read the staged grid
-            if (live) sg[pos] = 7;
+            if (IDX) { if (live && lane == 31 - __clz(same)) sg[pos] = (uint8_t)(p.agents_uniform ? 7 : agent_colour_index(lane)); }
+            else if (live) sg[pos] = 7;
             w.sync();
             const unsigned outm = TAG ? w.ballot(is_agent && !live) : 0u;
-            render(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm);
+            render<IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm);
         }
     }
 }
@@ -1121,6 +1167,27 @@ __global__ void incentive_kernel(const long long* __restrict__ a_inc, const floa
     if (recip) { const float inv = __fdiv_rn(1.0f, T); r_env[idx] = __fmul_rn(e, inv); r_inc[idx] = __fmul_rn(c, inv); }
     else { r_env[idx] = __fdiv_rn(e, T); r_inc[idx] = __fdiv_rn(c, T); }
     if (sgn) sgn[idx] = rv > 0.f ? 1.f : (rv < 0.f ? -1.f : 0.f);
+}
+
+// ------------------------------------------------------------------ index4 -> f32 RGB (ssd_expand_obs)
+// One CTA per agent view, one thread per pixel: f32 [3][N][N] = color_lut[nibble] / 256, exactly what u8 RGB / 256 gives.
+struct ExpandParams {
+    const uint8_t* in;                        // first view of the range in the index4 buffer
+    float* out;                               // [views][3][N][N]
+    int N, RS4, AS4;
+    uint32_t lut[16];                         // R | G << 8 | B << 16 per colour index
+};
+__global__ void __launch_bounds__(256) expand_obs_kernel(const __grid_constant__ ExpandParams p) {
+    const uint8_t* __restrict__ in = p.in + (size_t)blockIdx.x * p.AS4;
+    const int NN = p.N * p.N;
+    float* __restrict__ out = p.out + (size_t)blockIdx.x * 3 * NN;
+    for (int q = threadIdx.x; q < NN; q += blockDim.x) {
+        const int y = q / p.N, x = q - y * p.N;
+        const uint32_t rgb = p.lut[(__ldg(in + y * p.RS4 + (x >> 1)) >> (4 * (x & 1))) & 15u];
+        out[q] = (float)(rgb & 0xffu) * (1.0f / 256.0f);
+        out[NN + q] = (float)((rgb >> 8) & 0xffu) * (1.0f / 256.0f);
+        out[2 * NN + q] = (float)((rgb >> 16) & 0xffu) * (1.0f / 256.0f);
+    }
 }
 
 thread_local int g_last_cuda_error = 0;
@@ -1157,10 +1224,11 @@ struct ssd_handle {
     MapDev* d_map;
     int device;
     size_t smem_bytes;
-    int64_t launches;
+    mutable int64_t launches;                                 // also counts ssd_expand_obs, which takes a const handle
     int force_generic;                                        // SSD_B200_GENERIC=1: always use the runtime-geometry kernels
     int pdl;                                                  // programmatic dependent launch for small launches (SSD_B200_PDL=0 turns it off)
     int lanes_per_env;                                        // 16: two envs per warp (needs <= 16 spawn points); 32: one
+    int obs_format;                                           // SSD_OBS_RGB (at creation) or SSD_OBS_INDEX4
 };
 
 static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws* d, KParams& k) {
@@ -1176,7 +1244,7 @@ static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws
     return SSD_OK;
 }
 
-template <int MODE, class GEO, int LPE, bool TAG>
+template <int MODE, class GEO, int LPE, bool TAG, bool IDX>
 static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
@@ -1188,7 +1256,7 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         const int dev = h->device;
         if (dev < 0 || dev >= kMaxDevices) return SSD_ERR_INVALID;
         if ((int)h->smem_bytes > high_water[dev]) {
-            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, LPE, TAG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, LPE, TAG, IDX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
             high_water[dev] = (int)h->smem_bytes;
         }
     }
@@ -1204,9 +1272,9 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, LPE, TAG>, k));
+        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, LPE, TAG, IDX>, k));
     } else {
-        ssd_kernel<MODE, GEO, LPE, TAG><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
+        ssd_kernel<MODE, GEO, LPE, TAG, IDX><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
     }
     ++h->launches;
     SSD_CUDA(cudaGetLastError());
@@ -1223,13 +1291,15 @@ template <int MODE, class GEO>
 static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
     k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
+    const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
     if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation, one env per warp
-        if (k.tag_timeout != 0) return launch_lpe<MODE, GEO, 32, true>(h, k, stream);
+        if (k.tag_timeout != 0)
+            return idx ? launch_lpe<MODE, GEO, 32, true, true>(h, k, stream) : launch_lpe<MODE, GEO, 32, true, false>(h, k, stream);
     }
 #ifdef SSD_ENABLE_LPE16                                        // experiment: two envs per warp (measured slower, profiles/r1_notes.md)
-    if (h->lanes_per_env == 16) return launch_lpe<MODE, GEO, 16, false>(h, k, stream);
+    if (h->lanes_per_env == 16 && !idx) return launch_lpe<MODE, GEO, 16, false, false>(h, k, stream);
 #endif
-    return launch_lpe<MODE, GEO, 32, false>(h, k, stream);
+    return idx ? launch_lpe<MODE, GEO, 32, false, true>(h, k, stream) : launch_lpe<MODE, GEO, 32, false, false>(h, k, stream);
 }
 
 // The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
@@ -1320,6 +1390,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     k.kind = cfg->kind; k.B = cfg->n_envs; k.n = n; k.H = H; k.W = W; k.G = G; k.V = V; k.N = gv.N;
     k.GS = gv.GS; k.NA = round_up(n, 4);
     k.RP = gv.RP; k.PS = gv.PS; k.AS = gv.AS; k.ES = n * k.AS;
+    k.RS4 = gv.RS4; k.AS4 = gv.AS4;
     k.LPn = gv.LPn; k.nw8M = gv.nw8M; k.nw8T = gv.nw8T; k.maskM8 = gv.maskM8; k.maskT8 = gv.maskT8;
     k.pitchM = gv.pitchM; k.pitchT = gv.pitchT; k.PMS = gv.PMS;
     k.direct = gv.direct; k.padF = gv.padF; k.padB = gv.padB;
@@ -1397,6 +1468,21 @@ int ssd_get_layout(const ssd_handle* h, ssd_layout* o) {
     return SSD_OK;
 }
 
+int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* o) {
+    if (!h || !o || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
+    const KParams& k = h->kp;
+    o->format = format;
+    if (format == SSD_OBS_RGB) { o->row_stride = k.RP; o->plane_stride = k.PS; o->agent_stride = k.AS; o->env_stride = k.ES; }
+    else { o->row_stride = k.RS4; o->plane_stride = 0; o->agent_stride = k.AS4; o->env_stride = k.n * k.AS4; }
+    return SSD_OK;
+}
+
+int ssd_set_obs_format(ssd_handle* h, int32_t format) {
+    if (!h || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
+    h->obs_format = format;
+    return SSD_OK;
+}
+
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws, uint8_t* obs, void* stream) {
     KParams k;
     const int rc = fill_common(h, st, draws, k);
@@ -1453,7 +1539,8 @@ int ssd_step_host(ssd_handle* h, const ssd_state* st, const uint8_t* h_actions, 
     if (h_out->clean) SSD_CUDA(cudaMemcpyAsync(h_out->clean, d_out->clean, B * k.n, cudaMemcpyDeviceToHost, s));
     if (h_out->apple_cnt) SSD_CUDA(cudaMemcpyAsync(h_out->apple_cnt, d_out->apple_cnt, B * 2, cudaMemcpyDeviceToHost, s));
     if (h_out->done) SSD_CUDA(cudaMemcpyAsync(h_out->done, d_out->done, B, cudaMemcpyDeviceToHost, s));
-    if (h_out->obs && d_out->obs) SSD_CUDA(cudaMemcpyAsync(h_out->obs, d_out->obs, B * k.ES, cudaMemcpyDeviceToHost, s));
+    const size_t ES = h->obs_format == SSD_OBS_INDEX4 ? (size_t)k.n * k.AS4 : (size_t)k.ES;
+    if (h_out->obs && d_out->obs) SSD_CUDA(cudaMemcpyAsync(h_out->obs, d_out->obs, B * ES, cudaMemcpyDeviceToHost, s));
     if (h_out->state_rgb && d_out->state_rgb)
         SSD_CUDA(cudaMemcpyAsync(h_out->state_rgb, d_out->state_rgb, B * 3 * k.G, cudaMemcpyDeviceToHost, s));
     SSD_CUDA(cudaStreamSynchronize(s));
@@ -1474,6 +1561,24 @@ int ssd_incentive(const int64_t* actions_inc, const float* reward, int64_t rows,
     incentive_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const long long*>(actions_inc), reward, rows, n_agents, incentive, cost, ratio, T, recip,
         rewards_for_env, rewards_for_inc, recv_sign);
+    SSD_CUDA(cudaGetLastError());
+    return SSD_OK;
+}
+
+int ssd_expand_obs(const ssd_handle* h, const uint8_t* obs_index4, int32_t env_begin, int32_t env_count, float* out, void* stream) {
+    if (!h || !obs_index4 || !out) return SSD_ERR_INVALID;
+    const KParams& k = h->kp;
+    if (env_begin < 0 || env_count < 0 || (int64_t)env_begin + env_count > k.B) return SSD_ERR_INVALID;
+    if (env_count == 0) return SSD_OK;
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    ExpandParams e;
+    e.in = obs_index4 + (size_t)env_begin * k.n * k.AS4;
+    e.out = out;
+    e.N = k.N; e.RS4 = k.RS4; e.AS4 = k.AS4;
+    for (int i = 0; i < 16; ++i) e.lut[i] = k.lut[i];
+    expand_obs_kernel<<<(unsigned)(env_count * k.n), 256, 0, (cudaStream_t)stream>>>(e);
+    ++h->launches;
     SSD_CUDA(cudaGetLastError());
     return SSD_OK;
 }

@@ -53,6 +53,8 @@ class ObsFrontEnd:
 
     def forward_env(self, env, obs_buf=None, out=None):
         """All B*n agent views of an ``SSDBatchEnv`` (row order [B][n], as ``batch['obs'].reshape(bs * n, ...)``)."""
+        if env.obs_format != "rgb":
+            raise ValueError("the fused front end reads RGB planes; this env writes index4 observations")
         lay = env.layout
         return self.forward(env.obs_buf if obs_buf is None else obs_buf, env.B * env.n, lay.obs_agent_stride,
                             lay.obs_plane_stride, lay.obs_row_stride, out=out)

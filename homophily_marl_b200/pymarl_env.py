@@ -88,6 +88,8 @@ class _SSDEnv(MultiAgentEnv):
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
                      disable_fire_action=True, obs_color="simplified")
         extra.update(extra_args or {})
+        # get_obs is the reference's RGB list whatever extra_args says: the facade always runs the env in the "rgb" format
+        extra["obs_format"] = "rgb"
         # `ascii_map` is accepted and IGNORED, as in the reference: CleanupEnv / HarvestEnv replace it with the map that
         # `map=` selects (cleanup.py:31-54, harvest.py:18-22).  Custom maps: SSDBatchEnv(rows=...).
         device = device or os.environ.get("SSD_B200_DEVICE", "cuda:0")
@@ -178,7 +180,8 @@ class _SSDEnv(MultiAgentEnv):
         return np.lib.stride_tricks.as_strided(self._obs_host, shape=(n, 3, N, N), strides=self._obs_strides)
 
     def get_obs(self):
-        """List of n arrays (3, N, N) float = u8 / 256 (map_env.py:923-945)."""
+        """List of n arrays (3, N, N) float = u8 / 256 (map_env.py:923-945).  Always RGB: the facade ignores
+        ``extra_args["obs_format"]``."""
         return list(self._obs_u8() / 256)
 
     def get_obs_agent(self, agent_id):

@@ -50,6 +50,10 @@ extern "C" {
 #define SSD_CELL_RIVER  4
 #define SSD_CELL_STREAM 5
 
+/* observation formats (ssd_set_obs_format) */
+#define SSD_OBS_RGB    0   /* u8 RGB planes [n][3][N][N], rows padded (ssd_layout strides): the default            */
+#define SSD_OBS_INDEX4 1   /* packed colour indices [n][N][N], 4 bits per pixel (ssd_obs_layout strides; DESIGN.md §3) */
+
 typedef struct ssd_handle ssd_handle;
 
 /* Constructor arguments == the reference's env_args (config/envs/*.yaml:3-15,
@@ -95,6 +99,24 @@ typedef struct ssd_layout {
     int32_t obs_row_stride;   /* bytes between pixel rows (N rounded up to 4); pad bytes are 0 */
 } ssd_layout;
 
+/* Observation strides of one format, in bytes.
+ * SSD_OBS_RGB: the obs_* members of ssd_layout.
+ * SSD_OBS_INDEX4: pixel (y, x) of agent a's view is the colour index the RGB renderer looks up for it, so
+ *   color_lut[index] is the RGB pixel byte for byte: 0-5 cell codes, 6 outside the map, agents 7 in the simplified
+ *   scheme (every agent has one colour) and 6 + agent char of the highest index on the cell in the full scheme.  It
+ *   carries more than RGB: empty and outside (both black), or agents and walls (both blue when simplified), differ.
+ *   Two pixels per byte: pixel x of a row is byte x >> 1, low nibble when x is even.  An agent out of play (tagging-out)
+ *   sees all zero bytes and is absent from every view, as in RGB.  Every pad nibble and pad byte is 0.
+ *   row_stride = ceil(N/2) rounded up to 4, plane_stride = 0, agent_stride = N * row_stride rounded up to 16,
+ *   env_stride = n_agents * agent_stride. */
+typedef struct ssd_obs_layout {
+    int32_t format;           /* SSD_OBS_*                                       */
+    int32_t row_stride;       /* bytes between pixel rows                        */
+    int32_t plane_stride;     /* bytes between colour planes (0 for index4)      */
+    int32_t agent_stride;     /* bytes between agents                            */
+    int32_t env_stride;       /* bytes between envs                              */
+} ssd_obs_layout;
+
 /* Persistent per-env state (MapEnv.world_map, Agent.pos/orientation, _episode_steps, rewards). */
 typedef struct ssd_state {
     uint8_t*  grid;      /* [B][grid_stride]   cell codes, padding bytes stay 0           */
@@ -115,7 +137,8 @@ typedef struct ssd_step_out {
     uint8_t*  clean;      /* [B][n]   info["clean_num"]                                 */
     uint16_t* apple_cnt;  /* [B]      info["apple_den"] * H*W                           */
     uint8_t*  done;       /* [B]      terminated                                        */
-    uint8_t*  obs;        /* [B][obs_env_stride] u8 RGB planes, rows padded to obs_row_stride (get_obs * 256) or NULL */
+    uint8_t*  obs;        /* [B][env_stride] observations in the handle's format (ssd_set_obs_format): u8 RGB planes, rows
+                           * padded to obs_row_stride (get_obs * 256), or packed colour indices; or NULL              */
     uint8_t*  state_rgb;  /* [B][3][H][W] (get_state * 256) or NULL                     */
 } ssd_step_out;
 
@@ -143,6 +166,16 @@ uint32_t ssd_prob_to_threshold(double p);
 int ssd_create(const ssd_config* cfg, ssd_handle** out);
 int ssd_destroy(ssd_handle* h);
 int ssd_get_layout(const ssd_handle* h, ssd_layout* out);
+
+/* Strides of observation format `format` (SSD_OBS_*), whichever format the handle is in, so that a caller can allocate
+ * before switching.  ssd_get_layout always reports the RGB strides.  SSD_ERR_INVALID for a NULL handle or an unknown format. */
+int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* out);
+
+/* Selects the format of every later `obs` buffer of ssd_reset, ssd_step, ssd_step_range, ssd_render and ssd_step_host
+ * (which then copies B * env_stride bytes).  A handle starts in SSD_OBS_RGB.  It is a host-side property of the handle,
+ * serialised like every other call on it; a CUDA graph keeps the format it was captured with.  SSD_ERR_INVALID, before
+ * any CUDA call, for a NULL handle or an unknown format. */
+int ssd_set_obs_format(ssd_handle* h, int32_t format);
 
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */
@@ -209,7 +242,13 @@ int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int3
 int ssd_frontend_destroy(ssd_frontend* f);
 int ssd_frontend_last_cuda_error(void);
 
-/* Kernels launched through this handle since creation (bench.py's gpu_launches). */
+/* SSD_OBS_INDEX4 observations of envs [env_begin, env_begin + env_count) -> f32 out [env_count][n][3][N][N] contiguous,
+ * each value color_lut[index][c] / 256: bit-identical to the RGB observation / 256, zero views of agents out of play
+ * included.  obs_index4 is the base of the whole-batch buffer, `out` holds the range only.  One kernel launch on `stream`. */
+int ssd_expand_obs(const ssd_handle* h, const uint8_t* obs_index4, int32_t env_begin, int32_t env_count, float* out,
+                   void* stream);
+
+/* Kernels launched through this handle since creation (bench.py's gpu_launches), ssd_expand_obs included. */
 int64_t ssd_launch_count(const ssd_handle* h);
 
 /* Checked build only (-DSSD_BOUNDS_CHECK, libssd_b200_check.so): number of shared-memory index violations seen so

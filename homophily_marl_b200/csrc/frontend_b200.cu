@@ -665,7 +665,8 @@ int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int3
     // Load balance: 160 tiles on 148 persistent CTAs would leave a second, almost empty round, so the (tile, chunk) units are
     // dealt out as one sequence in equal contiguous shares (see the kernel).  Tiles cut by a share boundary are combined in CTA
     // order by whichever CTA stores its part last, so the result does not depend on timing.  The scratch slots and arrival
-    // counters belong to the handle: one forward at a time per handle (stream order is enough).
+    // counters belong to the handle: one forward at a time per handle (stream order is enough; concurrent streams need one
+    // handle each).
     const long long units = p.epi.units = (long long)p.n_tiles * p.n_chunks;
     // Grid: all SMs with equal shares, or -- few tiles -- s CTAs per tile (shares aligned with the tiles, one segment per CTA);
     // whichever has the cheaper busiest CTA at ~1.5 chunks of pipeline fill + accumulator drain per segment.

@@ -19,16 +19,16 @@ class ObsFrontEnd:
     def __init__(self, conv_w, conv_b, fc_w, fc_b, view, negative_slope=0.01, device="cuda:0"):
         if not torch.cuda.is_available():
             raise RuntimeError("ObsFrontEnd needs a CUDA device (sm_100a); there is no CPU fallback")
-        self.device = torch.device(device)
+        device = torch.device(device)
+        self.device = torch.device("cuda", device.index if device.index is not None else torch.cuda.current_device())
         self.view, self.N, self.P = int(view), 2 * int(view) + 1, 2 * int(view) - 1
         arrs = [np.ascontiguousarray(torch.as_tensor(t).detach().cpu().numpy(), dtype=np.float32) for t in (conv_w, conv_b, fc_w, fc_b)]
         if arrs[0].shape != (6, 3, 3, 3) or arrs[1].shape != (6,) or arrs[2].shape != (32, 6 * self.P * self.P) or arrs[3].shape != (32,):
             raise ValueError("expected Conv2d(3,6,3) and Linear(6*(N-2)^2, 32) parameters (config/default.yaml defaults)")
         self.lib = _capi.load()
         self._h = C.c_void_p()
-        idx = self.device.index if self.device.index is not None else torch.cuda.current_device()
         _capi.check(self.lib.ssd_frontend_create(self.view, arrs[0].ctypes.data, arrs[1].ctypes.data, arrs[2].ctypes.data,
-                                                 arrs[3].ctypes.data, float(negative_slope), idx, C.byref(self._h)))
+                                                 arrs[3].ctypes.data, float(negative_slope), self.device.index, C.byref(self._h)))
 
     @classmethod
     def from_module(cls, conv_to_fc, view, device=None):
@@ -38,17 +38,28 @@ class ObsFrontEnd:
         return cls(conv.weight, conv.bias, fc.weight, fc.bias, view, negative_slope=getattr(act, "negative_slope", 0.01), device=device)
 
     def forward(self, obs_buf: torch.Tensor, rows: int, agent_stride: int, plane_stride: int, row_stride: int, out=None):
-        """obs_buf: u8 CUDA buffer holding `rows` agent views `agent_stride` bytes apart.  Returns f32 [rows, 32]."""
+        """obs_buf: u8 CUDA buffer holding `rows` agent views `agent_stride` bytes apart.  Returns f32 [rows, 32].
+
+        One launch on the current stream of the handle's device.  The handle owns the scratch of tiles shared between CTAs, so
+        it must not run on two streams at once: concurrent callers (env ranges) each hold their own handle."""
+        rows = int(rows)
         if obs_buf.dtype != torch.uint8 or not obs_buf.is_cuda or not obs_buf.is_contiguous():
             raise ValueError("obs_buf must be a contiguous uint8 CUDA tensor")
+        if obs_buf.device != self.device:
+            raise ValueError(f"obs_buf is on {obs_buf.device}, the front end on {self.device}")
         if obs_buf.numel() < rows * agent_stride:
             raise ValueError("obs_buf is smaller than rows * agent_stride")
         if out is None:
-            out = torch.empty((rows, 32), dtype=torch.float32, device=obs_buf.device)
-        with torch.cuda.device(obs_buf.device):
-            _capi.check(self.lib.ssd_frontend_forward(self._h, obs_buf.data_ptr(), int(rows), int(agent_stride), int(plane_stride),
+            out = torch.empty((rows, 32), dtype=torch.float32, device=self.device)
+        elif (not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or out.device != self.device
+              or tuple(out.shape) != (rows, 32) or not out.is_contiguous()):
+            raise ValueError(f"out must be a contiguous float32 tensor of shape ({rows}, 32) on {self.device}")
+        if rows == 0:                                         # nothing to launch (an empty tensor may have no storage)
+            return out
+        with torch.cuda.device(self.device):
+            _capi.check(self.lib.ssd_frontend_forward(self._h, obs_buf.data_ptr(), rows, int(agent_stride), int(plane_stride),
                                                       int(row_stride), out.data_ptr(),
-                                                      C.c_void_p(torch.cuda.current_stream(obs_buf.device).cuda_stream)))
+                                                      C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
         return out
 
     def forward_env(self, env, obs_buf=None, out=None):
@@ -73,7 +84,10 @@ class ObsFrontEnd:
 
 class MacFrontEnd:
     """Reroutes ``mac.agent.rgb_preprocess`` (homophily_controller.py:132-136) to the fused kernel while a rollout is in
-    progress.  The packed weights follow the module's parameters (re-packed when an optimiser step bumped their versions)."""
+    progress.  The packed weights follow the module's parameters (re-packed when an optimiser step bumped their versions).
+
+    One ``ObsFrontEnd`` per env range, keyed by the range's first agent view: the batched runner rolls ranges out on their own
+    streams without host syncs, and a handle's scratch and tile counters serve one forward at a time."""
 
     def __init__(self, mac, env):
         self.mac, self.env = mac, env
@@ -81,24 +95,31 @@ class MacFrontEnd:
         self.original = mac.agent.rgb_preprocess
         self.active = False
         self.rows = None                                      # (first agent view, count) of the env range being rolled out
-        self._fe, self._stamp = None, None
+        self._fes, self._stamp = {}, None
         mac.agent.rgb_preprocess = self
 
-    def _front_end(self):
+    def _front_end(self, first=0):
         stamp = tuple((p.data_ptr(), p._version) for p in self.module.parameters())
-        if self._fe is None or stamp != self._stamp:
-            if self._fe is not None:
-                self._fe.close()
-            self._fe, self._stamp = ObsFrontEnd.from_module(self.module, self.env.spec.view, device=self.env.device), stamp
-        return self._fe
+        if stamp != self._stamp:                              # new weights: every range's handle is re-packed on its next use
+            self._close_all()
+            self._stamp = stamp
+        fe = self._fes.get(first)
+        if fe is None:
+            fe = self._fes[first] = ObsFrontEnd.from_module(self.module, self.env.spec.view, device=self.env.device)
+        return fe
+
+    def _close_all(self):
+        for fe in self._fes.values():
+            fe.close()
+        self._fes.clear()
 
     def __call__(self, x):
         first, count = self.rows if self.rows is not None else (0, self.env.B * self.env.n)
         if not self.active or x.shape[0] != count:            # learner path (autograd) / foreign batch: the module
             return self.original(x)
         lay = self.env.layout
-        return self._front_end().forward(self.env.obs_buf.view(-1)[first * lay.obs_agent_stride:], count, lay.obs_agent_stride,
-                                         lay.obs_plane_stride, lay.obs_row_stride)
+        return self._front_end(first).forward(self.env.obs_buf.view(-1)[first * lay.obs_agent_stride:], count, lay.obs_agent_stride,
+                                              lay.obs_plane_stride, lay.obs_row_stride)
 
     def __deepcopy__(self, memo):
         """``copy.deepcopy(mac)`` (the learner's target network, homophily_learner.py:47) must not copy the kernel handle: the
@@ -111,5 +132,4 @@ class MacFrontEnd:
 
     def detach(self):
         self.mac.agent.rgb_preprocess = self.original
-        if self._fe is not None:
-            self._fe.close()
+        self._close_all()

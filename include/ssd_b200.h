@@ -235,8 +235,9 @@ typedef struct ssd_frontend ssd_frontend;
 int ssd_frontend_create(int32_t view, const float* conv_w, const float* conv_b, const float* fc_w, const float* fc_b,
                         float negative_slope, int32_t device, ssd_frontend** out);
 /* obs: DEVICE u8, `rows` agent views `obs_agent_stride` bytes apart (ssd_layout strides); out: DEVICE f32 [rows][32].
- * One kernel launch on `stream`.  The handle owns scratch for tiles shared between CTAs: one forward at a time per handle
- * (stream order is enough); the result does not depend on timing. */
+ * One kernel launch on `stream`.  The handle owns scratch and counters for tiles shared between CTAs: one forward at a time
+ * per handle (stream order is enough), so a handle must not be shared across streams that run concurrently -- the batched
+ * runner holds one per env range.  The result does not depend on timing. */
 int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int32_t obs_agent_stride, int32_t obs_plane_stride,
                          int32_t obs_row_stride, float* out, void* stream);
 int ssd_frontend_destroy(ssd_frontend* f);

@@ -21,7 +21,8 @@ EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_pr
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_render",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
-           "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_destroy", "ssd_frontend_last_cuda_error")
+           "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
+           "ssd_frontend_last_cuda_error")
 
 
 class SsdConfig(C.Structure):
@@ -101,6 +102,8 @@ def load():
     L.ssd_frontend_create.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int32,
                                       C.POINTER(C.c_void_p)]
     L.ssd_frontend_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    L.ssd_frontend_forward_index4.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                              C.c_void_p]
     L.ssd_frontend_destroy.argtypes = [C.c_void_p]
     L.ssd_launch_count.restype = C.c_int64
     L.ssd_launch_count.argtypes = [C.c_void_p]

@@ -71,13 +71,19 @@ class BatchedEpisodeRunner:
                                  preprocess=preprocess, device=self.args.device)
         self.mac = mac
         # args.fused_frontend: during rollouts the MAC's rgb_preprocess (conv3x3 + FC on fp32 obs, homophily_controller.py:132-136)
-        # is served by the fused u8 front-end kernel reading the env's observation buffer (frontend.MacFrontEnd)
+        # is served by the fused u8 front-end kernel reading the env's observation buffer (frontend.MacFrontEnd).  True reads RGB
+        # planes, "index4" packed colour indices; each needs the env to write that format.
         self.front = None
-        if getattr(self.args, "fused_frontend", False) and self.env.obs_format != "rgb":
-            raise ValueError("fused_frontend reads RGB observation planes; it cannot run with obs_format 'index4'")
-        if getattr(self.args, "fused_frontend", False) and getattr(self.args, "rgb_input", False):
+        fused = getattr(self.args, "fused_frontend", False)
+        if fused is True and self.env.obs_format != "rgb":
+            raise ValueError("fused_frontend: True reads RGB observation planes; with obs_format 'index4' use fused_frontend: index4")
+        if fused == "index4" and self.env.obs_format != "index4":
+            raise ValueError(f"fused_frontend: index4 needs obs_format 'index4', the env writes {self.env.obs_format!r}")
+        if fused and fused is not True and fused != "index4":
+            raise ValueError(f"fused_frontend must be False, True or 'index4', got {fused!r}")
+        if fused and getattr(self.args, "rgb_input", False):
             from .frontend import MacFrontEnd
-            self.front = MacFrontEnd(mac, self.env)
+            self.front = MacFrontEnd(mac, self.env, obs_format="index4" if fused == "index4" else "rgb")
 
     def use_batch_factory(self, new_batch):
         """``new_batch()`` must return a fresh reference ``EpisodeBatch`` for B episodes of T+1 steps."""

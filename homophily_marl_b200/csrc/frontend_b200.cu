@@ -106,6 +106,8 @@ struct FrontParams {
     int n_tiles;
     const uint8_t* obs;
     EpilogueParams epi;
+    uint32_t pal[3][4];                      // index4 only: byte i of plane c = color_lut[i][c]; behind everything else, so the RGB
+                                             // kernel's parameter offsets (the tensor map's included) stay where they were
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -195,6 +197,19 @@ __device__ __forceinline__ float byte_to_float(uint32_t word, int b) {
     return __uint_as_float(v) - 8388608.0f;
 }
 
+__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
+    uint32_t v;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(v) : "r"(a), "r"(b), "r"(sel));
+    return v;
+}
+
+// Four colour indices -> four channel bytes of one plane through its 16-byte palette `pal`.  A PRMT selector nibble picks one
+// of 8 bytes by its low 3 bits (bit 3 would replicate the byte's sign), so `sel` holds the indices & 7, one lookup reads
+// entries 0-7, one entries 8-15, and `m` (0xff in the bytes whose index has bit 3 set) picks between them.
+__device__ __forceinline__ uint32_t palette4(const uint32_t (&pal)[4], uint32_t sel, uint32_t m) {
+    return (prmt(pal[2], pal[3], sel) & m) | (prmt(pal[0], pal[1], sel) & ~m);
+}
+
 // hi*hi accumulators each issuer rotates over in a segment of `stages` stages: chains of at most ~24 MMAs each (see `Precision`),
 // at most 7 (+ 1 for the lo terms) of the 8 accumulators an issuer owns
 __device__ __forceinline__ int rotation(int stages) {
@@ -203,7 +218,9 @@ __device__ __forceinline__ int rotation(int stages) {
 }
 
 // Epilogue of one segment, by warps 0-3 (TMEM lane = GEMM row = r).  Kept out of line so that its 32 + 32 live registers do not
-// weigh on the register allocation of the convolution loop.
+// weigh on the register allocation of the convolution loop.  One copy per kernel (IDX is otherwise unused): with a single
+// caller the compiler addresses that kernel's `arrivals_s` directly instead of through the pointer argument.
+template <bool IDX>
 __device__ __noinline__ void segment_epilogue(const EpilogueParams p, uint32_t tmem_base, uint32_t bar_tmem_full, uint32_t bar_tmem_empty,
                                           int* arrivals_s, uint32_t parity, int stages_here, int tile, bool whole_tile,
                                           bool first_segment) {
@@ -293,6 +310,10 @@ __device__ __noinline__ void segment_epilogue(const EpilogueParams p, uint32_t t
     }
 }
 
+// IDX: the views are SSD_OBS_INDEX4 rows (pixel x = nibble x of the row, p.RP bytes apart, p.PS unused) instead of RGB planes.
+// Only what a window row is loaded from differs: two nibble words instead of nine byte words, expanded through p.pal into
+// the same 3 planes x 3 words of channel bytes, so everything from byte_to_float on is the same code and the same arithmetic.
+template <bool IDX>
 __global__ void __launch_bounds__(kThreads, 1)
 obs_frontend_kernel(const __grid_constant__ FrontParams p, const __grid_constant__ CUtensorMap wmap) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -350,6 +371,10 @@ obs_frontend_kernel(const __grid_constant__ FrontParams p, const __grid_constant
             uint32_t win[3][9], nxt[9];
             // src points at (row yy, pixel x0) of plane 0; the three guards depend on the column only
             auto load_row = [&](uint32_t (&dst)[9], const uint8_t* src, bool g0, bool g1, bool g2) {
+                if constexpr (IDX) {                                           // raw nibble words: pixels x0..x0+7, x0+8..x0+15
+                    dst[0] = g0 ? __ldg(reinterpret_cast<const uint32_t*>(src)) : 0u;
+                    dst[1] = g2 ? __ldg(reinterpret_cast<const uint32_t*>(src + 4)) : 0u;   // only x0+8, x0+9 < N are used
+                } else {
 #pragma unroll
                 for (int ch = 0; ch < 3; ++ch, src += p.PS) {
 #ifdef FE_DIAG_NOLOAD                                                  // diagnostic build: one load per row instead of 9
@@ -361,6 +386,21 @@ obs_frontend_kernel(const __grid_constant__ FrontParams p, const __grid_constant
                     dst[ch * 3 + 2] = g2 ? __ldg(reinterpret_cast<const uint32_t*>(src + 8)) : 0u;   // only pixels x0+8, x0+9 < N are used
 #endif
                 }
+                }
+            };
+            // index4: the two nibble words of a row (raw[0], raw[1]) -> the RGB window row (in place when dst is raw)
+            auto expand_row = [&](uint32_t (&dst)[9], const uint32_t (&raw)[9]) {
+                const uint32_t w = raw[0], w1 = raw[1];
+                const uint32_t s = w & 0x77777777u, s1 = w1 & 0x77u;
+                // byte masks from bit 3 of each index: a PRMT selector nibble >= 8 replicates the chosen byte's top bit, which is
+                // bit 3 of the odd pixel of that byte of w, or of the even pixel in w << 4
+                const uint32_t m0 = prmt(w << 4, w, 0xD9C8u), m1 = prmt(w << 4, w, 0xFBEAu), m2 = prmt(w1 << 4, w1, 0xD9C8u);
+#pragma unroll
+                for (int ch = 0; ch < 3; ++ch) {
+                    dst[ch * 3] = palette4(p.pal[ch], s, m0);
+                    dst[ch * 3 + 1] = palette4(p.pal[ch], s >> 16, m1);
+                    dst[ch * 3 + 2] = palette4(p.pal[ch], s1, m2);
+                }
             };
             int xb = c_begin / p.P, y = c_begin - xb * p.P;                    // kept incrementally: no division per chunk
             const uint8_t* next_row = view;                                    // row y + 3 of the current column, at pixel x0
@@ -368,15 +408,22 @@ obs_frontend_kernel(const __grid_constant__ FrontParams p, const __grid_constant
             for (int c = c_begin; c < c_end; ++c) {
                 if (c == c_begin || y == 0) {                                  // first chunk of the item or of a column: whole window
                     const int x0 = xb * 16 + strip * 8;
-                    g0 = x0 < p.RP; g1 = x0 + 4 < p.RP; g2 = x0 + 8 < p.N;
-                    const uint8_t* src = view + y * p.RP + x0;
+                    // index4: x0 is a multiple of 8, so a nibble word at byte x0 / 2 < ceil(N / 2) <= RP (a multiple of 4) ends
+                    // inside the row stride
+                    g0 = x0 < (IDX ? p.N : p.RP); g1 = x0 + 4 < p.RP; g2 = x0 + 8 < p.N;
+                    const uint8_t* src = view + y * p.RP + (IDX ? x0 >> 1 : x0);
                     load_row(win[0], src, g0, g1, g2);
                     load_row(win[1], src + p.RP, g0, g1, g2);
                     load_row(nxt, src + 2 * p.RP, g0, g1, g2);
                     next_row = src + 3 * p.RP;
+                    if constexpr (IDX) { expand_row(win[0], win[0]); expand_row(win[1], win[1]); }
                 }
+                if constexpr (IDX) {
+                    expand_row(win[2], nxt);                                   // nxt stays raw: its loads landed during the last chunk
+                } else {
 #pragma unroll
-                for (int k = 0; k < 9; ++k) win[2][k] = nxt[k];
+                    for (int k = 0; k < 9; ++k) win[2][k] = nxt[k];
+                }
                 if (c + 1 < c_end && y + 1 < p.P) load_row(nxt, next_row, g0, g1, g2);   // the row the next chunk adds
                 next_row += p.RP;
                 if (++y == p.P) { y = 0; ++xb; }
@@ -464,7 +511,7 @@ obs_frontend_kernel(const __grid_constant__ FrontParams p, const __grid_constant
                 }
             }
             if (warp < 4)
-                segment_epilogue(p.epi, tmem_base, smem_u32(&bar_tmem_full), smem_u32(&bar_tmem_empty), &arrivals_s, item_n & 1u, stages_here,
+                segment_epilogue<IDX>(p.epi, tmem_base, smem_u32(&bar_tmem_full), smem_u32(&bar_tmem_empty), &arrivals_s, item_n & 1u, stages_here,
                                  tile, c_end - c_begin == p.n_chunks, first_segment);
         }
     } else if (warp != 9) {
@@ -564,6 +611,56 @@ struct ssd_frontend {
     size_t smem_bytes;
 };
 
+// Launch of either format: `p` is the handle's parameters with the obs strides (and, for index4, the palette) filled in.
+static int frontend_launch(ssd_frontend* f, FrontParams& p, bool index4, const uint8_t* obs, int64_t rows, float* out, void* stream) {
+    if ((rows + kTileM - 1) / kTileM * p.n_chunks >= (1ll << 31)) return SSD_ERR_INVALID;   // the kernel counts units in 32 bits
+    p.epi.rows = rows; p.n_tiles = (int)((rows + kTileM - 1) / kTileM);
+    p.obs = obs; p.epi.out = out;
+    // Load balance: 160 tiles on 148 persistent CTAs would leave a second, almost empty round, so the (tile, chunk) units are
+    // dealt out as one sequence in equal contiguous shares (see the kernel).  Tiles cut by a share boundary are combined in CTA
+    // order by whichever CTA stores its part last, so the result does not depend on timing.  The scratch slots and arrival
+    // counters belong to the handle: one forward at a time per handle (stream order is enough; concurrent streams need one
+    // handle each).
+    const long long units = p.epi.units = (long long)p.n_tiles * p.n_chunks;
+    // Grid: all SMs with equal shares, or -- few tiles -- s CTAs per tile (shares aligned with the tiles, one segment per CTA);
+    // whichever has the cheaper busiest CTA at ~1.5 chunks of pipeline fill + accumulator drain per segment.
+    int grid = units < f->sms ? (int)units : f->sms;
+    {
+        const double share = (double)units / grid;
+        double best = share + 1.5 * (share < p.n_chunks ? 2.0 : (double)((long long)(share / p.n_chunks) + 2));
+        for (int s_ = 1; s_ <= p.n_chunks && (long long)p.n_tiles * s_ <= f->sms; ++s_) {
+            const double cost = (double)((p.n_chunks + s_ - 1) / s_) + 1.5;
+            if (cost < best - 1e-9) { best = cost; grid = p.n_tiles * s_; }
+        }
+    }
+    { const char* e_ = getenv("SSD_B200_FRONTEND_GRID"); if (e_ && atoi(e_) >= 1 && atoi(e_) <= grid) grid = atoi(e_); }   // tuning
+    int prev = -1;
+    cudaError_t e = cudaGetDevice(&prev);
+    if (e == cudaSuccess && prev != f->device) e = cudaSetDevice(f->device);
+    if (e == cudaSuccess && !f->d_scratch)                     // first call (not capturable): two partial tiles per CTA
+        e = cudaMalloc(&f->d_scratch, (size_t)2 * f->sms * kTileM * kFeat * sizeof(float));
+    if (e == cudaSuccess && (size_t)p.n_tiles > f->arrivals_len) {             // first call / larger batch (not capturable)
+        if (f->d_arrivals) cudaFree(f->d_arrivals);
+        f->d_arrivals = nullptr; f->arrivals_len = 0;
+        const size_t len = ((size_t)p.n_tiles + 1023) / 1024 * 1024;
+        e = cudaMalloc(&f->d_arrivals, len * sizeof(int));
+        if (e == cudaSuccess) e = cudaMemsetAsync(f->d_arrivals, 0, len * sizeof(int), (cudaStream_t)stream);
+        if (e == cudaSuccess) f->arrivals_len = len;
+    }
+    p.epi.scratch = f->d_scratch;
+    p.epi.tile_arrivals = f->d_arrivals;
+    if (e == cudaSuccess) {
+        if (index4)
+            obs_frontend_kernel<true><<<grid, kThreads, f->smem_bytes, (cudaStream_t)stream>>>(p, f->wmap);
+        else
+            obs_frontend_kernel<false><<<grid, kThreads, f->smem_bytes, (cudaStream_t)stream>>>(p, f->wmap);
+        e = cudaGetLastError();
+    }
+    if (prev >= 0 && prev != f->device) cudaSetDevice(prev);
+    if (e != cudaSuccess) { g_front_cuda_error = (int)e; return SSD_ERR_CUDA; }
+    return SSD_OK;
+}
+
 extern "C" {
 
 int ssd_frontend_create(int32_t view, const float* conv_w, const float* conv_b, const float* fc_w, const float* fc_b,
@@ -637,7 +734,9 @@ int ssd_frontend_create(int32_t view, const float* conv_w, const float* conv_b, 
     }
     f->smem_bytes = (size_t)kSmemBytes + 1024;
     if (e == cudaSuccess && rc == SSD_OK)
-        e = cudaFuncSetAttribute(obs_frontend_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f->smem_bytes);
+        e = cudaFuncSetAttribute(obs_frontend_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f->smem_bytes);
+    if (e == cudaSuccess && rc == SSD_OK)
+        e = cudaFuncSetAttribute(obs_frontend_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f->smem_bytes);
     if (prev >= 0 && prev != device) cudaSetDevice(prev);
     if (e != cudaSuccess || rc != SSD_OK) {
         if (e != cudaSuccess) g_front_cuda_error = (int)e;
@@ -648,7 +747,6 @@ int ssd_frontend_create(int32_t view, const float* conv_w, const float* conv_b, 
     *out = f;
     return SSD_OK;
 }
-
 int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int32_t obs_agent_stride, int32_t obs_plane_stride,
                          int32_t obs_row_stride, float* out, void* stream) {
     if (!f || !obs || !out || rows < 0) return SSD_ERR_INVALID;
@@ -659,49 +757,23 @@ int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int3
         (reinterpret_cast<uintptr_t>(out) & 15))
         return SSD_ERR_INVALID;
     p.RP = obs_row_stride; p.PS = obs_plane_stride; p.AS = obs_agent_stride;
-    if ((rows + kTileM - 1) / kTileM * p.n_chunks >= (1ll << 31)) return SSD_ERR_INVALID;   // the kernel counts units in 32 bits
-    p.epi.rows = rows; p.n_tiles = (int)((rows + kTileM - 1) / kTileM);
-    p.obs = obs; p.epi.out = out;
-    // Load balance: 160 tiles on 148 persistent CTAs would leave a second, almost empty round, so the (tile, chunk) units are
-    // dealt out as one sequence in equal contiguous shares (see the kernel).  Tiles cut by a share boundary are combined in CTA
-    // order by whichever CTA stores its part last, so the result does not depend on timing.  The scratch slots and arrival
-    // counters belong to the handle: one forward at a time per handle (stream order is enough; concurrent streams need one
-    // handle each).
-    const long long units = p.epi.units = (long long)p.n_tiles * p.n_chunks;
-    // Grid: all SMs with equal shares, or -- few tiles -- s CTAs per tile (shares aligned with the tiles, one segment per CTA);
-    // whichever has the cheaper busiest CTA at ~1.5 chunks of pipeline fill + accumulator drain per segment.
-    int grid = units < f->sms ? (int)units : f->sms;
-    {
-        const double share = (double)units / grid;
-        double best = share + 1.5 * (share < p.n_chunks ? 2.0 : (double)((long long)(share / p.n_chunks) + 2));
-        for (int s_ = 1; s_ <= p.n_chunks && (long long)p.n_tiles * s_ <= f->sms; ++s_) {
-            const double cost = (double)((p.n_chunks + s_ - 1) / s_) + 1.5;
-            if (cost < best - 1e-9) { best = cost; grid = p.n_tiles * s_; }
-        }
-    }
-    { const char* e_ = getenv("SSD_B200_FRONTEND_GRID"); if (e_ && atoi(e_) >= 1 && atoi(e_) <= grid) grid = atoi(e_); }   // tuning
-    int prev = -1;
-    cudaError_t e = cudaGetDevice(&prev);
-    if (e == cudaSuccess && prev != f->device) e = cudaSetDevice(f->device);
-    if (e == cudaSuccess && !f->d_scratch)                     // first call (not capturable): two partial tiles per CTA
-        e = cudaMalloc(&f->d_scratch, (size_t)2 * f->sms * kTileM * kFeat * sizeof(float));
-    if (e == cudaSuccess && (size_t)p.n_tiles > f->arrivals_len) {             // first call / larger batch (not capturable)
-        if (f->d_arrivals) cudaFree(f->d_arrivals);
-        f->d_arrivals = nullptr; f->arrivals_len = 0;
-        const size_t len = ((size_t)p.n_tiles + 1023) / 1024 * 1024;
-        e = cudaMalloc(&f->d_arrivals, len * sizeof(int));
-        if (e == cudaSuccess) e = cudaMemsetAsync(f->d_arrivals, 0, len * sizeof(int), (cudaStream_t)stream);
-        if (e == cudaSuccess) f->arrivals_len = len;
-    }
-    p.epi.scratch = f->d_scratch;
-    p.epi.tile_arrivals = f->d_arrivals;
-    if (e == cudaSuccess) {
-        obs_frontend_kernel<<<grid, kThreads, f->smem_bytes, (cudaStream_t)stream>>>(p, f->wmap);
-        e = cudaGetLastError();
-    }
-    if (prev >= 0 && prev != f->device) cudaSetDevice(prev);
-    if (e != cudaSuccess) { g_front_cuda_error = (int)e; return SSD_ERR_CUDA; }
-    return SSD_OK;
+    return frontend_launch(f, p, false, obs, rows, out, stream);
+}
+
+int ssd_frontend_forward_index4(ssd_frontend* f, const uint8_t* obs, int64_t rows, int32_t obs_agent_stride,
+                                int32_t obs_row_stride, const uint8_t (*color_lut)[4], float* out, void* stream) {
+    if (!f || !obs || !out || !color_lut || rows < 0) return SSD_ERR_INVALID;
+    FrontParams p = f->fp;
+    if (obs_row_stride < (p.N + 1) / 2 || (obs_row_stride & 3) || obs_agent_stride < p.N * obs_row_stride || (obs_agent_stride & 3) ||
+        (reinterpret_cast<uintptr_t>(obs) & 3) || (reinterpret_cast<uintptr_t>(out) & 15))
+        return SSD_ERR_INVALID;
+    if (rows == 0) return SSD_OK;
+    p.RP = obs_row_stride; p.PS = 0; p.AS = obs_agent_stride;
+    for (int ch = 0; ch < 3; ++ch)
+        for (int j = 0; j < 4; ++j)
+            p.pal[ch][j] = (uint32_t)color_lut[4 * j][ch] | (uint32_t)color_lut[4 * j + 1][ch] << 8 |
+                           (uint32_t)color_lut[4 * j + 2][ch] << 16 | (uint32_t)color_lut[4 * j + 3][ch] << 24;
+    return frontend_launch(f, p, true, obs, rows, out, stream);
 }
 
 int ssd_frontend_destroy(ssd_frontend* f) {

@@ -240,6 +240,13 @@ int ssd_frontend_create(int32_t view, const float* conv_w, const float* conv_b, 
  * runner holds one per env range.  The result does not depend on timing. */
 int ssd_frontend_forward(ssd_frontend* f, const uint8_t* obs, int64_t rows, int32_t obs_agent_stride, int32_t obs_plane_stride,
                          int32_t obs_row_stride, float* out, void* stream);
+/* ssd_frontend_forward on SSD_OBS_INDEX4 agent views: pixel (y, x) of a view is nibble x of row y (byte x >> 1, low nibble
+ * when x is even), and stands for the RGB bytes color_lut[nibble][0..2] (RGB0 rows, the layout of ssd_config.color_lut;
+ * HOST pointer, copied into the launch).  The result is bit-identical to ssd_frontend_forward on the RGB planes
+ * color_lut[index] with any valid RGB strides.  Same handle rules: one forward at a time per handle, whatever the format.
+ * obs_row_stride >= ceil(N / 2) and obs_agent_stride >= N * obs_row_stride, both multiples of 4 (ssd_obs_layout strides). */
+int ssd_frontend_forward_index4(ssd_frontend* f, const uint8_t* obs, int64_t rows, int32_t obs_agent_stride,
+                                int32_t obs_row_stride, const uint8_t (*color_lut)[4], float* out, void* stream);
 int ssd_frontend_destroy(ssd_frontend* f);
 int ssd_frontend_last_cuda_error(void);
 

@@ -29,13 +29,9 @@
 
 namespace {
 
-#ifndef SSD_WARPS
-#define SSD_WARPS 4
-#endif
-#ifndef SSD_MIN_BLOCKS
-#define SSD_MIN_BLOCKS 8
-#endif
-constexpr int kWarps = SSD_WARPS;         // env instances per CTA
+constexpr int kWarps = 4;                 // env instances per CTA
+constexpr int kMinBlocks = 8;             // __launch_bounds__ minimum of resident CTAs per SM
+using ColourLuts = uint32_t[kWarps][16];  // ssd_kernel's static shared memory: one colour LUT per warp
 constexpr uint16_t kNoPoint = 0xFFFF;
 constexpr int kMaxDevices = 64;
 
@@ -60,22 +56,52 @@ struct MapDev {
     uint32_t thr_waste[SSD_MAX_CELLS + 1];
 };
 
+// ------------------------------------------------------------------ geometry
+// Everything that follows from (kind, H, W, V).  Computed by ONE constexpr function used by the host
+// (ssd_create) and, for the reference's shipped maps, at compile time by the kernels (GeoS), so that index
+// arithmetic folds into immediates; any other geometry runs the same code on runtime values (GeoD).
+struct GeoVals {
+    int kind, H, W, V, G, GS, N, RP, PS, AS, LPn, nw8M, nw8T, pitchM, pitchT, PMS;
+    int off_map[4];                           // byte offset of the nibble map read by orientation: 0,1 (LEFT/RIGHT) -> MT, 2,3 -> M
+    int direct, padF, padB;                   // small views (RP <= 16) are gathered straight from the staged grid: no maps, but
+                                              // V rows of slack before / after the grid so that column runs need no bounds test
+    uint32_t maskM8;                          // valid-nibble mask of the last word of a map row
+    int RS4, AS4;                             // SSD_OBS_INDEX4: bytes per row (ceil(N/2) rounded to 4) and per agent (rounded to 16)
+};
+__host__ __device__ constexpr int cround_up(int v, int m) { return (v + m - 1) / m * m; }
+__host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V) {
+    GeoVals g{};
+    g.kind = kind; g.H = H; g.W = W; g.V = V; g.G = H * W; g.GS = cround_up(H * W, 16);
+    g.N = 2 * V + 1; g.RP = cround_up(g.N, 4); g.PS = g.N * g.RP; g.AS = cround_up(3 * g.PS, 16);
+    // nibble-packed padded maps; word pitch kept odd so that lanes gathering consecutive rows hit distinct banks
+    g.LPn = cround_up(V, 8); g.nw8M = (W + 7) / 8; g.nw8T = (H + 7) / 8;
+    g.maskM8 = (W & 7) ? (1u << (4 * (W & 7))) - 1u : 0xffffffffu;
+    int wm = (g.LPn + W + V + 7) / 8; if (wm < g.LPn / 8 + g.nw8M) wm = g.LPn / 8 + g.nw8M; if ((wm & 1) == 0) ++wm;
+    int wt = (g.LPn + H + V + 7) / 8; if (wt < g.LPn / 8 + g.nw8T) wt = g.LPn / 8 + g.nw8T; if ((wt & 1) == 0) ++wt;
+    g.pitchM = 4 * wm; g.pitchT = 4 * wt;
+    const int szM = cround_up((H + 2 * V) * g.pitchM, 16) + 16, szT = cround_up((W + 2 * V) * g.pitchT, 16) + 16;
+    g.off_map[0] = 16; g.off_map[1] = 16; g.off_map[2] = 16 + szT; g.off_map[3] = 16 + szT;
+    g.PMS = szT + szM + 32;
+    g.direct = g.RP <= 16;
+    g.padF = g.direct ? cround_up(V * W + 48, 16) : 16;      // + 32 bytes at the very front for the (class, rank) -> lane table
+    g.padB = g.direct ? cround_up(V * W + 32, 16) : 32;
+    if (g.direct) g.PMS = 0;
+    g.RS4 = cround_up((g.N + 1) / 2, 4); g.AS4 = cround_up(g.N * g.RS4, 16);
+    return g;
+}
+
 struct KParams {
-    int kind, B, n, H, W, G, V, N;
+    GeoVals geo;                              // make_geo(kind, H, W, V)
+    int B, n;
     int env0, env1;                           // this launch covers env instances [env0, env1) of the B resident ones
     int pdl;                                  // launched with the programmatic-serialization attribute (set per launch)
-    int GS, NA, RP, PS, AS, ES;               // strides (ssd_layout)
-    int pitchM, pitchT, off_map[4], PMS;      // nibble maps M / MT: row pitches, byte offset by orientation (0,1 -> MT; 2,3 -> M), total bytes
-    int direct, padF, padB;                   // direct-gather render (small views): slack bytes before / after the staged grid
-    int LPn, nw8M, nw8T;                      // left pad in nibbles (V rounded up to 8), words per map row holding cells
-    uint32_t maskM8, maskT8;                  // valid-nibble mask of the last word of a map row
+    int NA;                                   // agent stride (ssd_layout)
     int agents_uniform;                       // all agent colours equal -> no per-agent repaint
     int episode_limit, fire_cost, hit_penalty, beam_len, n_actions;
     int n_apple, n_waste, n_spawn, n_apple4, n_waste2;
     int random_spawn, spawn_rot;
     int base_apples, base_waste;              // 'A' / 'H' cells of the reset grid (cell counts are carried in ssd_state.counts)
-    int smem_per_warp, off_pmap;
-    uint32_t invN20, invW20, invMW20, invMTW20;   // floor(x / d) == (x * inv) >> 20 on the used ranges
+    uint32_t invN20, invW20, invMW20;         // GeoD's divisions: floor(x / d) == (x * inv) >> 20 on the used ranges
     uint32_t seed_lo, seed_hi, gid_base;
     uint32_t thr_harvest[4];
     uint32_t lut[16];
@@ -87,102 +113,57 @@ struct KParams {
     const uint32_t* d_prio; const uint32_t* d_uapple; const uint32_t* d_uwaste; const uint32_t* d_wkey;
     const uint32_t* d_spawnkey; const uint8_t* d_rot;
     int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
-    int RS4, AS4;                             // packed colour-index observations (SSD_OBS_INDEX4): row / agent strides
 };
 
-
-// ------------------------------------------------------------------ geometry
-// Everything that follows from (kind, H, W, V).  Computed by ONE constexpr function used by the host
-// (ssd_create) and, for the reference's shipped maps, at compile time by the kernels (GeoS), so that index
-// arithmetic folds into immediates; any other geometry runs the same code on runtime values (GeoD).
-struct GeoVals {
-    int kind, H, W, V, G, GS, N, RP, PS, AS, LPn, nw8M, nw8T, pitchM, pitchT, off0, off1, off2, off3, PMS;
-    int direct, padF, padB;                   // small views (RP <= 16) are gathered straight from the staged grid: no maps, but
-                                              // V rows of slack before / after the grid so that column runs need no bounds test
-    uint32_t maskM8, maskT8;
-    int RS4, AS4;                             // SSD_OBS_INDEX4: bytes per row (ceil(N/2) rounded to 4) and per agent (rounded to 16)
+// The geometry accessors, over D::vals(): compile-time constants (GeoS) or the launch's KParams::geo (GeoD).  Only the
+// divisions and the by-orientation map offset are written per class: GeoS folds constants where GeoD indexes its values.
+template <class D>
+struct GeoAccess {
+    __device__ __forceinline__ int kind() const { return v().kind; }
+    __device__ __forceinline__ int H() const { return v().H; }
+    __device__ __forceinline__ int W() const { return v().W; }
+    __device__ __forceinline__ int V() const { return v().V; }
+    __device__ __forceinline__ int G() const { return v().G; }
+    __device__ __forceinline__ int GS() const { return v().GS; }
+    __device__ __forceinline__ int N() const { return v().N; }
+    __device__ __forceinline__ int RP() const { return v().RP; }
+    __device__ __forceinline__ int PS() const { return v().PS; }
+    __device__ __forceinline__ int AS() const { return v().AS; }
+    __device__ __forceinline__ int RS4() const { return v().RS4; }
+    __device__ __forceinline__ int AS4() const { return v().AS4; }
+    __device__ __forceinline__ int LPn() const { return v().LPn; }
+    __device__ __forceinline__ int nw8M() const { return v().nw8M; }
+    __device__ __forceinline__ int nw8T() const { return v().nw8T; }
+    __device__ __forceinline__ int pitchM() const { return v().pitchM; }
+    __device__ __forceinline__ int pitchT() const { return v().pitchT; }
+    __device__ __forceinline__ int PMS() const { return v().PMS; }
+    __device__ __forceinline__ bool direct() const { return v().direct != 0; }
+    __device__ __forceinline__ int padF() const { return v().padF; }
+    __device__ __forceinline__ int padB() const { return v().padB; }
+    __device__ __forceinline__ uint32_t maskM8() const { return v().maskM8; }
+private:
+    __device__ __forceinline__ decltype(auto) v() const { return static_cast<const D*>(this)->vals(); }
 };
-__host__ __device__ constexpr int cround_up(int v, int m) { return (v + m - 1) / m * m; }
-__host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V) {
-    GeoVals g{};
-    g.kind = kind; g.H = H; g.W = W; g.V = V; g.G = H * W; g.GS = cround_up(H * W, 16);
-    g.N = 2 * V + 1; g.RP = cround_up(g.N, 4); g.PS = g.N * g.RP; g.AS = cround_up(3 * g.PS, 16);
-    // nibble-packed padded maps; word pitch kept odd so that lanes gathering consecutive rows hit distinct banks
-    g.LPn = cround_up(V, 8); g.nw8M = (W + 7) / 8; g.nw8T = (H + 7) / 8;
-    g.maskM8 = (W & 7) ? (1u << (4 * (W & 7))) - 1u : 0xffffffffu;
-    g.maskT8 = (H & 7) ? (1u << (4 * (H & 7))) - 1u : 0xffffffffu;
-    int wm = (g.LPn + W + V + 7) / 8; if (wm < g.LPn / 8 + g.nw8M) wm = g.LPn / 8 + g.nw8M; if ((wm & 1) == 0) ++wm;
-    int wt = (g.LPn + H + V + 7) / 8; if (wt < g.LPn / 8 + g.nw8T) wt = g.LPn / 8 + g.nw8T; if ((wt & 1) == 0) ++wt;
-    g.pitchM = 4 * wm; g.pitchT = 4 * wt;
-    const int szM = cround_up((H + 2 * V) * g.pitchM, 16) + 16, szT = cround_up((W + 2 * V) * g.pitchT, 16) + 16;
-    g.off0 = 16; g.off1 = 16; g.off2 = 16 + szT; g.off3 = 16 + szT;        // by orientation: LEFT/RIGHT -> MT, UP/DOWN -> M
-    g.PMS = szT + szM + 32;
-    g.direct = g.RP <= 16;
-    g.padF = g.direct ? cround_up(V * W + 48, 16) : 16;      // + 32 bytes at the very front for the (class, rank) -> lane table
-    g.padB = g.direct ? cround_up(V * W + 32, 16) : 32;
-    if (g.direct) g.PMS = 0;
-    g.RS4 = cround_up((g.N + 1) / 2, 4); g.AS4 = cround_up(g.N * g.RS4, 16);
-    return g;
-}
 
 template <int KIND_, int H_, int W_, int V_>
-struct GeoS {                                                 // compile-time geometry
+struct GeoS : GeoAccess<GeoS<KIND_, H_, W_, V_>> {          // compile-time geometry
     static constexpr GeoVals v = make_geo(KIND_, H_, W_, V_);
     __device__ __forceinline__ explicit GeoS(const KParams&) {}
-    __device__ __forceinline__ int kind() const { return v.kind; }
-    __device__ __forceinline__ int H() const { return v.H; }
-    __device__ __forceinline__ int W() const { return v.W; }
-    __device__ __forceinline__ int V() const { return v.V; }
-    __device__ __forceinline__ int G() const { return v.G; }
-    __device__ __forceinline__ int GS() const { return v.GS; }
-    __device__ __forceinline__ int N() const { return v.N; }
-    __device__ __forceinline__ int RP() const { return v.RP; }
-    __device__ __forceinline__ int PS() const { return v.PS; }
-    __device__ __forceinline__ int AS() const { return v.AS; }
-    __device__ __forceinline__ int RS4() const { return v.RS4; }
-    __device__ __forceinline__ int AS4() const { return v.AS4; }
-    __device__ __forceinline__ int LPn() const { return v.LPn; }
-    __device__ __forceinline__ int nw8M() const { return v.nw8M; }
-    __device__ __forceinline__ int nw8T() const { return v.nw8T; }
-    __device__ __forceinline__ int pitchM() const { return v.pitchM; }
-    __device__ __forceinline__ int pitchT() const { return v.pitchT; }
-    __device__ __forceinline__ int PMS() const { return v.PMS; }
-    __device__ __forceinline__ bool direct() const { return v.direct != 0; }
-    __device__ __forceinline__ int padF() const { return v.padF; }
-    __device__ __forceinline__ int padB() const { return v.padB; }
-    __device__ __forceinline__ uint32_t maskM8() const { return v.maskM8; }
-    __device__ __forceinline__ int off_map(int o) const { return o == 0 ? v.off0 : (o == 1 ? v.off1 : (o == 2 ? v.off2 : v.off3)); }
+    __device__ __forceinline__ static constexpr GeoVals vals() { return v; }
+    __device__ __forceinline__ int off_map(int o) const {
+        constexpr int o0 = v.off_map[0], o1 = v.off_map[1], o2 = v.off_map[2], o3 = v.off_map[3];
+        return o == 0 ? o0 : (o == 1 ? o1 : (o == 2 ? o2 : o3));
+    }
     __device__ __forceinline__ int divW(int x) const { return (int)((unsigned)x / (unsigned)v.W); }
     __device__ __forceinline__ int divN(int x) const { return (int)((unsigned)x / (unsigned)v.N); }
     __device__ __forceinline__ int divMW(int x) const { return (int)((unsigned)x / (unsigned)v.nw8M); }
 };
 
-struct GeoD {                                                 // runtime geometry (any wall-enclosed map)
+struct GeoD : GeoAccess<GeoD> {                               // runtime geometry (any wall-enclosed map)
     const KParams& p;
     __device__ __forceinline__ explicit GeoD(const KParams& p_) : p(p_) {}
-    __device__ __forceinline__ int kind() const { return p.kind; }
-    __device__ __forceinline__ int H() const { return p.H; }
-    __device__ __forceinline__ int W() const { return p.W; }
-    __device__ __forceinline__ int V() const { return p.V; }
-    __device__ __forceinline__ int G() const { return p.G; }
-    __device__ __forceinline__ int GS() const { return p.GS; }
-    __device__ __forceinline__ int N() const { return p.N; }
-    __device__ __forceinline__ int RP() const { return p.RP; }
-    __device__ __forceinline__ int PS() const { return p.PS; }
-    __device__ __forceinline__ int AS() const { return p.AS; }
-    __device__ __forceinline__ int RS4() const { return p.RS4; }
-    __device__ __forceinline__ int AS4() const { return p.AS4; }
-    __device__ __forceinline__ int LPn() const { return p.LPn; }
-    __device__ __forceinline__ int nw8M() const { return p.nw8M; }
-    __device__ __forceinline__ int nw8T() const { return p.nw8T; }
-    __device__ __forceinline__ int pitchM() const { return p.pitchM; }
-    __device__ __forceinline__ int pitchT() const { return p.pitchT; }
-    __device__ __forceinline__ int PMS() const { return p.PMS; }
-    __device__ __forceinline__ bool direct() const { return p.direct != 0; }
-    __device__ __forceinline__ int padF() const { return p.padF; }
-    __device__ __forceinline__ int padB() const { return p.padB; }
-    __device__ __forceinline__ uint32_t maskM8() const { return p.maskM8; }
-    __device__ __forceinline__ int off_map(int o) const { return p.off_map[o]; }
+    __device__ __forceinline__ const GeoVals& vals() const { return p.geo; }
+    __device__ __forceinline__ int off_map(int o) const { return p.geo.off_map[o]; }
     __device__ __forceinline__ int divW(int x) const { return (int)(((uint32_t)x * p.invW20) >> 20); }
     __device__ __forceinline__ int divN(int x) const { return (int)(((uint32_t)x * p.invN20) >> 20); }
     __device__ __forceinline__ int divMW(int x) const { return (int)(((uint32_t)x * p.invMW20) >> 20); }
@@ -204,32 +185,22 @@ __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_
 __device__ __forceinline__ uint32_t pick(const uint4& v, int i) {
     return i == 0 ? v.x : (i == 1 ? v.y : (i == 2 ? v.z : v.w));
 }
-// A sub-warp of LPE lanes owns one env instance.  The shipped configuration is LPE = 32 (one env per warp).  LPE = 16 (two
-// envs per warp, so that the agent-lane phases issue one instruction for two envs; -DSSD_ENABLE_LPE16) passes the parity
-// suite but measured 7-20 % slower on every workload: the lane-parallel render phases take twice the trips per warp.
-// Every collective is restricted to the sub-warp's member mask, so the halves of a warp may diverge freely.
-template <int LPE>
-struct SubWarp {
-    static constexpr int kLanes = LPE, kEnvs = 32 / LPE;
-    int lane, sub, base;                                     // lane within the sub-warp, sub-warp index, first warp lane
-    unsigned mask;
-    __device__ __forceinline__ explicit SubWarp(int warp_lane)
-        : lane(warp_lane % LPE), sub(warp_lane / LPE), base(warp_lane / LPE * LPE),
-          mask(LPE == 32 ? 0xffffffffu : (0xffffu << (warp_lane / LPE * LPE))) {}
-    __device__ __forceinline__ unsigned ballot(bool pred) const { return __ballot_sync(mask, pred) >> base; }
-    template <typename T> __device__ __forceinline__ T shfl(T v, int src) const { return __shfl_sync(mask, v, base + src); }
-    template <typename T> __device__ __forceinline__ unsigned match(T v) const { return __match_any_sync(mask, v) >> base; }
-    template <typename T> __device__ __forceinline__ T rmin(T v) const { return __reduce_min_sync(mask, v); }
-    template <typename T> __device__ __forceinline__ T rmax(T v) const { return __reduce_max_sync(mask, v); }
-    template <typename T> __device__ __forceinline__ T radd(T v) const { return __reduce_add_sync(mask, v); }
-    __device__ __forceinline__ unsigned ror(unsigned v) const { return __reduce_or_sync(mask, v); }
-    __device__ __forceinline__ void sync() const { __syncwarp(mask); }
+// The lanes of the warp that owns an env instance, and the full-warp collectives the device functions use.
+struct Warp {
+    int lane;
+    __device__ __forceinline__ explicit Warp(int lane_) : lane(lane_) {}
+    __device__ __forceinline__ unsigned ballot(bool pred) const { return __ballot_sync(0xffffffffu, pred); }
+    template <typename T> __device__ __forceinline__ T shfl(T v, int src) const { return __shfl_sync(0xffffffffu, v, src); }
+    template <typename T> __device__ __forceinline__ T rmin(T v) const { return __reduce_min_sync(0xffffffffu, v); }
+    template <typename T> __device__ __forceinline__ T rmax(T v) const { return __reduce_max_sync(0xffffffffu, v); }
+    template <typename T> __device__ __forceinline__ T radd(T v) const { return __reduce_add_sync(0xffffffffu, v); }
+    __device__ __forceinline__ unsigned ror(unsigned v) const { return __reduce_or_sync(0xffffffffu, v); }
+    __device__ __forceinline__ void sync() const { __syncwarp(); }
 };
 
 // lanes j < n whose value equals this lane's: what __match_any_sync returns for the agent lanes, from n pipelined shuffles
 // (MATCH.ANY costs 3-4 % of a Cleanup step per use, profiles/r2_notes.md)
-template <class SW>
-__device__ __forceinline__ unsigned equal_lanes(const SW& w, int v, int n) {
+__device__ __forceinline__ unsigned equal_lanes(const Warp& w, int v, int n) {
     unsigned m = 0;
     for (int j = 0; j < n; ++j) m |= (unsigned)(w.shfl(v, j) == v) << j;
     return m;
@@ -237,8 +208,7 @@ __device__ __forceinline__ unsigned equal_lanes(const SW& w, int v, int n) {
 // Cheap sufficient test for "the values of the lanes in `who` are pairwise distinct": two 32-bucket bit filters, OR-reduced over
 // the warp (REDUX.OR); if either filter shows one bit per participating lane there is no duplicate.  False alarms (hash
 // collisions) only send the caller to the exact shuffle loop.
-template <class SW>
-__device__ __forceinline__ bool surely_distinct(const SW& w, int v, bool in, unsigned who) {
+__device__ __forceinline__ bool surely_distinct(const Warp& w, int v, bool in, unsigned who) {
     const int cnt = __popc(who);
     const unsigned f0 = w.ror(in ? 1u << (v & 31) : 0u);
     if (__popc(f0) == cnt) return true;
@@ -246,12 +216,12 @@ __device__ __forceinline__ bool surely_distinct(const SW& w, int v, bool in, uns
     return __popc(f1) == cnt;
 }
 
-// sub-warp-strided loop with the first trip peeled (trip counts here are almost always 0 or 1)
-template <int STRIDE, typename F>
+// warp-strided loop with the first trip peeled (trip counts here are almost always 0 or 1)
+template <typename F>
 __device__ __forceinline__ void warp_for(int n, int lane, F f) {
     int i = lane;
     if (i < n) f(i);
-    for (i += STRIDE; i < n; i += STRIDE) f(i);
+    for (i += 32; i < n; i += 32) f(i);
 }
 // draw streams: 0 mover priority, 1 apple, 2 waste (u, order key), 3 spawn key, 4 spawn rotation
 __device__ __forceinline__ uint32_t philox_word(const KParams& p, uint32_t gid, uint32_t tick, uint32_t stream, uint32_t idx) {
@@ -268,8 +238,8 @@ __device__ __forceinline__ int agent_colour_index(int i) {
 // ------------------------------------------------------------------ update_moves (map_env.py:477-661)
 // lanes < n hold one agent each: pos (cell index), ori, act.  Non-agent lanes carry unique
 // negative positions so they never match a cell.
-template <class SW, class GEO>
-__device__ __forceinline__ void update_moves(const SW& w, const GEO& g, const KParams& p, const uint8_t* __restrict__ sg, int lane, bool is_agent,
+template <class GEO>
+__device__ __forceinline__ void update_moves(const Warp& w, const GEO& g, const KParams& p, const uint8_t* __restrict__ sg, int lane, bool is_agent,
                                              int act, int& pos, int& ori, int env, uint32_t gid, uint32_t tick) {
     // turns take effect immediately (map_env.py:509-511, 843-861)
     if (act == 5) ori = (0x0132 >> (4 * ori)) & 3;           // CW : LEFT->UP, RIGHT->DOWN, UP->RIGHT, DOWN->LEFT
@@ -385,8 +355,8 @@ constexpr uint8_t kOcc = 0x80;
 
 // ------------------------------------------------------------------ beams (map_env.py:663-769)
 // TAG: every agent a FIRE ray hits (the one hit_penalty charges) sets `tagged`; it stays on the map until all beams are done.
-template <bool TAG, class SW, class GEO>
-__device__ __forceinline__ void beams(const SW& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent,
+template <bool TAG, class GEO>
+__device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent,
                                       int act, int pos, int ori, int& reward, int& clean_num, int& waste, bool& tagged) {
     const bool fire = is_agent && act == 7;
     const bool clean = is_agent && act == 8 && g.kind() == SSD_KIND_CLEANUP;
@@ -440,8 +410,8 @@ __device__ __forceinline__ void beams(const SW& w, const GEO& g, const KParams& 
 // ------------------------------------------------------------------ spawning (cleanup.py:165-204, harvest.py:92-122)
 // `apples` / `waste` are the env's running cell counts (ssd_state.counts): the reference recounts the map every step
 // (map_env.py:291-292, cleanup.py:206-212); here consume / clean / spawn keep them up to date, which is the same number.
-template <class SW, class GEO>
-__device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, int env, uint32_t gid, uint32_t tick,
+template <class GEO>
+__device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, int env, uint32_t gid, uint32_t tick,
                                       int& apples, int& waste) {
     const MapDev* __restrict__ m = p.map;
     uint32_t tA = 1, tW = 0;
@@ -457,7 +427,7 @@ __device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& 
     int n_new = 0;
     if (tA != 0) {
         int it = 0;
-        for (int j = lane; j < p.n_apple4; j += SW::kLanes, ++it) {
+        for (int j = lane; j < p.n_apple4; j += 32, ++it) {
             const ushort4 pts = __ldg(reinterpret_cast<const ushort4*>(m->apple_pts) + j);
             const uint16_t c4[4] = { pts.x, pts.y, pts.z, pts.w };
             uint4 r = make_uint4(0, 0, 0, 0);
@@ -491,7 +461,7 @@ __device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& 
     int wcell = -1;
     if (tW != 0) {
         uint32_t bk = 0xffffffffu, bc = 0xffffffffu;
-        for (int j = lane; j < p.n_waste2; j += SW::kLanes) {
+        for (int j = lane; j < p.n_waste2; j += 32) {
             const ushort2 pts = __ldg(reinterpret_cast<const ushort2*>(m->waste_pts) + j);
             uint4 r = make_uint4(0, 0, 0, 0);
             if (!p.d_uwaste) r = philox4x32_10(gid, tick, 2u, (uint32_t)j, p.seed_lo, p.seed_hi);
@@ -513,7 +483,7 @@ __device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& 
     w.sync();                                             // every decision read the pre-spawn grid
     if (g.kind() == SSD_KIND_HARVEST && decided) {
         int it = 0;
-        for (int j = lane; j < p.n_apple4; j += SW::kLanes, ++it) {
+        for (int j = lane; j < p.n_apple4; j += 32, ++it) {
             const ushort4 pts = __ldg(reinterpret_cast<const ushort4*>(m->apple_pts) + j);
             const uint16_t c4[4] = { pts.x, pts.y, pts.z, pts.w };
 #pragma unroll
@@ -530,8 +500,8 @@ __device__ __forceinline__ void spawn(const SW& w, const GEO& g, const KParams& 
 // ------------------------------------------------------------------ agent placement (map_env.py:771-793)
 // The agents in `who` take, in index order, the free spawn point with the largest (key, cell); lanes are spawn points.  At reset
 // every point is free; a respawn after tagging-out (RESPAWN) also skips the points in-play agents stand on (occupancy bits).
-template <bool RESPAWN, class SW, class GEO>
-__device__ __forceinline__ void place_agents(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, int lane, int env,
+template <bool RESPAWN, class GEO>
+__device__ __forceinline__ void place_agents(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, int lane, int env,
                                              uint32_t gid, uint32_t tick, unsigned who, int& pos) {
     const bool is_sp = lane < p.n_spawn;
     const int mycell = is_sp ? (int)__ldg(&p.map->spawn_pts[lane]) : -1;
@@ -558,18 +528,15 @@ __device__ __forceinline__ int spawn_orientation(const KParams& p, int env, uint
 }
 
 // ------------------------------------------------------------------ render (map_env.py:360-379, 418-446, 795-815, 923-957)
-#ifndef SSD_ST_HINT
-#define SSD_ST_HINT ""                                        // cache operator of the observation stores (see profiles/r1_notes.md)
-#endif
 __device__ __forceinline__ void st_row32(uint8_t* dst, const uint32_t* w) {     // one full 32-byte sector per lane
-    asm volatile("st.global" SSD_ST_HINT ".v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
+    asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                  :: "l"(dst), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7]) : "memory");
 }
 __device__ __forceinline__ void st_row16(uint8_t* dst, const uint32_t* w) {
-    asm volatile("st.global" SSD_ST_HINT ".v4.b32 [%0], {%1,%2,%3,%4};" :: "l"(dst), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
+    asm volatile("st.global.v4.b32 [%0], {%1,%2,%3,%4};" :: "l"(dst), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
 }
 __device__ __forceinline__ void st_row8(uint8_t* dst, uint32_t w0, uint32_t w1) {
-    asm volatile("st.global" SSD_ST_HINT ".v2.b32 [%0], {%1,%2};" :: "l"(dst), "r"(w0), "r"(w1) : "memory");
+    asm volatile("st.global.v2.b32 [%0], {%1,%2};" :: "l"(dst), "r"(w0), "r"(w1) : "memory");
 }
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {   // raw PRMT: no selector masking
     uint32_t d;
@@ -607,10 +574,10 @@ struct RowUnit {                                              // one (agent, y) 
     bool valid;
 };
 
-template <int OCT_T, bool IDX, class SW, class GEO>
-__device__ __forceinline__ void fetch_row(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane, int it, int units,
+template <int OCT_T, bool IDX, class GEO>
+__device__ __forceinline__ void fetch_row(const Warp& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane, int it, int units,
                                           uint32_t abase_sh, int astep, unsigned outm, RowUnit<OCT_T>& U) {
-    const int u = it * SW::kLanes + lane;
+    const int u = it * 32 + lane;
     U.valid = u < units;
     const int al = U.valid ? g.divN(u) : 0;
     U.keep = ((outm >> al) & 1u) ? 0u : 0xffffffffu;
@@ -691,12 +658,12 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
     }
 }
 
-template <int OCT_T, bool IDX, class SW, class GEO>
-__device__ __forceinline__ void gather_rows(const SW& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane,
+template <int OCT_T, bool IDX, class GEO>
+__device__ __forceinline__ void gather_rows(const Warp& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane,
                                             uint32_t abase_sh, int astep, unsigned outm) {
     const int WR = g.RP() >> 2;
     const uint32_t lastmask = IDX ? 0xffffffffu >> (4 * (8 * ((WR + 1) >> 1) - g.N())) : 0xffffffffu >> (8 * (4 * WR - g.N()));
-    const int units = p.n * g.N(), iters = (units + SW::kLanes - 1) / SW::kLanes;
+    const int units = p.n * g.N(), iters = (units + 31) / 32;
     RowUnit<OCT_T> cur, nxt;
     fetch_row<OCT_T, IDX>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, outm, cur);
     for (int it = 0; it < iters; ++it) {                      // software pipeline: row it+1 is fetched while row it is emitted
@@ -708,12 +675,12 @@ __device__ __forceinline__ void gather_rows(const SW& w, const GEO& g, const KPa
 
 // Nibble-packed padded maps, built one aligned 32-bit word (8 cells) at a time.  Map cells start at nibble
 // LPn (V rounded up to 8) of a padded row, so only the last word of a row needs its tail set to "outside".
-template <class SW, class GEO>
-__device__ __forceinline__ void build_rowmap(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* map, int lane) {
+template <class GEO>
+__device__ __forceinline__ void build_rowmap(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* map, int lane) {
     const uint32_t* sgw = reinterpret_cast<const uint32_t*>(sg);
     const int total = g.H() * g.nw8M();
 #pragma unroll 4
-    for (int i = lane; i < total; i += SW::kLanes) {
+    for (int i = lane; i < total; i += 32) {
         const int r = g.divMW(i), j = i - r * g.nw8M();
         const int sb = r * g.W() + 8 * j, wi = sb >> 2;       // first source byte of this word (grid row r, col 8j)
         const uint32_t sel = 0x3210u + 0x1111u * (sb & 3);
@@ -729,10 +696,10 @@ __device__ __forceinline__ void build_rowmap(const SW& w, const GEO& g, const KP
 // Transposed map from M: one lane transposes one 8 x 8 block of nibbles (8 words in, 8 words out) with three butterfly
 // stages (swap 1-, 2-, 4-nibble sub-blocks across the diagonal).  Rows below the map come from M's first padding row and
 // columns right of the map from M's tail nibbles, both "outside", which is exactly what MT's own padding holds.
-template <class SW, class GEO>
-__device__ __forceinline__ void build_colmap(const SW& w, const GEO& g, const KParams& p, const uint8_t* M, uint8_t* MT, int lane) {
+template <class GEO>
+__device__ __forceinline__ void build_colmap(const Warp& w, const GEO& g, const KParams& p, const uint8_t* M, uint8_t* MT, int lane) {
     const int total = g.nw8T() * g.nw8M();
-    for (int blk = lane; blk < total; blk += SW::kLanes) {
+    for (int blk = lane; blk < total; blk += 32) {
         const int i = g.divMW(blk), j = blk - i * g.nw8M();   // rows 8i.., columns 8j..
         uint32_t a[8];
 #pragma unroll
@@ -768,13 +735,13 @@ __device__ __forceinline__ void build_colmap(const SW& w, const GEO& g, const KP
 }
 
 // "outside the map" everywhere (utility_funcs.py:58-116 without np.pad); issued while the state loads are in flight
-template <class SW, class GEO>
-__device__ __forceinline__ void fill_outside(const SW& w, const GEO& g, const KParams& p, uint8_t* pmap, int lane) {
+template <class GEO>
+__device__ __forceinline__ void fill_outside(const Warp& w, const GEO& g, const KParams& p, uint8_t* pmap, int lane) {
     const uint4 v6 = make_uint4(0x66666666u, 0x66666666u, 0x66666666u, 0x66666666u);
     uint4* q = reinterpret_cast<uint4*>(pmap);
     const int n16 = g.PMS() >> 4;
 #pragma unroll 8
-    for (int i = lane; i < n16; i += SW::kLanes) q[i] = v6;           // trip count is a compile-time constant for the shipped maps
+    for (int i = lane; i < n16; i += 32) q[i] = v6;           // trip count is a compile-time constant for the shipped maps
 }
 
 // Direct gather for small views (N <= 16, i.e. every Cleanup configuration): a lane owns one (agent, y) output row and
@@ -783,12 +750,12 @@ __device__ __forceinline__ void fill_outside(const SW& w, const GEO& g, const KP
 // index 6, reverses the run for DOWN / RIGHT, and colours 4 pixels per PRMT as the map path does.  No padded maps are built.
 // The grid tile has V rows of slack on both sides (zeroed at kernel start), so no load needs a bounds test; agents were
 // written into the staged grid as index 7 by the caller.
-template <bool COLS, bool IDX, class SW, class GEO>
-__device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, const uint8_t* rank2lane,
+template <bool COLS, bool IDX, class GEO>
+__device__ __forceinline__ void gather_class(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, const uint8_t* rank2lane,
                                              uint8_t* gobs, int lane, uint32_t apack, int n_in_class, unsigned outm) {
     const int N = g.N(), V = g.V(), W = g.W(), units = n_in_class * N, WR = g.RP() >> 2;
     const uint32_t lastmask = 0xffffffffu >> (8 * (4 * WR - N));
-    for (int u0 = 0; u0 < units; u0 += SW::kLanes) {
+    for (int u0 = 0; u0 < units; u0 += 32) {
         const int u = u0 + lane;
         const bool valid = u < units;
         const int rank = valid ? g.divN(u) : 0;
@@ -868,8 +835,8 @@ __device__ __forceinline__ void gather_class(const SW& w, const GEO& g, const KP
 // The rows of UP / DOWN agents and of LEFT / RIGHT agents are gathered in two separate passes, so that a trip of the warp runs
 // ONE of the two load schemes instead of both under divergence.  `tbl` (32 bytes at the very start of the tile's front slack,
 // never touched by a gather load) maps (class, rank within class) -> agent lane.
-template <bool IDX, class SW, class GEO>
-__device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* tbl, uint8_t* gobs, int lane,
+template <bool IDX, class GEO>
+__device__ __forceinline__ void gather_direct(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* tbl, uint8_t* gobs, int lane,
                                               bool is_agent, int r0, int c0, int ori, unsigned outm) {
     const uint32_t apack = (uint32_t)r0 | ((uint32_t)c0 << 8) | ((uint32_t)ori << 16);
     const unsigned m_rows = w.ballot(is_agent && ori >= 2), m_cols = w.ballot(is_agent && ori < 2);
@@ -884,8 +851,8 @@ __device__ __forceinline__ void gather_direct(const SW& w, const GEO& g, const K
 
 // live: the lane's agent is on the map; outm: agents out of play (tagged out), whose views are written as zeros.  Their rows go
 // through the same gather at cell (0, 0), masked, so that a warp trip never mixes two kinds of row.
-template <bool IDX, class SW, class GEO>
-__device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
+template <bool IDX, class GEO>
+__device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
                                        int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm) {
     const bool top = live && lane == 31 - __clz(same);       // later index overwrites (map_env.py:370); same = lanes on this lane's cell
     int r0 = 0, c0 = 0;
@@ -893,7 +860,7 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
 
     if (p.state_rgb) {                                        // get_state: unrotated full map (map_env.py:950-957)
         uint8_t* out = p.state_rgb + (size_t)env * 3 * g.G();
-        for (int c = lane; c < g.G(); c += SW::kLanes) {
+        for (int c = lane; c < g.G(); c += 32) {
             const uint32_t rgb = lut_s[sg[c]];
             out[c] = (uint8_t)rgb; out[g.G() + c] = (uint8_t)(rgb >> 8); out[2 * g.G() + c] = (uint8_t)(rgb >> 16);
         }
@@ -935,20 +902,20 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
     }
     if constexpr (IDX) {                                          // pad bytes per agent block (8 for N = 15)
         const int body = g.N() * g.RS4(), tail = g.AS4() - body;
-        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
+        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += 32)
             *reinterpret_cast<uint32_t*>(gobs + (i / (tail >> 2)) * g.AS4() + body + 4 * (i % (tail >> 2))) = 0u;
     } else {
         const int tail = g.AS() - 3 * g.PS();                     // pad bytes per agent block (0 for the shipped views)
-        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += SW::kLanes)
+        if (tail) for (int i = lane; i < p.n * (tail >> 2); i += 32)
             *reinterpret_cast<uint32_t*>(gobs + (i / (tail >> 2)) * g.AS() + 3 * g.PS() + 4 * (i % (tail >> 2))) = 0u;
     }
     if (!IDX && !p.agents_uniform) {
         // full-colour scheme: every visible agent is re-painted with its own colour (after the row stores)
         w.sync();
         const uint32_t apack = (uint32_t)r0 | ((uint32_t)c0 << 10) | ((uint32_t)ori << 20);
-        const int pairs = p.n * p.n, iters = (pairs + SW::kLanes - 1) / SW::kLanes;
+        const int pairs = p.n * p.n, iters = (pairs + 31) / 32;
         for (int it = 0; it < iters; ++it) {
-            const int q = it * SW::kLanes + lane;
+            const int q = it * 32 + lane;
             const bool valid = q < pairs;
             const int al = valid ? q / p.n : 0, j = valid ? q - al * p.n : 0;
             const uint32_t api = w.shfl(apack, al), apj = w.shfl(apack, j);
@@ -970,26 +937,26 @@ __device__ __forceinline__ void render(const SW& w, const GEO& g, const KParams&
 // ------------------------------------------------------------------ the kernel
 // TAG: tagging-out timers are on (p.tag_timeout > 0; MODE_STEP and MODE_RENDER only, DESIGN.md §3 item 11).
 // IDX: observations are written as packed colour indices (SSD_OBS_INDEX4, DESIGN.md §3 item 12) instead of RGB planes.
-template <int MODE, class GEO, int LPE, bool TAG, bool IDX>
-__global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const __grid_constant__ KParams p) {
-    using SW = SubWarp<LPE>;
+template <int MODE, class GEO, bool TAG, bool IDX>
+__global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __grid_constant__ KParams p) {
     const GEO g(p);
     extern __shared__ __align__(16) uint8_t smem[];
-    __shared__ uint32_t lut_all[kWarps * 2][16];              // colour LUT, one private copy per (sub-)warp: no CTA barrier anywhere
+    __shared__ ColourLuts lut_all;                            // colour LUT, one private copy per warp: no CTA barrier anywhere
     const int warp = threadIdx.x >> 5;
-    const SW w(threadIdx.x & 31);
-    const int lane = w.lane;                                  // lane within the sub-warp that owns an env
-    uint32_t* lut_s = lut_all[warp * SW::kEnvs + w.sub];
+    const Warp w(threadIdx.x & 31);
+    const int lane = w.lane;
+    uint32_t* lut_s = lut_all[warp];
     // per-env tile: [front slack][grid GS][back slack][nibble maps (map path only)]
-    uint8_t* tile = smem + ((size_t)warp * SW::kEnvs + w.sub) * (g.padF() + g.GS() + g.padB() + g.PMS());
+    uint8_t* tile = smem + (size_t)warp * (g.padF() + g.GS() + g.padB() + g.PMS());
     uint8_t* sg = tile + g.padF();
     uint8_t* pmap = sg + g.GS() + g.padB();
     const bool is_agent = lane < p.n;
     // One env instance per warp and per launch.  (A persistent loop over env instances was measured and dropped: warps that
     // start together stay phase-locked -- everybody resolves moves, then everybody stores observations -- which turns a
     // 65536-env launch into 14 back-to-back single-wave steps: Harvest 204 us instead of 167 us.  Letting the block scheduler
-    // start a fresh CTA whenever one retires decorrelates the phases; profiles/r2_notes.md.)
-    const int env = p.env0 + (blockIdx.x * kWarps + warp) * SW::kEnvs + w.sub;
+    // start a fresh CTA whenever one retires decorrelates the phases; profiles/r2_notes.md.)  Two envs per warp (16 lanes each)
+    // was measured slower on every workload but the largest Cleanup launch (profiles/r1_notes.md, profiles/r2_notes.md §2).
+    const int env = p.env0 + blockIdx.x * kWarps + warp;
     if (env >= p.env1) return;
     // Prologue that touches nothing an earlier launch writes (colour LUT, slack / "outside" fill of the staging tile).  Under
     // programmatic dependent launch (small launches, p.pdl) it runs first, while the previous launch of the stream is still
@@ -998,8 +965,8 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
         if (lane < 16) lut_s[lane] = p.lut[lane];             // (made visible by w.sync below)
         if (p.obs) {
             if (g.direct()) {                                 // zero the slack around the grid (read, then masked, by the gather)
-                for (int i = lane; i < (g.padF() >> 4); i += SW::kLanes) reinterpret_cast<uint4*>(tile)[i] = make_uint4(0, 0, 0, 0);
-                for (int i = lane; i < (g.padB() >> 4); i += SW::kLanes) reinterpret_cast<uint4*>(sg + g.GS())[i] = make_uint4(0, 0, 0, 0);
+                for (int i = lane; i < (g.padF() >> 4); i += 32) reinterpret_cast<uint4*>(tile)[i] = make_uint4(0, 0, 0, 0);
+                for (int i = lane; i < (g.padB() >> 4); i += 32) reinterpret_cast<uint4*>(sg + g.GS())[i] = make_uint4(0, 0, 0, 0);
             } else fill_outside(w, g, p, pmap, lane);         // "outside the map"
         }
     };
@@ -1031,7 +998,7 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
             if (lane < n16) g0 = __ldcg(src + lane);
             if (!p.pdl) prologue();                           // while the state loads are in flight
             if (lane < n16) reinterpret_cast<uint4*>(sg)[lane] = g0;
-            for (int i = lane + SW::kLanes; i < n16; i += SW::kLanes) reinterpret_cast<uint4*>(sg)[i] = __ldcg(src + i);
+            for (int i = lane + 32; i < n16; i += 32) reinterpret_cast<uint4*>(sg)[i] = __ldcg(src + i);
         }
         // Tagging-out (TAG): an agent whose timer (bits 24..31 of its record) is non-zero is out of play for the whole step.  Its
         // lane then acts like a lane without an agent (unique negative pos, no action), and `home` keeps the cell of its record.
@@ -1122,7 +1089,7 @@ __global__ void __launch_bounds__(kWarps * 32, SSD_MIN_BLOCKS) ssd_kernel(const 
             if (live && lane == __ffs(same) - 1) sg[pos] &= 0x7f;
             w.sync();
             uint4* dst = reinterpret_cast<uint4*>(p.grid + (size_t)env * g.GS());
-            warp_for<SW::kLanes>(g.GS() >> 4, lane, [&](int i) { dst[i] = reinterpret_cast<const uint4*>(sg)[i]; });
+            warp_for(g.GS() >> 4, lane, [&](int i) { dst[i] = reinterpret_cast<const uint4*>(sg)[i]; });
             if (is_agent) {                                        // an agent out of play keeps the cell it left the map from
                 const int cell = (TAG && !live) ? home : pos;
                 const int r = g.divW(cell);
@@ -1217,6 +1184,13 @@ uint32_t magic20(int d, int max_x) {
     return m;
 }
 
+// Observation strides of one format (ssd_get_obs_layout; ssd_step_host copies B * env_stride bytes).
+ssd_obs_layout obs_layout(const KParams& k, int32_t format) {
+    const GeoVals& g = k.geo;
+    if (format == SSD_OBS_INDEX4) return { format, g.RS4, 0, g.AS4, k.n * g.AS4 };
+    return { format, g.RP, g.PS, g.AS, k.n * g.AS };
+}
+
 }  // namespace
 
 struct ssd_handle {
@@ -1227,7 +1201,6 @@ struct ssd_handle {
     mutable int64_t launches;                                 // also counts ssd_expand_obs, which takes a const handle
     int force_generic;                                        // SSD_B200_GENERIC=1: always use the runtime-geometry kernels
     int pdl;                                                  // programmatic dependent launch for small launches (SSD_B200_PDL=0 turns it off)
-    int lanes_per_env;                                        // 16: two envs per warp (needs <= 16 spawn points); 32: one
     int obs_format;                                           // SSD_OBS_RGB (at creation) or SSD_OBS_INDEX4
 };
 
@@ -1244,8 +1217,8 @@ static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws
     return SSD_OK;
 }
 
-template <int MODE, class GEO, int LPE, bool TAG, bool IDX>
-static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
+template <int MODE, class GEO, bool TAG, bool IDX>
+static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
     {   // cudaFuncAttributeMaxDynamicSharedMemorySize belongs to the kernel FUNCTION (per device), not to a handle: all
@@ -1256,12 +1229,11 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         const int dev = h->device;
         if (dev < 0 || dev >= kMaxDevices) return SSD_ERR_INVALID;
         if ((int)h->smem_bytes > high_water[dev]) {
-            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, LPE, TAG, IDX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, TAG, IDX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
             high_water[dev] = (int)h->smem_bytes;
         }
     }
-    const int envs_per_cta = kWarps * (32 / LPE);
-    int grid = (k.env1 - k.env0 + envs_per_cta - 1) / envs_per_cta;
+    const int grid = (k.env1 - k.env0 + kWarps - 1) / kWarps;
     if (grid <= 0) return SSD_OK;
 
     if (k.pdl) {                                               // programmatic dependent launch (see launch_geo)
@@ -1272,9 +1244,9 @@ static int launch_lpe(ssd_handle* h, const KParams& k, void* stream) {
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, LPE, TAG, IDX>, k));
+        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, TAG, IDX>, k));
     } else {
-        ssd_kernel<MODE, GEO, LPE, TAG, IDX><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
+        ssd_kernel<MODE, GEO, TAG, IDX><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
     }
     ++h->launches;
     SSD_CUDA(cudaGetLastError());
@@ -1292,25 +1264,23 @@ static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
     k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
     const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
-    if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation, one env per warp
+    if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation
         if (k.tag_timeout != 0)
-            return idx ? launch_lpe<MODE, GEO, 32, true, true>(h, k, stream) : launch_lpe<MODE, GEO, 32, true, false>(h, k, stream);
+            return idx ? launch_kernel<MODE, GEO, true, true>(h, k, stream) : launch_kernel<MODE, GEO, true, false>(h, k, stream);
     }
-#ifdef SSD_ENABLE_LPE16                                        // experiment: two envs per warp (measured slower, profiles/r1_notes.md)
-    if (h->lanes_per_env == 16 && !idx) return launch_lpe<MODE, GEO, 16, false, false>(h, k, stream);
-#endif
-    return idx ? launch_lpe<MODE, GEO, 32, false, true>(h, k, stream) : launch_lpe<MODE, GEO, 32, false, false>(h, k, stream);
+    return idx ? launch_kernel<MODE, GEO, false, true>(h, k, stream) : launch_kernel<MODE, GEO, false, false>(h, k, stream);
 }
 
 // The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
 template <int MODE>
 static int launch(ssd_handle* h, const KParams& k, void* stream) {
+    const GeoVals& v = k.geo;
     if (!h->force_generic) {
-        if (k.kind == SSD_KIND_HARVEST && k.H == 9 && k.W == 38 && k.V == 15) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 15>>(h, k, stream);
-        if (k.kind == SSD_KIND_HARVEST && k.H == 9 && k.W == 38 && k.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 7>>(h, k, stream);
-        if (k.kind == SSD_KIND_CLEANUP && k.H == 25 && k.W == 18 && k.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 25, 18, 7>>(h, k, stream);
-        if (k.kind == SSD_KIND_CLEANUP && k.H == 48 && k.W == 18 && k.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 48, 18, 7>>(h, k, stream);
-        if (k.kind == SSD_KIND_CLEANUP && k.H == 10 && k.W == 10 && k.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 10, 10, 7>>(h, k, stream);
+        if (v.kind == SSD_KIND_HARVEST && v.H == 9 && v.W == 38 && v.V == 15) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 15>>(h, k, stream);
+        if (v.kind == SSD_KIND_HARVEST && v.H == 9 && v.W == 38 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 7>>(h, k, stream);
+        if (v.kind == SSD_KIND_CLEANUP && v.H == 25 && v.W == 18 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 25, 18, 7>>(h, k, stream);
+        if (v.kind == SSD_KIND_CLEANUP && v.H == 48 && v.W == 18 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 48, 18, 7>>(h, k, stream);
+        if (v.kind == SSD_KIND_CLEANUP && v.H == 10 && v.W == 10 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 10, 10, 7>>(h, k, stream);
     }
     return launch_geo<MODE, GeoD>(h, k, stream);
 }
@@ -1386,15 +1356,9 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     if (!h) { delete hm; return SSD_ERR_INVALID; }
     memset(h, 0, sizeof(*h));
     KParams& k = h->kp;
-    const GeoVals gv = make_geo(cfg->kind, H, W, V);
-    k.kind = cfg->kind; k.B = cfg->n_envs; k.n = n; k.H = H; k.W = W; k.G = G; k.V = V; k.N = gv.N;
-    k.GS = gv.GS; k.NA = round_up(n, 4);
-    k.RP = gv.RP; k.PS = gv.PS; k.AS = gv.AS; k.ES = n * k.AS;
-    k.RS4 = gv.RS4; k.AS4 = gv.AS4;
-    k.LPn = gv.LPn; k.nw8M = gv.nw8M; k.nw8T = gv.nw8T; k.maskM8 = gv.maskM8; k.maskT8 = gv.maskT8;
-    k.pitchM = gv.pitchM; k.pitchT = gv.pitchT; k.PMS = gv.PMS;
-    k.direct = gv.direct; k.padF = gv.padF; k.padB = gv.padB;
-    k.off_map[0] = gv.off0; k.off_map[1] = gv.off1; k.off_map[2] = gv.off2; k.off_map[3] = gv.off3;
+    k.geo = make_geo(cfg->kind, H, W, V);
+    const GeoVals& gv = k.geo;
+    k.B = cfg->n_envs; k.n = n; k.NA = round_up(n, 4);
     k.episode_limit = cfg->episode_limit; k.fire_cost = cfg->fire_cost; k.hit_penalty = cfg->hit_penalty;
     k.tag_timeout = cfg->tag_timeout;
     k.beam_len = cfg->beam_len; k.n_actions = cfg->kind == SSD_KIND_CLEANUP ? 9 : 8;
@@ -1402,7 +1366,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     k.base_apples = 0; k.base_waste = 0;
     for (int c = 0; c < G; ++c) { k.base_apples += hm->base_grid[c] == SSD_CELL_APPLE; k.base_waste += hm->base_grid[c] == SSD_CELL_WASTE; }
     k.random_spawn = cfg->random_spawn_point != 0; k.spawn_rot = cfg->spawn_rotation < 0 ? -1 : cfg->spawn_rotation;
-    k.invN20 = magic20(k.N, SSD_MAX_AGENTS * k.N + 64); k.invW20 = magic20(W, G + 1);
+    k.invN20 = magic20(gv.N, SSD_MAX_AGENTS * gv.N + 64); k.invW20 = magic20(W, G + 1);
     k.seed_lo = (uint32_t)cfg->seed; k.seed_hi = (uint32_t)(cfg->seed >> 32); k.gid_base = cfg->env_gid_base;
     for (int i = 0; i < 4; ++i) k.thr_harvest[i] = cfg->thr_harvest[i];
     for (int i = 0; i < 16; ++i)
@@ -1416,27 +1380,19 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     }
     if (k.invN20 == 0 || k.invW20 == 0 || k.n_apple4 > 32 * 16) { delete hm; delete h; return SSD_ERR_INVALID; }
 
-    k.invMW20 = magic20(k.nw8M, H * k.nw8M + 32); k.invMTW20 = magic20(k.nw8T, W * k.nw8T + 32);
-    if (k.invMW20 == 0 || k.invMTW20 == 0 || k.PMS >= 60000) { delete hm; delete h; return SSD_ERR_INVALID; }
-    k.off_pmap = k.padF + k.GS + k.padB;
-    k.smem_per_warp = k.off_pmap + k.PMS;
-    // two envs per warp need the spawn points (reset) and the per-lane apple decision bits (64) to fit 16 lanes
-    h->lanes_per_env = 32;
-#ifdef SSD_ENABLE_LPE16
-    if (ns <= 16 && k.n_apple4 <= 16 * 16 && k.tag_timeout == 0) h->lanes_per_env = 16;
-    { const char* e = getenv("SSD_B200_LPE"); if (e && atoi(e) == 32) h->lanes_per_env = 32; }
-#endif
-    h->smem_bytes = (size_t)kWarps * (32 / h->lanes_per_env) * k.smem_per_warp;
+    k.invMW20 = magic20(gv.nw8M, H * gv.nw8M + 32);
+    if (k.invMW20 == 0 || gv.PMS >= 60000) { delete hm; delete h; return SSD_ERR_INVALID; }
+    h->smem_bytes = (size_t)kWarps * (gv.padF + gv.GS + gv.padB + gv.PMS);     // one staging tile per warp
     { const char* e = getenv("SSD_B200_GENERIC"); h->force_generic = e && e[0] == '1'; }
     { const char* e = getenv("SSD_B200_PDL"); h->pdl = !(e && e[0] == '0'); }
     h->device = cfg->device;
 
     DeviceGuard guard(cfg->device);
     cudaError_t e = guard.err;
-    if (e == cudaSuccess) {                                   // the launch needs smem_bytes dynamic + the static LUT
+    if (e == cudaSuccess) {                                   // the launch needs smem_bytes dynamic + the static LUTs
         int optin = 0;
         e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
-        if (e == cudaSuccess && h->smem_bytes + 256 > (size_t)optin) { delete hm; delete h; return SSD_ERR_INVALID; }
+        if (e == cudaSuccess && h->smem_bytes + sizeof(ColourLuts) > (size_t)optin) { delete hm; delete h; return SSD_ERR_INVALID; }
     }
     if (e == cudaSuccess) e = cudaMalloc(&h->d_map, sizeof(MapDev));
     if (e == cudaSuccess) e = cudaMemcpy(h->d_map, hm, sizeof(MapDev), cudaMemcpyHostToDevice);
@@ -1462,18 +1418,16 @@ int ssd_destroy(ssd_handle* h) {
 int ssd_get_layout(const ssd_handle* h, ssd_layout* o) {
     if (!h || !o) return SSD_ERR_INVALID;
     const KParams& k = h->kp;
-    o->n_actions = k.n_actions; o->n_cells = k.G; o->obs_n = k.N; o->grid_stride = k.GS; o->agent_stride = k.NA;
-    o->obs_plane_stride = k.PS; o->obs_agent_stride = k.AS; o->obs_env_stride = k.ES;
-    o->n_apple_pts = k.n_apple; o->n_waste_pts = k.n_waste; o->n_spawn_pts = k.n_spawn; o->obs_row_stride = k.RP;
+    const GeoVals& g = k.geo;
+    o->n_actions = k.n_actions; o->n_cells = g.G; o->obs_n = g.N; o->grid_stride = g.GS; o->agent_stride = k.NA;
+    o->obs_plane_stride = g.PS; o->obs_agent_stride = g.AS; o->obs_env_stride = obs_layout(k, SSD_OBS_RGB).env_stride;
+    o->n_apple_pts = k.n_apple; o->n_waste_pts = k.n_waste; o->n_spawn_pts = k.n_spawn; o->obs_row_stride = g.RP;
     return SSD_OK;
 }
 
 int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* o) {
     if (!h || !o || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
-    const KParams& k = h->kp;
-    o->format = format;
-    if (format == SSD_OBS_RGB) { o->row_stride = k.RP; o->plane_stride = k.PS; o->agent_stride = k.AS; o->env_stride = k.ES; }
-    else { o->row_stride = k.RS4; o->plane_stride = 0; o->agent_stride = k.AS4; o->env_stride = k.n * k.AS4; }
+    *o = obs_layout(h->kp, format);
     return SSD_OK;
 }
 
@@ -1493,13 +1447,7 @@ int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd
 
 int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
              const ssd_step_out* out, void* stream) {
-    KParams k;
-    const int rc = fill_common(h, st, draws, k);
-    if (rc) return rc;
-    if (!actions || !out || !out->reward || !out->clean || !out->apple_cnt || !out->done) return SSD_ERR_INVALID;
-    k.actions = actions; k.reward = out->reward; k.clean = out->clean; k.apple_cnt = out->apple_cnt; k.done = out->done;
-    k.obs = out->obs; k.state_rgb = out->state_rgb;
-    return launch<MODE_STEP>(h, k, stream);
+    return ssd_step_range(h, st, actions, draws, out, 0, h ? h->kp.B : 0, stream);
 }
 
 int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
@@ -1539,10 +1487,10 @@ int ssd_step_host(ssd_handle* h, const ssd_state* st, const uint8_t* h_actions, 
     if (h_out->clean) SSD_CUDA(cudaMemcpyAsync(h_out->clean, d_out->clean, B * k.n, cudaMemcpyDeviceToHost, s));
     if (h_out->apple_cnt) SSD_CUDA(cudaMemcpyAsync(h_out->apple_cnt, d_out->apple_cnt, B * 2, cudaMemcpyDeviceToHost, s));
     if (h_out->done) SSD_CUDA(cudaMemcpyAsync(h_out->done, d_out->done, B, cudaMemcpyDeviceToHost, s));
-    const size_t ES = h->obs_format == SSD_OBS_INDEX4 ? (size_t)k.n * k.AS4 : (size_t)k.ES;
+    const size_t ES = (size_t)obs_layout(k, h->obs_format).env_stride;
     if (h_out->obs && d_out->obs) SSD_CUDA(cudaMemcpyAsync(h_out->obs, d_out->obs, B * ES, cudaMemcpyDeviceToHost, s));
     if (h_out->state_rgb && d_out->state_rgb)
-        SSD_CUDA(cudaMemcpyAsync(h_out->state_rgb, d_out->state_rgb, B * 3 * k.G, cudaMemcpyDeviceToHost, s));
+        SSD_CUDA(cudaMemcpyAsync(h_out->state_rgb, d_out->state_rgb, B * 3 * k.geo.G, cudaMemcpyDeviceToHost, s));
     SSD_CUDA(cudaStreamSynchronize(s));
     return SSD_OK;
 }
@@ -1573,9 +1521,9 @@ int ssd_expand_obs(const ssd_handle* h, const uint8_t* obs_index4, int32_t env_b
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
     ExpandParams e;
-    e.in = obs_index4 + (size_t)env_begin * k.n * k.AS4;
+    e.in = obs_index4 + (size_t)env_begin * k.n * k.geo.AS4;
     e.out = out;
-    e.N = k.N; e.RS4 = k.RS4; e.AS4 = k.AS4;
+    e.N = k.geo.N; e.RS4 = k.geo.RS4; e.AS4 = k.geo.AS4;
     for (int i = 0; i < 16; ++i) e.lut[i] = k.lut[i];
     expand_obs_kernel<<<(unsigned)(env_count * k.n), 256, 0, (cudaStream_t)stream>>>(e);
     ++h->launches;

@@ -18,6 +18,7 @@ SSD_OBS_RGB, SSD_OBS_INDEX4 = 0, 1
 # every symbol include/ssd_b200.h declares (checked by tests/test_capi_symbols.py against the header text)
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
+           "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_render",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
@@ -44,6 +45,10 @@ class SsdLayout(C.Structure):
 
 class SsdObsLayout(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("format", "row_stride", "plane_stride", "agent_stride", "env_stride")]
+
+
+class SsdStateLayout(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("format", "row_stride", "plane_stride", "env_stride")]
 
 
 class SsdState(C.Structure):
@@ -88,6 +93,9 @@ def load():
     L.ssd_get_obs_layout.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdObsLayout)]
     L.ssd_set_obs_format.argtypes = [C.c_void_p, C.c_int32]
     L.ssd_expand_obs.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    L.ssd_get_state_layout.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdStateLayout)]
+    L.ssd_set_state_format.argtypes = [C.c_void_p, C.c_int32]
+    L.ssd_expand_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

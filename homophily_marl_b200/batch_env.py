@@ -41,11 +41,13 @@ class SSDBatchEnv:
                  fire_cost=1, hit_penalty=0, want_state=False, check_actions=False):
         # tag_timeout: steps an agent hit by a FIRE ray is out of play (off the map, action ignored, zero view); 0 = never
         # obs_format: "rgb" (u8 RGB planes, the reference's get_obs * 256) or "index4" (packed 4-bit colour indices)
+        # state_format: the same choice for the state image (get_state * 256), independent of obs_format
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
-                     disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb")
+                     disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb")
         extra.update(extra_args or {})
-        if extra["obs_format"] not in OBS_FORMATS:
-            raise ValueError(f"obs_format must be one of {sorted(OBS_FORMATS)}, got {extra['obs_format']!r}")
+        for key in ("obs_format", "state_format"):
+            if extra[key] not in OBS_FORMATS:
+                raise ValueError(f"{key} must be one of {sorted(OBS_FORMATS)}, got {extra[key]!r}")
         self.extra_args = extra
         self.name = name
         self.spec = mapspec.compile_map(name, map, num_agents, view_size, episode_limit,
@@ -91,6 +93,9 @@ class SSDBatchEnv:
         self.obs_format, self.obs_layout = "rgb", self.get_obs_layout("rgb")
         if extra["obs_format"] != "rgb":
             self._set_format(extra["obs_format"])
+        self.state_format, self.state_layout = "rgb", self.get_state_layout("rgb")
+        if extra["state_format"] != "rgb":
+            self._set_state_format(extra["state_format"])
 
         dev, B, n = self.device, self.B, self.n
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
@@ -105,7 +110,8 @@ class SSDBatchEnv:
         self.apple_cnt = z((B,), torch.int16)
         self.done = z((B,), torch.uint8)
         self.obs_buf = self.new_obs_buffer()
-        self.state_rgb = z((B, 3, self.H, self.W), torch.uint8) if want_state else None
+        self.want_state = bool(want_state)
+        self._alloc_state()
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
                                                             self.t_buf, self.tick_buf, self.counts_buf)])
         self._keep = None
@@ -129,6 +135,67 @@ class SSDBatchEnv:
         self._set_format(fmt)
         self.extra_args["obs_format"] = fmt
         self.obs_buf = self.new_obs_buffer()
+
+    # ------------------------------------------------------------------ state image format
+    def get_state_layout(self, fmt):
+        """``ssd_state_layout`` (format, row_stride, plane_stride, env_stride) of "rgb" or "index4"."""
+        lay = _capi.SsdStateLayout()
+        _capi.check(self.lib.ssd_get_state_layout(self._h, OBS_FORMATS[fmt], C.byref(lay)))
+        return lay
+
+    def _set_state_format(self, fmt):
+        _capi.check(self.lib.ssd_set_state_format(self._h, OBS_FORMATS[fmt]))
+        self.state_format, self.state_layout = fmt, self.get_state_layout(fmt)
+
+    def _alloc_state(self):
+        """``state_buf``: the state image buffer of the current format, u8 [B, 3, H, W] for RGB (also ``state_rgb``) or
+        [B, env_stride] for index4 (``state_rgb`` is then None); both None without ``want_state``."""
+        self.state_buf = self.state_rgb = None
+        if self.want_state:
+            shape = (self.B, 3, self.H, self.W) if self.state_format == "rgb" else (self.B, self.state_layout.env_stride)
+            self.state_buf = torch.zeros(shape, dtype=torch.uint8, device=self.device)
+            if self.state_format == "rgb":
+                self.state_rgb = self.state_buf
+
+    def set_state_format(self, fmt):
+        """Switches the format every later step / render writes the state image in, and reallocates ``state_buf``.
+        Host-side: a CUDA graph captured before keeps the format it was captured with."""
+        if fmt not in OBS_FORMATS:
+            raise ValueError(f"state_format must be one of {sorted(OBS_FORMATS)}, got {fmt!r}")
+        self._set_state_format(fmt)
+        self.extra_args["state_format"] = fmt
+        self._alloc_state()
+
+    def _state_index4(self, what):
+        if self.state_format != "index4" or self.state_buf is None:
+            raise ValueError(f"{what} needs state_format 'index4' and want_state=True")
+
+    def state_packed(self, buf=None):
+        """[B, H, row_stride] u8 view (no copy) of an index4 state buffer: cell c of a row is byte c >> 1, low nibble when c
+        is even."""
+        self._state_index4("state_packed()")
+        buf = self.state_buf if buf is None else buf
+        lay = self.state_layout
+        return buf.as_strided((self.B, self.H, lay.row_stride), (lay.env_stride, lay.row_stride, 1))
+
+    def state_index(self, buf=None):
+        """[B, H, W] u8 colour indices (unpacked copy): ``spec.lut[state_index()]`` is the RGB state image."""
+        p = self.state_packed(buf)
+        return torch.stack((p & 15, p >> 4), dim=-1).reshape(self.B, self.H, -1)[..., :self.W]
+
+    def state_float(self, env_begin=0, env_count=None, out=None):
+        """f32 [env_count, 3, H, W] of envs [env_begin, env_begin + env_count) of the index4 state buffer, through one
+        ``ssd_expand_state`` launch on the current stream: bit-identical to ``state_rgb.float() / 256`` of an RGB env."""
+        self._state_index4("state_float()")
+        env_count = self.B - env_begin if env_count is None else int(env_count)
+        shape = (env_count, 3, self.H, self.W)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        elif out.dtype != torch.float32 or not out.is_cuda or not out.is_contiguous() or tuple(out.shape) != shape:
+            raise ValueError(f"out must be a contiguous float32 CUDA tensor of shape {shape}")
+        _capi.check(self.lib.ssd_expand_state(self._h, _ptr(self.state_buf), int(env_begin), env_count, _ptr(out),
+                                              self._stream()))
+        return out
 
     # ------------------------------------------------------------------ buffers / views
     def new_obs_buffer(self):
@@ -290,7 +357,7 @@ class SSDBatchEnv:
         return _capi.SsdStepOut(self.reward.data_ptr(), self.clean.data_ptr(), self.apple_cnt.data_ptr(),
                                 self.done.data_ptr(),
                                 (self.obs_buf if obs_out is None else obs_out).data_ptr() if want_obs else None,
-                                self.state_rgb.data_ptr() if (want_state and self.state_rgb is not None) else None)
+                                self.state_buf.data_ptr() if (want_state and self.state_buf is not None) else None)
 
     def step(self, actions, draws=None, obs_out=None, want_obs=True, want_state=False, auto_reset=False):
         """actions: u8 CUDA tensor [B, n].  Results land in self.reward / clean / apple_cnt / done / obs.
@@ -307,7 +374,7 @@ class SSDBatchEnv:
         if auto_reset:
             out = None if not want_obs else (self.obs_buf if obs_out is None else obs_out)
             _capi.check(self.lib.ssd_reset(self._h, C.byref(self._st), _ptr(self.done), None, _ptr(out), self._stream()))
-            if want_state and self.state_rgb is not None:
+            if want_state and self.state_buf is not None:
                 self.render(want_obs=False, want_state=True)
 
     def step_range(self, actions, env_begin, env_count, draws=None, obs_out=None, want_obs=True, want_state=False):
@@ -322,7 +389,7 @@ class SSDBatchEnv:
 
     def render(self, obs_out=None, want_obs=True, want_state=False):
         o = (self.obs_buf if obs_out is None else obs_out) if want_obs else None
-        s = self.state_rgb if want_state else None
+        s = self.state_buf if want_state else None
         _capi.check(self.lib.ssd_render(self._h, C.byref(self._st), _ptr(o), _ptr(s), self._stream()))
 
     def make_host_io(self, with_obs=True, with_state=False):
@@ -331,7 +398,7 @@ class SSDBatchEnv:
         io = dict(actions=torch.zeros((self.B, self.n), dtype=torch.uint8).pin_memory(),
                   reward=pin(self.reward), clean=pin(self.clean), apple_cnt=pin(self.apple_cnt), done=pin(self.done),
                   obs=pin(self.obs_buf) if with_obs else None,
-                  state=pin(self.state_rgb) if (with_state and self.state_rgb is not None) else None,
+                  state=pin(self.state_buf) if (with_state and self.state_buf is not None) else None,
                   agent=pin(self.agent_buf))
         io["d_actions"] = torch.zeros((self.B, self.n), dtype=torch.uint8, device=self.device)
         return io
@@ -339,6 +406,8 @@ class SSDBatchEnv:
     def step_host(self, io):
         """H2D actions -> step -> D2H reward/clean/apple_cnt/done(/obs/state) -> stream sync, all inside the C call."""
         want_state = io.get("state") is not None
+        if want_state and self.state_buf is not None and io["state"].numel() != self.B * self.state_layout.env_stride:
+            raise ValueError("io['state'] does not match the current state format: call make_host_io again after set_state_format")
         d_out = self._step_out(None, io["obs"] is not None, want_state)
         h_out = _capi.SsdStepOut(io["reward"].data_ptr(), io["clean"].data_ptr(), io["apple_cnt"].data_ptr(),
                                  io["done"].data_ptr(), io["obs"].data_ptr() if io["obs"] is not None else None,
@@ -352,7 +421,7 @@ class SSDBatchEnv:
             io["obs"].copy_(self.obs_buf, non_blocking=True)
         if state and io.get("state") is not None:
             self.render(want_obs=False, want_state=True)
-            io["state"].copy_(self.state_rgb, non_blocking=True)
+            io["state"].copy_(self.state_buf, non_blocking=True)
         if agent:
             io["agent"].copy_(self.agent_buf, non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()

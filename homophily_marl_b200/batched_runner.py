@@ -110,12 +110,16 @@ class BatchedEpisodeRunner:
     # ---- device-side views of what the reference env returns per step -------------------------------------
     def _pre_transition(self, sl=slice(None)):
         e = self.env                                          # obs AND state image were written by the last step / reset launch
+        lo, hi, _ = sl.indices(e.B)
         if e.obs_format == "rgb":
             obs = e.obs_view()[sl].float() / 256
         else:                                                 # index4: expanded on the current (the range's) stream
-            lo, hi, _ = sl.indices(e.B)
             obs = e.obs_float(lo, hi - lo)
-        return {"state": e.state_rgb[sl].float() / 256, "avail_actions": self._avail[sl],
+        if e.state_format == "rgb":
+            state = e.state_rgb[sl].float() / 256
+        else:                                                 # index4 state image: expanded the same way
+            state = e.state_float(lo, hi - lo)
+        return {"state": state, "avail_actions": self._avail[sl],
                 "obs": obs, "agent_pos": e.agent_pos[sl].float(),
                 "agent_orientation": self._orient_vec[e.agent_orient[sl].long()]}
 

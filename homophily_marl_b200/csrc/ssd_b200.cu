@@ -113,6 +113,7 @@ struct KParams {
     const uint32_t* d_prio; const uint32_t* d_uapple; const uint32_t* d_uwaste; const uint32_t* d_wkey;
     const uint32_t* d_spawnkey; const uint8_t* d_rot;
     int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
+    int state_idx4;                           // state_rgb holds packed colour indices (SSD_OBS_INDEX4; DESIGN.md §3 item 13)
 };
 
 // The geometry accessors, over D::vals(): compile-time constants (GeoS) or the launch's KParams::geo (GeoD).  Only the
@@ -855,22 +856,51 @@ template <bool IDX, class GEO>
 __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
                                        int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm) {
     const bool top = live && lane == 31 - __clz(same);       // later index overwrites (map_env.py:370); same = lanes on this lane's cell
-    int r0 = 0, c0 = 0;
-    if (live) { r0 = g.divW(pos); c0 = pos - r0 * g.W(); }
-
-    if (p.state_rgb) {                                        // get_state: unrotated full map (map_env.py:950-957)
-        uint8_t* out = p.state_rgb + (size_t)env * 3 * g.G();
-        for (int c = lane; c < g.G(); c += 32) {
-            const uint32_t rgb = lut_s[sg[c]];
-            out[c] = (uint8_t)rgb; out[g.G() + c] = (uint8_t)(rgb >> 8); out[2 * g.G() + c] = (uint8_t)(rgb >> 16);
-        }
-        w.sync();                                         // orders the agent overlay after the cell colours
-        if (top) {
-            const uint32_t rgb = lut_s[agent_colour_index(lane)];
-            out[pos] = (uint8_t)rgb; out[g.G() + pos] = (uint8_t)(rgb >> 8); out[2 * g.G() + pos] = (uint8_t)(rgb >> 16);
+    if (p.state_rgb) {
+        if (p.state_idx4) {                                   // get_state as packed colour indices (DESIGN.md §3 item 13)
+            // One lane assembles one 32-bit word, 8 cells of a row, as build_rowmap does, and stores it.  A row is nw8M
+            // words (ceil(W/2) rounded up to 4 bytes); the nibbles past W and the words past the last row are 0.
+            // RGB-observation kernels staged every agent as 7, so in the full-colour scheme the top agent's own colour index
+            // is staged for the pack and 7 restored before the observation gather.  (r0, c0 are computed after this block:
+            // live across the pack loop they cost the render kernels registers.)
+            uint8_t* sgm = const_cast<uint8_t*>(sg);
+            const bool repaint = !IDX && !p.agents_uniform;
+            if (repaint) { if (top) sgm[pos] = (uint8_t)agent_colour_index(lane); w.sync(); }
+            const int words = cround_up(g.H() * g.nw8M(), 4);
+            uint32_t* out = reinterpret_cast<uint32_t*>(p.state_rgb) + (size_t)env * words;
+            const uint32_t* sgw = reinterpret_cast<const uint32_t*>(sg);
+#pragma unroll 1                                              // 1-5 trips on the shipped maps
+            for (int i = lane; i < words; i += 32) {
+                const int r = g.divMW(i), j = i - r * g.nw8M();
+                uint32_t v = 0u;
+                if (r < g.H()) {
+                    const int sb = r * g.W() + 8 * j, wi = sb >> 2;   // first cell of this word (row r, column 8j)
+                    const uint32_t sel = 0x3210u + 0x1111u * (sb & 3);
+                    SSD_CHECK(wi >= 0 && 4 * (wi + 3) <= g.GS() + g.padB());   // the last words may read into the back slack
+                    const uint32_t a0 = sgw[wi], a1 = sgw[wi + 1], a2 = sgw[wi + 2];
+                    const uint32_t x0 = prmt(a0, a1, sel), x1 = prmt(a1, a2, sel);
+                    v = prmt(x0 | (x0 >> 4), x1 | (x1 >> 4), 0x6420);          // 8 bytes -> 8 nibbles
+                    if (j == g.nw8M() - 1) v &= g.maskM8();
+                }
+                out[i] = v;
+            }
+            if (repaint) { w.sync(); if (top) sgm[pos] = 7; w.sync(); }
+        } else {                                              // get_state: unrotated full map (map_env.py:950-957)
+            uint8_t* out = p.state_rgb + (size_t)env * 3 * g.G();
+            for (int c = lane; c < g.G(); c += 32) {
+                const uint32_t rgb = lut_s[sg[c]];
+                out[c] = (uint8_t)rgb; out[g.G() + c] = (uint8_t)(rgb >> 8); out[2 * g.G() + c] = (uint8_t)(rgb >> 16);
+            }
+            w.sync();                                         // orders the agent overlay after the cell colours
+            if (top) {
+                const uint32_t rgb = lut_s[agent_colour_index(lane)];
+                out[pos] = (uint8_t)rgb; out[g.G() + pos] = (uint8_t)(rgb >> 8); out[2 * g.G() + pos] = (uint8_t)(rgb >> 16);
+            }
         }
     }
     if (!p.obs) return;
+    int r0 = 0, c0 = 0;
+    if (live) { r0 = g.divW(pos); c0 = pos - r0 * g.W(); }
     uint8_t* gobs = p.obs + (size_t)env * (p.n * (IDX ? g.AS4() : g.AS()));
 
     if (g.direct()) {
@@ -1136,21 +1166,22 @@ __global__ void incentive_kernel(const long long* __restrict__ a_inc, const floa
     if (sgn) sgn[idx] = rv > 0.f ? 1.f : (rv < 0.f ? -1.f : 0.f);
 }
 
-// ------------------------------------------------------------------ index4 -> f32 RGB (ssd_expand_obs)
-// One CTA per agent view, one thread per pixel: f32 [3][N][N] = color_lut[nibble] / 256, exactly what u8 RGB / 256 gives.
+// ------------------------------------------------------------------ index4 -> f32 RGB (ssd_expand_obs, ssd_expand_state)
+// One CTA per block of rows x cols nibbles (an agent view, or an env's state image), one thread per pixel:
+// f32 [3][rows][cols] = color_lut[nibble] / 256, exactly what u8 RGB / 256 gives.
 struct ExpandParams {
-    const uint8_t* in;                        // first view of the range in the index4 buffer
-    float* out;                               // [views][3][N][N]
-    int N, RS4, AS4;
+    const uint8_t* in;                        // first block of the range in the index4 buffer
+    float* out;                               // [blocks][3][rows][cols]
+    int rows, cols, row_stride, block_stride; // block_stride: bytes between blocks (agent or env stride)
     uint32_t lut[16];                         // R | G << 8 | B << 16 per colour index
 };
-__global__ void __launch_bounds__(256) expand_obs_kernel(const __grid_constant__ ExpandParams p) {
-    const uint8_t* __restrict__ in = p.in + (size_t)blockIdx.x * p.AS4;
-    const int NN = p.N * p.N;
+__global__ void __launch_bounds__(256) expand_index4_kernel(const __grid_constant__ ExpandParams p) {
+    const uint8_t* __restrict__ in = p.in + (size_t)blockIdx.x * p.block_stride;
+    const int NN = p.rows * p.cols;
     float* __restrict__ out = p.out + (size_t)blockIdx.x * 3 * NN;
     for (int q = threadIdx.x; q < NN; q += blockDim.x) {
-        const int y = q / p.N, x = q - y * p.N;
-        const uint32_t rgb = p.lut[(__ldg(in + y * p.RS4 + (x >> 1)) >> (4 * (x & 1))) & 15u];
+        const int y = q / p.cols, x = q - y * p.cols;
+        const uint32_t rgb = p.lut[(__ldg(in + y * p.row_stride + (x >> 1)) >> (4 * (x & 1))) & 15u];
         out[q] = (float)(rgb & 0xffu) * (1.0f / 256.0f);
         out[NN + q] = (float)((rgb >> 8) & 0xffu) * (1.0f / 256.0f);
         out[2 * NN + q] = (float)((rgb >> 16) & 0xffu) * (1.0f / 256.0f);
@@ -1191,6 +1222,14 @@ ssd_obs_layout obs_layout(const KParams& k, int32_t format) {
     return { format, g.RP, g.PS, g.AS, k.n * g.AS };
 }
 
+// State image strides of one format (ssd_get_state_layout; ssd_step_host copies B * env_stride bytes).  An index4 row is
+// nw8M words, which is ceil(W/2) rounded up to 4 bytes.
+ssd_state_layout state_layout(const KParams& k, int32_t format) {
+    const GeoVals& g = k.geo;
+    if (format == SSD_OBS_INDEX4) return { format, 4 * g.nw8M, 0, 4 * round_up(g.H * g.nw8M, 4) };
+    return { format, g.W, g.G, 3 * g.G };
+}
+
 }  // namespace
 
 struct ssd_handle {
@@ -1198,16 +1237,18 @@ struct ssd_handle {
     MapDev* d_map;
     int device;
     size_t smem_bytes;
-    mutable int64_t launches;                                 // also counts ssd_expand_obs, which takes a const handle
+    mutable int64_t launches;                                 // also counts ssd_expand_obs / _state, which take a const handle
     int force_generic;                                        // SSD_B200_GENERIC=1: always use the runtime-geometry kernels
     int pdl;                                                  // programmatic dependent launch for small launches (SSD_B200_PDL=0 turns it off)
     int obs_format;                                           // SSD_OBS_RGB (at creation) or SSD_OBS_INDEX4
+    int state_format;                                         // the same, for the state image
 };
 
 static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws* d, KParams& k) {
     if (!h || !st || !st->grid || !st->agent || !st->ep_ret || !st->t || !st->tick || !st->counts) return SSD_ERR_INVALID;
     k = h->kp;
     k.env0 = 0; k.env1 = k.B;
+    k.state_idx4 = h->state_format == SSD_OBS_INDEX4;
     k.grid = st->grid; k.agent = st->agent; k.ep_ret = st->ep_ret; k.t = st->t; k.tick = st->tick; k.counts = st->counts;
     if (d) {
         if ((d->u_waste == nullptr) != (d->wkey == nullptr)) return SSD_ERR_INVALID;
@@ -1437,6 +1478,18 @@ int ssd_set_obs_format(ssd_handle* h, int32_t format) {
     return SSD_OK;
 }
 
+int ssd_get_state_layout(const ssd_handle* h, int32_t format, ssd_state_layout* o) {
+    if (!h || !o || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
+    *o = state_layout(h->kp, format);
+    return SSD_OK;
+}
+
+int ssd_set_state_format(ssd_handle* h, int32_t format) {
+    if (!h || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
+    h->state_format = format;
+    return SSD_OK;
+}
+
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws, uint8_t* obs, void* stream) {
     KParams k;
     const int rc = fill_common(h, st, draws, k);
@@ -1490,7 +1543,8 @@ int ssd_step_host(ssd_handle* h, const ssd_state* st, const uint8_t* h_actions, 
     const size_t ES = (size_t)obs_layout(k, h->obs_format).env_stride;
     if (h_out->obs && d_out->obs) SSD_CUDA(cudaMemcpyAsync(h_out->obs, d_out->obs, B * ES, cudaMemcpyDeviceToHost, s));
     if (h_out->state_rgb && d_out->state_rgb)
-        SSD_CUDA(cudaMemcpyAsync(h_out->state_rgb, d_out->state_rgb, B * 3 * k.geo.G, cudaMemcpyDeviceToHost, s));
+        SSD_CUDA(cudaMemcpyAsync(h_out->state_rgb, d_out->state_rgb, B * (size_t)state_layout(k, h->state_format).env_stride,
+                                 cudaMemcpyDeviceToHost, s));
     SSD_CUDA(cudaStreamSynchronize(s));
     return SSD_OK;
 }
@@ -1513,22 +1567,40 @@ int ssd_incentive(const int64_t* actions_inc, const float* reward, int64_t rows,
     return SSD_OK;
 }
 
+// One expand_index4_kernel launch over `blocks` blocks of rows x cols nibbles, `block_stride` bytes apart from `in`.
+static int launch_expand(const ssd_handle* h, const uint8_t* in, int64_t blocks, int rows, int cols, int row_stride,
+                         int block_stride, float* out, void* stream) {
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    ExpandParams e;
+    e.in = in; e.out = out;
+    e.rows = rows; e.cols = cols; e.row_stride = row_stride; e.block_stride = block_stride;
+    for (int i = 0; i < 16; ++i) e.lut[i] = h->kp.lut[i];
+    expand_index4_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(e);
+    ++h->launches;
+    SSD_CUDA(cudaGetLastError());
+    return SSD_OK;
+}
+
 int ssd_expand_obs(const ssd_handle* h, const uint8_t* obs_index4, int32_t env_begin, int32_t env_count, float* out, void* stream) {
     if (!h || !obs_index4 || !out) return SSD_ERR_INVALID;
     const KParams& k = h->kp;
     if (env_begin < 0 || env_count < 0 || (int64_t)env_begin + env_count > k.B) return SSD_ERR_INVALID;
     if (env_count == 0) return SSD_OK;
-    DeviceGuard guard(h->device);
-    SSD_CUDA(guard.err);
-    ExpandParams e;
-    e.in = obs_index4 + (size_t)env_begin * k.n * k.geo.AS4;
-    e.out = out;
-    e.N = k.geo.N; e.RS4 = k.geo.RS4; e.AS4 = k.geo.AS4;
-    for (int i = 0; i < 16; ++i) e.lut[i] = k.lut[i];
-    expand_obs_kernel<<<(unsigned)(env_count * k.n), 256, 0, (cudaStream_t)stream>>>(e);
-    ++h->launches;
-    SSD_CUDA(cudaGetLastError());
-    return SSD_OK;
+    const GeoVals& g = k.geo;
+    return launch_expand(h, obs_index4 + (size_t)env_begin * k.n * g.AS4, (int64_t)env_count * k.n, g.N, g.N, g.RS4, g.AS4,
+                         out, stream);
+}
+
+int ssd_expand_state(const ssd_handle* h, const uint8_t* state_index4, int32_t env_begin, int32_t env_count, float* out,
+                     void* stream) {
+    if (!h || !state_index4 || !out) return SSD_ERR_INVALID;
+    const KParams& k = h->kp;
+    if (env_begin < 0 || env_count < 0 || (int64_t)env_begin + env_count > k.B) return SSD_ERR_INVALID;
+    if (env_count == 0) return SSD_OK;
+    const ssd_state_layout s = state_layout(k, SSD_OBS_INDEX4);
+    return launch_expand(h, state_index4 + (size_t)env_begin * s.env_stride, env_count, k.geo.H, k.geo.W, s.row_stride,
+                         s.env_stride, out, stream);
 }
 
 int64_t ssd_launch_count(const ssd_handle* h) { return h ? h->launches : -1; }

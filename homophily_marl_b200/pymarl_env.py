@@ -88,8 +88,9 @@ class _SSDEnv(MultiAgentEnv):
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
                      disable_fire_action=True, obs_color="simplified")
         extra.update(extra_args or {})
-        # get_obs is the reference's RGB list whatever extra_args says: the facade always runs the env in the "rgb" format
-        extra["obs_format"] = "rgb"
+        # get_obs / get_state are the reference's RGB arrays whatever extra_args says: the facade always runs the env in the
+        # "rgb" formats
+        extra["obs_format"] = extra["state_format"] = "rgb"
         # `ascii_map` is accepted and IGNORED, as in the reference: CleanupEnv / HarvestEnv replace it with the map that
         # `map=` selects (cleanup.py:31-54, harvest.py:18-22).  Custom maps: SSDBatchEnv(rows=...).
         device = device or os.environ.get("SSD_B200_DEVICE", "cuda:0")

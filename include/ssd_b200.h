@@ -117,6 +117,21 @@ typedef struct ssd_obs_layout {
     int32_t env_stride;       /* bytes between envs                              */
 } ssd_obs_layout;
 
+/* State image strides of one format, in bytes (ssd_set_state_format).
+ * SSD_OBS_RGB: u8 [3][H][W] per env (get_state * 256): row_stride = W, plane_stride = H*W, env_stride = 3*H*W.
+ * SSD_OBS_INDEX4: cell (r, c) is the colour index the RGB state renderer looks up for it, so color_lut[index] is the RGB
+ *   state pixel byte for byte: 0-5 the cell code; where an agent in play stands, the colour index of the highest agent
+ *   index on the cell (7 in the simplified scheme, 6 + agent char in the full scheme).  An agent out of play (tagging-out)
+ *   is absent, as in RGB, and index 6 (outside) never occurs.  Two cells per byte: cell c of row r is byte c >> 1 of the
+ *   row, low nibble when c is even.  Every pad nibble and pad byte is 0.
+ *   row_stride = ceil(W/2) rounded up to 4, plane_stride = 0, env_stride = H * row_stride rounded up to 16. */
+typedef struct ssd_state_layout {
+    int32_t format;           /* SSD_OBS_*                                       */
+    int32_t row_stride;       /* bytes between map rows                          */
+    int32_t plane_stride;     /* bytes between colour planes (0 for index4)      */
+    int32_t env_stride;       /* bytes between envs                              */
+} ssd_state_layout;
+
 /* Persistent per-env state (MapEnv.world_map, Agent.pos/orientation, _episode_steps, rewards). */
 typedef struct ssd_state {
     uint8_t*  grid;      /* [B][grid_stride]   cell codes, padding bytes stay 0           */
@@ -139,7 +154,8 @@ typedef struct ssd_step_out {
     uint8_t*  done;       /* [B]      terminated                                        */
     uint8_t*  obs;        /* [B][env_stride] observations in the handle's format (ssd_set_obs_format): u8 RGB planes, rows
                            * padded to obs_row_stride (get_obs * 256), or packed colour indices; or NULL              */
-    uint8_t*  state_rgb;  /* [B][3][H][W] (get_state * 256) or NULL                     */
+    uint8_t*  state_rgb;  /* [B][env_stride] state image in the handle's state format (ssd_set_state_format): u8 RGB
+                           * [B][3][H][W] (get_state * 256, the default), or packed colour indices; or NULL             */
 } ssd_step_out;
 
 /* Injected, position-indexed random draws (parity harness).  NULL members fall
@@ -177,6 +193,16 @@ int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* out)
  * any CUDA call, for a NULL handle or an unknown format. */
 int ssd_set_obs_format(ssd_handle* h, int32_t format);
 
+/* Strides of state image format `format` (SSD_OBS_*), whichever format the handle is in.  SSD_ERR_INVALID for a NULL
+ * handle or an unknown format. */
+int ssd_get_state_layout(const ssd_handle* h, int32_t format, ssd_state_layout* out);
+
+/* Selects the format of every later state image (the state_rgb buffer of ssd_step, ssd_step_range, ssd_render and
+ * ssd_step_host, which then copies B * env_stride bytes), independently of the observation format.  A handle starts in
+ * SSD_OBS_RGB.  Host-side and serialised like ssd_set_obs_format; a CUDA graph keeps the format it was captured with.
+ * SSD_ERR_INVALID, before any CUDA call, for a NULL handle or an unknown format. */
+int ssd_set_state_format(ssd_handle* h, int32_t format);
+
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws,
@@ -195,7 +221,8 @@ int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const s
 int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
                    const ssd_step_out* out, int32_t env_begin, int32_t env_count, void* stream);
 
-/* get_obs / get_state without stepping (map_env.py:923-957).  Either pointer may be NULL. */
+/* get_obs / get_state without stepping (map_env.py:923-957).  Either pointer may be NULL; state_rgb is written in the
+ * handle's state format. */
 int ssd_render(ssd_handle* h, const ssd_state* st, uint8_t* obs, uint8_t* state_rgb, void* stream);
 
 /* Host-buffer variant of ssd_step: copies h_actions -> d_actions, steps, copies every non-NULL
@@ -256,7 +283,13 @@ int ssd_frontend_last_cuda_error(void);
 int ssd_expand_obs(const ssd_handle* h, const uint8_t* obs_index4, int32_t env_begin, int32_t env_count, float* out,
                    void* stream);
 
-/* Kernels launched through this handle since creation (bench.py's gpu_launches), ssd_expand_obs included. */
+/* SSD_OBS_INDEX4 state images of envs [env_begin, env_begin + env_count) -> f32 out [env_count][3][H][W] contiguous, each
+ * value color_lut[index][c] / 256: bit-identical to the RGB state image / 256.  state_index4 is the base of the
+ * whole-batch buffer, `out` holds the range only.  One kernel launch on `stream` (the kernel of ssd_expand_obs). */
+int ssd_expand_state(const ssd_handle* h, const uint8_t* state_index4, int32_t env_begin, int32_t env_count, float* out,
+                     void* stream);
+
+/* Kernels launched through this handle since creation (bench.py's gpu_launches), ssd_expand_obs / _state included. */
 int64_t ssd_launch_count(const ssd_handle* h);
 
 /* Checked build only (-DSSD_BOUNDS_CHECK, libssd_b200_check.so): number of shared-memory index violations seen so

@@ -19,7 +19,7 @@ SSD_OBS_RGB, SSD_OBS_INDEX4 = 0, 1
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state",
-           "ssd_reset", "ssd_step", "ssd_step_range", "ssd_render",
+           "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
@@ -63,6 +63,10 @@ class SsdDraws(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("prio", "u_apple", "u_waste", "wkey", "spawn_key", "rot")]
 
 
+class SsdEpisodeEnd(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("obs", "state_rgb", "ep_ret")]
+
+
 class SsdError(RuntimeError):
     def __init__(self, code, cuda_error=0, msg=""):
         self.code, self.cuda_error = code, cuda_error
@@ -100,6 +104,8 @@ def load():
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),
                                  C.c_int32, C.c_int32, C.c_void_p]
+    L.ssd_step_autoreset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),
+                                     C.POINTER(SsdEpisodeEnd), C.c_int32, C.c_int32, C.c_void_p]
     L.ssd_render.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.c_void_p, C.c_void_p]
     L.ssd_step_host.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.c_void_p,
                                 C.POINTER(SsdStepOut), C.POINTER(SsdStepOut), C.c_void_p]

@@ -38,7 +38,9 @@ def _ptr(t):
 class SSDBatchEnv:
     def __init__(self, name, n_envs, num_agents, map="default", view_size=7, episode_limit=100,
                  extra_args=None, seed=0, device="cuda:0", env_gid_base=0, rows=None, params=None,
-                 fire_cost=1, hit_penalty=0, want_state=False, check_actions=False):
+                 fire_cost=1, hit_penalty=0, want_state=False, check_actions=False, keep_episode_end=False):
+        # keep_episode_end: allocate end_obs_buf / end_state_buf / end_ep_ret_buf, which step / step_range with auto_reset fill
+        #   with what an env whose episode ended saw before its reset
         # tag_timeout: steps an agent hit by a FIRE ray is out of play (off the map, action ignored, zero view); 0 = never
         # obs_format: "rgb" (u8 RGB planes, the reference's get_obs * 256) or "index4" (packed 4-bit colour indices)
         # state_format: the same choice for the state image (get_state * 256), independent of obs_format
@@ -109,7 +111,10 @@ class SSDBatchEnv:
         self.clean = z((B, n), torch.uint8)
         self.apple_cnt = z((B,), torch.int16)
         self.done = z((B,), torch.uint8)
+        self.keep_episode_end = bool(keep_episode_end)
         self.obs_buf = self.new_obs_buffer()
+        self.end_obs_buf = self.new_obs_buffer() if self.keep_episode_end else None
+        self.end_ep_ret_buf = z((B, lay.agent_stride), torch.int32) if self.keep_episode_end else None
         self.want_state = bool(want_state)
         self._alloc_state()
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
@@ -135,6 +140,8 @@ class SSDBatchEnv:
         self._set_format(fmt)
         self.extra_args["obs_format"] = fmt
         self.obs_buf = self.new_obs_buffer()
+        if self.keep_episode_end:
+            self.end_obs_buf = self.new_obs_buffer()
 
     # ------------------------------------------------------------------ state image format
     def get_state_layout(self, fmt):
@@ -149,13 +156,16 @@ class SSDBatchEnv:
 
     def _alloc_state(self):
         """``state_buf``: the state image buffer of the current format, u8 [B, 3, H, W] for RGB (also ``state_rgb``) or
-        [B, env_stride] for index4 (``state_rgb`` is then None); both None without ``want_state``."""
-        self.state_buf = self.state_rgb = None
+        [B, env_stride] for index4 (``state_rgb`` is then None); both None without ``want_state``.  ``end_state_buf``, with
+        ``keep_episode_end``, has the same shape."""
+        self.state_buf = self.state_rgb = self.end_state_buf = None
         if self.want_state:
             shape = (self.B, 3, self.H, self.W) if self.state_format == "rgb" else (self.B, self.state_layout.env_stride)
             self.state_buf = torch.zeros(shape, dtype=torch.uint8, device=self.device)
             if self.state_format == "rgb":
                 self.state_rgb = self.state_buf
+            if self.keep_episode_end:
+                self.end_state_buf = torch.zeros(shape, dtype=torch.uint8, device=self.device)
 
     def set_state_format(self, fmt):
         """Switches the format every later step / render writes the state image in, and reallocates ``state_buf``.
@@ -183,18 +193,21 @@ class SSDBatchEnv:
         p = self.state_packed(buf)
         return torch.stack((p & 15, p >> 4), dim=-1).reshape(self.B, self.H, -1)[..., :self.W]
 
-    def state_float(self, env_begin=0, env_count=None, out=None):
-        """f32 [env_count, 3, H, W] of envs [env_begin, env_begin + env_count) of the index4 state buffer, through one
-        ``ssd_expand_state`` launch on the current stream: bit-identical to ``state_rgb.float() / 256`` of an RGB env."""
+    def state_float(self, env_begin=0, env_count=None, buf=None, out=None):
+        """f32 [env_count, 3, H, W] of envs [env_begin, env_begin + env_count) of an index4 state buffer (``state_buf`` by
+        default, or ``end_state_buf``), through one ``ssd_expand_state`` launch on the current stream: bit-identical to
+        ``state_rgb.float() / 256`` of an RGB env."""
         self._state_index4("state_float()")
+        buf = self.state_buf if buf is None else buf
         env_count = self.B - env_begin if env_count is None else int(env_count)
         shape = (env_count, 3, self.H, self.W)
         if out is None:
             out = torch.empty(shape, dtype=torch.float32, device=self.device)
         elif out.dtype != torch.float32 or not out.is_cuda or not out.is_contiguous() or tuple(out.shape) != shape:
             raise ValueError(f"out must be a contiguous float32 CUDA tensor of shape {shape}")
-        _capi.check(self.lib.ssd_expand_state(self._h, _ptr(self.state_buf), int(env_begin), env_count, _ptr(out),
-                                              self._stream()))
+        if buf.dtype != torch.uint8 or not buf.is_cuda or buf.numel() < self.B * self.state_layout.env_stride:
+            raise ValueError("buf must be a uint8 CUDA index4 state buffer of B * env_stride bytes")
+        _capi.check(self.lib.ssd_expand_state(self._h, _ptr(buf), int(env_begin), env_count, _ptr(out), self._stream()))
         return out
 
     # ------------------------------------------------------------------ buffers / views
@@ -261,6 +274,11 @@ class SSDBatchEnv:
     @property
     def ep_ret(self):
         return self.ep_ret_buf[:, :self.n]
+
+    @property
+    def end_ep_ret(self):
+        """[B, n] int32 episode returns written by an auto-reset step for the envs whose episode it ended (keep_episode_end)."""
+        return None if self.end_ep_ret_buf is None else self.end_ep_ret_buf[:, :self.n]
 
     @property
     def tag_out(self):
@@ -359,31 +377,45 @@ class SSDBatchEnv:
                                 (self.obs_buf if obs_out is None else obs_out).data_ptr() if want_obs else None,
                                 self.state_buf.data_ptr() if (want_state and self.state_buf is not None) else None)
 
+    def _episode_end(self, want_obs, want_state):
+        if not self.keep_episode_end:
+            return None
+        return _capi.SsdEpisodeEnd(self.end_obs_buf.data_ptr() if want_obs else None,
+                                   self.end_state_buf.data_ptr() if (want_state and self.end_state_buf is not None) else None,
+                                   self.end_ep_ret_buf.data_ptr())
+
     def step(self, actions, draws=None, obs_out=None, want_obs=True, want_state=False, auto_reset=False):
         """actions: u8 CUDA tensor [B, n].  Results land in self.reward / clean / apple_cnt / done / obs.
 
-        ``auto_reset=True``: every env whose ``done`` flag this step raised is reset by a masked ``ssd_reset`` launch on the same
-        stream (no host sync), and its slot of the observation buffer then holds the FIRST observation of the new episode;
-        ``done`` / ``reward`` keep the values of the finished step.  Envs may therefore run on different episode clocks
+        ``auto_reset=True`` (``ssd_step_autoreset``, one launch): every env whose ``done`` flag this step raised is reset in
+        the same launch, and its slot of the observation buffer (and of the state image) then holds the FIRST observation of
+        the new episode; ``done`` / ``reward`` keep the values of the finished step.  With ``keep_episode_end``, the finished
+        step's observation, state image and ``ep_ret`` of those envs land in ``end_obs_buf`` / ``end_state_buf`` /
+        ``end_ep_ret``; the slots of other envs are not written.  Envs may therefore run on different episode clocks
         (``load_state(t=...)``), which the reference -- one env, ``get_done()`` constantly False -- never needs."""
+        if auto_reset:
+            return self.step_range(actions, 0, self.B, draws, obs_out, want_obs, want_state, auto_reset=True)
         self._check_actions(actions)
         d = self._draws(draws)
         so = self._step_out(obs_out, want_obs, want_state)
         _capi.check(self.lib.ssd_step(self._h, C.byref(self._st), _ptr(actions), C.byref(d) if d else None,
                                       C.byref(so), self._stream()))
-        if auto_reset:
-            out = None if not want_obs else (self.obs_buf if obs_out is None else obs_out)
-            _capi.check(self.lib.ssd_reset(self._h, C.byref(self._st), _ptr(self.done), None, _ptr(out), self._stream()))
-            if want_state and self.state_buf is not None:
-                self.render(want_obs=False, want_state=True)
 
-    def step_range(self, actions, env_begin, env_count, draws=None, obs_out=None, want_obs=True, want_state=False):
-        """``step`` restricted to envs [env_begin, env_begin + env_count) (``ssd_step_range``).  ``actions`` is the
-        whole-batch [B, n] tensor; disjoint ranges may run concurrently on different CUDA streams (the launch goes to the
-        caller's current stream), which lets one group's policy / logic overlap another group's observation stores."""
+    def step_range(self, actions, env_begin, env_count, draws=None, obs_out=None, want_obs=True, want_state=False,
+                   auto_reset=False):
+        """``step`` restricted to envs [env_begin, env_begin + env_count) (``ssd_step_range``, or ``ssd_step_autoreset``
+        with ``auto_reset``).  ``actions`` is the whole-batch [B, n] tensor; disjoint ranges may run concurrently on
+        different CUDA streams (the launch goes to the caller's current stream), which lets one group's policy / logic
+        overlap another group's observation stores."""
         self._check_actions(actions)
         d = self._draws(draws)
         so = self._step_out(obs_out, want_obs, want_state)
+        if auto_reset:
+            end = self._episode_end(want_obs, want_state)
+            _capi.check(self.lib.ssd_step_autoreset(self._h, C.byref(self._st), _ptr(actions), C.byref(d) if d else None,
+                                                    C.byref(so), C.byref(end) if end else None, int(env_begin),
+                                                    int(env_count), self._stream()))
+            return
         _capi.check(self.lib.ssd_step_range(self._h, C.byref(self._st), _ptr(actions), C.byref(d) if d else None,
                                             C.byref(so), int(env_begin), int(env_count), self._stream()))
 

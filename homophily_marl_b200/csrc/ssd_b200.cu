@@ -35,7 +35,7 @@ using ColourLuts = uint32_t[kWarps][16];  // ssd_kernel's static shared memory: 
 constexpr uint16_t kNoPoint = 0xFFFF;
 constexpr int kMaxDevices = 64;
 
-enum { MODE_STEP = 0, MODE_RESET = 1, MODE_RENDER = 2 };
+enum { MODE_STEP = 0, MODE_RESET = 1, MODE_RENDER = 2, MODE_STEP_RESET = 3 };   // MODE_STEP_RESET: ssd_step_autoreset
 
 // -DSSD_BOUNDS_CHECK builds the checked variant (libssd_b200_check.so): every data-dependent shared-memory index is
 // tested against its tile and violations are counted (compute-sanitizer is closed on the GPU pool).
@@ -114,6 +114,7 @@ struct KParams {
     const uint32_t* d_spawnkey; const uint8_t* d_rot;
     int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
     int state_idx4;                           // state_rgb holds packed colour indices (SSD_OBS_INDEX4; DESIGN.md §3 item 13)
+    uint8_t* end_obs; uint8_t* end_state; int32_t* end_ep_ret;   // MODE_STEP_RESET: ssd_episode_end (DESIGN.md §3 item 14)
 };
 
 // The geometry accessors, over D::vals(): compile-time constants (GeoS) or the launch's KParams::geo (GeoD).  Only the
@@ -854,9 +855,13 @@ __device__ __forceinline__ void gather_direct(const Warp& w, const GEO& g, const
 // through the same gather at cell (0, 0), masked, so that a warp trip never mixes two kinds of row.
 template <bool IDX, class GEO>
 __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
-                                       int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm) {
+                                       int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm,
+                                       bool end) {
+    // end (MODE_STEP_RESET): into the episode-end buffers instead of the step outputs.  Each pointer is read from the launch
+    // parameters where it is used, as before: a pointer held in registers across the state block costs the fused kernels spills.
+    uint8_t* const state = end ? p.end_state : p.state_rgb;
     const bool top = live && lane == 31 - __clz(same);       // later index overwrites (map_env.py:370); same = lanes on this lane's cell
-    if (p.state_rgb) {
+    if (state) {
         if (p.state_idx4) {                                   // get_state as packed colour indices (DESIGN.md §3 item 13)
             // One lane assembles one 32-bit word, 8 cells of a row, as build_rowmap does, and stores it.  A row is nw8M
             // words (ceil(W/2) rounded up to 4 bytes); the nibbles past W and the words past the last row are 0.
@@ -867,7 +872,7 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             const bool repaint = !IDX && !p.agents_uniform;
             if (repaint) { if (top) sgm[pos] = (uint8_t)agent_colour_index(lane); w.sync(); }
             const int words = cround_up(g.H() * g.nw8M(), 4);
-            uint32_t* out = reinterpret_cast<uint32_t*>(p.state_rgb) + (size_t)env * words;
+            uint32_t* out = reinterpret_cast<uint32_t*>(state) + (size_t)env * words;
             const uint32_t* sgw = reinterpret_cast<const uint32_t*>(sg);
 #pragma unroll 1                                              // 1-5 trips on the shipped maps
             for (int i = lane; i < words; i += 32) {
@@ -886,7 +891,7 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             }
             if (repaint) { w.sync(); if (top) sgm[pos] = 7; w.sync(); }
         } else {                                              // get_state: unrotated full map (map_env.py:950-957)
-            uint8_t* out = p.state_rgb + (size_t)env * 3 * g.G();
+            uint8_t* out = state + (size_t)env * 3 * g.G();
             for (int c = lane; c < g.G(); c += 32) {
                 const uint32_t rgb = lut_s[sg[c]];
                 out[c] = (uint8_t)rgb; out[g.G() + c] = (uint8_t)(rgb >> 8); out[2 * g.G() + c] = (uint8_t)(rgb >> 16);
@@ -898,10 +903,11 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             }
         }
     }
-    if (!p.obs) return;
+    uint8_t* const obs = end ? p.end_obs : p.obs;
+    if (!obs) return;
     int r0 = 0, c0 = 0;
     if (live) { r0 = g.divW(pos); c0 = pos - r0 * g.W(); }
-    uint8_t* gobs = p.obs + (size_t)env * (p.n * (IDX ? g.AS4() : g.AS()));
+    uint8_t* gobs = obs + (size_t)env * (p.n * (IDX ? g.AS4() : g.AS()));
 
     if (g.direct()) {
         gather_direct<IDX>(w, g, p, sg, const_cast<uint8_t*>(sg) - g.padF(), gobs, lane, is_agent, r0, c0, ori, outm);
@@ -964,11 +970,64 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
     }
 }
 
+// ------------------------------------------------------------------ the kernel's stages
+// setup_agents (map_env.py:771-784) and custom_map_update (313) on the base grid staged in sg: MODE_RESET's body.  The reset
+// env's t, tick and counts are stored; its agents are all in play.
+template <class GEO>
+__device__ __forceinline__ void reset_env(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent, int env,
+                                          uint32_t gid, uint32_t tick, int& pos, int& ori, int& apples, int& waste) {
+    place_agents<false>(w, g, p, sg, lane, env, gid, tick, ~0u, pos);
+    if (is_agent) ori = spawn_orientation(p, env, gid, tick, lane);
+    if (is_agent) sg[pos] |= kOcc;                         // distinct spawn points: no two lanes share a cell
+    w.sync();
+    apples = p.base_apples; waste = p.base_waste;
+    spawn(w, g, p, sg, lane, env, gid, tick, apples, waste);
+    if (lane == 0) { p.t[env] = 0; p.tick[env] = tick + 1; p.counts[env] = (uint32_t)apples | ((uint32_t)waste << 16); }
+}
+
+// The write-back of a reset env (every agent in play on a cell of its own, no timer, ep_ret 0).  The step's write-back in
+// ssd_kernel stays written out there: calling a shared function from it moves the register allocation of the Harvest V=15
+// tagging step kernels.
+template <class GEO>
+__device__ __forceinline__ void write_back_reset(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent,
+                                                 int env, int pos, int ori) {
+    if (is_agent) sg[pos] &= 0x7f;
+    w.sync();
+    uint4* dst = reinterpret_cast<uint4*>(p.grid + (size_t)env * g.GS());
+    warp_for(g.GS() >> 4, lane, [&](int i) { dst[i] = reinterpret_cast<const uint4*>(sg)[i]; });
+    if (is_agent) {
+        const int r = g.divW(pos);
+        p.agent[(size_t)env * p.NA + lane] = (uint32_t)r | ((uint32_t)(pos - r * g.W()) << 8) | ((uint32_t)ori << 16);
+        p.ep_ret[(size_t)env * p.NA + lane] = 0;
+    }
+}
+
+// The agent overlay, then render (`end`: into the episode-end buffers).
+template <bool TAG, bool IDX, class GEO>
+__device__ __forceinline__ void draw(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s, int lane,
+                                     bool is_agent, bool live, int pos, int ori, int env, unsigned same, bool end) {
+    // agent overlay: every occupied cell shows an agent (index 7; which agent only matters for the full-colour repaint and
+    // the state image, both handled in render).  Same value from every lane on a shared cell: no race.
+    // IDX: the top agent of a cell is staged as its own colour index (7 in the simplified scheme), so no repaint follows.
+    w.sync();                                          // the write-back has read the staged grid
+    if (IDX) { if (live && lane == 31 - __clz(same)) sg[pos] = (uint8_t)(p.agents_uniform ? 7 : agent_colour_index(lane)); }
+    else if (live) sg[pos] = 7;
+    w.sync();
+    const unsigned outm = TAG ? w.ballot(is_agent && !live) : 0u;
+    render<IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm, end);
+}
+
 // ------------------------------------------------------------------ the kernel
-// TAG: tagging-out timers are on (p.tag_timeout > 0; MODE_STEP and MODE_RENDER only, DESIGN.md §3 item 11).
+// TAG: tagging-out timers are on (p.tag_timeout > 0; every mode but MODE_RESET, DESIGN.md §3 item 11).
 // IDX: observations are written as packed colour indices (SSD_OBS_INDEX4, DESIGN.md §3 item 12) instead of RGB planes.
+// MODE_STEP_RESET: MODE_STEP, then an env whose episode the step ended renders the finished step into the episode-end
+// buffers, runs MODE_RESET's body keyed by the post-step tick and renders its first observation (DESIGN.md §3 item 14).  A mode
+// of its own, not a runtime flag, so that the other instantiations keep their code.  Its two render call sites inline two copies
+// of the render: a two-pass loop around one call site spilled in the Harvest V=15 and runtime-geometry kernels
+// (profiles/r7_notes.md).
 template <int MODE, class GEO, bool TAG, bool IDX>
 __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __grid_constant__ KParams p) {
+    constexpr bool STEP = MODE == MODE_STEP || MODE == MODE_STEP_RESET;
     const GEO g(p);
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ ColourLuts lut_all;                            // colour LUT, one private copy per warp: no CTA barrier anywhere
@@ -993,7 +1052,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
     // storing observations, and the state loads follow the grid dependency; otherwise it runs under the state loads.
     auto prologue = [&]() {
         if (lane < 16) lut_s[lane] = p.lut[lane];             // (made visible by w.sync below)
-        if (p.obs) {
+        if (p.obs || (MODE == MODE_STEP_RESET && p.end_obs)) {
             if (g.direct()) {                                 // zero the slack around the grid (read, then masked, by the gather)
                 for (int i = lane; i < (g.padF() >> 4); i += 32) reinterpret_cast<uint4*>(tile)[i] = make_uint4(0, 0, 0, 0);
                 for (int i = lane; i < (g.padB() >> 4); i += 32) reinterpret_cast<uint4*>(sg + g.GS())[i] = make_uint4(0, 0, 0, 0);
@@ -1011,9 +1070,9 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
         // per step anyway, and a launch that became resident before its predecessors finished (programmatic dependent launch,
         // concurrent env ranges sharing a cache line at a range boundary) must never see a line an earlier CTA left in this SM's L1.
         const uint32_t tick = __ldcg(p.tick + env);
-        const int t_prev = MODE == MODE_STEP ? __ldcg(p.t + env) : 0;
-        const uint32_t cnt = MODE == MODE_STEP ? __ldcg(p.counts + env) : 0u;
-        int act = (MODE == MODE_STEP && is_agent) ? (int)__ldcg(p.actions + (size_t)env * p.n + lane) : 255;
+        const int t_prev = STEP ? __ldcg(p.t + env) : 0;
+        const uint32_t cnt = STEP ? __ldcg(p.counts + env) : 0u;
+        int act = (STEP && is_agent) ? (int)__ldcg(p.actions + (size_t)env * p.n + lane) : 255;
         int pos = -1 - lane, ori = 0, ep_ret = 0;
         uint32_t a_rec = 0;
         if (MODE != MODE_RESET && is_agent) {
@@ -1050,7 +1109,8 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
         // after update_moves, so it is evaluated once and shared by consume, the occupancy strip and the render
         unsigned same = 1u << lane;                            // reset: distinct spawn points
         if (MODE == MODE_RENDER) same = equal_lanes(w, pos, p.n);
-        if (MODE == MODE_STEP) {
+        bool ended = false;                                        // MODE_STEP_RESET: this step ended the episode
+        if (STEP) {
             int reward = 0, clean_num = 0;
             bool tagged = false;
             update_moves(w, g, p, sg, lane, live, act, pos, ori, env, gid, tick);                     // map_env.py:251
@@ -1101,15 +1161,10 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                 p.tick[env] = tick + 1;
                 p.counts[env] = (uint32_t)apples | ((uint32_t)waste << 16);
             }
+            if (MODE == MODE_STEP_RESET) ended = t >= p.episode_limit;
         } else if (MODE == MODE_RESET) {
-            place_agents<false>(w, g, p, sg, lane, env, gid, tick, ~0u, pos);                          // setup_agents (771-784)
-            if (is_agent) ori = spawn_orientation(p, env, gid, tick, lane);
-            if (is_agent) sg[pos] |= kOcc;                         // distinct spawn points: no two lanes share a cell
-            w.sync();
-            apples = p.base_apples; waste = p.base_waste;
-            spawn(w, g, p, sg, lane, env, gid, tick, apples, waste);                                  // custom_map_update (313)
+            reset_env(w, g, p, sg, lane, is_agent, env, gid, tick, pos, ori, apples, waste);
             ep_ret = 0;
-            if (lane == 0) { p.t[env] = 0; p.tick[env] = tick + 1; p.counts[env] = (uint32_t)apples | ((uint32_t)waste << 16); }
         }
 
         // the next launch of this stream may become resident now (its prologue overlaps this launch's stores; it still waits
@@ -1128,17 +1183,25 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                 p.ep_ret[(size_t)env * p.NA + lane] = ep_ret;
             }
         }
-        if (p.obs || p.state_rgb) {
-            // agent overlay: every occupied cell shows an agent (index 7; which agent only matters for the full-colour repaint and
-            // the state image, both handled in render).  Same value from every lane on a shared cell: no race.
-            // IDX: the top agent of a cell is staged as its own colour index (7 in the simplified scheme), so no repaint follows.
-            w.sync();                                          // the write-back above has read the staged grid
-            if (IDX) { if (live && lane == 31 - __clz(same)) sg[pos] = (uint8_t)(p.agents_uniform ? 7 : agent_colour_index(lane)); }
-            else if (live) sg[pos] = 7;
-            w.sync();
-            const unsigned outm = TAG ? w.ballot(is_agent && !live) : 0u;
-            render<IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm);
+        if constexpr (MODE == MODE_STEP_RESET) {
+            // An env whose episode ended renders the finished step into the episode-end buffers and is reset (MODE_RESET's body on
+            // the base grid staged again, the draws keyed by the post-step tick, as a masked ssd_reset after this step would key
+            // them); every env then renders into the step outputs below.
+            if (ended) {
+                if (is_agent && p.end_ep_ret) p.end_ep_ret[(size_t)env * p.NA + lane] = ep_ret;
+                if (p.end_obs || p.end_state) draw<TAG, IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, true);
+                // The base grid is staged again.  Nothing else needs restoring: a render never writes the slack or the "outside"
+                // fill of the maps, and it rebuilds every map cell it reads.
+                w.sync();                                          // the render has read the staged grid
+                const uint4* src = reinterpret_cast<const uint4*>(p.map->base_grid);
+                warp_for(g.GS() >> 4, lane, [&](int i) { reinterpret_cast<uint4*>(sg)[i] = __ldcg(src + i); });
+                w.sync();
+                reset_env(w, g, p, sg, lane, is_agent, env, gid, tick + 1, pos, ori, apples, waste);
+                write_back_reset(w, g, p, sg, lane, is_agent, env, pos, ori);
+                live = is_agent; same = 1u << lane;
+            }
         }
+        if (p.obs || p.state_rgb) draw<TAG, IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, false);
     }
 }
 
@@ -1503,9 +1566,9 @@ int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const s
     return ssd_step_range(h, st, actions, draws, out, 0, h ? h->kp.B : 0, stream);
 }
 
-int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
-                   const ssd_step_out* out, int32_t env_begin, int32_t env_count, void* stream) {
-    KParams k;
+// The arguments of a step over envs [env_begin, env_begin + env_count), validated before any CUDA call.
+static int fill_step(const ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
+                     const ssd_step_out* out, int32_t env_begin, int32_t env_count, KParams& k) {
     const int rc = fill_common(h, st, draws, k);
     if (rc) return rc;
     if (!actions || !out || !out->reward || !out->clean || !out->apple_cnt || !out->done) return SSD_ERR_INVALID;
@@ -1513,7 +1576,25 @@ int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, c
     k.env0 = env_begin; k.env1 = env_begin + env_count;
     k.actions = actions; k.reward = out->reward; k.clean = out->clean; k.apple_cnt = out->apple_cnt; k.done = out->done;
     k.obs = out->obs; k.state_rgb = out->state_rgb;
+    return SSD_OK;
+}
+
+int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
+                   const ssd_step_out* out, int32_t env_begin, int32_t env_count, void* stream) {
+    KParams k;
+    const int rc = fill_step(h, st, actions, draws, out, env_begin, env_count, k);
+    if (rc) return rc;
     return launch<MODE_STEP>(h, k, stream);
+}
+
+int ssd_step_autoreset(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
+                       const ssd_step_out* out, const ssd_episode_end* end, int32_t env_begin, int32_t env_count,
+                       void* stream) {
+    KParams k;
+    const int rc = fill_step(h, st, actions, draws, out, env_begin, env_count, k);
+    if (rc) return rc;
+    if (end) { k.end_obs = end->obs; k.end_state = end->state_rgb; k.end_ep_ret = end->ep_ret; }
+    return launch<MODE_STEP_RESET>(h, k, stream);
 }
 
 int ssd_render(ssd_handle* h, const ssd_state* st, uint8_t* obs, uint8_t* state_rgb, void* stream) {

@@ -13,7 +13,7 @@
  * pointers unless the name starts with h_ (host, pinned); `stream` is a
  * cudaStream_t passed as void*; every call returns 0 or a negative SSD_ERR_*
  * code and never throws; no internal threads; calls on one handle must be
- * serialised by the caller (except ssd_step_range on disjoint ranges).  There is no CPU fallback: without a CUDA device
+ * serialised by the caller (except ssd_step_range / ssd_step_autoreset on disjoint ranges).  There is no CPU fallback: without a CUDA device
  * ssd_create fails with SSD_ERR_CUDA.
  * Launches of at most 2048 envs are chained to the preceding kernel of `stream` by programmatic dependent launch: their
  * CTAs may become resident early, but they read nothing before all earlier work of the stream has completed, so stream
@@ -220,6 +220,26 @@ int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const s
  * batch is split, because draws are keyed by the global env id. */
 int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
                    const ssd_step_out* out, int32_t env_begin, int32_t env_count, void* stream);
+
+/* Episode-end outputs of ssd_step_autoreset: what an env whose episode ended in the step saw before its reset.  Written
+ * only for those envs; the slots of every other env are left as they are.  Every member may be NULL. */
+typedef struct ssd_episode_end {
+    uint8_t* obs;         /* [B][obs env_stride]   the finished step's observations, in the handle's observation format */
+    uint8_t* state_rgb;   /* [B][state env_stride] its state image, in the handle's state format                          */
+    int32_t* ep_ret;      /* [B][agent_stride]     the finished episode's return, this step's reward included            */
+} ssd_episode_end;
+
+/* ssd_step_range with auto-reset in the same launch (DESIGN.md §3 item 14).  In every buffer, pads included, the result is
+ * bit-identical to ssd_step_range(h, st, actions, draws, out, env_begin, env_count), then ssd_reset(h, st, mask = done,
+ * draws) of the envs of the range whose `done` the step raised, with the same `draws`, then ssd_render of their
+ * observations (out->obs) and state images (out->state_rgb).  So for a reset env: done, reward, clean and apple_cnt are
+ * those of the finished step; out->obs / out->state_rgb hold the first observation / state image of the new episode;
+ * t = 0, ep_ret = 0, every agent is in play, and tick advances by 2 (the reset draws are keyed by the post-step tick).
+ * `end` (or NULL) receives the episode-end outputs.  Validated like ssd_step_range before any CUDA call; disjoint ranges may
+ * run concurrently on different streams.  One kernel launch. */
+int ssd_step_autoreset(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
+                       const ssd_step_out* out, const ssd_episode_end* end, int32_t env_begin, int32_t env_count,
+                       void* stream);
 
 /* get_obs / get_state without stepping (map_env.py:923-957).  Either pointer may be NULL; state_rgb is written in the
  * handle's state format. */

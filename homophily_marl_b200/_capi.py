@@ -14,12 +14,14 @@ LIB_PATH = os.environ.get("SSD_B200_LIB") or os.path.join(
 
 SSD_OK, SSD_ERR_INVALID, SSD_ERR_CUDA, SSD_ERR_SPAWN, SSD_ERR_MAP = 0, -1, -2, -3, -4
 SSD_OBS_RGB, SSD_OBS_INDEX4 = 0, 1
+SSD_MAX_VARIANTS = 256
 
 # every symbol include/ssd_b200.h declares (checked by tests/test_capi_symbols.py against the header text)
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
+           "ssd_set_variants", "ssd_set_env_variants",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
@@ -35,6 +37,11 @@ class SsdConfig(C.Structure):
                 ("seed", C.c_uint64), ("env_gid_base", C.c_uint32), ("n_waste_lut", C.c_uint32),
                 ("ascii_map", C.c_char_p), ("thr_apple", C.c_void_p), ("thr_waste", C.c_void_p),
                 ("thr_harvest", C.c_uint32 * 4), ("color_lut", (C.c_uint8 * 4) * 16)]
+
+
+class SsdVariant(C.Structure):
+    _fields_ = [("ascii_map", C.c_char_p), ("n_waste_lut", C.c_uint32), ("thr_apple", C.c_void_p), ("thr_waste", C.c_void_p),
+                ("thr_harvest", C.c_uint32 * 4), ("fire_cost", C.c_int32), ("hit_penalty", C.c_int32), ("tag_timeout", C.c_int32)]
 
 
 class SsdLayout(C.Structure):
@@ -100,6 +107,8 @@ def load():
     L.ssd_get_state_layout.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdStateLayout)]
     L.ssd_set_state_format.argtypes = [C.c_void_p, C.c_int32]
     L.ssd_expand_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    L.ssd_set_variants.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdVariant)]
+    L.ssd_set_env_variants.argtypes = [C.c_void_p, C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

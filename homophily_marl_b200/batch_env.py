@@ -38,12 +38,15 @@ def _ptr(t):
 class SSDBatchEnv:
     def __init__(self, name, n_envs, num_agents, map="default", view_size=7, episode_limit=100,
                  extra_args=None, seed=0, device="cuda:0", env_gid_base=0, rows=None, params=None,
-                 fire_cost=1, hit_penalty=0, want_state=False, check_actions=False, keep_episode_end=False):
+                 fire_cost=1, hit_penalty=0, want_state=False, check_actions=False, keep_episode_end=False, variants=None,
+                 variant_of=None):
         # keep_episode_end: allocate end_obs_buf / end_state_buf / end_ep_ret_buf, which step / step_range with auto_reset fill
         #   with what an env whose episode ended saw before its reset
         # tag_timeout: steps an agent hit by a FIRE ray is out of play (off the map, action ignored, zero view); 0 = never
         # obs_format: "rgb" (u8 RGB planes, the reference's get_obs * 256) or "index4" (packed 4-bit colour indices)
         # state_format: the same choice for the state image (get_state * 256), independent of obs_format
+        # variants (also extra_args["variants"]): per-env variants of this config, a list of mapspec.compile_variant override
+        #   dicts ({} = this config); env b runs variant variant_of[b], by default (env_gid_base + b) % len(variants)
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
                      disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb")
         extra.update(extra_args or {})
@@ -98,6 +101,12 @@ class SSDBatchEnv:
         self.state_format, self.state_layout = "rgb", self.get_state_layout("rgb")
         if extra["state_format"] != "rgb":
             self._set_state_format(extra["state_format"])
+        self.variant, self.variant_specs = None, [self.spec]
+        variants = extra.get("variants") if variants is None else variants
+        if variants is not None:
+            self._set_variants(variants, variant_of)
+        elif variant_of is not None:
+            raise ValueError("variant_of needs variants")
 
         dev, B, n = self.device, self.B, self.n
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)  # noqa: E731
@@ -120,6 +129,33 @@ class SSDBatchEnv:
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
                                                             self.t_buf, self.tick_buf, self.counts_buf)])
         self._keep = None
+
+    # ------------------------------------------------------------------ per-env variants
+    def _set_variants(self, variants, variant_of):
+        """``ssd_set_variants`` with the compiled ``variants``, then ``ssd_set_env_variants`` with ``self.variant``."""
+        specs = [mapspec.compile_variant(self.spec, v) for v in variants]
+        if not 1 <= len(specs) <= _capi.SSD_MAX_VARIANTS:
+            raise ValueError(f"variants needs 1..{_capi.SSD_MAX_VARIANTS} entries, got {len(specs)}")
+        recs, keep = (_capi.SsdVariant * len(specs))(), []
+        for r, sp in zip(recs, specs):
+            a = sp.ascii_bytes()
+            ta = np.ascontiguousarray(sp.thr_apple, dtype=np.uint32)
+            tw = np.ascontiguousarray(sp.thr_waste, dtype=np.uint32)
+            keep += [a, ta, tw]
+            r.ascii_map, r.n_waste_lut, r.thr_apple, r.thr_waste = a, len(ta), ta.ctypes.data, tw.ctypes.data
+            for k in range(4):
+                r.thr_harvest[k] = int(sp.thr_harvest[k])
+            r.fire_cost, r.hit_penalty, r.tag_timeout = sp.fire_cost, sp.hit_penalty, sp.tag_timeout
+        if variant_of is None:
+            variant_of = (np.arange(self.B, dtype=np.int64) + self.env_gid_base) % len(specs)
+        ids = torch.as_tensor(np.asarray(variant_of.cpu() if torch.is_tensor(variant_of) else variant_of, dtype=np.int64))
+        if ids.shape != (self.B,) or int(ids.min()) < 0 or int(ids.max()) >= len(specs):
+            raise ValueError(f"variant_of must be [B] ids in 0..{len(specs) - 1}")
+        _capi.check(self.lib.ssd_set_variants(self._h, len(specs), recs))
+        # the kernels read this tensor in every later launch: write it (and reset the env for a new layout) to move an env
+        self.variant = ids.to(device=self.device, dtype=torch.uint8).contiguous()
+        _capi.check(self.lib.ssd_set_env_variants(self._h, _ptr(self.variant)))
+        self.variant_specs = specs
 
     # ------------------------------------------------------------------ observation format
     def get_obs_layout(self, fmt):
@@ -307,14 +343,17 @@ class SSDBatchEnv:
 
     def load_state(self, grid=None, pos_rc=None, orient=None, t=None, tag_out=None):
         """Batched variant of ``set_state``: NumPy arrays [B,H,W] / [B,n,2] / [B,n] / [B]; ``tag_out`` [B,n] sets the
-        tagging-out timers (non-zero only with ``tag_timeout`` > 0)."""
+        tagging-out timers (non-zero only on envs whose variant has ``tag_timeout`` > 0)."""
         if grid is not None:
             g = np.ascontiguousarray(grid, dtype=np.uint8).reshape(self.B, self.G)
             self.grid_buf[:, :self.G] = torch.as_tensor(g, device=self.device)
             self._recount(slice(None))
         if tag_out is not None:
             tag_out = np.asarray(tag_out, dtype=np.int64)
-            if tag_out.any() and self.spec.tag_timeout == 0:
+            tags = np.array([sp.tag_timeout for sp in self.variant_specs])
+            vid = np.zeros(self.B, dtype=np.int64) if self.variant is None else \
+                np.minimum(self.variant.cpu().numpy().astype(np.int64), len(tags) - 1)
+            if (tag_out.reshape(self.B, -1).any(1) & (tags[vid] == 0)).any():
                 raise ValueError("tag_out needs tag_timeout > 0: with tag_timeout 0 the kernels ignore the timers")
             if tag_out.min(initial=0) < 0 or tag_out.max(initial=0) > 255:
                 raise ValueError("tag_out must be in 0..255")

@@ -61,6 +61,7 @@ class BatchedEpisodeRunner:
         self._streams = [torch.cuda.Stream(device=e.device) for _ in range(self.groups)] if self.groups > 1 else []
         self._actions_u8 = torch.zeros((e.B, e.n), dtype=torch.uint8, device=e.device)
         self.front = None
+        self._vstats = {}                                     # per-variant sums since the last flush, by test_mode
 
     # ---- reference surface ------------------------------------------------------------------------------
     def setup(self, scheme, groups, preprocess, mac, batch_cls=None):
@@ -219,8 +220,20 @@ class BatchedEpisodeRunner:
         eq = np.where(coll != 0, 1 - pair / np.where(denom == 0, 1, denom), 1.0)
         env_info = {"collective_return": float(coll.sum()), "equality_metric": float(eq.sum())}
         self.last_env_info = {"collective_return": coll, "equality_metric": eq}
+        returns = episode_return.cpu().numpy()
+        if len(e.variant_specs) > 1:                          # a sweep: the pooled means alone average the variants away
+            vid = np.minimum(e.variant.cpu().numpy().astype(np.int64), len(e.variant_specs) - 1)
+            self.last_env_info["variant"] = vid
+            acc = self._vstats.setdefault(bool(test_mode), {})
+            for k in np.unique(vid):
+                m = vid == k
+                a = acc.setdefault(int(k), {"n": 0, "return": 0.0, "collective_return": 0.0, "equality_metric": 0.0})
+                a["n"] += int(m.sum())
+                a["return"] += float(returns[m].mean(axis=1).sum())
+                a["collective_return"] += float(coll[m].sum())
+                a["equality_metric"] += float(eq[m].sum())
 
-        self._account(env_info, episode_return.cpu().numpy(), test_mode)
+        self._account(env_info, returns, test_mode)
         return self.batch
 
     # ---- statistics: same keys and denominators as episode_runner.py:121-152, accumulated over B episodes at once ----
@@ -253,5 +266,8 @@ class BatchedEpisodeRunner:
         skip = {"n_episodes", "clean_num", "apple_den", "agent_pos", "agent_orientation"}
         for key in [k for k in stats if k not in skip]:
             log(prefix + key + "_mean", stats[key] / episodes, self.t_env)
+        for k, a in sorted(self._vstats.pop(prefix == "test_", {}).items()):
+            for key in ("return", "collective_return", "equality_metric"):
+                log(f"{prefix}v{k}_{key}_mean", a[key] / a["n"], self.t_env)
         rets.clear()
         stats.clear()

@@ -56,6 +56,15 @@ struct MapDev {
     uint32_t thr_waste[SSD_MAX_CELLS + 1];
 };
 
+// One env variant (ssd_set_variants): its map tables and the scalars that may differ between the variants of a handle.
+struct VarDev {
+    MapDev map;
+    int n_apple, n_waste, n_spawn, n_apple4, n_waste2;
+    int base_apples, base_waste;
+    int fire_cost, hit_penalty, tag_timeout;
+    uint32_t thr_harvest[4];
+};
+
 // ------------------------------------------------------------------ geometry
 // Everything that follows from (kind, H, W, V).  Computed by ONE constexpr function used by the host
 // (ssd_create) and, for the reference's shipped maps, at compile time by the kernels (GeoS), so that index
@@ -115,6 +124,27 @@ struct KParams {
     int tag_timeout;                          // steps a FIRE-hit agent stays off the map (0: never; DESIGN.md §3 item 11)
     int state_idx4;                           // state_rgb holds packed colour indices (SSD_OBS_INDEX4; DESIGN.md §3 item 13)
     uint8_t* end_obs; uint8_t* end_state; int32_t* end_ep_ret;   // MODE_STEP_RESET: ssd_episode_end (DESIGN.md §3 item 14)
+    const uint8_t* variant_of;                // [B] variant id per env (ssd_set_env_variants), or NULL: the fields above (variant 0)
+    const VarDev* variants;                   // the variant table (n_variants records), read only when variant_of is set
+    int n_variants;
+};
+
+// The variant an env runs (DESIGN.md §3 item 15).  VAR = false (no id array): every read is the KParams field it always was, and
+// the kernel is the code it was before variants existed.  VAR: a load from the env's record in the variant table.  Warp-uniform:
+// one warp owns one env.
+template <bool VAR>
+struct Var {
+    static constexpr bool kVar = VAR;
+    const KParams& p;
+    int id;
+    __device__ __forceinline__ const VarDev* d() const { return p.variants + id; }
+    __device__ __forceinline__ const MapDev* map() const { return VAR ? &d()->map : p.map; }
+#define SSD_VAR_FIELD(f) __device__ __forceinline__ int f() const { return VAR ? __ldg(&d()->f) : p.f; }
+    SSD_VAR_FIELD(n_apple4) SSD_VAR_FIELD(n_waste) SSD_VAR_FIELD(n_waste2) SSD_VAR_FIELD(n_spawn)
+    SSD_VAR_FIELD(base_apples) SSD_VAR_FIELD(base_waste) SSD_VAR_FIELD(fire_cost) SSD_VAR_FIELD(hit_penalty)
+    SSD_VAR_FIELD(tag_timeout)
+#undef SSD_VAR_FIELD
+    __device__ __forceinline__ uint32_t thr_harvest(int k) const { return VAR ? __ldg(&d()->thr_harvest[k]) : p.thr_harvest[k]; }
 };
 
 // The geometry accessors, over D::vals(): compile-time constants (GeoS) or the launch's KParams::geo (GeoD).  Only the
@@ -357,13 +387,14 @@ constexpr uint8_t kOcc = 0x80;
 
 // ------------------------------------------------------------------ beams (map_env.py:663-769)
 // TAG: every agent a FIRE ray hits (the one hit_penalty charges) sets `tagged`; it stays on the map until all beams are done.
-template <bool TAG, class GEO>
-__device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent,
+// In a TAG launch an env whose variant has tag_timeout 0 tags nobody, exactly like the kernel without TAG.
+template <bool TAG, class GEO, class VR>
+__device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams& p, const VR& vr, uint8_t* sg, int lane, bool is_agent,
                                       int act, int pos, int ori, int& reward, int& clean_num, int& waste, bool& tagged) {
     const bool fire = is_agent && act == 7;
     const bool clean = is_agent && act == 8 && g.kind() == SSD_KIND_CLEANUP;
-    if (fire) reward -= p.fire_cost;                          // agent.py:188-190, 239-241
-    unsigned need = w.ballot(clean || (fire && (TAG || p.hit_penalty != 0)));
+    if (fire) reward -= vr.fire_cost();                       // agent.py:188-190, 239-241
+    unsigned need = w.ballot(clean || (fire && (TAG || vr.hit_penalty() != 0)));
     while (need) {                                            // agent index order, map effects applied per agent (669-671)
         const int i = __ffs(need) - 1;
         need &= need - 1;
@@ -395,14 +426,14 @@ __device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams
         const unsigned um = w.ballot(upd >= 0);
         if (lane == i && is_clean) clean_num = __popc(um);    // 672-673
         waste -= __popc(um);                                  // only CLEAN produces updates: 'H' -> 'R'
-        if (TAG || p.hit_penalty != 0) {                      // hit(): the LAST index standing on the cell (agent.py:184-186)
+        if (TAG || vr.hit_penalty() != 0) {                   // hit(): the LAST index standing on the cell (agent.py:184-186)
 #pragma unroll
             for (int s = 0; s < 3; ++s) {
                 const int hq = w.shfl(hit, s);
                 const unsigned on = w.ballot(hq >= 0 && pos == hq);
                 if (on && lane == 31 - __clz(on)) {
-                    reward -= p.hit_penalty;
-                    if (TAG) tagged = true;
+                    reward -= vr.hit_penalty();
+                    if (TAG && (!VR::kVar || vr.tag_timeout() != 0)) tagged = true;   // without variants TAG means tag_timeout > 0
                 }
             }
         }
@@ -412,13 +443,13 @@ __device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams
 // ------------------------------------------------------------------ spawning (cleanup.py:165-204, harvest.py:92-122)
 // `apples` / `waste` are the env's running cell counts (ssd_state.counts): the reference recounts the map every step
 // (map_env.py:291-292, cleanup.py:206-212); here consume / clean / spawn keep them up to date, which is the same number.
-template <class GEO>
-__device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, int env, uint32_t gid, uint32_t tick,
-                                      int& apples, int& waste) {
-    const MapDev* __restrict__ m = p.map;
+template <class GEO, class VR>
+__device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams& p, const VR& vr, uint8_t* sg, int lane, int env,
+                                      uint32_t gid, uint32_t tick, int& apples, int& waste) {
+    const MapDev* __restrict__ m = vr.map();
     uint32_t tA = 1, tW = 0;
     if (g.kind() == SSD_KIND_CLEANUP) {
-        SSD_CHECK(waste >= 0 && waste <= p.n_waste);
+        SSD_CHECK(waste >= 0 && waste <= vr.n_waste());
         tA = __ldg(&m->thr_apple[waste]);
         tW = __ldg(&m->thr_waste[waste]);
     }
@@ -429,7 +460,7 @@ __device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams
     int n_new = 0;
     if (tA != 0) {
         int it = 0;
-        for (int j = lane; j < p.n_apple4; j += 32, ++it) {
+        for (int j = lane; j < vr.n_apple4(); j += 32, ++it) {
             const ushort4 pts = __ldg(reinterpret_cast<const ushort4*>(m->apple_pts) + j);
             const uint16_t c4[4] = { pts.x, pts.y, pts.z, pts.w };
             uint4 r = make_uint4(0, 0, 0, 0);
@@ -449,7 +480,7 @@ __device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams
                     for (int a = -1; a <= 1; ++a)
 #pragma unroll
                         for (int b = -1; b <= 1; ++b) cnt += sg[c + a * g.W() + b] == SSD_CELL_APPLE;
-                    thr = p.thr_harvest[cnt < 3 ? cnt : 3];
+                    thr = vr.thr_harvest(cnt < 3 ? cnt : 3);
                 }
                 const uint32_t u = p.d_uapple ? p.d_uapple[(size_t)env * g.G() + c] : pick(r, q);
                 if (u < thr) {
@@ -463,7 +494,7 @@ __device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams
     int wcell = -1;
     if (tW != 0) {
         uint32_t bk = 0xffffffffu, bc = 0xffffffffu;
-        for (int j = lane; j < p.n_waste2; j += 32) {
+        for (int j = lane; j < vr.n_waste2(); j += 32) {
             const ushort2 pts = __ldg(reinterpret_cast<const ushort2*>(m->waste_pts) + j);
             uint4 r = make_uint4(0, 0, 0, 0);
             if (!p.d_uwaste) r = philox4x32_10(gid, tick, 2u, (uint32_t)j, p.seed_lo, p.seed_hi);
@@ -485,7 +516,7 @@ __device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams
     w.sync();                                             // every decision read the pre-spawn grid
     if (g.kind() == SSD_KIND_HARVEST && decided) {
         int it = 0;
-        for (int j = lane; j < p.n_apple4; j += 32, ++it) {
+        for (int j = lane; j < vr.n_apple4(); j += 32, ++it) {
             const ushort4 pts = __ldg(reinterpret_cast<const ushort4*>(m->apple_pts) + j);
             const uint16_t c4[4] = { pts.x, pts.y, pts.z, pts.w };
 #pragma unroll
@@ -502,18 +533,18 @@ __device__ __forceinline__ void spawn(const Warp& w, const GEO& g, const KParams
 // ------------------------------------------------------------------ agent placement (map_env.py:771-793)
 // The agents in `who` take, in index order, the free spawn point with the largest (key, cell); lanes are spawn points.  At reset
 // every point is free; a respawn after tagging-out (RESPAWN) also skips the points in-play agents stand on (occupancy bits).
-template <bool RESPAWN, class GEO>
-__device__ __forceinline__ void place_agents(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, int lane, int env,
-                                             uint32_t gid, uint32_t tick, unsigned who, int& pos) {
-    const bool is_sp = lane < p.n_spawn;
-    const int mycell = is_sp ? (int)__ldg(&p.map->spawn_pts[lane]) : -1;
+template <bool RESPAWN, class GEO, class VR>
+__device__ __forceinline__ void place_agents(const Warp& w, const GEO& g, const KParams& p, const VR& vr, const uint8_t* sg, int lane,
+                                             int env, uint32_t gid, uint32_t tick, unsigned who, int& pos) {
+    const bool is_sp = lane < vr.n_spawn();
+    const int mycell = is_sp ? (int)__ldg(&vr.map()->spawn_pts[lane]) : -1;
     bool taken = RESPAWN && is_sp && (sg[mycell] & kOcc);
     for (int i = 0; i < p.n; ++i) {
         if (!((who >> i) & 1u)) continue;
         uint32_t key = 0;
         if (p.random_spawn && is_sp)
             key = p.d_spawnkey ? p.d_spawnkey[((size_t)env * p.n + i) * g.G() + mycell]
-                               : philox_word(p, gid, tick, 3u, (uint32_t)(i * p.n_spawn + lane));
+                               : philox_word(p, gid, tick, 3u, (uint32_t)(i * vr.n_spawn() + lane));
         const bool cand = is_sp && !taken;
         const uint32_t mk = w.rmax(cand ? key : 0u);
         const unsigned eq = w.ballot(cand && key == mk);
@@ -973,15 +1004,15 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
 // ------------------------------------------------------------------ the kernel's stages
 // setup_agents (map_env.py:771-784) and custom_map_update (313) on the base grid staged in sg: MODE_RESET's body.  The reset
 // env's t, tick and counts are stored; its agents are all in play.
-template <class GEO>
-__device__ __forceinline__ void reset_env(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, int lane, bool is_agent, int env,
-                                          uint32_t gid, uint32_t tick, int& pos, int& ori, int& apples, int& waste) {
-    place_agents<false>(w, g, p, sg, lane, env, gid, tick, ~0u, pos);
+template <class GEO, class VR>
+__device__ __forceinline__ void reset_env(const Warp& w, const GEO& g, const KParams& p, const VR& vr, uint8_t* sg, int lane, bool is_agent,
+                                          int env, uint32_t gid, uint32_t tick, int& pos, int& ori, int& apples, int& waste) {
+    place_agents<false>(w, g, p, vr, sg, lane, env, gid, tick, ~0u, pos);
     if (is_agent) ori = spawn_orientation(p, env, gid, tick, lane);
     if (is_agent) sg[pos] |= kOcc;                         // distinct spawn points: no two lanes share a cell
     w.sync();
-    apples = p.base_apples; waste = p.base_waste;
-    spawn(w, g, p, sg, lane, env, gid, tick, apples, waste);
+    apples = vr.base_apples(); waste = vr.base_waste();
+    spawn(w, g, p, vr, sg, lane, env, gid, tick, apples, waste);
     if (lane == 0) { p.t[env] = 0; p.tick[env] = tick + 1; p.counts[env] = (uint32_t)apples | ((uint32_t)waste << 16); }
 }
 
@@ -1018,14 +1049,16 @@ __device__ __forceinline__ void draw(const Warp& w, const GEO& g, const KParams&
 }
 
 // ------------------------------------------------------------------ the kernel
-// TAG: tagging-out timers are on (p.tag_timeout > 0; every mode but MODE_RESET, DESIGN.md §3 item 11).
+// TAG: tagging-out timers are on (p.tag_timeout > 0, or with variants any variant's; every mode but MODE_RESET, DESIGN.md §3 item 11).
 // IDX: observations are written as packed colour indices (SSD_OBS_INDEX4, DESIGN.md §3 item 12) instead of RGB planes.
 // MODE_STEP_RESET: MODE_STEP, then an env whose episode the step ended renders the finished step into the episode-end
 // buffers, runs MODE_RESET's body keyed by the post-step tick and renders its first observation (DESIGN.md §3 item 14).  A mode
 // of its own, not a runtime flag, so that the other instantiations keep their code.  Its two render call sites inline two copies
 // of the render: a two-pass loop around one call site spilled in the Harvest V=15 and runtime-geometry kernels
 // (profiles/r7_notes.md).
-template <int MODE, class GEO, bool TAG, bool IDX>
+// VAR: envs run the variants of p.variant_of (DESIGN.md §3 item 15).  A template parameter, not a runtime switch on variant_of,
+// because the switch moved the register allocation of most kernels without variants and spilled one (profiles/r8_notes.md).
+template <int MODE, class GEO, bool TAG, bool IDX, bool VAR>
 __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __grid_constant__ KParams p) {
     constexpr bool STEP = MODE == MODE_STEP || MODE == MODE_STEP_RESET;
     const GEO g(p);
@@ -1066,6 +1099,13 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
     {
         if (MODE == MODE_RESET && p.mask && __ldcg(p.mask + env) == 0) return;
         const uint32_t gid = p.gid_base + (uint32_t)env;
+        int vid = 0;                                          // the env's variant: ids past the table run the last variant
+        if (VAR) {
+            vid = __ldcg(p.variant_of + env);
+            SSD_CHECK(vid < p.n_variants);
+            vid = min(vid, p.n_variants - 1);
+        }
+        const Var<VAR> vr{p, vid};
         // every global load of the step is issued up front.  Mutable state is read past L1 (ld.global.cg): each entry is read once
         // per step anyway, and a launch that became resident before its predecessors finished (programmatic dependent launch,
         // concurrent env ranges sharing a cache line at a range boundary) must never see a line an earlier CTA left in this SM's L1.
@@ -1081,7 +1121,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
         }
         const int n16 = g.GS() >> 4;
         {
-            const uint4* src = MODE == MODE_RESET ? reinterpret_cast<const uint4*>(p.map->base_grid)
+            const uint4* src = MODE == MODE_RESET ? reinterpret_cast<const uint4*>(vr.map()->base_grid)
                                                   : reinterpret_cast<const uint4*>(p.grid + (size_t)env * g.GS());
             uint4 g0 = make_uint4(0, 0, 0, 0);
             if (lane < n16) g0 = __ldcg(src + lane);
@@ -1126,7 +1166,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
             }
             apples -= __popc(ate);
             w.sync();
-            beams<TAG>(w, g, p, sg, lane, live, act, pos, ori, reward, clean_num, waste, tagged);    // 259-260
+            beams<TAG>(w, g, p, vr, sg, lane, live, act, pos, ori, reward, clean_num, waste, tagged);    // 259-260
             unsigned gone = 0;
             if (TAG) {                                 // the tagged leave the map; a cell stays occupied while an untagged agent is on it
                 gone = w.ballot(tagged);
@@ -1136,13 +1176,13 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                     if (tagged) { home = pos; pos = -1 - lane; live = false; }
                 }
             }
-            spawn(w, g, p, sg, lane, env, gid, tick, apples, waste);                                  // 263, 291-292
+            spawn(w, g, p, vr, sg, lane, env, gid, tick, apples, waste);                              // 263, 291-292
             if (TAG) {                                 // the agents out during this step count down; those reaching 0 return
                 const bool back = timer == 1;
-                timer = tagged ? p.tag_timeout : (timer ? timer - 1 : 0);
+                timer = tagged ? vr.tag_timeout() : (timer ? timer - 1 : 0);
                 const unsigned who = w.ballot(back);
                 if (who) {
-                    place_agents<true>(w, g, p, sg, lane, env, gid, tick, who, pos);
+                    place_agents<true>(w, g, p, vr, sg, lane, env, gid, tick, who, pos);
                     if (back) { ori = spawn_orientation(p, env, gid, tick, lane); live = true; sg[pos] |= kOcc; }
                     w.sync();
                 }
@@ -1163,7 +1203,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
             }
             if (MODE == MODE_STEP_RESET) ended = t >= p.episode_limit;
         } else if (MODE == MODE_RESET) {
-            reset_env(w, g, p, sg, lane, is_agent, env, gid, tick, pos, ori, apples, waste);
+            reset_env(w, g, p, vr, sg, lane, is_agent, env, gid, tick, pos, ori, apples, waste);
             ep_ret = 0;
         }
 
@@ -1193,10 +1233,10 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                 // The base grid is staged again.  Nothing else needs restoring: a render never writes the slack or the "outside"
                 // fill of the maps, and it rebuilds every map cell it reads.
                 w.sync();                                          // the render has read the staged grid
-                const uint4* src = reinterpret_cast<const uint4*>(p.map->base_grid);
+                const uint4* src = reinterpret_cast<const uint4*>(vr.map()->base_grid);
                 warp_for(g.GS() >> 4, lane, [&](int i) { reinterpret_cast<uint4*>(sg)[i] = __ldcg(src + i); });
                 w.sync();
-                reset_env(w, g, p, sg, lane, is_agent, env, gid, tick + 1, pos, ori, apples, waste);
+                reset_env(w, g, p, vr, sg, lane, is_agent, env, gid, tick + 1, pos, ori, apples, waste);
                 write_back_reset(w, g, p, sg, lane, is_agent, env, pos, ori);
                 live = is_agent; same = 1u << lane;
             }
@@ -1305,6 +1345,9 @@ struct ssd_handle {
     int pdl;                                                  // programmatic dependent launch for small launches (SSD_B200_PDL=0 turns it off)
     int obs_format;                                           // SSD_OBS_RGB (at creation) or SSD_OBS_INDEX4
     int state_format;                                         // the same, for the state image
+    VarDev* d_vars;                                           // variant table: SSD_MAX_VARIANTS records, allocated once when first needed
+    VarDev* base;                                             // host copy of the creation config's record (ssd_set_variants(h, 0, ...))
+    int tag_any;                                              // some variant of the table has tag_timeout > 0
 };
 
 static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws* d, KParams& k) {
@@ -1321,7 +1364,7 @@ static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws
     return SSD_OK;
 }
 
-template <int MODE, class GEO, bool TAG, bool IDX>
+template <int MODE, class GEO, bool TAG, bool IDX, bool VAR>
 static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
@@ -1333,7 +1376,7 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
         const int dev = h->device;
         if (dev < 0 || dev >= kMaxDevices) return SSD_ERR_INVALID;
         if ((int)h->smem_bytes > high_water[dev]) {
-            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, TAG, IDX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, TAG, IDX, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
             high_water[dev] = (int)h->smem_bytes;
         }
     }
@@ -1348,9 +1391,9 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, TAG, IDX>, k));
+        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, TAG, IDX, VAR>, k));
     } else {
-        ssd_kernel<MODE, GEO, TAG, IDX><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
+        ssd_kernel<MODE, GEO, TAG, IDX, VAR><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
     }
     ++h->launches;
     SSD_CUDA(cudaGetLastError());
@@ -1363,16 +1406,26 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
 // launches gain nothing and pay for the prologue no longer running under the state loads, so they keep the plain launch.
 constexpr int kPdlMaxEnvs = 2048;
 
+template <int MODE, class GEO, bool VAR>
+static int launch_var(ssd_handle* h, const KParams& k, void* stream) {
+    const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
+    if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation
+        if (k.variant_of ? h->tag_any : k.tag_timeout != 0)
+            return idx ? launch_kernel<MODE, GEO, true, true, VAR>(h, k, stream) : launch_kernel<MODE, GEO, true, false, VAR>(h, k, stream);
+    }
+    return idx ? launch_kernel<MODE, GEO, false, true, VAR>(h, k, stream) : launch_kernel<MODE, GEO, false, false, VAR>(h, k, stream);
+}
+
 template <int MODE, class GEO>
 static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
     k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
-    const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
-    if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation
-        if (k.tag_timeout != 0)
-            return idx ? launch_kernel<MODE, GEO, true, true>(h, k, stream) : launch_kernel<MODE, GEO, true, false>(h, k, stream);
+    // per-env variants: their own instantiations (a render reads nothing a variant sets, but draws no agent out of play when
+    // any variant tags)
+    if constexpr (MODE != MODE_RENDER) {
+        if (k.variant_of) return launch_var<MODE, GEO, true>(h, k, stream);
     }
-    return idx ? launch_kernel<MODE, GEO, false, true>(h, k, stream) : launch_kernel<MODE, GEO, false, false>(h, k, stream);
+    return launch_var<MODE, GEO, false>(h, k, stream);
 }
 
 // The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
@@ -1387,6 +1440,78 @@ static int launch(ssd_handle* h, const KParams& k, void* stream) {
         if (v.kind == SSD_KIND_CLEANUP && v.H == 10 && v.W == 10 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_CLEANUP, 10, 10, 7>>(h, k, stream);
     }
     return launch_geo<MODE, GeoD>(h, k, stream);
+}
+
+// One variant of a handle of kind `kind`, H x W and n agents, checked as ssd_create checks its config: the int8 reward bound and the
+// 8-bit timer (SSD_ERR_INVALID), a wall-enclosed map in the kind's alphabet (SSD_ERR_MAP), at least n spawn points (SSD_ERR_SPAWN),
+// at most SSD_MAX_SPAWN of them, the Cleanup LUT length (#waste points + 1) and the apple point limit of spawn (SSD_ERR_INVALID).
+// Every point slot past the lists holds kNoPoint, so a launch that pairs a table with a stale count never reads a bogus cell.
+static int compile_variant(int kind, int H, int W, int n, const char* ascii_map, uint32_t n_waste_lut, const uint32_t* thr_apple,
+                           const uint32_t* thr_waste, const uint32_t thr_harvest[4], int fire_cost, int hit_penalty, int tag_timeout,
+                           VarDev* v) {
+    if (!ascii_map) return SSD_ERR_INVALID;
+    if (abs(fire_cost) + n * abs(hit_penalty) + 1 > 127) return SSD_ERR_INVALID;   // reward is int8
+    if (tag_timeout < 0 || tag_timeout > 255) return SSD_ERR_INVALID;              // 8-bit timer in the agent record
+    memset(v, 0, sizeof(VarDev));
+    MapDev* hm = &v->map;
+    for (int k = 0; k < SSD_MAX_CELLS + 4; ++k) hm->apple_pts[k] = hm->waste_pts[k] = kNoPoint;
+    const int G = H * W;
+    int na = 0, nw = 0, ns = 0;
+    for (int c = 0; c < G; ++c) {
+        const char ch = ascii_map[c];
+        const int r = c / W, col = c % W;
+        const bool border = r == 0 || col == 0 || r == H - 1 || col == W - 1;
+        if (border && ch != '@') return SSD_ERR_MAP;
+        uint8_t code = SSD_CELL_EMPTY;
+        switch (ch) {
+            case '@': code = SSD_CELL_WALL; break;
+            case ' ': break;
+            case 'P': if (ns < SSD_MAX_SPAWN) hm->spawn_pts[ns] = (uint16_t)c; ++ns; break;   // map_env.py:143-146
+            case 'A': if (kind == SSD_KIND_HARVEST) { code = SSD_CELL_APPLE; hm->apple_pts[na++] = (uint16_t)c; } break;
+            case 'B': if (kind == SSD_KIND_CLEANUP) hm->apple_pts[na++] = (uint16_t)c; break;   // cleanup.py:81-82
+            case 'H': if (kind == SSD_KIND_CLEANUP) { code = SSD_CELL_WASTE; hm->waste_pts[nw++] = (uint16_t)c; } break;
+            case 'R': if (kind == SSD_KIND_CLEANUP) code = SSD_CELL_RIVER; break;
+            case 'S': if (kind == SSD_KIND_CLEANUP) code = SSD_CELL_STREAM; break;
+            default: return SSD_ERR_MAP;
+        }
+        hm->base_grid[c] = code;
+    }
+    if (ns < n) return SSD_ERR_SPAWN;
+    if (ns > SSD_MAX_SPAWN) return SSD_ERR_INVALID;
+    if (kind == SSD_KIND_CLEANUP) {
+        if (n_waste_lut != (uint32_t)nw + 1 || !thr_apple || !thr_waste) return SSD_ERR_INVALID;
+        memcpy(hm->thr_apple, thr_apple, sizeof(uint32_t) * (nw + 1));
+        memcpy(hm->thr_waste, thr_waste, sizeof(uint32_t) * (nw + 1));
+    }
+    v->n_apple = na; v->n_waste = nw; v->n_spawn = ns; v->n_apple4 = (na + 3) / 4; v->n_waste2 = (nw + 1) / 2;
+    if (v->n_apple4 > 32 * 16) return SSD_ERR_INVALID;                               // spawn's 64-bit decision mask
+    for (int c = 0; c < G; ++c) { v->base_apples += hm->base_grid[c] == SSD_CELL_APPLE; v->base_waste += hm->base_grid[c] == SSD_CELL_WASTE; }
+    v->fire_cost = fire_cost; v->hit_penalty = hit_penalty; v->tag_timeout = tag_timeout;
+    for (int i = 0; i < 4; ++i) v->thr_harvest[i] = thr_harvest[i];
+    return SSD_OK;
+}
+
+// The scalars of variant 0 live in KParams, where every launch without an id array reads them.
+static void set_variant0(KParams& k, const VarDev& v) {
+    k.n_apple = v.n_apple; k.n_waste = v.n_waste; k.n_spawn = v.n_spawn; k.n_apple4 = v.n_apple4; k.n_waste2 = v.n_waste2;
+    k.base_apples = v.base_apples; k.base_waste = v.base_waste;
+    k.fire_cost = v.fire_cost; k.hit_penalty = v.hit_penalty; k.tag_timeout = v.tag_timeout;
+    for (int i = 0; i < 4; ++i) k.thr_harvest[i] = v.thr_harvest[i];
+}
+
+// Allocates the variant table at its full size, every record the creation config, the first time a call needs it.  It is never
+// reallocated, so no launch, queued or captured in a CUDA graph, can read a freed table.
+static int ensure_variant_table(ssd_handle* h) {
+    if (h->d_vars) return SSD_OK;
+    VarDev* d = nullptr;
+    SSD_CUDA(cudaMalloc(&d, sizeof(VarDev) * SSD_MAX_VARIANTS));
+    for (int i = 0; i < SSD_MAX_VARIANTS; ++i) {
+        const cudaError_t e = cudaMemcpy(d + i, h->base, sizeof(VarDev), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) { cudaFree(d); return cuda_fail(e); }
+    }
+    h->d_vars = d;
+    h->kp.variants = d;
+    return SSD_OK;
 }
 
 extern "C" {
@@ -1423,56 +1548,30 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     if (abs(cfg->fire_cost) + n * abs(cfg->hit_penalty) + 1 > 127) return SSD_ERR_INVALID;   // reward is int8
     if (cfg->tag_timeout < 0 || cfg->tag_timeout > 255) return SSD_ERR_INVALID;              // 8-bit timer in the agent record
 
-    MapDev* hm = new (std::nothrow) MapDev;
-    if (!hm) return SSD_ERR_INVALID;
-    memset(hm, 0, sizeof(MapDev));
-    int na = 0, nw = 0, ns = 0;
-    for (int c = 0; c < G; ++c) {
-        const char ch = cfg->ascii_map[c];
-        const int r = c / W, col = c % W;
-        const bool border = r == 0 || col == 0 || r == H - 1 || col == W - 1;
-        if (border && ch != '@') { delete hm; return SSD_ERR_MAP; }
-        uint8_t code = SSD_CELL_EMPTY;
-        switch (ch) {
-            case '@': code = SSD_CELL_WALL; break;
-            case ' ': break;
-            case 'P': if (ns < SSD_MAX_SPAWN) hm->spawn_pts[ns] = (uint16_t)c; ++ns; break;   // map_env.py:143-146
-            case 'A': if (cfg->kind == SSD_KIND_HARVEST) { code = SSD_CELL_APPLE; hm->apple_pts[na++] = (uint16_t)c; } break;
-            case 'B': if (cfg->kind == SSD_KIND_CLEANUP) hm->apple_pts[na++] = (uint16_t)c; break;   // cleanup.py:81-82
-            case 'H': if (cfg->kind == SSD_KIND_CLEANUP) { code = SSD_CELL_WASTE; hm->waste_pts[nw++] = (uint16_t)c; } break;
-            case 'R': if (cfg->kind == SSD_KIND_CLEANUP) code = SSD_CELL_RIVER; break;
-            case 'S': if (cfg->kind == SSD_KIND_CLEANUP) code = SSD_CELL_STREAM; break;
-            default: delete hm; return SSD_ERR_MAP;
-        }
-        hm->base_grid[c] = code;
+    VarDev* v0 = new (std::nothrow) VarDev;
+    if (!v0) return SSD_ERR_INVALID;
+    {
+        const int rc = compile_variant(cfg->kind, H, W, n, cfg->ascii_map, cfg->n_waste_lut, cfg->thr_apple, cfg->thr_waste,
+                                       cfg->thr_harvest, cfg->fire_cost, cfg->hit_penalty, cfg->tag_timeout, v0);
+        if (rc) { delete v0; return rc; }
     }
-    if (ns < n) { delete hm; return SSD_ERR_SPAWN; }
-    if (ns > SSD_MAX_SPAWN) { delete hm; return SSD_ERR_INVALID; }
-    for (int k = na; k < round_up(na, 4) + 4 && k < SSD_MAX_CELLS + 4; ++k) hm->apple_pts[k] = kNoPoint;
-    for (int k = nw; k < round_up(nw, 2) + 2 && k < SSD_MAX_CELLS + 4; ++k) hm->waste_pts[k] = kNoPoint;
-    if (cfg->kind == SSD_KIND_CLEANUP) {
-        if (cfg->n_waste_lut != (uint32_t)nw + 1 || !cfg->thr_apple || !cfg->thr_waste) { delete hm; return SSD_ERR_INVALID; }
-        memcpy(hm->thr_apple, cfg->thr_apple, sizeof(uint32_t) * (nw + 1));
-        memcpy(hm->thr_waste, cfg->thr_waste, sizeof(uint32_t) * (nw + 1));
-    }
+    const MapDev* hm = &v0->map;
 
     ssd_handle* h = new (std::nothrow) ssd_handle;
-    if (!h) { delete hm; return SSD_ERR_INVALID; }
+    if (!h) { delete v0; return SSD_ERR_INVALID; }
     memset(h, 0, sizeof(*h));
     KParams& k = h->kp;
     k.geo = make_geo(cfg->kind, H, W, V);
     const GeoVals& gv = k.geo;
     k.B = cfg->n_envs; k.n = n; k.NA = round_up(n, 4);
-    k.episode_limit = cfg->episode_limit; k.fire_cost = cfg->fire_cost; k.hit_penalty = cfg->hit_penalty;
-    k.tag_timeout = cfg->tag_timeout;
+    k.episode_limit = cfg->episode_limit;
     k.beam_len = cfg->beam_len; k.n_actions = cfg->kind == SSD_KIND_CLEANUP ? 9 : 8;
-    k.n_apple = na; k.n_waste = nw; k.n_spawn = ns; k.n_apple4 = (na + 3) / 4; k.n_waste2 = (nw + 1) / 2;
-    k.base_apples = 0; k.base_waste = 0;
-    for (int c = 0; c < G; ++c) { k.base_apples += hm->base_grid[c] == SSD_CELL_APPLE; k.base_waste += hm->base_grid[c] == SSD_CELL_WASTE; }
+    set_variant0(k, *v0);
+    k.n_variants = 1;
+    h->base = v0;
     k.random_spawn = cfg->random_spawn_point != 0; k.spawn_rot = cfg->spawn_rotation < 0 ? -1 : cfg->spawn_rotation;
     k.invN20 = magic20(gv.N, SSD_MAX_AGENTS * gv.N + 64); k.invW20 = magic20(W, G + 1);
     k.seed_lo = (uint32_t)cfg->seed; k.seed_hi = (uint32_t)(cfg->seed >> 32); k.gid_base = cfg->env_gid_base;
-    for (int i = 0; i < 4; ++i) k.thr_harvest[i] = cfg->thr_harvest[i];
     for (int i = 0; i < 16; ++i)
         k.lut[i] = (uint32_t)cfg->color_lut[i][0] | ((uint32_t)cfg->color_lut[i][1] << 8) | ((uint32_t)cfg->color_lut[i][2] << 16);
     k.agents_uniform = 1;
@@ -1482,10 +1581,10 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
         for (int i = 0; i < 4; ++i) { lo |= (uint32_t)cfg->color_lut[i][ch] << (8 * i); hi |= (uint32_t)cfg->color_lut[4 + i][ch] << (8 * i); }
         k.lut8[2 * ch] = lo; k.lut8[2 * ch + 1] = hi;
     }
-    if (k.invN20 == 0 || k.invW20 == 0 || k.n_apple4 > 32 * 16) { delete hm; delete h; return SSD_ERR_INVALID; }
+    if (k.invN20 == 0 || k.invW20 == 0) { delete v0; delete h; return SSD_ERR_INVALID; }
 
     k.invMW20 = magic20(gv.nw8M, H * gv.nw8M + 32);
-    if (k.invMW20 == 0 || gv.PMS >= 60000) { delete hm; delete h; return SSD_ERR_INVALID; }
+    if (k.invMW20 == 0 || gv.PMS >= 60000) { delete v0; delete h; return SSD_ERR_INVALID; }
     h->smem_bytes = (size_t)kWarps * (gv.padF + gv.GS + gv.padB + gv.PMS);     // one staging tile per warp
     { const char* e = getenv("SSD_B200_GENERIC"); h->force_generic = e && e[0] == '1'; }
     { const char* e = getenv("SSD_B200_PDL"); h->pdl = !(e && e[0] == '0'); }
@@ -1496,13 +1595,13 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     if (e == cudaSuccess) {                                   // the launch needs smem_bytes dynamic + the static LUTs
         int optin = 0;
         e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
-        if (e == cudaSuccess && h->smem_bytes + sizeof(ColourLuts) > (size_t)optin) { delete hm; delete h; return SSD_ERR_INVALID; }
+        if (e == cudaSuccess && h->smem_bytes + sizeof(ColourLuts) > (size_t)optin) { delete v0; delete h; return SSD_ERR_INVALID; }
     }
     if (e == cudaSuccess) e = cudaMalloc(&h->d_map, sizeof(MapDev));
     if (e == cudaSuccess) e = cudaMemcpy(h->d_map, hm, sizeof(MapDev), cudaMemcpyHostToDevice);
-    delete hm;
     if (e != cudaSuccess) {
         if (h->d_map) cudaFree(h->d_map);
+        delete v0;
         delete h;
         return cuda_fail(e);
     }
@@ -1515,6 +1614,8 @@ int ssd_destroy(ssd_handle* h) {
     if (!h) return SSD_ERR_INVALID;
     DeviceGuard guard(h->device);
     cudaFree(h->d_map);
+    if (h->d_vars) cudaFree(h->d_vars);
+    delete h->base;
     delete h;
     return SSD_OK;
 }
@@ -1550,6 +1651,49 @@ int ssd_get_state_layout(const ssd_handle* h, int32_t format, ssd_state_layout* 
 int ssd_set_state_format(ssd_handle* h, int32_t format) {
     if (!h || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
     h->state_format = format;
+    return SSD_OK;
+}
+
+int ssd_set_variants(ssd_handle* h, int32_t n_variants, const ssd_variant* variants) {
+    if (!h || n_variants < 0 || n_variants > SSD_MAX_VARIANTS || (n_variants > 0 && !variants)) return SSD_ERR_INVALID;
+    const int m = n_variants > 0 ? n_variants : 1;
+    VarDev* recs = new (std::nothrow) VarDev[m];
+    if (!recs) return SSD_ERR_INVALID;
+    const GeoVals& g = h->kp.geo;
+    if (n_variants == 0) recs[0] = *h->base;
+    for (int i = 0; i < n_variants; ++i) {
+        const ssd_variant& v = variants[i];
+        const int rc = compile_variant(g.kind, g.H, g.W, h->kp.n, v.ascii_map, v.n_waste_lut, v.thr_apple, v.thr_waste, v.thr_harvest,
+                                       v.fire_cost, v.hit_penalty, v.tag_timeout, &recs[i]);
+        if (rc) { delete[] recs; return rc; }
+    }
+    DeviceGuard guard(h->device);
+    cudaError_t e = guard.err;
+    if (e == cudaSuccess) {
+        const int rc = ensure_variant_table(h);
+        if (rc) { delete[] recs; return rc; }
+        e = cudaDeviceSynchronize();                          // no launch in flight reads the table or the map while they change
+    }
+    if (e == cudaSuccess) e = cudaMemcpy(h->d_vars, recs, sizeof(VarDev) * m, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(h->d_map, &recs[0].map, sizeof(MapDev), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { delete[] recs; return cuda_fail(e); }
+    set_variant0(h->kp, recs[0]);
+    h->kp.n_variants = m;
+    h->tag_any = 0;
+    for (int i = 0; i < m; ++i) h->tag_any |= recs[i].tag_timeout != 0;
+    delete[] recs;
+    return SSD_OK;
+}
+
+int ssd_set_env_variants(ssd_handle* h, const uint8_t* variant_of) {
+    if (!h) return SSD_ERR_INVALID;
+    if (variant_of) {
+        DeviceGuard guard(h->device);
+        SSD_CUDA(guard.err);
+        const int rc = ensure_variant_table(h);
+        if (rc) return rc;
+    }
+    h->kp.variant_of = variant_of;
     return SSD_OK;
 }
 

@@ -15,6 +15,7 @@ run-length encoded: ``<char><count>`` with ``_`` standing for a blank cell.
 """
 from __future__ import annotations
 
+import dataclasses
 import hashlib
 import math
 import re
@@ -228,6 +229,43 @@ def compile_map(name: str, map_name: str, n_agents: int, view: int, episode_limi
                    base_grid=base, wall=wall.astype(np.uint8), apple_pts=apple, waste_pts=waste,
                    spawn_pts=spawn, thr_apple=thr_a, thr_waste=thr_w, thr_harvest=thr_h,
                    lut=color_lut(p.kind, obs_color))
+
+
+VARIANT_KEYS_COMMON = ("rows", "fire_cost", "hit_penalty", "tag_timeout")
+VARIANT_KEYS = {KIND_CLEANUP: VARIANT_KEYS_COMMON + ("threshold_depletion", "threshold_restoration", "waste_spawn_prob",
+                                                    "apple_respawn_prob"),
+                KIND_HARVEST: VARIANT_KEYS_COMMON + ("spawn_prob",)}
+
+
+def compile_variant(base: MapSpec, overrides: dict) -> MapSpec:
+    """One env variant (``ssd_set_variants``): ``base`` (the handle's creation spec) with ``overrides`` applied.  Keys:
+    ``rows`` (an ASCII layout of base's exact H x W), ``fire_cost``, ``hit_penalty``, ``tag_timeout``, and the spawn
+    dynamics of the kind -- Cleanup ``threshold_depletion``, ``threshold_restoration``, ``waste_spawn_prob``,
+    ``apple_respawn_prob``; Harvest ``spawn_prob`` (4 probabilities).  ``{}`` is the base config.  Everything else (kind,
+    size, view, agents, episode limit, colours) stays the handle's."""
+    ov = dict(overrides or {})
+    allowed = VARIANT_KEYS[base.kind]
+    other = set(VARIANT_KEYS[KIND_HARVEST if base.kind == KIND_CLEANUP else KIND_CLEANUP]) - set(allowed)
+    for key in ov:
+        if key in other:
+            kind = "cleanup" if base.kind == KIND_CLEANUP else "harvest"
+            raise ValueError(f"variant key {key!r} does not apply to {kind}")
+        if key not in allowed:
+            raise ValueError(f"unknown variant key {key!r}; allowed: {sorted(allowed)}")
+    rows = list(ov.pop("rows", base.rows))
+    if len(rows) != base.H or any(len(r) != base.W for r in rows):
+        raise ValueError(f"variant rows must be {base.H} rows of {base.W} characters")
+    pk = {k: ov.pop(k) for k in list(ov) if k not in VARIANT_KEYS_COMMON}
+    if "spawn_prob" in pk:
+        sp = tuple(float(x) for x in pk["spawn_prob"])
+        if len(sp) != 4:
+            raise ValueError("spawn_prob needs 4 probabilities")
+        pk["spawn_prob"] = sp
+    params = dataclasses.replace(base.params, **{k: (v if k == "spawn_prob" else float(v)) for k, v in pk.items()})
+    return compile_map("", "", base.n_agents, base.view, base.episode_limit, obs_color=base.obs_color, rows=rows,
+                       params=params, fire_cost=int(ov.get("fire_cost", base.fire_cost)),
+                       hit_penalty=int(ov.get("hit_penalty", base.hit_penalty)),
+                       tag_timeout=int(ov.get("tag_timeout", base.tag_timeout)))
 
 
 def dump_maps() -> str:

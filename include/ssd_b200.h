@@ -41,6 +41,7 @@ extern "C" {
 #define SSD_MAX_AGENTS 16
 #define SSD_MAX_CELLS  2048
 #define SSD_MAX_SPAWN  32
+#define SSD_MAX_VARIANTS 256   /* variant ids are u8 (ssd_set_env_variants) */
 
 /* cell codes stored in the device grid (one byte per cell) */
 #define SSD_CELL_EMPTY  0
@@ -84,6 +85,19 @@ typedef struct ssd_config {
     uint32_t thr_harvest[4];      /* harvest: ceil(SPAWN_PROB[k] * 2^32) (harvest.py:118) */
     uint8_t color_lut[16][4];     /* RGB0 per colour index: 0-5 cell codes, 6 outside, 6+c agent char c */
 } ssd_config;
+
+/* One env variant (ssd_set_variants): the fields of ssd_config that may differ between the envs of one handle.  Everything else
+ * (kind, size, view, n_agents, episode_limit, beam_len, colours, formats, spawn options, seed, env_gid_base) is the handle's. */
+typedef struct ssd_variant {
+    const char* ascii_map;        /* [height*width] row-major, the handle's size and kind alphabet                      */
+    uint32_t n_waste_lut;         /* entries in thr_apple / thr_waste (= #waste points of this map + 1); cleanup only    */
+    const uint32_t* thr_apple;    /* cleanup: as ssd_config.thr_apple                                                    */
+    const uint32_t* thr_waste;    /* cleanup: as ssd_config.thr_waste                                                    */
+    uint32_t thr_harvest[4];      /* harvest: as ssd_config.thr_harvest                                                  */
+    int32_t fire_cost;            /* as ssd_config.fire_cost                                                             */
+    int32_t hit_penalty;          /* as ssd_config.hit_penalty                                                           */
+    int32_t tag_timeout;          /* 0..255, as ssd_config.tag_timeout                                                   */
+} ssd_variant;
 
 /* Strides the caller must allocate with (all in elements of the buffer type). */
 typedef struct ssd_layout {
@@ -202,6 +216,26 @@ int ssd_get_state_layout(const ssd_handle* h, int32_t format, ssd_state_layout* 
  * SSD_OBS_RGB.  Host-side and serialised like ssd_set_obs_format; a CUDA graph keeps the format it was captured with.
  * SSD_ERR_INVALID, before any CUDA call, for a NULL handle or an unknown format. */
 int ssd_set_state_format(ssd_handle* h, int32_t format);
+
+/* Sets the handle's variant table to variants[0 .. n_variants) (DESIGN.md §3 item 15), entry 0 included; n_variants = 0 restores
+ * the creation config as the only variant.  Env b running variant v is bit-identical, in every buffer and pad byte, to env b of a
+ * handle created with v's config alone (same seed and env_gid_base), in every call.  Each entry is validated as ssd_create
+ * validates its config, before any CUDA call: SSD_ERR_MAP (not wall-enclosed, or a character outside the kind's alphabet),
+ * SSD_ERR_SPAWN (fewer spawn points than agents), SSD_ERR_INVALID (NULL map, n_waste_lut != #waste points + 1 or NULL LUTs for
+ * Cleanup, more than SSD_MAX_SPAWN spawn points, too many apple points, |fire_cost| + n|hit_penalty| + 1 > 127, tag_timeout
+ * outside 0..255, n_variants outside 0..SSD_MAX_VARIANTS).  On an error nothing changes.  A configuration call, serialised like
+ * ssd_set_obs_format: it synchronises the device before it overwrites the table, which is allocated once at its full size, so no
+ * launch ever reads a freed table.  A CUDA graph captured before it reads the new table with the launch parameters it was captured
+ * with (capture again).  A launch uses the tagging-out kernels when any variant has tag_timeout > 0; an env whose variant has
+ * tag_timeout 0 is then never tagged. */
+int ssd_set_variants(ssd_handle* h, int32_t n_variants, const ssd_variant* variants);
+
+/* variant_of: caller-owned DEVICE array [B] of variant ids indexed by env index, read by every later launch (a step, auto-reset or
+ * render uses the env's current id; a reset builds the env from its current variant's layout, so an env moves to a variant with
+ * another layout by writing its id and resetting it).  An id >= n_variants runs the last variant (the checked build counts it).
+ * NULL (the default) runs every env as variant 0, with no per-env load.  Host-side and serialised like ssd_set_obs_format; a CUDA
+ * graph keeps the pointer it was captured with. */
+int ssd_set_env_variants(ssd_handle* h, const uint8_t* variant_of);
 
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */

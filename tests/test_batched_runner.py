@@ -1,92 +1,27 @@
 """GPU suite (SURVEY 8f f1): the batched runner fills an EpisodeBatch exactly as B runs of the reference's single-env
 runner loop would (src/runners/episode_runner.py:48-141), while keeping every tensor on the device."""
-import types
-
 import numpy as np
 import pytest
+
+from harness import FakeBatch, ScriptedMAC, _scheme, action_tables, make_runner
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 
-class FakeBatch:
-    """EpisodeBatch stand-in with the update() semantics of src/components/episode_buffer.py:87-116:
-    per-key dtype, th.tensor() for non-tensors, clone for tensors, view_as into [B, T, ...] storage."""
-
-    def __init__(self, scheme, B, T, device):
-        self.scheme, self.batch_size, self.max_seq_length, self.device = scheme, B, T, device
-        self.data = {k: torch.zeros((B, T) + tuple(v["shape"]), dtype=v.get("dtype", torch.float32), device=device)
-                     for k, v in scheme.items()}
-        self.data["filled"] = torch.zeros((B, T, 1), dtype=torch.long, device=device)
-
-    def update(self, data, bs=slice(None), ts=slice(None)):
-        ts = slice(ts, ts + 1) if isinstance(ts, int) else ts
-        self.data["filled"][bs, ts] = 1
-        for k, v in data.items():
-            dtype = self.scheme[k].get("dtype", torch.float32)
-            v = v.clone().detach() if isinstance(v, torch.Tensor) else torch.tensor(v, dtype=dtype, device=self.device)
-            dest = self.data[k][bs, ts]
-            self.data[k][bs, ts] = v.view_as(dest)
-
-    def __getitem__(self, k):
-        if isinstance(k, slice):                              # EpisodeBatch[lo:hi]: a view on the same storage
-            view = FakeBatch.__new__(FakeBatch)
-            view.scheme, view.max_seq_length, view.device = self.scheme, self.max_seq_length, self.device
-            view.data = {name: t[k] for name, t in self.data.items()}
-            view.batch_size, view.offset = view.data["filled"].shape[0], k.start or 0
-            return view
-        return self.data[k]
-
-
-class ScriptedMAC:
-    """Actions come from a fixed table (independent of the observations) so two runners can be compared."""
-
-    def __init__(self, table, table_inc):
-        self.table, self.table_inc = table, table_inc
-
-    def init_hidden(self, batch_size):
-        self.bs = batch_size
-
-    def select_actions_env(self, batch, t_ep, t_env, test_mode=False):
-        lo = getattr(batch, "offset", 0)
-        return self.table[lo:lo + batch.batch_size, t_ep].clone()
-
-    def select_actions_inc(self, actions, batch, t_ep, t_env, test_mode=False, agent_pos_replay=None):
-        assert agent_pos_replay.shape[-1] == 2
-        lo = getattr(batch, "offset", 0)
-        return self.table_inc[lo:lo + batch.batch_size, t_ep].clone()
-
-
-def _scheme(n, A, H, W, N):
-    return {"state": {"shape": (3, H, W)}, "obs": {"shape": (n, 3, N, N)}, "actions": {"shape": (n, 1), "dtype": torch.long},
-            "avail_actions": {"shape": (n, A), "dtype": torch.int}, "reward": {"shape": (n,)},
-            "terminated": {"shape": (1,), "dtype": torch.uint8}, "clean_num": {"shape": (n,)}, "apple_den": {"shape": (n,)},
-            "agent_pos": {"shape": (n, 2)}, "agent_orientation": {"shape": (n, 2)}, "actions_inc": {"shape": (n, n, 1), "dtype": torch.long}}
-
-
 @pytest.mark.parametrize("name,mp,n,view,groups", [("cleanup", "default3", 3, 7, 1), ("harvest", "default10", 5, 15, 1),
                                                     ("cleanup", "default3", 3, 7, 3)])
 def test_batched_runner_equals_sequential_facade_runs(name, mp, n, view, groups):
-    from homophily_marl_b200.batched_runner import BatchedEpisodeRunner
     from homophily_marl_b200 import REGISTRY
     B, T = 6, 9
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, disable_rotation_action=False,
-                 disable_fire_action=False, obs_color="full")
-    env_args = dict(num_agents=n, render=False, episode_limit=T, is_replay=False, view_size=view, map=mp, extra_args=extra, seed=3)
-    args = types.SimpleNamespace(batch_size_run=B, env=name, env_args=env_args, device="cuda:0", name="homophily", mac="homophily_mac",
-                                 n_actions=None, ind_reward=True, runner_log_interval=10 ** 9, test_nepisode=B, env_groups=groups)
     logged = {}
-    logger = types.SimpleNamespace(log_stat=lambda k, v, t: logged.__setitem__(k, v))
-    runner = BatchedEpisodeRunner(args, logger)
-    info = runner.get_env_info()
-    A, dev = info["n_actions"], runner.env.device
-    args.n_actions = A
-    g = torch.Generator().manual_seed(0)
-    table = torch.randint(0, 2 * A, (B, T + 1, n, 1), generator=g).to(dev)          # exercises `actions % n_actions`
-    table_inc = torch.randint(0, 3, (B, T + 1, n, n, 1), generator=g).to(dev)
-    scheme = _scheme(n, A, *info["state_dims"], info["obs_dims"][0])
-    runner.use_batch_factory(lambda: FakeBatch(scheme, B, T + 1, dev))
+    runner = make_runner(name, mp, n, view, B=B, T=T, groups=groups, extra=dict(obs_color="full"),
+                         log_stat=lambda k, v, t: logged.__setitem__(k, v))
+    env_args, A, dev = runner.args.env_args, runner.env.n_actions, runner.env.device
+    table, table_inc = action_tables(runner, 0, high=2 * A)                          # exercises `actions % n_actions`
     runner.mac = ScriptedMAC(table, table_inc)
+    info = runner.get_env_info()
+    scheme = _scheme(n, A, *info["state_dims"], info["obs_dims"][0])
     batch = runner.run(test_mode=True)
     assert runner.t == T and runner.t_env == 0 and bool(batch["filled"].all())
     assert set(logged) >= {"test_return_mean", "test_collective_return_mean", "test_equality_metric_mean", "test_ep_length_mean"}

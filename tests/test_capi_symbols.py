@@ -10,6 +10,8 @@ import sys
 import numpy as np
 import pytest
 
+from harness import ssd_config
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HDR = os.path.join(ROOT, "include", "ssd_b200.h")
 
@@ -70,32 +72,16 @@ def test_prob_to_threshold_matches_host_compiler(lib):
         assert np.array_equal(k / 2.0 ** 32 < p, k < T)
 
 
-def _cfg(rows, kind=0, n=1, view=7, **kw):
-    from homophily_marl_b200 import _capi
-    cfg = _capi.SsdConfig()
-    cfg.kind, cfg.n_envs, cfg.n_agents, cfg.height, cfg.width, cfg.view = kind, 4, n, len(rows), len(rows[0]), view
-    cfg.episode_limit, cfg.fire_cost, cfg.hit_penalty, cfg.beam_len = 10, 1, 0, 5
-    cfg.ascii_map = "".join(rows).encode()
-    thr = (C.c_uint32 * 8)()
-    cfg.thr_apple = C.cast(thr, C.c_void_p)
-    cfg.thr_waste = C.cast(thr, C.c_void_p)
-    cfg.n_waste_lut = kw.pop("n_waste_lut", 1)
-    for k2, v in kw.items():
-        setattr(cfg, k2, v)
-    cfg._keep = thr
-    return cfg
-
-
 def test_create_validates_before_touching_cuda(lib):
     from homophily_marl_b200 import _capi
     h = C.c_void_p()
     ok_rows = ["@@@@@", "@P B@", "@ P @", "@@@@@"]
-    assert lib.ssd_create(C.byref(_cfg(["@@@@@", "@P B ", "@ P @", "@@@@@"])), C.byref(h)) == _capi.SSD_ERR_MAP      # open border
-    assert lib.ssd_create(C.byref(_cfg(["@@@@@", "@P x@", "@ P @", "@@@@@"])), C.byref(h)) == _capi.SSD_ERR_MAP      # unknown char
-    assert lib.ssd_create(C.byref(_cfg(ok_rows, n=3)), C.byref(h)) == _capi.SSD_ERR_SPAWN                            # map_env.py:783
-    assert lib.ssd_create(C.byref(_cfg(ok_rows, n=17)), C.byref(h)) == _capi.SSD_ERR_INVALID
-    assert lib.ssd_create(C.byref(_cfg(ok_rows, kind=5)), C.byref(h)) == _capi.SSD_ERR_INVALID
-    assert lib.ssd_create(C.byref(_cfg(ok_rows, hit_penalty=127)), C.byref(h)) == _capi.SSD_ERR_INVALID              # int8 reward
+    assert lib.ssd_create(C.byref(ssd_config(["@@@@@", "@P B ", "@ P @", "@@@@@"])), C.byref(h)) == _capi.SSD_ERR_MAP      # open border
+    assert lib.ssd_create(C.byref(ssd_config(["@@@@@", "@P x@", "@ P @", "@@@@@"])), C.byref(h)) == _capi.SSD_ERR_MAP      # unknown char
+    assert lib.ssd_create(C.byref(ssd_config(ok_rows, n=3)), C.byref(h)) == _capi.SSD_ERR_SPAWN                            # map_env.py:783
+    assert lib.ssd_create(C.byref(ssd_config(ok_rows, n=17)), C.byref(h)) == _capi.SSD_ERR_INVALID
+    assert lib.ssd_create(C.byref(ssd_config(ok_rows, kind=5)), C.byref(h)) == _capi.SSD_ERR_INVALID
+    assert lib.ssd_create(C.byref(ssd_config(ok_rows, hit_penalty=127)), C.byref(h)) == _capi.SSD_ERR_INVALID              # int8 reward
     assert lib.ssd_create(None, C.byref(h)) == _capi.SSD_ERR_INVALID
     assert lib.ssd_step(None, None, None, None, None, None) == _capi.SSD_ERR_INVALID
     assert lib.ssd_destroy(None) == _capi.SSD_ERR_INVALID
@@ -114,7 +100,7 @@ def test_no_cpu_fallback():
         REGISTRY["harvest"](num_agents=5, map="default10", view_size=15, quiet=True)
     lib = _capi.load()
     h = C.c_void_p()
-    rc = lib.ssd_create(C.byref(_cfg(["@@@@@", "@P B@", "@ P @", "@@@@@"])), C.byref(h))
+    rc = lib.ssd_create(C.byref(ssd_config(["@@@@@", "@P B@", "@ P @", "@@@@@"])), C.byref(h))
     assert rc == _capi.SSD_ERR_CUDA and lib.ssd_last_cuda_error() != 0
 
 

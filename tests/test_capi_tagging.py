@@ -3,6 +3,8 @@ import ctypes as C
 
 import pytest
 
+from harness import ssd_config
+
 
 @pytest.fixture(scope="module")
 def lib():
@@ -11,27 +13,11 @@ def lib():
     return _capi.load()
 
 
-def _cfg(**kw):
-    from homophily_marl_b200 import _capi
-    rows = ["@@@@@", "@P B@", "@ P @", "@@@@@"]
-    cfg = _capi.SsdConfig()
-    cfg.kind, cfg.n_envs, cfg.n_agents, cfg.height, cfg.width, cfg.view = 0, 4, 1, len(rows), len(rows[0]), 7
-    cfg.episode_limit, cfg.fire_cost, cfg.hit_penalty, cfg.beam_len = 10, 1, 0, 5
-    cfg.ascii_map = "".join(rows).encode()
-    thr = (C.c_uint32 * 8)()
-    cfg.thr_apple = cfg.thr_waste = C.cast(thr, C.c_void_p)
-    cfg.n_waste_lut = 1
-    for k, v in kw.items():
-        setattr(cfg, k, v)
-    cfg._keep = thr
-    return cfg
-
-
 @pytest.mark.parametrize("T", [-1, 256, 1 << 20])
 def test_create_rejects_out_of_range_tag_timeout(lib, T):
     from homophily_marl_b200 import _capi
     h = C.c_void_p()
-    assert lib.ssd_create(C.byref(_cfg(tag_timeout=T)), C.byref(h)) == _capi.SSD_ERR_INVALID
+    assert lib.ssd_create(C.byref(ssd_config(tag_timeout=T)), C.byref(h)) == _capi.SSD_ERR_INVALID
     assert not h.value
 
 
@@ -42,4 +28,4 @@ def test_in_range_tag_timeout_passes_validation(lib):
     from homophily_marl_b200 import _capi
     h = C.c_void_p()
     for T in (0, 1, 255):                                          # reaches the CUDA calls, which fail without a device
-        assert lib.ssd_create(C.byref(_cfg(tag_timeout=T)), C.byref(h)) == _capi.SSD_ERR_CUDA
+        assert lib.ssd_create(C.byref(ssd_config(tag_timeout=T)), C.byref(h)) == _capi.SSD_ERR_CUDA

@@ -5,32 +5,17 @@ envs the step finished with the same draws, ssd_render -- are stepped from one s
 every buffer, pads included; the twin's observation, state image and ep_ret just before its reset must equal the fused env's
 episode-end buffers.  Also: the C oracle (and the tagging reference) with per-env resets on every shipped config and a
 runtime-geometry map, sentinel bytes in the slots of envs that did not finish or lie outside the range, 8 ranges on 8 streams
-with and without programmatic dependent launch, 65 536 envs, CUDA-graph capture and the checked build."""
-import os
-import subprocess
-import sys
-
+with and without programmatic dependent launch, 65 536 envs and CUDA-graph capture."""
 import numpy as np
 import pytest
 
 import lockstep
-from test_gpu_obs_index import STATE, actions, make_ref
+from harness import (BUFS, COMBOS, END_BUFS, assert_same_buffers, custom_params, env_var, make_env, make_ref, random_actions,
+                     random_draws, random_map)
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-FIRE = 7
-COMBOS = [(o, s) for o in ("rgb", "index4") for s in ("rgb", "index4")]
 SENTINEL = 0xEE
-
-
-def make_env(key, B, obs="rgb", state="rgb", color=None, T=0, seed=9, limit=7, **kw):
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    name, mp, n, view, c = lockstep.CONFIGS[key]
-    extra = dict(obs_color=color or c, random_spawn_point=True, random_spawn_rotation=None, tag_timeout=T, obs_format=obs,
-                 state_format=state)
-    return SSDBatchEnv(name, B, n, map=mp, view_size=view, episode_limit=limit, extra_args=extra, seed=seed,
-                       want_state=True, **kw)
 
 
 def stagger(env, limit):
@@ -45,13 +30,6 @@ def fill_end(env):
     env.end_ep_ret_buf.fill_(-7)
 
 
-def random_draws(rs, env):
-    B, n, G = env.B, env.n, env.G
-    u = lambda *s: rs.randint(0, 2 ** 32, size=s, dtype=np.uint64).astype(np.uint32)  # noqa: E731
-    return dict(prio=u(B, n), u_apple=u(B, G), u_waste=u(B, G), wkey=u(B, G), spawn_key=u(B, n * G),
-                rot=rs.randint(0, 4, size=(B, n)).astype(np.uint8))
-
-
 def sequence_step(env, act, draws=None):
     """The three launches the fused step must equal; returns the pre-reset obs / state / ep_ret and the done mask."""
     env.step(act, draws=draws, want_state=True)
@@ -63,8 +41,7 @@ def sequence_step(env, act, draws=None):
 
 
 def assert_twins(fused, seq, pre, done, what):
-    for k in STATE + ("obs_buf", "state_buf"):
-        assert torch.equal(getattr(fused, k), getattr(seq, k)), (what, k)
+    assert_same_buffers(fused, seq, BUFS, what)
     obs, state, ep_ret = pre
     d = done.cpu().numpy().astype(bool)
     assert np.array_equal(fused.end_obs_buf.cpu().numpy()[d], obs.cpu().numpy()[d]), (what, "end obs")
@@ -84,14 +61,14 @@ def test_fused_equals_the_three_launch_sequence(key, color, T):
     B, L = 24, 7
     resets = back_at_end = 0
     for obs, state in COMBOS:
-        fused = make_env(key, B, obs, state, color, T, limit=L, keep_episode_end=True)
-        seq = make_env(key, B, obs, state, color, T, limit=L)
+        fused = make_env(key, B, obs=obs, state=state, color=color, T=T, limit=L, keep_episode_end=True)
+        seq = make_env(key, B, obs=obs, state=state, color=color, T=T, limit=L)
         for e in (fused, seq):
             e.reset()
             stagger(e, L)
         rs = np.random.RandomState(B + T)
         for t in range(2 * L + 3):
-            act = torch.as_tensor(actions(rs, fused, T > 0), device=fused.device)
+            act = torch.as_tensor(random_actions(rs, fused, fire=0.35 if T else 0), device=fused.device)
             timers = seq.tag_out.clone()
             fill_end(fused)
             fused.obs_buf.fill_(SENTINEL)
@@ -111,8 +88,8 @@ def test_fused_equals_the_three_launch_sequence(key, color, T):
 def test_injected_draws_and_teleports(key, T):
     B, L = 6, 5
     for obs, state in COMBOS:
-        fused = make_env(key, B, obs, state, T=T, limit=L, keep_episode_end=True)
-        seq = make_env(key, B, obs, state, T=T, limit=L)
+        fused = make_env(key, B, obs=obs, state=state, T=T, limit=L, keep_episode_end=True)
+        seq = make_env(key, B, obs=obs, state=state, T=T, limit=L)
         sched = lockstep.schedule_for(key, seed=40 + T, teleport_every=3)
         rs = np.random.RandomState(T)
         d0 = random_draws(rs, fused)
@@ -121,7 +98,7 @@ def test_injected_draws_and_teleports(key, T):
             stagger(e, L)
         for t in range(3 * L):
             draws = random_draws(rs, fused)
-            act = actions(rs, fused, T > 0)
+            act = random_actions(rs, fused, fire=0.35 if T else 0)
             _, _, tele = sched.step_inputs(t)
             if tele is not None:                                # clustered agents, duplicate occupancy: collisions
                 for e in (fused, seq):
@@ -143,7 +120,7 @@ def oracle_run(env, ora, L, steps, envs=None):
     envs = np.arange(env.B) if envs is None else envs
     resets = 0
     for t in range(steps):
-        act = actions(rs, env, env.spec.tag_timeout > 0)
+        act = random_actions(rs, env, fire=0.35 if env.spec.tag_timeout else 0)
         env.end_obs_buf.fill_(SENTINEL)
         env.step(torch.as_tensor(act, device=env.device), want_state=True, auto_reset=True)
         out = ora.step(act, want_obs=True, threads=8)
@@ -177,51 +154,34 @@ def test_every_shipped_config_matches_the_oracle(key):
 
 def test_runtime_geometry_matches_the_oracle():
     """SSD_B200_GENERIC=1 (the GeoD kernels) on a shipped map, and a custom map that only the runtime geometry serves."""
-    code = ("import test_gpu_autoreset as m; m.generic_case(); print('OK')")
-    r = subprocess.run([sys.executable, "-c", "import sys; sys.path[:0] = ['tests', '.']; " + code], cwd=ROOT,
-                       env={**os.environ, "SSD_B200_GENERIC": "1"}, capture_output=True, text=True, timeout=1200)
-    assert r.returncode == 0 and "OK" in r.stdout, r.stdout[-1000:] + r.stderr[-3000:]
-    custom_map_case()
-
-
-def generic_case():
-    env = make_env("cleanup10_full", 16, limit=5, keep_episode_end=True)
-    ora = make_ref(env)
-    env.reset()
-    ora.reset()
-    assert oracle_run(env, ora, 5, 12) > 0
-
-
-def custom_map_case():
-    from homophily_marl_b200 import mapspec
     from homophily_marl_b200.batch_env import SSDBatchEnv
-    from oracle import oracle as O
-    from test_gpu_generic_geometry import random_map
+    with env_var("SSD_B200_GENERIC", "1"):
+        env = make_env("cleanup10_full", 16, limit=5, keep_episode_end=True)
     rows = random_map(np.random.RandomState(5), "harvest", 13, 15, n_spawn=9)
-    params = mapspec.EnvParams(mapspec.KIND_HARVEST, "custom", spawn_prob=(0.01, 0.1, 0.2, 0.4))
-    env = SSDBatchEnv("harvest", 16, 6, view_size=9, episode_limit=5, rows=rows, params=params, seed=3, want_state=True,
-                      extra_args=dict(random_spawn_point=True, random_spawn_rotation=None, obs_color="full"),
-                      keep_episode_end=True)
-    ora = O.OracleBatch.from_spec(env.spec, n_envs=16, seed=3, random_spawn_point=True, spawn_rotation=None)
-    env.reset()
-    ora.reset()
-    assert oracle_run(env, ora, 5, 12) > 0
+    custom = SSDBatchEnv("harvest", 16, 6, view_size=9, episode_limit=5, rows=rows, params=custom_params("harvest"), seed=3,
+                         want_state=True, extra_args=dict(random_spawn_point=True, random_spawn_rotation=None, obs_color="full"),
+                         keep_episode_end=True)
+    for e in (env, custom):
+        ora = make_ref(e)
+        e.reset()
+        ora.reset()
+        assert oracle_run(e, ora, 5, 12) > 0
 
 
-def ranges_case(pdl_expected):
+def ranges_case():
     """8 disjoint ranges on 8 streams, no host sync between steps, == one whole-batch launch.  Ranges of 23 and 40 envs start
     inside cache lines of the state arrays."""
     sizes = [23, 40, 64, 23, 40, 96, 33, 65]
     B, L = sum(sizes), 6
     starts = np.concatenate([[0], np.cumsum(sizes)[:-1]])
-    one = make_env("harvest5", B, "index4", "index4", T=2, limit=L, keep_episode_end=True)
-    grp = make_env("harvest5", B, "index4", "index4", T=2, limit=L, keep_episode_end=True)
+    one = make_env("harvest5", B, obs="index4", state="index4", T=2, limit=L, keep_episode_end=True)
+    grp = make_env("harvest5", B, obs="index4", state="index4", T=2, limit=L, keep_episode_end=True)
     for e in (one, grp):
         e.reset()
         stagger(e, L)
         fill_end(e)
     rs = np.random.RandomState(3)
-    acts = torch.as_tensor(np.stack([actions(rs, one, True) for _ in range(3 * L)]), device=one.device)
+    acts = torch.as_tensor(np.stack([random_actions(rs, one, fire=0.35) for _ in range(3 * L)]), device=one.device)
     streams = [torch.cuda.Stream() for _ in sizes]
     main = torch.cuda.current_stream()
     for g, s in enumerate(streams):
@@ -234,8 +194,7 @@ def ranges_case(pdl_expected):
     for t in range(len(acts)):
         one.step(acts[t], want_state=True, auto_reset=True)
     torch.cuda.synchronize()
-    for k in STATE + ("obs_buf", "state_buf", "end_obs_buf", "end_state_buf", "end_ep_ret_buf"):
-        assert torch.equal(getattr(one, k), getattr(grp, k)), k
+    assert_same_buffers(one, grp, BUFS + END_BUFS, "ranges")
     # a range never writes outside itself
     e = make_env("cleanup5", 64, limit=1, keep_episode_end=True)
     e.reset()
@@ -248,23 +207,20 @@ def ranges_case(pdl_expected):
         b = buf.cpu().numpy()
         assert (b[:10] == SENTINEL).all() and (b[33:] == SENTINEL).all() and not (b[10:33] == SENTINEL).all()
     assert (e.t_buf.cpu().numpy()[10:33] == 0).all()
-    return pdl_expected
 
 
 def test_ranges_on_streams_equal_one_launch_with_pdl():
-    ranges_case(True)
+    ranges_case()
 
 
 def test_ranges_on_streams_equal_one_launch_without_pdl():
-    r = subprocess.run([sys.executable, "-c", "import sys; sys.path[:0] = ['tests', '.']; import test_gpu_autoreset as m; "
-                        "m.ranges_case(False); print('OK')"], cwd=ROOT, env={**os.environ, "SSD_B200_PDL": "0"},
-                       capture_output=True, text=True, timeout=1200)
-    assert r.returncode == 0 and "OK" in r.stdout, r.stdout[-1000:] + r.stderr[-3000:]
+    with env_var("SSD_B200_PDL", "0"):
+        ranges_case()
 
 
 def test_65536_envs():
     B, L = 65536, 50
-    env = make_env("cleanup5", B, "index4", "index4", limit=L, keep_episode_end=True)
+    env = make_env("cleanup5", B, obs="index4", state="index4", limit=L, keep_episode_end=True)
     ora = make_ref(env)
     env.reset()
     ora.reset(threads=8)
@@ -273,7 +229,7 @@ def test_65536_envs():
     rs = np.random.RandomState(2)
     sample = np.sort(rs.choice(B, 48, replace=False))
     for t in range(3):
-        act = actions(rs, env, False)
+        act = random_actions(rs, env)
         env.step(torch.as_tensor(act, device=env.device), want_state=True, auto_reset=True)
         out = ora.step(act, want_obs=False, threads=8)
         done = out["done"].astype(bool)
@@ -292,13 +248,13 @@ def test_65536_envs():
 
 def test_cuda_graph_capture_equals_eager():
     B, L, K = 64, 4, 9
-    a = make_env("cleanup10_full", B, "index4", "rgb", T=2, limit=L, keep_episode_end=True)
-    b = make_env("cleanup10_full", B, "index4", "rgb", T=2, limit=L, keep_episode_end=True)
+    a = make_env("cleanup10_full", B, obs="index4", T=2, limit=L, keep_episode_end=True)
+    b = make_env("cleanup10_full", B, obs="index4", T=2, limit=L, keep_episode_end=True)
     for e in (a, b):
         e.reset()
         stagger(e, L)
     rs = np.random.RandomState(0)
-    acts = torch.as_tensor(np.stack([actions(rs, a, True) for _ in range(K)]), device=a.device)
+    acts = torch.as_tensor(np.stack([random_actions(rs, a, fire=0.35) for _ in range(K)]), device=a.device)
     before = a.launch_count
     for t in range(K):
         a.step(acts[t], want_state=True, auto_reset=True)
@@ -312,12 +268,11 @@ def test_cuda_graph_capture_equals_eager():
     torch.cuda.synchronize()
     graph.replay()
     torch.cuda.synchronize()
-    for k in STATE + ("obs_buf", "state_buf", "end_obs_buf", "end_state_buf", "end_ep_ret_buf"):
-        assert torch.equal(getattr(a, k), getattr(b, k)), k
+    assert_same_buffers(a, b, BUFS + END_BUFS, "graph")
 
 
 def test_format_switch_reallocates_the_episode_end_buffers():
-    e = make_env("harvest5", 8, keep_episode_end=True)
+    e = make_env("harvest5", 8, limit=7, keep_episode_end=True)
     assert e.end_obs_buf.shape == e.obs_buf.shape and e.end_state_buf.shape == e.state_buf.shape
     assert e.end_ep_ret.shape == (8, e.n) and e.end_ep_ret.dtype == torch.int32
     e.set_obs_format("index4")
@@ -330,17 +285,5 @@ def test_format_switch_reallocates_the_episode_end_buffers():
     assert e.done.all()
     end = e.state_float(buf=e.end_state_buf)
     assert end.shape == (8, 3, e.H, e.W) and not torch.equal(end, e.state_float())   # the last state, not the new episode's
-    f = make_env("harvest5", 8, keep_episode_end=False)
+    f = make_env("harvest5", 8, limit=7, keep_episode_end=False)
     assert f.end_obs_buf is None and f.end_state_buf is None and f.end_ep_ret is None
-
-
-def test_checked_build_sees_no_shared_memory_violation():
-    from homophily_marl_b200 import _build
-    _build.build_checked()
-    code = ("import test_gpu_autoreset as m; "
-            "[m.test_fused_equals_the_three_launch_sequence(k, c, T) for k in ('cleanup5', 'harvest5', 'harvest10_full') "
-            " for c in ('simplified', 'full') for T in (0, 3)]; m.generic_case(); m.custom_map_case(); "
-            "from homophily_marl_b200 import _capi; print('OOB', _capi.load().ssd_debug_oob_count())")
-    r = subprocess.run([sys.executable, "-c", "import sys; sys.path[:0] = ['tests', '.']; " + code], cwd=ROOT,
-                       env={**os.environ, "SSD_B200_CHECKED": "1"}, capture_output=True, text=True, timeout=2400)
-    assert r.returncode == 0 and "OOB 0" in r.stdout, r.stdout[-1000:] + r.stderr[-3000:]

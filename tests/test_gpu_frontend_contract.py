@@ -11,60 +11,19 @@ tf32 (a kernel that lost its lo terms) miss that bound by at least 10x, so the b
 its measured error as ``frontend-err <case> V=<v> err=<e> tol=<t> hi_only=<h>``.
 """
 import ctypes as C
-import types
 
 import numpy as np
 import pytest
 
 import frontend_ref as R
+from harness import DEV, _auto_grid, _expect, _front_end, _weights, action_tables, feature_mac, make_runner
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
-DEV = "cuda:0"
-
-
-def _weights(view, seed, conv_scale=1.0, fc_scale=1.0):
-    """conv_w, conv_b, fc_w, fc_b as float32 numpy arrays (PyTorch's default init of the reference module)."""
-    torch.manual_seed(seed)
-    P = 2 * view - 1
-    conv, fc = torch.nn.Conv2d(3, 6, 3, 1), torch.nn.Linear(6 * P * P, 32)
-    w = [t.detach().numpy().astype(np.float32).copy() for t in (conv.weight, conv.bias, fc.weight, fc.bias)]
-    w[0] *= np.float32(conv_scale)
-    w[2] *= np.float32(fc_scale)
-    return w
-
-
-def _front_end(w, view, slope=0.01):
-    from homophily_marl_b200.frontend import ObsFrontEnd
-    return ObsFrontEnd(*w, view, negative_slope=slope, device=DEV)
-
 
 def _random_buf(n, seed):
     return np.random.RandomState(seed).randint(0, 256, size=n).astype(np.uint8)
-
-
-def _expect(case, view, got, host, rows, lay, w, slope, hi_check=True, scale="y"):
-    """Asserts the bound on `got` (numpy [rows, 32]) and, with hi_check, that the hi-only FC misses it by >= 10x.
-
-    scale="M" measures the error against 1 + M, M = |fc_b| + sum |W||a| the condition scale of the FC sum, instead of
-    1 + |y|: with trained-like weights the sum cancels (M / (1 + |y|) reaches ~1 000 at 16x the default init) and no fp32
-    contraction meets the 1 + |y| form there -- torch's own fp32 matmul of the exact activations measures 2.2e-5."""
-    slope = float(np.float32(slope))                          # the kernel's slope is the float32 one
-    y, M = R.forward64(host, rows, lay["AS"], lay["PS"], lay["RP"], view, *w, slope)
-    tol = R.tolerance(view)
-
-    def rel(v):
-        return float((np.abs(np.asarray(v, np.float64) - y) / (1 + (M if scale == "M" else np.abs(y)))).max()) if y.size else 0.0
-    err = rel(got)
-    herr = rel(R.forward64_hi_only(host, rows, lay["AS"], lay["PS"], lay["RP"], view, *w, slope)) if hi_check else float("nan")
-    print(f"frontend-err {case} V={view} err={err:.3e} tol={tol:.2e} hi_only={herr:.3e}"
-          + (f" scale=1+M (vs 1+|y|: {R.rel_err(got, y):.3e})" if scale == "M" else ""))
-    assert np.isfinite(got).all(), case
-    assert err <= tol, (case, view, err, tol)
-    if hi_check:
-        assert herr >= 10 * tol, (case, view, herr, tol)
-    return y
 
 
 def _run(fe, host, rows, lay, offset=0, out=None):
@@ -81,24 +40,6 @@ def _used_bytes(size, rows, lay, view):
     used = np.zeros(size, dtype=bool)
     used[(r * lay["AS"] + c * lay["PS"] + y * lay["RP"] + x).ravel()] = True
     return used
-
-
-def _auto_grid(view, rows):
-    """The grid ssd_frontend_forward picks without SSD_B200_FRONTEND_GRID (restated), and the number of (tile, chunk) units."""
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    P = 2 * view - 1
-    n_chunks, tiles = P * ((P + 15) // 16), -(-rows // 128)
-    units = tiles * n_chunks
-    grid = min(units, sms)
-    share = units / grid
-    best = share + 1.5 * (2.0 if share < n_chunks else float(int(share / n_chunks) + 2))
-    for s in range(1, n_chunks + 1):
-        if tiles * s > sms:
-            break
-        cost = (n_chunks + s - 1) // s + 1.5
-        if cost < best - 1e-9:
-            best, grid = cost, tiles * s
-    return grid, units
 
 
 # ---------------------------------------------------------------------------------------------------- numeric contract
@@ -383,48 +324,16 @@ def test_two_handles_on_two_streams_without_a_host_sync():
 
 def test_batched_runner_ranges_each_use_their_own_handle(monkeypatch):
     """env_groups = 4 with the fused front end: every range's features equal fp64 on exactly the rows the runner stored."""
-    from homophily_marl_b200.batched_runner import BatchedEpisodeRunner
     from homophily_marl_b200.frontend import MacFrontEnd, ObsFrontEnd
-    from test_batched_runner import FakeBatch, _scheme
     B, T, n, view, G = 128, 20, 3, 7, 4
     N = 2 * view + 1
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, disable_rotation_action=False,
-                 disable_fire_action=False, obs_color="full")
-    env_args = dict(num_agents=n, render=False, episode_limit=T, is_replay=False, view_size=view, map="default3", extra_args=extra, seed=5)
-    args = types.SimpleNamespace(batch_size_run=B, env="cleanup", env_args=env_args, device=DEV, name="homophily", mac="homophily_mac",
-                                 n_actions=None, ind_reward=True, runner_log_interval=10 ** 9, test_nepisode=B, env_groups=G)
-    runner = BatchedEpisodeRunner(args, types.SimpleNamespace(log_stat=lambda k, v, t: None))
-    info = runner.get_env_info()
-    A = args.n_actions = info["n_actions"]
-    g = torch.Generator().manual_seed(3)
-    table = torch.randint(0, A, (B, T + 1, n, 1), generator=g).to(DEV)
-    table_inc = torch.randint(0, 3, (B, T + 1, n, n, 1), generator=g).to(DEV)
-    runner.use_batch_factory(lambda: FakeBatch(_scheme(n, A, *info["state_dims"], N), B, T + 1, DEV))
+    runner = make_runner(n=n, view=view, B=B, T=T, groups=G, seed=5, extra=dict(obs_color="full"))
+    table, table_inc = action_tables(runner, 3)
 
     torch.manual_seed(19)
     P = 2 * view - 1
     module = torch.nn.Sequential(torch.nn.Conv2d(3, 6, 3, 1), torch.nn.LeakyReLU(), torch.nn.Flatten(),
                                  torch.nn.Linear(6 * P * P, 32), torch.nn.LeakyReLU()).to(DEV)
-
-    class Agent:
-        conv_to_fc = module
-
-        def rgb_preprocess(self, x):
-            return module(x)
-
-    class MAC:                                                # scripted actions; the features go through rgb_preprocess
-        agent = Agent()
-
-        def init_hidden(self, batch_size):
-            pass
-
-        def select_actions_env(self, batch, t_ep, t_env, test_mode=False):
-            feats = self.agent.rgb_preprocess(batch["obs"][:, t_ep].reshape(-1, 3, N, N))
-            assert feats.shape == (batch.batch_size * n, 32)
-            return table[batch.offset:batch.offset + batch.batch_size, t_ep].clone()
-
-        def select_actions_inc(self, actions, batch, t_ep, t_env, test_mode=False, agent_pos_replay=None):
-            return table_inc[batch.offset:batch.offset + batch.batch_size, t_ep].clone()
 
     records = []
     forward = ObsFrontEnd.forward
@@ -435,7 +344,7 @@ def test_batched_runner_ranges_each_use_their_own_handle(monkeypatch):
         return got                                            # the clones run on the current (the range's) stream
 
     monkeypatch.setattr(ObsFrontEnd, "forward", recording)
-    runner.mac = MAC()
+    runner.mac = feature_mac(module, N, n, table, table_inc)
     runner.front = MacFrontEnd(runner.mac, runner.env)
     batch = runner.run(test_mode=True)
     torch.cuda.synchronize()

@@ -6,19 +6,17 @@ same views: every check here is ``torch.equal`` against that, except the fp64 co
 15 and 31 so that the identity cannot hide a bug both paths share.
 """
 import ctypes as C
-import types
 
 import numpy as np
 import pytest
 
 import frontend_ref as R
+from harness import DEV, _auto_grid, _cfg, _expect, _front_end, _weights, action_tables, feature_mac, make_runner
 from obs_index_ref import obs_layout, pack, rgb_of
-from test_gpu_frontend_contract import _auto_grid, _expect, _front_end, _weights
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
-DEV = "cuda:0"
 ROWS = 3 * 128 + 5                                            # a partial last tile
 
 
@@ -356,49 +354,15 @@ def test_two_handles_on_two_streams_without_a_host_sync():
 
 # ---------------------------------------------------------------------------------------------------- batched runner
 
-def _index4_runner(fused, obs_format="index4", B=128, T=20, G=4):
-    from homophily_marl_b200.batched_runner import BatchedEpisodeRunner
-    n, view = 3, 7
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, disable_rotation_action=False,
-                 disable_fire_action=False, obs_color="full", tag_timeout=2, obs_format=obs_format)
-    env_args = dict(num_agents=n, render=False, episode_limit=T, is_replay=False, view_size=view, map="default3", extra_args=extra, seed=5)
-    args = types.SimpleNamespace(batch_size_run=B, env="cleanup", env_args=env_args, device=DEV, name="homophily", mac="homophily_mac",
-                                 n_actions=None, ind_reward=True, runner_log_interval=10 ** 9, test_nepisode=B, env_groups=G,
-                                 fused_frontend=fused, rgb_input=True)
-    return BatchedEpisodeRunner(args, types.SimpleNamespace(log_stat=lambda k, v, t: None))
-
-
-def _mac(module, N, n, table, table_inc):
-    class Agent:
-        conv_to_fc = module
-
-        def rgb_preprocess(self, x):
-            return module(x)
-
-    class MAC:                                                # scripted actions; the features go through rgb_preprocess
-        agent = Agent()
-
-        def init_hidden(self, batch_size):
-            pass
-
-        def select_actions_env(self, batch, t_ep, t_env, test_mode=False):
-            feats = self.agent.rgb_preprocess(batch["obs"][:, t_ep].reshape(-1, 3, N, N))
-            assert feats.shape == (batch.batch_size * n, 32)
-            return table[batch.offset:batch.offset + batch.batch_size, t_ep].clone()
-
-        def select_actions_inc(self, actions, batch, t_ep, t_env, test_mode=False, agent_pos_replay=None):
-            return table_inc[batch.offset:batch.offset + batch.batch_size, t_ep].clone()
-    return MAC()
-
-
 def test_batched_runner_setup_selects_the_front_end_by_format():
     from homophily_marl_b200.frontend import MacFrontEnd
     torch.manual_seed(0)
     module = torch.nn.Sequential(torch.nn.Conv2d(3, 6, 3, 1), torch.nn.LeakyReLU(), torch.nn.Flatten(),
                                  torch.nn.Linear(6 * 13 * 13, 32), torch.nn.LeakyReLU()).to(DEV)
-    mac = _mac(module, 15, 3, None, None)
+    mac = feature_mac(module, 15, 3, None, None)
     factory = dict(batch_cls=lambda *a, **k: None)
-    runner = _index4_runner("index4", B=8, G=1)
+    runner = make_runner(B=8, T=20, seed=5, extra=dict(obs_color="full", tag_timeout=2, obs_format="index4"),
+                         fused_frontend="index4", rgb_input=True)
     runner.setup(None, None, None, mac, **factory)
     assert isinstance(runner.front, MacFrontEnd) and runner.front.obs_format == "index4"
     runner.front.detach()
@@ -407,7 +371,8 @@ def test_batched_runner_setup_selects_the_front_end_by_format():
         with pytest.raises(ValueError):
             runner.setup(None, None, None, mac, **factory)
     runner.close_env()
-    rgb = _index4_runner("index4", obs_format="rgb", B=8, G=1)
+    rgb = make_runner(B=8, T=20, seed=5, extra=dict(obs_color="full", tag_timeout=2, obs_format="rgb"),
+                      fused_frontend="index4", rgb_input=True)
     with pytest.raises(ValueError, match="index4"):
         rgb.setup(None, None, None, mac, **factory)
     rgb.args.fused_frontend = True
@@ -421,16 +386,11 @@ def test_batched_runner_ranges_read_index4_bit_identical_to_rgb(monkeypatch):
     """env_groups = 4, index4 env, fused front end on index4: each fused call equals, bit for bit, the RGB front end (same
     handle) on the fp32 observations the runner stored for that step."""
     from homophily_marl_b200.frontend import MacFrontEnd, ObsFrontEnd
-    from test_batched_runner import FakeBatch, _scheme
     B, T, n, view, G = 128, 20, 3, 7, 4
     N = 2 * view + 1
-    runner = _index4_runner("index4", B=B, T=T, G=G)
-    info = runner.get_env_info()
-    A = runner.args.n_actions = info["n_actions"]
-    g = torch.Generator().manual_seed(3)
-    table = torch.randint(0, A, (B, T + 1, n, 1), generator=g).to(DEV)
-    table_inc = torch.randint(0, 3, (B, T + 1, n, n, 1), generator=g).to(DEV)
-    runner.use_batch_factory(lambda: FakeBatch(_scheme(n, A, *info["state_dims"], N), B, T + 1, DEV))
+    runner = make_runner(n=n, view=view, B=B, T=T, groups=G, seed=5, extra=dict(obs_color="full", tag_timeout=2, obs_format="index4"),
+                         fused_frontend="index4", rgb_input=True)
+    table, table_inc = action_tables(runner, 3)
     torch.manual_seed(19)
     P = 2 * view - 1
     module = torch.nn.Sequential(torch.nn.Conv2d(3, 6, 3, 1), torch.nn.LeakyReLU(), torch.nn.Flatten(),
@@ -444,7 +404,7 @@ def test_batched_runner_ranges_read_index4_bit_identical_to_rgb(monkeypatch):
         return got
 
     monkeypatch.setattr(ObsFrontEnd, "forward_index4", recording)
-    runner.mac = _mac(module, N, n, table, table_inc)
+    runner.mac = feature_mac(module, N, n, table, table_inc)
     runner.front = MacFrontEnd(runner.mac, runner.env, obs_format="index4")
     batch = runner.run(test_mode=True)
     torch.cuda.synchronize()
@@ -474,7 +434,6 @@ def test_refloop_components_with_index4_and_the_fused_front_end():
     from baseline import refloop
     if not refloop.available():
         pytest.skip("reference sources absent (baseline/_ref)")
-    from test_train_loop import _cfg
     B = 128
     env_args = dict(num_agents=3, map="default3", episode_limit=20, extra_args=dict(obs_format="index4"))
     cfg = _cfg(runner="batched", batch_size_run=B, buffer_size=2 * B, batch_size=8, buffer_cpu_only=False, fused_frontend="index4",

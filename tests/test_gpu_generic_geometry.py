@@ -1,29 +1,17 @@
 """GPU suite: geometries outside the compile-time specialisations -- custom ASCII maps, odd view sizes (generic row
 pitch, non-zero agent-block tail), up to 16 agents, tiny and near-maximum maps -- against the oracle, Philox mode."""
+import os
+import runpy
+
 import numpy as np
 import pytest
 
+from harness import custom_params, random_map
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
-
-
-def random_map(rs, kind, H, W, n_spawn):
-    """Wall-enclosed random map in the reference alphabet with at least n_spawn 'P' cells."""
-    g = np.full((H, W), " ", dtype="<U1")
-    g[0, :] = g[-1, :] = "@"
-    g[:, 0] = g[:, -1] = "@"
-    inner = [(r, c) for r in range(1, H - 1) for c in range(1, W - 1)]
-    rs.shuffle(inner)
-    it = iter(inner)
-    for _ in range(n_spawn):
-        r, c = next(it)
-        g[r, c] = "P"
-    alphabet = ("B", "H", "R", "S", "@", " ", " ") if kind == "cleanup" else ("A", "A", "@", " ", " ", " ")
-    for r, c in it:
-        g[r, c] = alphabet[rs.randint(len(alphabet))]
-    return ["".join(row) for row in g]
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 CASES = [  # kind, H, W, n_agents, view
@@ -35,14 +23,10 @@ CASES = [  # kind, H, W, n_agents, view
 
 @pytest.mark.parametrize("kind,H,W,n,view", CASES)
 def test_generic_geometry_matches_oracle(kind, H, W, n, view):
-    from homophily_marl_b200 import mapspec
     from homophily_marl_b200.batch_env import SSDBatchEnv
     rs = np.random.RandomState(H * 1000 + W * 10 + n)
     rows = random_map(rs, kind, H, W, n_spawn=min(32, n + 3))
-    if kind == "cleanup":
-        params = mapspec.EnvParams(mapspec.KIND_CLEANUP, "custom", 0.7, 0.1, 0.4, 0.25)
-    else:
-        params = mapspec.EnvParams(mapspec.KIND_HARVEST, "custom", spawn_prob=(0.01, 0.1, 0.2, 0.4))
+    params = custom_params(kind)
     B, T = 24, 30
     color = "full" if (H + W) % 2 else "simplified"
     env = SSDBatchEnv(kind, B, n, view_size=view, episode_limit=11, rows=rows, params=params, seed=42, env_gid_base=7,
@@ -95,19 +79,10 @@ def test_maximum_map_size_and_rejects():
     assert ei.value.code == _capi.SSD_ERR_MAP
 
 
-def test_checked_build_sees_no_shared_memory_violation():
-    """compute-sanitizer is closed on the GPU pool, so the library has its own checked variant (-DSSD_BOUNDS_CHECK):
-    every data-dependent shared-memory index is tested against its tile.  Runs the all-paths workload in a subprocess."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = ("import runpy, sys; sys.argv=['x']; runpy.run_path(%r, run_name='__main__'); "
-            "from homophily_marl_b200 import _capi; n = _capi.load().ssd_debug_oob_count(); print('OOB', n); assert n == 0, n"
-            % os.path.join(root, "profiles", "sanitizer_case.py"))
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env={**os.environ, "SSD_B200_CHECKED": "1"},
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "OOB 0" in r.stdout, r.stdout[-500:] + r.stderr[-1500:]
+def test_all_paths_workload():
+    """profiles/sanitizer_case.py: both envs, both colour schemes, every kernel mode, the specialised and the runtime geometry,
+    injected draws.  tests/test_gpu_checked_build.py runs it on the checked build."""
+    runpy.run_path(os.path.join(ROOT, "profiles", "sanitizer_case.py"), run_name="__main__")
 
 
 @pytest.mark.parametrize("B,n", [(1, 1), (3, 1), (5, 2), (4097, 5)])

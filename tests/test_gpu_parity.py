@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import lockstep as ls
+from harness import assert_outputs_match_oracle, assert_state_matches_oracle, make_env, make_ref
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -15,39 +16,6 @@ torch = pytest.importorskip("torch")
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 KEYS = sorted(ls.CONFIGS)
-
-
-def _make_pair(key, B, episode_limit, seed=5, random_spawn=True, gid0=0, **kw):
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    name, map_name, n, view, color = ls.CONFIGS[key]
-    extra = dict(obs_color=color)
-    if random_spawn:
-        extra.update(random_spawn_point=True, random_spawn_rotation=None)
-    env = SSDBatchEnv(name, B, n, map=map_name, view_size=view, episode_limit=episode_limit, extra_args=extra,
-                      seed=seed, env_gid_base=gid0, want_state=True, **kw)
-    ora = O.OracleBatch.from_spec(env.spec, n_envs=B, seed=seed, env_gid0=gid0, random_spawn_point=random_spawn,
-                                  spawn_rotation=None if random_spawn else 0)
-    return env, ora
-
-
-def _assert_state_equal(env, ora, what):
-    assert np.array_equal(env.grid.cpu().numpy(), ora.grid), f"{what}: grid"
-    assert np.array_equal(env.agent_pos.cpu().numpy(), ora.pos_rc), f"{what}: pos"
-    assert np.array_equal(env.agent_orient.cpu().numpy(), ora.orient), f"{what}: orient"
-    assert np.array_equal(env.ep_ret.cpu().numpy(), ora.ep_ret), f"{what}: ep_ret"
-    assert np.array_equal(env.t_buf.cpu().numpy(), ora.envs["t"]), f"{what}: t"
-
-
-def _assert_out_equal(env, out, what):
-    assert np.array_equal(env.reward.cpu().numpy(), out["reward"]), f"{what}: reward"
-    assert np.array_equal(env.clean.cpu().numpy(), out["clean"]), f"{what}: clean"
-    assert np.array_equal(env.apple_cnt.cpu().numpy().view(np.uint16), out["apple_cnt"]), f"{what}: apple_cnt"
-    assert np.array_equal(env.done.cpu().numpy(), out["done"]), f"{what}: done"
-    if out.get("obs") is not None:
-        got = env.obs_view().cpu().numpy()
-        if not np.array_equal(got, out["obs"]):
-            bad = np.argwhere(got != out["obs"])
-            raise AssertionError(f"{what}: obs mismatch at {bad[0].tolist()} ({len(bad)} bytes)")
 
 
 @pytest.mark.parametrize("key", KEYS)
@@ -73,11 +41,12 @@ def test_cuda_matches_oracle_lockstep_injected(key):
 def test_cuda_matches_oracle_philox_batched(key):
     """B envs, on-device Philox draws, episode resets, clustered restarts every 8 steps."""
     B, limit, T = 192, 25, 70
-    env, ora = _make_pair(key, B, limit, seed=1234, gid0=1000)
+    env = make_env(key, B, limit=limit, seed=1234, env_gid_base=1000)
+    ora = make_ref(env)
     rs = np.random.RandomState(99)
     env.reset()
     ora.reset(threads=4)
-    _assert_state_equal(env, ora, "reset")
+    assert_state_matches_oracle(env, ora, "reset")
     assert np.array_equal(env.obs_view().cpu().numpy(), np.stack([ora.obs_one(b) for b in range(B)]))
     for t in range(T):
         if t % 8 == 3:
@@ -90,21 +59,22 @@ def test_cuda_matches_oracle_philox_batched(key):
             act[:, : env.n // 2 + 1] = rs.randint(0, 4, size=(B, env.n // 2 + 1))
         env.step(torch.as_tensor(act, device=env.device), want_state=True)
         out = ora.step(act, threads=4)
-        _assert_out_equal(env, out, f"{key} t={t}")
-        _assert_state_equal(env, ora, f"{key} t={t}")
+        assert_outputs_match_oracle(env, out, f"{key} t={t}")
+        assert_state_matches_oracle(env, ora, f"{key} t={t}")
         assert np.array_equal(env.state_rgb.cpu().numpy(), np.stack([ora.state_one(b) for b in range(B)]))
         if out["done"].any():
             assert out["done"].all()
             env.reset()
             ora.reset(threads=4)
-            _assert_state_equal(env, ora, f"{key} reset@{t}")
+            assert_state_matches_oracle(env, ora, f"{key} reset@{t}")
     assert int(ora.envs["error"].sum()) == 0
 
 
 def test_full_size_harvest_4096_vs_oracle_and_invariants():
     """BASELINE configs[1]: Harvest default5, 5 agents, 4096 envs (yaml-default extra_args)."""
     B, T = 4096, 30
-    env, ora = _make_pair("harvest5", B, 100, seed=3, random_spawn=False)
+    env = make_env("harvest5", B, limit=100, seed=3, random_spawn=False)
+    ora = make_ref(env)
     env.reset()
     ora.reset(threads=8)
     rs = np.random.RandomState(1)
@@ -112,8 +82,8 @@ def test_full_size_harvest_4096_vs_oracle_and_invariants():
         act = rs.randint(0, env.n_actions, size=(B, env.n)).astype(np.uint8)
         env.step(torch.as_tensor(act, device=env.device))
         out = ora.step(act, threads=8)
-        _assert_out_equal(env, out, f"t={t}")
-    _assert_state_equal(env, ora, "final")
+        assert_outputs_match_oracle(env, out, f"t={t}")
+    assert_state_matches_oracle(env, ora, "final")
     grid = env.grid.cpu().numpy()
     assert np.array_equal((grid == 2).reshape(B, -1).sum(1), env.apple_cnt.cpu().numpy().view(np.uint16))
     pos = env.agent_pos.cpu().numpy()
@@ -144,7 +114,8 @@ def test_cleanup10_16384_sharded_matches_single():
 
 
 def test_step_host_equals_device_step():
-    env, ora = _make_pair("cleanup5", 64, 100, seed=21)
+    env = make_env("cleanup5", 64, limit=100, seed=21)
+    ora = make_ref(env)
     env.reset()
     ora.reset()
     io = env.make_host_io(with_obs=True)
@@ -164,7 +135,7 @@ def test_step_host_equals_device_step():
 
 
 def test_reset_mask_only_touches_selected_envs():
-    env, ora = _make_pair("cleanup3", 32, 100, seed=4)
+    env = make_env("cleanup3", 32, limit=100, seed=4)
     env.reset()
     rs = np.random.RandomState(8)
     for t in range(12):
@@ -182,7 +153,8 @@ def test_reset_mask_only_touches_selected_envs():
 
 
 def test_obs_padding_bytes_stay_zero_and_ring_buffers_work():
-    env, ora = _make_pair("harvest10_n5", 16, 100, seed=6)
+    env = make_env("harvest10_n5", 16, limit=100, seed=6)
+    ora = make_ref(env)
     ring = [env.new_obs_buffer() for _ in range(3)]
     env.reset(obs_out=ring[0])
     ora.reset()
@@ -220,7 +192,7 @@ def test_hit_penalty_and_fire_cost_parameters():
         act = rs.choice([0, 1, 2, 3, 4, 7, 7, 7], size=(B, 10)).astype(np.uint8)
         env.step(torch.as_tensor(act, device=env.device))
         out = ora.step(act)
-        _assert_out_equal(env, out, f"t={t}")
+        assert_outputs_match_oracle(env, out, f"t={t}")
         hits += int((out["reward"] <= -5).sum())
     assert hits > 0
 
@@ -261,7 +233,8 @@ def test_incentive_bookkeeping_matches_torch():
 def test_env_on_second_device_leaves_current_device_alone():
     """The C ABI makes the handle's device current only for the duration of a call (one process may hold several)."""
     assert torch.cuda.current_device() == 0
-    env1, ora = _make_pair("cleanup5", 32, 50, seed=8)
+    env1 = make_env("cleanup5", 32, limit=50, seed=8)
+    ora = make_ref(env1)
     from homophily_marl_b200.batch_env import SSDBatchEnv
     env2 = SSDBatchEnv("cleanup", 32, 5, map="default5", view_size=7, episode_limit=50, seed=8, device="cuda:1",
                        extra_args=dict(random_spawn_point=True, random_spawn_rotation=None))
@@ -322,7 +295,8 @@ def test_full_size_harvest_65536_properties_and_sampled_oracle():
 def test_full_size_cleanup10_16384_vs_oracle():
     """BASELINE configs[2] on one GPU: Cleanup default10, 10 agents, 16384 envs, a few steps against the oracle."""
     B = 16384
-    env, ora = _make_pair("cleanup10", B, 100, seed=23)
+    env = make_env("cleanup10", B, limit=100, seed=23)
+    ora = make_ref(env)
     env.reset()
     ora.reset(threads=8)
     rs = np.random.RandomState(6)
@@ -331,13 +305,14 @@ def test_full_size_cleanup10_16384_vs_oracle():
         act[:, :4] = 8 if t % 2 else act[:, :4]                    # plenty of CLEAN beams so that spawning switches on
         env.step(torch.as_tensor(act, device=env.device))
         out = ora.step(act, threads=8)
-        _assert_out_equal(env, out, f"t={t}")
-    _assert_state_equal(env, ora, "final")
+        assert_outputs_match_oracle(env, out, f"t={t}")
+    assert_state_matches_oracle(env, ora, "final")
 
 
 def test_single_env_1000_steps_like_baseline_config0():
     """BASELINE configs[0] shape: Cleanup default5, 5 agents, ONE env, 1000 random-action steps in a single episode."""
-    env, ora = _make_pair("cleanup5", 1, 1000, seed=0, random_spawn=False)
+    env = make_env("cleanup5", 1, limit=1000, seed=0, random_spawn=False)
+    ora = make_ref(env)
     env.reset()
     ora.reset()
     rs = np.random.RandomState(123)
@@ -348,8 +323,8 @@ def test_single_env_1000_steps_like_baseline_config0():
         env.step(dev_acts[t])
         out = ora.step(acts[t])
         if t % 50 == 49 or t == 999:
-            _assert_out_equal(env, out, f"t={t}")
-            _assert_state_equal(env, ora, f"t={t}")
+            assert_outputs_match_oracle(env, out, f"t={t}")
+            assert_state_matches_oracle(env, ora, f"t={t}")
         obs_sum += int(out["obs"].sum())
     assert bool(env.done[0].item()) and obs_sum > 0
     assert np.array_equal(env.ep_ret.cpu().numpy(), ora.ep_ret)

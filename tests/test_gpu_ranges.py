@@ -3,6 +3,7 @@
 import numpy as np
 import pytest
 
+from harness import custom_params, random_map
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -52,11 +53,9 @@ def test_groups_on_streams_equal_one_batch(name, mp, n, view, groups, per):
 def test_interleaved_generic_handles_of_different_sizes():
     """Two runtime-geometry handles share ONE kernel instantiation; the larger one must keep working after the smaller one
     made its first launch (cudaFuncAttributeMaxDynamicSharedMemorySize is per function, only ever raised)."""
-    from homophily_marl_b200 import mapspec
     from homophily_marl_b200.batch_env import SSDBatchEnv
-    from test_gpu_generic_geometry import random_map
     rs = np.random.RandomState(3)
-    params = mapspec.EnvParams(mapspec.KIND_HARVEST, "custom", spawn_prob=(0.01, 0.1, 0.2, 0.4))
+    params = custom_params("harvest")
     big = SSDBatchEnv("harvest", 8, 4, view_size=31, episode_limit=50, rows=random_map(rs, "harvest", 32, 64, 6), params=params, seed=1)
     small = SSDBatchEnv("harvest", 8, 2, view_size=3, episode_limit=50, rows=random_map(rs, "harvest", 6, 7, 4), params=params, seed=2)
     ob = O.OracleBatch.from_spec(big.spec, n_envs=8, seed=1)

@@ -4,34 +4,19 @@ Four envs -- RGB and index4 observations, each with an RGB and an index4 state i
 In every shipped configuration, both colour schemes, with and without tagging-out timers, with injected draws and teleports:
 ``lut[unpack(state)]`` is the RGB state image byte for byte, the packed bytes (pads included, buffers pre-filled with 0xFF)
 equal the NumPy restatement (tests/state_index_ref.py) of the reference's state, and ``state_float`` equals
-``state_rgb.float() / 256``.  Also covered: ssd_render, env ranges on streams, 65 536 envs, the runtime geometry, the checked
-build, ``step_host``, switching formats, ``auto_reset`` and the batched runner's ``batch["state"]``."""
-import os
-import subprocess
-import sys
-import types
-
+``state_rgb.float() / 256``.  Also covered: ssd_render, env ranges on streams, 65 536 envs, the runtime geometry, ``step_host``,
+switching formats, ``auto_reset`` and the batched runner's ``batch["state"]``."""
 import numpy as np
 import pytest
 
+import harness
 import lockstep
+from harness import (COMBOS, FIRE, STATE, ScriptedMAC, action_tables, assert_same_buffers, env_var, make_custom_env, make_env,
+                     make_ref, make_runner, random_actions)
 from state_index_ref import index_state, ora_state, pack, rgb_of, state_layout, unpack
-from test_gpu_obs_index import STATE, actions, make_ref
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-FIRE = 7
-COMBOS = [(o, s) for o in ("rgb", "index4") for s in ("rgb", "index4")]     # (obs_format, state_format)
-
-
-def make_env(key, B, obs, state, color=None, T=0, seed=9, episode_limit=1000, **kw):
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    name, mp, n, view, c = lockstep.CONFIGS[key]
-    extra = dict(obs_color=color or c, random_spawn_point=True, random_spawn_rotation=None, tag_timeout=T, obs_format=obs,
-                 state_format=state)
-    return SSDBatchEnv(name, B, n, map=mp, view_size=view, episode_limit=episode_limit, extra_args=extra, seed=seed,
-                       want_state=True, **kw)
 
 
 def ref_state(env, ora, envs=None):
@@ -51,8 +36,7 @@ def check_quad(envs, what, ora=None, with_float=True):
     """envs: {(obs, state): env} stepped with the same inputs; index4 state buffers were pre-filled with 0xFF."""
     base = envs[("rgb", "rgb")]
     for e in envs.values():
-        for k in STATE:
-            assert torch.equal(getattr(base, k), getattr(e, k)), (what, k)
+        assert_same_buffers(base, e, STATE, what)
     for obs in ("rgb", "index4"):
         a, b = envs[(obs, "rgb")], envs[(obs, "index4")]
         assert b.state_rgb is None and b.state_buf.shape == (b.B, b.state_layout.env_stride)
@@ -72,11 +56,11 @@ def fill_state(envs):
             e.state_buf.fill_(0xFF)
 
 
-def run_lockstep(make, B=32, steps=40, seed=9):
+def run_lockstep(make, B=32, steps=40):
     """Four envs and the reference, all from one seed, Philox draws."""
     envs = {c: make(*c) for c in COMBOS}
     any_env = envs[("rgb", "index4")]
-    ora = make_ref(any_env, seed=seed)
+    ora = make_ref(any_env)
     for e in envs.values():
         e.reset()
     ora.reset()
@@ -87,7 +71,7 @@ def run_lockstep(make, B=32, steps=40, seed=9):
     rs = np.random.RandomState(B + steps)
     tagged = 0
     for t in range(steps):
-        act = actions(rs, any_env, any_env.spec.tag_timeout > 0)
+        act = random_actions(rs, any_env, fire=0.35 if any_env.spec.tag_timeout else 0)
         at = torch.as_tensor(act, device=any_env.device)
         fill_state(envs)
         for e in envs.values():
@@ -111,7 +95,7 @@ def run_lockstep(make, B=32, steps=40, seed=9):
 @pytest.mark.parametrize("color", ["simplified", "full"])
 @pytest.mark.parametrize("key", sorted(lockstep.CONFIGS))
 def test_every_config_matches_reference(key, color, T):
-    tagged = run_lockstep(lambda o, s: make_env(key, 32, o, s, color=color, T=T))
+    tagged = run_lockstep(lambda o, s: make_env(key, 32, obs=o, state=s, color=color, T=T))
     assert T == 0 or tagged > 0
 
 
@@ -119,10 +103,9 @@ def test_every_config_matches_reference(key, color, T):
                                    ("harvest10_n5", 2), ("cleanup3", 0)])
 def test_injected_draws_and_teleports(key, T):
     """One env, every draw injected, teleports (duplicate occupancy included) every 7 steps."""
-    from tag_oracle import TagOracleBatch
-    envs = {c: make_env(key, 1, *c, T=T) for c in COMBOS}
+    envs = {(o, s): make_env(key, 1, obs=o, state=s, T=T) for o, s in COMBOS}
     b = envs[("rgb", "index4")]
-    ora = TagOracleBatch.from_spec(b.spec, n_envs=1, random_spawn_point=True, spawn_rotation=None)
+    ora = make_ref(b, seed=0)
     n = b.n
     sched = lockstep.schedule_for(key, seed=300 + T, teleport_every=7)
     rs = np.random.RandomState(T + 1)
@@ -157,7 +140,7 @@ def test_layout_strides_every_shipped_geometry():
     from homophily_marl_b200 import _capi
     seen = {}
     for key in sorted(lockstep.CONFIGS):
-        e = make_env(key, 2, "rgb", "rgb")
+        e = make_env(key, 2)
         rs_, env_stride = state_layout(e.H, e.W)
         lay = e.get_state_layout("index4")
         assert (lay.format, lay.row_stride, lay.plane_stride, lay.env_stride) == (_capi.SSD_OBS_INDEX4, rs_, 0, env_stride)
@@ -181,15 +164,15 @@ def test_layout_strides_every_shipped_geometry():
 
 def test_env_ranges_on_streams_equal_one_launch():
     B, G = 4096, 8
-    a = make_env("harvest5", B, "rgb", "rgb", T=3, seed=4)
-    b = make_env("harvest5", B, "index4", "index4", T=3, seed=4)
+    a = make_env("harvest5", B, T=3, seed=4)
+    b = make_env("harvest5", B, obs="index4", state="index4", T=3, seed=4)
     a.reset()
     b.reset()
     rs = np.random.RandomState(8)
     streams = [torch.cuda.Stream(device=b.device) for _ in range(G)]
     fl = torch.empty((B, 3, b.H, b.W), dtype=torch.float32, device=b.device)
     for t in range(30):
-        act = torch.as_tensor(actions(rs, a, True), device=a.device)
+        act = torch.as_tensor(random_actions(rs, a, fire=0.35), device=a.device)
         a.step(act, want_state=True)
         b.state_buf.fill_(0xFF)
         cur = torch.cuda.current_stream(b.device)
@@ -201,8 +184,7 @@ def test_env_ranges_on_streams_equal_one_launch():
         for s in streams:
             cur.wait_stream(s)
         torch.cuda.synchronize()
-        for k in STATE:
-            assert torch.equal(getattr(a, k), getattr(b, k)), (t, k)
+        assert_same_buffers(a, b, STATE, t)
         assert torch.equal(fl, a.state_rgb.float() / 256), t
         assert np.array_equal(b.state_buf.cpu().numpy(), pack(device_state(b, range(B)))), t
 
@@ -210,8 +192,8 @@ def test_env_ranges_on_streams_equal_one_launch():
 @pytest.mark.parametrize("key", ["harvest5", "cleanup10"])
 def test_65536_envs_sampled(key):
     B = 65536
-    a = make_env(key, B, "rgb", "rgb", seed=13)
-    b = make_env(key, B, "index4", "index4", seed=13)
+    a = make_env(key, B, seed=13)
+    b = make_env(key, B, obs="index4", state="index4", seed=13)
     a.reset()
     b.reset()
     rs = np.random.RandomState(2)
@@ -219,12 +201,11 @@ def test_65536_envs_sampled(key):
     st = torch.as_tensor(sample, device=b.device)
     before = b.launch_count
     for t in range(6):
-        act = torch.as_tensor(actions(rs, a, False), device=a.device)
+        act = torch.as_tensor(random_actions(rs, a), device=a.device)
         a.step(act, want_state=True)
         b.state_buf.fill_(0xFF)
         b.step(act, want_state=True)
-        for k in STATE:
-            assert torch.equal(getattr(a, k), getattr(b, k)), (t, k)
+        assert_same_buffers(a, b, STATE, t)
         got = b.state_buf[st].cpu().numpy()
         assert np.array_equal(got, pack(device_state(b, sample))), t
         assert np.array_equal(rgb_of(b.spec.lut, unpack(got, b.H, b.W)), a.state_rgb[st].cpu().numpy()), t
@@ -236,8 +217,8 @@ def test_65536_envs_sampled(key):
 
 def test_step_host_copies_the_state_format():
     B = 64
-    b = make_env("harvest5", B, "rgb", "index4", seed=3)
-    a = make_env("harvest5", B, "rgb", "rgb", seed=3)
+    b = make_env("harvest5", B, state="index4", seed=3)
+    a = make_env("harvest5", B, seed=3)
     ES = b.state_layout.env_stride
     io, ioa = b.make_host_io(with_obs=True, with_state=True), a.make_host_io(with_obs=True, with_state=True)
     assert io["state"].shape == (B, ES) and ioa["state"].shape == (B, 3, a.H, a.W)
@@ -247,7 +228,7 @@ def test_step_host_copies_the_state_format():
     b.reset()
     rs = np.random.RandomState(1)
     for t in range(5):
-        act = torch.as_tensor(actions(rs, b, False))
+        act = torch.as_tensor(random_actions(rs, b))
         io["actions"].copy_(act)
         ioa["actions"].copy_(act)
         io["state"].fill_(0xEE)
@@ -268,8 +249,8 @@ def test_step_host_copies_the_state_format():
 
 def test_switching_format_between_steps_and_auto_reset():
     B, L = 16, 12
-    a = make_env("cleanup10_full", B, "index4", "rgb", T=2, seed=6, episode_limit=L)
-    b = make_env("cleanup10_full", B, "index4", "index4", T=2, seed=6, episode_limit=L)
+    a = make_env("cleanup10_full", B, obs="index4", T=2, seed=6, limit=L)
+    b = make_env("cleanup10_full", B, obs="index4", state="index4", T=2, seed=6, limit=L)
     a.reset()
     b.reset()
     rs = np.random.RandomState(4)
@@ -283,11 +264,10 @@ def test_switching_format_between_steps_and_auto_reset():
         rgb, idx = (b, a) if 8 <= t < 20 else (a, b)
         assert rgb.state_rgb is not None and idx.state_rgb is None
         idx.state_buf.fill_(0xFF)
-        act = torch.as_tensor(actions(rs, a, True), device=a.device)
+        act = torch.as_tensor(random_actions(rs, a, fire=0.35), device=a.device)
         a.step(act, want_state=True, auto_reset=True)
         b.step(act, want_state=True, auto_reset=True)
-        for k in STATE:
-            assert torch.equal(getattr(a, k), getattr(b, k)), (t, k)
+        assert_same_buffers(a, b, STATE, t)
         got = idx.state_buf.cpu().numpy()
         assert np.array_equal(got, pack(device_state(idx, range(B)))), t
         assert np.array_equal(rgb_of(idx.spec.lut, unpack(got, idx.H, idx.W)), rgb.state_rgb.cpu().numpy()), t
@@ -302,7 +282,7 @@ def test_switching_format_between_steps_and_auto_reset():
 
 
 def test_state_float_validates_out():
-    b = make_env("cleanup5", 8, "rgb", "index4")
+    b = make_env("cleanup5", 8, state="index4")
     b.reset()
     b.render(want_obs=False, want_state=True)
     with pytest.raises(ValueError):
@@ -314,38 +294,16 @@ def test_state_float_validates_out():
     assert torch.equal(out, b.state_float()[2:5])
 
 
-def _subprocess(env_extra, code):
-    r = subprocess.run([sys.executable, "-c", "import sys; sys.path[:0] = ['tests', '.']; " + code], cwd=ROOT,
-                       env={**os.environ, **env_extra}, capture_output=True, text=True, timeout=1200)
-    assert r.returncode == 0, r.stdout[-1000:] + r.stderr[-3000:]
-    return r.stdout
-
-
-# kind, H, W, n_agents, view, colour.  ceil(W/2) is a multiple of 4 for W = 15, 16, 64 and not for 11, 13, 33, 38, 50;
-# H * row_stride is a multiple of 16 for (12, 11), (20, 33), (16, 16), (40, 50), (32, 64) and not for the others.
-CUSTOM = [
-    ("cleanup", 12, 11, 16, 3, "full"), ("cleanup", 20, 33, 7, 5, "simplified"), ("harvest", 16, 16, 16, 11, "full"),
-    ("cleanup", 40, 50, 10, 9, "full"), ("harvest", 32, 64, 16, 31, "full"), ("harvest", 9, 38, 5, 13, "simplified"),
-    ("cleanup", 7, 16, 4, 5, "full"), ("harvest", 13, 15, 6, 7, "full"), ("harvest", 11, 13, 6, 7, "simplified"),
-]
-
-
-def run_custom(kind, H, W, n, view, color, T=2, B=16, steps=25):
-    from homophily_marl_b200 import mapspec
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    from test_gpu_generic_geometry import random_map
-    rows = random_map(np.random.RandomState(H * W + n), kind, H, W, n_spawn=min(32, n + 3))
-    params = (mapspec.EnvParams(mapspec.KIND_CLEANUP, "custom", 0.7, 0.1, 0.4, 0.25) if kind == "cleanup"
-              else mapspec.EnvParams(mapspec.KIND_HARVEST, "custom", spawn_prob=(0.01, 0.1, 0.2, 0.4)))
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, obs_color=color, tag_timeout=T)
-    return run_lockstep(lambda o, s: SSDBatchEnv(kind, B, n, view_size=view, episode_limit=1000, rows=rows, params=params, seed=9,
-                                                 extra_args=dict(extra, obs_format=o, state_format=s), want_state=True),
-                        B=B, steps=steps)
+# the shared custom maps plus three more, so that both stride cases occur: ceil(W/2) is a multiple of 4 for W = 15, 16, 64 and
+# not for 11, 13, 33, 38, 50; H * row_stride is a multiple of 16 for (12, 11), (20, 33), (16, 16), (40, 50), (32, 64) and not
+# for the others.
+CUSTOM = harness.CUSTOM + [("cleanup", 7, 16, 4, 5, "full"), ("harvest", 13, 15, 6, 7, "full"),
+                           ("harvest", 11, 13, 6, 7, "simplified")]
 
 
 @pytest.mark.parametrize("case", CUSTOM, ids=lambda c: "%s_%dx%d_n%d_v%d" % c[:5])
 def test_runtime_geometry_custom_maps(case):
-    assert run_custom(*case) > 0
+    assert run_lockstep(lambda o, s: make_custom_env(case, 16, obs=o, state=s, T=2), B=16, steps=25) > 0
 
 
 def test_custom_maps_cover_both_stride_cases():
@@ -357,55 +315,19 @@ def test_custom_maps_cover_both_stride_cases():
 
 def test_runtime_geometry_on_shipped_maps():
     """SSD_B200_GENERIC=1: the GeoD instantiations on the shipped maps."""
-    out = _subprocess({"SSD_B200_GENERIC": "1"},
-                      "import test_gpu_state_index as m; "
-                      "[m.run_lockstep(lambda o, s, k=k, T=T: m.make_env(k, 16, o, s, T=T), B=16, steps=20) "
-                      " for k in ('cleanup5', 'cleanup10_full', 'harvest5', 'harvest10_full') for T in (0, 3)]; print('OK')")
-    assert "OK" in out
-
-
-def test_checked_build_sees_no_shared_memory_violation():
-    from homophily_marl_b200 import _build
-    _build.build_checked()
-    out = _subprocess({"SSD_B200_CHECKED": "1"},
-                      "import test_gpu_state_index as m; "
-                      "[m.run_lockstep(lambda o, s, k=k, T=T: m.make_env(k, 16, o, s, T=T), B=16, steps=20) "
-                      " for k in ('cleanup3', 'cleanup10_full', 'harvest5', 'harvest10_full') for T in (0, 3)]; "
-                      "[m.run_custom(*c, B=8, steps=10) for c in m.CUSTOM]; "
-                      "from homophily_marl_b200 import _capi; print('OOB', _capi.load().ssd_debug_oob_count())")
-    assert "OOB 0" in out, out[-500:]
-
-
-def _runner(obs_format, state_format, groups, B=6, T=9):
-    from test_batched_runner import FakeBatch, ScriptedMAC, _scheme
-    from homophily_marl_b200.batched_runner import BatchedEpisodeRunner
-    n = 3
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, disable_rotation_action=False,
-                 disable_fire_action=False, obs_color="full", tag_timeout=2, obs_format=obs_format, state_format=state_format)
-    env_args = dict(num_agents=n, render=False, episode_limit=T, is_replay=False, view_size=7, map="default3",
-                    extra_args=extra, seed=3)
-    args = types.SimpleNamespace(batch_size_run=B, env="cleanup", env_args=env_args, device="cuda:0", name="homophily",
-                                 mac="homophily_mac", n_actions=None, ind_reward=True, runner_log_interval=10 ** 9,
-                                 test_nepisode=B, env_groups=groups, fused_frontend=False, rgb_input=False)
-    runner = BatchedEpisodeRunner(args, types.SimpleNamespace(log_stat=lambda *a: None))
-    info = runner.get_env_info()
-    A, dev = info["n_actions"], runner.env.device
-    args.n_actions = A
-    g = torch.Generator().manual_seed(0)
-    table = torch.randint(0, 2 * A, (B, T + 1, n, 1), generator=g).to(dev)
-    table_inc = torch.randint(0, 3, (B, T + 1, n, n, 1), generator=g).to(dev)
-    scheme = _scheme(n, A, *info["state_dims"], info["obs_dims"][0])
-    return runner, (lambda: FakeBatch(scheme, B, T + 1, dev)), ScriptedMAC(table, table_inc)
+    for key in ("cleanup5", "cleanup10_full", "harvest5", "harvest10_full"):
+        for T in (0, 3):
+            with env_var("SSD_B200_GENERIC", "1"):
+                run_lockstep(lambda o, s, key=key, T=T: make_env(key, 16, obs=o, state=s, T=T), B=16, steps=20)
 
 
 @pytest.mark.parametrize("groups", [1, 3])
 def test_batched_runner_fills_the_same_batch(groups):
     batches = {}
     for obs, state in COMBOS:
-        runner, factory, mac = _runner(obs, state, groups)
+        runner = make_runner(groups=groups, extra=dict(obs_color="full", tag_timeout=2, obs_format=obs, state_format=state))
+        runner.mac = ScriptedMAC(*action_tables(runner, 0, high=2 * runner.env.n_actions))
         assert runner.env.state_format == state
-        runner.use_batch_factory(factory)
-        runner.mac = mac
         batches[(obs, state)] = runner.run(test_mode=True)
         runner.close_env()
     a = batches[("rgb", "rgb")]

@@ -1,72 +1,36 @@
 """GPU suite: tagging-out timers (tag_timeout > 0) are bit-exact against the tagging reference (tests/tag_oracle.c) -- grid, positions, orientations, timers,
 rewards, clean counts, apple counts, done flags, u8 observations and state images -- in every shipped configuration, with
-injected draws and teleports, with Philox draws at scale across episodes, split into env ranges, on the runtime geometry and
-in the checked build; and the PyMARL facade and the batched runner carry the feature through ``extra_args``."""
-import os
-import subprocess
-import sys
-import types
-
+injected draws and teleports, with Philox draws at scale across episodes, split into env ranges and on the runtime geometry; and
+the PyMARL facade and the batched runner carry the feature through ``extra_args``."""
 import numpy as np
 import pytest
 
 import lockstep
-from tag_oracle import TagOracleBatch
+from harness import (FIRE, STATE, ScriptedMAC, assert_outputs_match_oracle, assert_same_buffers, assert_state_matches_oracle,
+                     env_var, make_env, make_ref, make_runner, random_actions, step_one_outputs)
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-FIRE = 7
-
-
-def fire_heavy(rs, B, n, n_actions, p_fire=0.35):
-    a = rs.randint(0, n_actions, size=(B, n))
-    return np.where(rs.rand(B, n) < p_fire, FIRE, a).astype(np.uint8)
-
-
-def make_pair(key, B, T, seed=9, episode_limit=1000, **kw):
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    name, mp, n, view, color = lockstep.CONFIGS[key]
-    extra = dict(obs_color=color, random_spawn_point=True, random_spawn_rotation=None, tag_timeout=T)
-    env = SSDBatchEnv(name, B, n, map=mp, view_size=view, episode_limit=episode_limit, extra_args=extra, seed=seed,
-                      want_state=True, **kw)
-    ora = TagOracleBatch.from_spec(env.spec, n_envs=B, seed=seed, random_spawn_point=True, spawn_rotation=None)
-    assert ora.tag_timeout == T
-    return env, ora
-
-
-def assert_state_equal(env, ora, what):
-    assert np.array_equal(env.grid.cpu().numpy(), ora.grid), (what, "grid")
-    assert np.array_equal(env.agent_pos.cpu().numpy(), ora.pos_rc), (what, "pos")
-    assert np.array_equal(env.agent_orient.cpu().numpy(), ora.orient), (what, "orient")
-    assert np.array_equal(env.tag_out.cpu().numpy(), ora.tag_out), (what, "tag_out")
-    assert np.array_equal(env.ep_ret.cpu().numpy(), ora.ep_ret), (what, "ep_ret")
-
-
-def assert_outputs_equal(env, out, what):
-    for k in ("reward", "clean", "done"):
-        assert np.array_equal(getattr(env, k).cpu().numpy(), out[k]), (what, k)
-    assert np.array_equal(env.apple_cnt.cpu().numpy().view(np.uint16), out["apple_cnt"]), (what, "apple_cnt")
-    if out.get("obs") is not None:
-        assert np.array_equal(env.obs_view().cpu().numpy(), out["obs"]), (what, "obs")
 
 
 def run_philox_case(key, B=48, T=3, steps=60):
     """B envs, Philox draws, FIRE-heavy random play; step outputs and ssd_render both checked.  Returns (tags, respawns)."""
-    env, ora = make_pair(key, B, T, episode_limit=steps + 5)
+    env = make_env(key, B, T=T, limit=steps + 5)
+    ora = make_ref(env)
+    assert ora.tag_timeout == T
     env.reset()
     ora.reset()
     rs = np.random.RandomState(len(key) * 7 + T)
     tags = respawns = 0
     for t in range(steps):
-        act = fire_heavy(rs, B, env.n, env.n_actions)
+        act = random_actions(rs, env, fire=0.35)
         before = ora.tag_out.copy()
         env.step(torch.as_tensor(act, device=env.device), want_state=True)
         out = ora.step(act, threads=8)
         tags += int(((ora.tag_out == T) & (before == 0)).sum())
         respawns += int(((before == 1) & (ora.tag_out == 0)).sum())
-        assert_outputs_equal(env, out, (key, t))
-        assert_state_equal(env, ora, (key, t))
+        assert_outputs_match_oracle(env, out, (key, t))
+        assert_state_matches_oracle(env, ora, (key, t))
         state = np.stack([ora.state_one(b) for b in range(B)])
         assert np.array_equal(env.state_rgb.cpu().numpy(), state), (key, t, "state")
         if t % 10 == 9:                                            # ssd_render honours the timers too
@@ -88,11 +52,9 @@ def test_every_config_matches_oracle_with_tagging(key):
 @pytest.mark.parametrize("key,T", [("cleanup5", 1), ("harvest5", 3), ("cleanup10_full", 25), ("harvest10_full", 3)])
 def test_injected_draws_and_teleports(key, T):
     """One env, every draw injected (spawn_key / rot included, so respawns read them), FIRE-heavy, teleports every 7 steps."""
-    from homophily_marl_b200.batch_env import SSDBatchEnv
-    name, mp, n, view, color = lockstep.CONFIGS[key]
-    extra = dict(obs_color=color, random_spawn_point=True, random_spawn_rotation=None, tag_timeout=T)
-    env = SSDBatchEnv(name, 1, n, map=mp, view_size=view, episode_limit=1000, extra_args=extra, want_state=True)
-    ora = TagOracleBatch.from_spec(env.spec, n_envs=1, random_spawn_point=True, spawn_rotation=None)
+    env = make_env(key, 1, T=T, seed=0)
+    ora = make_ref(env)
+    n = env.n
     sched = lockstep.schedule_for(key, seed=100 + T, teleport_every=7)
     rs = np.random.RandomState(T)
     d0 = sched.reset_draws()
@@ -110,12 +72,11 @@ def test_injected_draws_and_teleports(key, T):
         before = ora.tag_out.copy()
         env.step(torch.as_tensor(actions.reshape(1, n), device=env.device),
                  draws={k: v.reshape(1, -1) for k, v in draws.items()}, want_state=True)
-        r, c, cnt, done = ora.step_one(actions, 0, {k: v.reshape(-1) for k, v in draws.items()})
+        out = step_one_outputs(ora, actions, draws)
         tags += int(((ora.tag_out == T) & (before == 0)).sum())
         respawns += int(((before == 1) & (ora.tag_out == 0)).sum())
-        assert_outputs_equal(env, dict(reward=r[None], clean=c[None], done=np.array([done], np.uint8),
-                                       apple_cnt=np.array([cnt], np.uint16), obs=ora.obs_one(0)[None]), (key, t))
-        assert_state_equal(env, ora, (key, t))
+        assert_outputs_match_oracle(env, out, (key, t))
+        assert_state_matches_oracle(env, ora, (key, t))
         assert np.array_equal(env.state_rgb[0].cpu().numpy(), ora.state_one(0)), (key, t, "state")
     assert tags > 0 and respawns > 0, (tags, respawns)
 
@@ -123,19 +84,20 @@ def test_injected_draws_and_teleports(key, T):
 def test_philox_at_scale_with_masked_reset_and_auto_reset():
     """4 096 envs over more than two episodes: auto_reset at the episode end, plus masked resets of some envs mid-episode."""
     B, T, L = 4096, 4, 30
-    env, ora = make_pair("cleanup5", B, T, seed=21, episode_limit=L)
+    env = make_env("cleanup5", B, T=T, seed=21, limit=L)
+    ora = make_ref(env)
     env.reset()
     ora.reset(threads=8)
     rs = np.random.RandomState(5)
     tags = respawns = cleared = 0
     for t in range(75):
-        act = fire_heavy(rs, B, env.n, env.n_actions)
+        act = random_actions(rs, env, fire=0.35)
         before = ora.tag_out.copy()
         env.step(torch.as_tensor(act, device=env.device), auto_reset=True)
         out = ora.step(act, threads=8)
         tags += int(((ora.tag_out == T) & (before == 0)).sum())
         respawns += int(((before == 1) & (ora.tag_out == 0)).sum())
-        assert_outputs_equal(env, dict(out, obs=None), t)
+        assert_outputs_match_oracle(env, dict(out, obs=None), t)
         done = np.flatnonzero(out["done"])
         for b in done:
             ora.reset_one(int(b))
@@ -145,7 +107,7 @@ def test_philox_at_scale_with_masked_reset_and_auto_reset():
             env.reset(mask=torch.as_tensor(mask.astype(np.uint8)))
             for b in np.flatnonzero(mask):
                 ora.reset_one(int(b))
-        assert_state_equal(env, ora, t)
+        assert_state_matches_oracle(env, ora, t)
         if t % 5 == 0 or len(done):                                # the step's views; first views of the envs just reset
             want = np.stack([ora.obs_one(b) for b in range(B)])
             assert np.array_equal(env.obs_view().cpu().numpy(), want), (t, "obs")
@@ -155,15 +117,15 @@ def test_philox_at_scale_with_masked_reset_and_auto_reset():
 
 def test_env_ranges_equal_one_launch():
     B, T = 4096, 3
-    a, _ = make_pair("harvest5", B, T, seed=4)
-    b, _ = make_pair("harvest5", B, T, seed=4)
+    a = make_env("harvest5", B, T=T, seed=4)
+    b = make_env("harvest5", B, T=T, seed=4)
     a.reset()
     b.reset()
     rs = np.random.RandomState(8)
     streams = [torch.cuda.Stream(device=b.device) for _ in range(8)]
     obs_b = b.new_obs_buffer()
     for t in range(40):
-        act = torch.as_tensor(fire_heavy(rs, B, a.n, a.n_actions), device=a.device)
+        act = torch.as_tensor(random_actions(rs, a, fire=0.35), device=a.device)
         a.step(act)
         cur = torch.cuda.current_stream(b.device)
         for g, s in enumerate(streams):
@@ -173,34 +135,17 @@ def test_env_ranges_equal_one_launch():
         for s in streams:
             cur.wait_stream(s)
         torch.cuda.synchronize()
-        for k in ("reward", "clean", "done", "apple_cnt", "grid_buf", "agent_buf", "ep_ret_buf", "counts_buf"):
-            assert torch.equal(getattr(a, k), getattr(b, k)), (t, k)
+        assert_same_buffers(a, b, STATE, t)
         assert torch.equal(a.obs_buf, obs_b), t
     assert int((a.tag_out > 0).sum()) > 0
 
 
-def _subprocess_cases(env_extra, keys):
-    code = ("import sys; sys.path[:0] = ['tests', '.']; import test_gpu_tagging as m; "
-            "n = [m.run_philox_case(k, B=24, steps=30) for k in %r]; print('CASES', n); "
-            "assert all(t > 0 and r > 0 for t, r in n); "
-            "from homophily_marl_b200 import _capi; print('OOB', _capi.load().ssd_debug_oob_count())" % (keys,))
-    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env={**os.environ, **env_extra}, capture_output=True, text=True,
-                       timeout=900)
-    assert r.returncode == 0, r.stdout[-1000:] + r.stderr[-3000:]
-    return r.stdout
-
-
 def test_runtime_geometry_kernels():
     """SSD_B200_GENERIC=1: the GeoD instantiations (tagging variant) on the shipped maps."""
-    out = _subprocess_cases({"SSD_B200_GENERIC": "1"}, ["cleanup5", "harvest5", "harvest10_full"])
-    assert "CASES" in out
-
-
-def test_checked_build_sees_no_shared_memory_violation():
-    from homophily_marl_b200 import _build
-    _build.build_checked()
-    out = _subprocess_cases({"SSD_B200_CHECKED": "1"}, ["cleanup10_full", "harvest5", "harvest10_full"])
-    assert "OOB 0" in out, out[-500:]
+    for key in ("cleanup5", "harvest5", "harvest10_full"):
+        with env_var("SSD_B200_GENERIC", "1"):
+            tags, respawns = run_philox_case(key, B=24, steps=30)
+        assert tags > 0 and respawns > 0, (key, tags, respawns)
 
 
 def test_pymarl_facade_with_tagging():
@@ -227,30 +172,19 @@ def test_pymarl_facade_with_tagging():
 
 def test_batched_runner_with_tagging():
     """One runner episode with tagging on: the stored observation rows of agents out of play are zero, all others are not."""
-    from test_batched_runner import FakeBatch, ScriptedMAC, _scheme
     from homophily_marl_b200.batch_env import SSDBatchEnv
-    from homophily_marl_b200.batched_runner import BatchedEpisodeRunner
     B, T, n = 8, 40, 5
-    extra = dict(random_spawn_point=True, random_spawn_rotation=None, disable_rotation_action=False,
-                 disable_fire_action=False, tag_timeout=6)
-    env_args = dict(num_agents=n, render=False, episode_limit=T, is_replay=False, view_size=7, map="default5",
-                    extra_args=extra, seed=3)
-    args = types.SimpleNamespace(batch_size_run=B, env="cleanup", env_args=env_args, device="cuda:0", name="homophily",
-                                 mac="homophily_mac", n_actions=None, ind_reward=True, runner_log_interval=10 ** 9,
-                                 test_nepisode=B, env_groups=1)
-    runner = BatchedEpisodeRunner(args, types.SimpleNamespace(log_stat=lambda *a: None))
-    info = runner.get_env_info()
-    A, dev = info["n_actions"], runner.env.device
-    args.n_actions = A
+    runner = make_runner(mp="default5", n=n, B=B, T=T, extra=dict(tag_timeout=6))
+    A, dev = runner.env.n_actions, runner.env.device
     g = torch.Generator().manual_seed(1)
     table = torch.randint(0, A, (B, T + 1, n, 1), generator=g)
     table = torch.where(torch.rand(table.shape, generator=g) < 0.4, torch.full_like(table, FIRE), table).to(dev)
     table_inc = torch.zeros((B, T + 1, n, n, 1), dtype=torch.long, device=dev)
-    runner.use_batch_factory(lambda: FakeBatch(_scheme(n, A, *info["state_dims"], info["obs_dims"][0]), B, T + 1, dev))
     runner.mac = ScriptedMAC(table, table_inc)
     batch = runner.run(test_mode=True)
     # the same episode on a twin env gives the timers at every stored step
-    twin = SSDBatchEnv("cleanup", B, n, map="default5", view_size=7, episode_limit=T, extra_args=extra, seed=3)
+    twin = SSDBatchEnv("cleanup", B, n, map="default5", view_size=7, episode_limit=T, extra_args=runner.args.env_args["extra_args"],
+                       seed=3)
     twin.reset()
     out_steps = 0
     for t in range(T + 1):

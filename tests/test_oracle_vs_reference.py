@@ -55,13 +55,13 @@ def test_seeded_anchor_hashes_of_the_reference():
 
 
 def test_fakebatch_has_the_update_semantics_of_the_reference_episodebatch():
-    """tests/test_batched_runner.py checks the batched runner through a stand-in EpisodeBatch; this pins the stand-in
+    """The batched-runner tests check the runner through a stand-in EpisodeBatch (harness.FakeBatch); this pins the stand-in
     against the reference's EpisodeBatch.update (src/components/episode_buffer.py:87-116) on the CPU."""
     import numpy as np
     import torch
     refshim._import_registry()
     from components.episode_buffer import EpisodeBatch
-    from test_batched_runner import FakeBatch, _scheme
+    from harness import FakeBatch, _scheme
     n, A, H, W, N, B, T = 3, 9, 10, 10, 15, 2, 4
     fs = _scheme(n, A, H, W, N)
     scheme = {"state": {"vshape": (3, H, W)}, "obs": {"vshape": (3, N, N), "group": "agents"},

@@ -14,18 +14,10 @@ import numpy as np
 import pytest
 
 from baseline import refloop
+from harness import _cfg
 
 pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not refloop.available(), reason="reference sources absent (baseline/_ref)")]
 torch = pytest.importorskip("torch")
-
-
-def _cfg(**kw):
-    base = dict(seed=3, use_cuda=True, save_model=False, t_max=300, batch_size=4, buffer_size=16, test_nepisode=2,
-                test_interval=10 ** 9, log_interval=10 ** 9, runner_log_interval=10 ** 9, learner_log_interval=1,
-                env_args=dict(num_agents=3, map="default3"))
-    base.update(kw)
-    seed = base.pop("seed")
-    return refloop.load_config("cleanup", seed=seed, **base)
 
 
 def _oracle_replay(batch, spec, seed, b0=0, ticks_before=0):

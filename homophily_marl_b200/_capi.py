@@ -15,13 +15,18 @@ LIB_PATH = os.environ.get("SSD_B200_LIB") or os.path.join(
 SSD_OK, SSD_ERR_INVALID, SSD_ERR_CUDA, SSD_ERR_SPAWN, SSD_ERR_MAP = 0, -1, -2, -3, -4
 SSD_OBS_RGB, SSD_OBS_INDEX4 = 0, 1
 SSD_MAX_VARIANTS = 256
+# per-agent episode counters (ssd_set_stats): field index = position in STAT_NAMES
+STAT_NAMES = ("apples", "apple_t", "fires", "hits_dealt", "hits_taken", "out_steps", "cleaned")
+SSD_N_STATS = len(STAT_NAMES)
+(SSD_STAT_APPLES, SSD_STAT_APPLE_T, SSD_STAT_FIRES, SSD_STAT_HITS_DEALT, SSD_STAT_HITS_TAKEN, SSD_STAT_OUT_STEPS,
+ SSD_STAT_CLEANED) = range(SSD_N_STATS)
 
 # every symbol include/ssd_b200.h declares (checked by tests/test_capi_symbols.py against the header text)
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
-           "ssd_set_variants", "ssd_set_env_variants",
+           "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
@@ -109,6 +114,7 @@ def load():
     L.ssd_expand_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.ssd_set_variants.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdVariant)]
     L.ssd_set_env_variants.argtypes = [C.c_void_p, C.c_void_p]
+    L.ssd_set_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

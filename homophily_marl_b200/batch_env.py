@@ -47,8 +47,11 @@ class SSDBatchEnv:
         # state_format: the same choice for the state image (get_state * 256), independent of obs_format
         # variants (also extra_args["variants"]): per-env variants of this config, a list of mapspec.compile_variant override
         #   dicts ({} = this config); env b runs variant variant_of[b], by default (env_gid_base + b) % len(variants)
+        # episode_stats: per-agent episode counters in stats_buf (and, with keep_episode_end, end_stats_buf), the inputs of
+        #   social_metrics(); without it nothing is allocated and no kernel counts
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
-                     disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb")
+                     disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb",
+                     episode_stats=False)
         extra.update(extra_args or {})
         for key in ("obs_format", "state_format"):
             if extra[key] not in OBS_FORMATS:
@@ -124,6 +127,11 @@ class SSDBatchEnv:
         self.obs_buf = self.new_obs_buffer()
         self.end_obs_buf = self.new_obs_buffer() if self.keep_episode_end else None
         self.end_ep_ret_buf = z((B, lay.agent_stride), torch.int32) if self.keep_episode_end else None
+        self.stats_buf = self.end_stats_buf = None
+        if extra["episode_stats"]:
+            self.stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32)
+            self.end_stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32) if self.keep_episode_end else None
+            _capi.check(self.lib.ssd_set_stats(self._h, _ptr(self.stats_buf), _ptr(self.end_stats_buf)))
         self.want_state = bool(want_state)
         self._alloc_state()
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
@@ -315,6 +323,43 @@ class SSDBatchEnv:
     def end_ep_ret(self):
         """[B, n] int32 episode returns written by an auto-reset step for the envs whose episode it ended (keep_episode_end)."""
         return None if self.end_ep_ret_buf is None else self.end_ep_ret_buf[:, :self.n]
+
+    # ------------------------------------------------------------------ episode counters and social metrics
+    def stats(self, buf=None):
+        """[B, 7, n] int32 view (no copy) of the per-agent episode counters (``stats_buf``, or ``end_stats_buf``), field k being
+        ``_capi.STAT_NAMES[k]``: apples eaten, sum of the 1-based step index t over them, FIREs, FIRE rays dealt that hit an agent,
+        rays taken, steps started tagged out, waste cells cleaned; each counted since the env's last reset (extra_args
+        ``episode_stats``)."""
+        if self.stats_buf is None:
+            raise ValueError("stats() needs extra_args episode_stats=True")
+        return (self.stats_buf if buf is None else buf)[:, :, :self.n]
+
+    def social_metrics(self, end=False):
+        """Efficiency, equality, sustainability and peace (Perolat et al., 2017) of every env's current episode after ``t``
+        steps, or with ``end=True`` of the episode an auto-reset step last finished (``end_stats_buf`` / ``end_ep_ret``, t =
+        episode_limit; needs keep_episode_end).  A dict of fp64 [B] device tensors, computed without a host sync:
+        efficiency = sum of ep_ret / t; equality = 1 - Gini of ep_ret, as the runners compute ``equality_metric`` (1 when the
+        collective return is 0); sustainability = mean over the agents that ate of APPLE_T / APPLES (0 when none ate);
+        peace = n - sum of OUT_STEPS / t.  An env at t = 0 has efficiency 0 and peace n."""
+        if end:
+            if self.end_stats_buf is None:
+                raise ValueError("social_metrics(end=True) needs episode_stats and keep_episode_end")
+            ret, st = self.end_ep_ret.double(), self.stats(self.end_stats_buf).double()
+            t = torch.full((self.B,), float(self.episode_limit), dtype=torch.float64, device=self.device)
+        else:
+            ret, st = self.ep_ret.double(), self.stats().double()
+            t = self.t_buf.double().clamp(min=1.0)
+        coll = ret.sum(1)
+        denom = 2 * self.n * ret.abs().sum(1)
+        pair = (ret[:, None, :] - ret[:, :, None]).abs().sum((1, 2))
+        equality = torch.where(coll != 0, 1 - pair / torch.where(denom == 0, 1.0, denom), 1.0)
+        apples, apple_t = st[:, _capi.SSD_STAT_APPLES], st[:, _capi.SSD_STAT_APPLE_T]
+        ate = apples > 0
+        n_ate = ate.sum(1)
+        per = torch.where(ate, apple_t / apples.clamp(min=1.0), 0.0)
+        sustainability = torch.where(n_ate > 0, per.sum(1) / n_ate.clamp(min=1), 0.0)
+        peace = self.n - st[:, _capi.SSD_STAT_OUT_STEPS].sum(1) / t
+        return dict(efficiency=coll / t, equality=equality, sustainability=sustainability, peace=peace)
 
     @property
     def tag_out(self):

@@ -23,8 +23,13 @@ from functools import partial
 import numpy as np
 import torch
 
-from . import mapspec
+from . import _capi, mapspec
 from .batch_env import SSDBatchEnv
+
+# extra_args episode_stats: the social metrics and per-env event totals (summed over agents) added to env_info at episode end
+SOCIAL_KEYS = ("efficiency", "sustainability", "peace")
+EVENT_FIELDS = {"apples": _capi.SSD_STAT_APPLES, "fires": _capi.SSD_STAT_FIRES, "hits": _capi.SSD_STAT_HITS_DEALT,
+                "cleaned": _capi.SSD_STAT_CLEANED}
 
 
 class BatchedEpisodeRunner:
@@ -213,13 +218,21 @@ class BatchedEpisodeRunner:
         # termination info of every env (map_env.py:897-912), accumulated like B single-env episodes
         if not bool(e.done.all().item()):                     # first host sync of the episode
             raise RuntimeError("device-side done flags disagree with the host step count")
-        R = e.ep_ret.double().cpu().numpy()
+        R = e.ep_ret.double()
+        if e.stats_buf is not None:                           # episode_stats: metrics and event totals ride on the same copy
+            m, tot = e.social_metrics(), e.stats().double().sum(2)
+            R = torch.cat([R] + [m[k][:, None] for k in SOCIAL_KEYS] + [tot[:, k, None] for k in EVENT_FIELDS.values()], 1)
+        R = R.cpu().numpy()
+        R, X = R[:, :e.n], R[:, e.n:]
         coll = R.sum(axis=1)
         denom = 2 * e.n * np.abs(R).sum(axis=1)
         pair = np.abs(R[:, None, :] - R[:, :, None]).sum(axis=(1, 2))
         eq = np.where(coll != 0, 1 - pair / np.where(denom == 0, 1, denom), 1.0)
         env_info = {"collective_return": float(coll.sum()), "equality_metric": float(eq.sum())}
         self.last_env_info = {"collective_return": coll, "equality_metric": eq}
+        for j, k in enumerate(SOCIAL_KEYS + tuple(EVENT_FIELDS) if X.shape[1] else ()):
+            env_info[k] = float(X[:, j].sum())
+            self.last_env_info[k] = X[:, j]
         returns = episode_return.cpu().numpy()
         if len(e.variant_specs) > 1:                          # a sweep: the pooled means alone average the variants away
             vid = np.minimum(e.variant.cpu().numpy().astype(np.int64), len(e.variant_specs) - 1)
@@ -232,6 +245,8 @@ class BatchedEpisodeRunner:
                 a["return"] += float(returns[m].mean(axis=1).sum())
                 a["collective_return"] += float(coll[m].sum())
                 a["equality_metric"] += float(eq[m].sum())
+                for j, key in enumerate(SOCIAL_KEYS if X.shape[1] else ()):
+                    a[key] = a.get(key, 0.0) + float(X[m, j].sum())
 
         self._account(env_info, returns, test_mode)
         return self.batch
@@ -267,7 +282,7 @@ class BatchedEpisodeRunner:
         for key in [k for k in stats if k not in skip]:
             log(prefix + key + "_mean", stats[key] / episodes, self.t_env)
         for k, a in sorted(self._vstats.pop(prefix == "test_", {}).items()):
-            for key in ("return", "collective_return", "equality_metric"):
+            for key in ("return", "collective_return", "equality_metric") + tuple(q for q in SOCIAL_KEYS if q in a):
                 log(f"{prefix}v{k}_{key}_mean", a[key] / a["n"], self.t_env)
         rets.clear()
         stats.clear()

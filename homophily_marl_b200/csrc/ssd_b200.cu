@@ -127,7 +127,14 @@ struct KParams {
     const uint8_t* variant_of;                // [B] variant id per env (ssd_set_env_variants), or NULL: the fields above (variant 0)
     const VarDev* variants;                   // the variant table (n_variants records), read only when variant_of is set
     int n_variants;
+    uint32_t* stats; uint32_t* end_stats;     // STATS kernels: per-agent episode counters (ssd_set_stats; DESIGN.md §3 item 16)
 };
+
+// STATS: one agent's counter deltas of a step, packed in one register so that the step's live registers stay flat.  Bits: 0 ate an
+// apple, 1 fired, 2 started the step out of play, 3-4 FIRE rays of its beam that hit an agent (<= 3), 5-10 rays that hit it
+// (<= 3 per shooter, <= 48).
+constexpr uint32_t kSdAte = 1u, kSdFire = 2u, kSdOut = 4u;
+constexpr int kSdDealt = 3, kSdTaken = 5;
 
 // The variant an env runs (DESIGN.md §3 item 15).  VAR = false (no id array): every read is the KParams field it always was, and
 // the kernel is the code it was before variants existed.  VAR: a load from the env's record in the variant table.  Warp-uniform:
@@ -438,6 +445,46 @@ __device__ __forceinline__ void beams(const Warp& w, const GEO& g, const KParams
             }
         }
     }
+}
+
+// STATS: the FIRE rays of the step once more, for the episode counters (DESIGN.md §3 item 16), after beams() and before the tagged
+// leave the map.  A FIRE ray stops at a wall or at the first cell an agent in play stands on, and neither changes during the beam
+// phase (CLEAN only turns waste into river; tagged agents stay on the map until every beam is done), so this walk finds the cells
+// beams() hit, whatever order the beams ran in.  Returns the lane's kSdFire, kSdDealt and kSdTaken bits.  A pass of its own:
+// walking FIRE rays inside beams() whatever hit_penalty is spilled the Harvest V=15 auto-reset kernel with variants.
+template <class GEO>
+__device__ __forceinline__ uint32_t fire_counts(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, int lane, bool is_agent,
+                                                int act, int pos, int ori) {
+    const bool fire = is_agent && act == 7;
+    uint32_t sd = fire ? kSdFire : 0u;
+    unsigned need = w.ballot(fire);
+    while (need) {
+        const int i = __ffs(need) - 1;
+        need &= need - 1;
+        const int posi = w.shfl(pos, i), orii = w.shfl(ori, i);
+        const int dr = orii == 0 ? -1 : (orii == 1 ? 1 : 0), dc = orii == 2 ? -1 : (orii == 3 ? 1 : 0);
+        const int rr = orii == 2 ? 1 : (orii == 3 ? -1 : 0), rc = orii == 0 ? -1 : (orii == 1 ? 1 : 0);
+        const int d = dr * g.W() + dc, rs = rr * g.W() + rc;
+        int hit = -1;
+        if (lane < 3) {
+            int q = posi + (lane == 0 ? d : (lane == 1 ? rs : -rs));
+            for (int k = 0; k < p.beam_len; ++k) {
+                SSD_CHECK(q >= 0 && q < g.G());
+                const int v = sg[q];
+                if ((v & 0x7f) == SSD_CELL_WALL) break;
+                if (v & kOcc) { hit = q; break; }
+                q += d;
+            }
+        }
+#pragma unroll
+        for (int s = 0; s < 3; ++s) {
+            const int hq = w.shfl(hit, s);
+            const unsigned on = w.ballot(hq >= 0 && pos == hq);
+            if (on && lane == 31 - __clz(on)) sd += 1u << kSdTaken;   // the agent hit_penalty charges
+            if (on && lane == i) sd += 1u << kSdDealt;
+        }
+    }
+    return sd;
 }
 
 // ------------------------------------------------------------------ spawning (cleanup.py:165-204, harvest.py:92-122)
@@ -1058,7 +1105,9 @@ __device__ __forceinline__ void draw(const Warp& w, const GEO& g, const KParams&
 // (profiles/r7_notes.md).
 // VAR: envs run the variants of p.variant_of (DESIGN.md §3 item 15).  A template parameter, not a runtime switch on variant_of,
 // because the switch moved the register allocation of most kernels without variants and spilled one (profiles/r8_notes.md).
-template <int MODE, class GEO, bool TAG, bool IDX, bool VAR>
+// STATS (MODE_STEP, MODE_STEP_RESET): the step adds its events to the per-agent episode counters p.stats (DESIGN.md §3 item 16).
+// A template parameter for the same reason as VAR: the kernels without counters keep their code.
+template <int MODE, class GEO, bool TAG, bool IDX, bool VAR, bool STATS>
 __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __grid_constant__ KParams p) {
     constexpr bool STEP = MODE == MODE_STEP || MODE == MODE_STEP_RESET;
     const GEO g(p);
@@ -1153,6 +1202,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
         if (STEP) {
             int reward = 0, clean_num = 0;
             bool tagged = false;
+            uint32_t sd = 0;                                       // STATS: the step's counter deltas (kSd* bits)
             update_moves(w, g, p, sg, lane, live, act, pos, ori, env, gid, tick);                     // map_env.py:251
             // consume in index order: the lowest index on a cell eats the apple (253-256); mark occupancy
             same = surely_distinct(w, pos, live, w.ballot(live)) ? (1u << lane) : equal_lanes(w, pos, p.n);
@@ -1165,8 +1215,37 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                 else sg[pos] = (uint8_t)(kOcc | here);
             }
             apples -= __popc(ate);
+            if (STATS && ((ate >> lane) & 1u)) sd = kSdAte;
             w.sync();
             beams<TAG>(w, g, p, vr, sg, lane, live, act, pos, ori, reward, clean_num, waste, tagged);    // 259-260
+            if (STATS) sd |= fire_counts(w, g, p, sg, lane, live, act, pos, ori);
+            if (STATS && is_agent) {
+                // Every count of the step is known here (t, whether the step ends the episode, the stage-in timer), so the
+                // counters are updated before spawn and nothing of them is live across spawn or the render: the non-zero deltas
+                // are added in L2 (RED.ADD, no register waits for a load).  Loading the seven counters and storing them with the
+                // agent records spilled in the Harvest V=15 and runtime-geometry auto-reset kernels.  An episode that ends in a
+                // MODE_STEP_RESET step loads its counters (past L1, after griddepcontrol.wait), writes them to end_stats if set
+                // and stores zeros: the reset that follows starts from 0.
+                const uint32_t t = (uint32_t)t_prev + 1u;
+                if (TAG && timer != 0) sd |= kSdOut;
+                const uint32_t d[SSD_N_STATS] = { sd & 1u, (sd & 1u) ? t : 0u, (sd >> 1) & 1u, (sd >> kSdDealt) & 3u,
+                                                  (sd >> kSdTaken) & 63u, (sd >> 2) & 1u, (uint32_t)clean_num };
+                uint32_t* const s = p.stats + (size_t)env * SSD_N_STATS * p.NA + lane;
+                if (MODE == MODE_STEP_RESET && (int)t >= p.episode_limit) {
+                    uint32_t v[SSD_N_STATS];
+#pragma unroll
+                    for (int f = 0; f < SSD_N_STATS; ++f) v[f] = __ldcg(s + f * p.NA) + d[f];
+                    uint32_t* const e = p.end_stats + (size_t)env * SSD_N_STATS * p.NA + lane;
+#pragma unroll
+                    for (int f = 0; f < SSD_N_STATS; ++f) {
+                        if (p.end_stats) e[f * p.NA] = v[f];
+                        s[f * p.NA] = 0u;
+                    }
+                } else {
+#pragma unroll
+                    for (int f = 0; f < SSD_N_STATS; ++f) if (d[f]) atomicAdd(s + f * p.NA, d[f]);
+                }
+            }
             unsigned gone = 0;
             if (TAG) {                                 // the tagged leave the map; a cell stays occupied while an untagged agent is on it
                 gone = w.ballot(tagged);
@@ -1269,6 +1348,17 @@ __global__ void incentive_kernel(const long long* __restrict__ a_inc, const floa
     if (sgn) sgn[idx] = rv > 0.f ? 1.f : (rv < 0.f ? -1.f : 0.f);
 }
 
+// ------------------------------------------------------------------ episode counters of a reset (ssd_reset with ssd_set_stats)
+// Zeroes the SSD_N_STATS x agent_stride counters of every env whose mask byte is non-zero (mask NULL: every env).  A kernel of its
+// own, so that the MODE_RESET instantiations keep their code.
+__global__ void __launch_bounds__(256) zero_stats_kernel(uint32_t* __restrict__ stats, const uint8_t* __restrict__ mask,
+                                                         long long total, int per_env) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    if (mask && mask[i / per_env] == 0) return;
+    stats[i] = 0u;
+}
+
 // ------------------------------------------------------------------ index4 -> f32 RGB (ssd_expand_obs, ssd_expand_state)
 // One CTA per block of rows x cols nibbles (an agent view, or an env's state image), one thread per pixel:
 // f32 [3][rows][cols] = color_lut[nibble] / 256, exactly what u8 RGB / 256 gives.
@@ -1364,7 +1454,7 @@ static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws
     return SSD_OK;
 }
 
-template <int MODE, class GEO, bool TAG, bool IDX, bool VAR>
+template <int MODE, class GEO, bool TAG, bool IDX, bool VAR, bool STATS>
 static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
     DeviceGuard guard(h->device);
     SSD_CUDA(guard.err);
@@ -1376,7 +1466,7 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
         const int dev = h->device;
         if (dev < 0 || dev >= kMaxDevices) return SSD_ERR_INVALID;
         if ((int)h->smem_bytes > high_water[dev]) {
-            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, TAG, IDX, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
+            SSD_CUDA(cudaFuncSetAttribute(ssd_kernel<MODE, GEO, TAG, IDX, VAR, STATS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
             high_water[dev] = (int)h->smem_bytes;
         }
     }
@@ -1391,9 +1481,9 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, TAG, IDX, VAR>, k));
+        SSD_CUDA(cudaLaunchKernelEx(&cfg, ssd_kernel<MODE, GEO, TAG, IDX, VAR, STATS>, k));
     } else {
-        ssd_kernel<MODE, GEO, TAG, IDX, VAR><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
+        ssd_kernel<MODE, GEO, TAG, IDX, VAR, STATS><<<grid, kWarps * 32, h->smem_bytes, (cudaStream_t)stream>>>(k);
     }
     ++h->launches;
     SSD_CUDA(cudaGetLastError());
@@ -1406,26 +1496,32 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
 // launches gain nothing and pay for the prologue no longer running under the state loads, so they keep the plain launch.
 constexpr int kPdlMaxEnvs = 2048;
 
-template <int MODE, class GEO, bool VAR>
+template <int MODE, class GEO, bool VAR, bool STATS>
 static int launch_var(ssd_handle* h, const KParams& k, void* stream) {
     const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
     if constexpr (MODE != MODE_RESET) {                        // tagging-out timers: their own instantiation
         if (k.variant_of ? h->tag_any : k.tag_timeout != 0)
-            return idx ? launch_kernel<MODE, GEO, true, true, VAR>(h, k, stream) : launch_kernel<MODE, GEO, true, false, VAR>(h, k, stream);
+            return idx ? launch_kernel<MODE, GEO, true, true, VAR, STATS>(h, k, stream)
+                       : launch_kernel<MODE, GEO, true, false, VAR, STATS>(h, k, stream);
     }
-    return idx ? launch_kernel<MODE, GEO, false, true, VAR>(h, k, stream) : launch_kernel<MODE, GEO, false, false, VAR>(h, k, stream);
+    return idx ? launch_kernel<MODE, GEO, false, true, VAR, STATS>(h, k, stream)
+               : launch_kernel<MODE, GEO, false, false, VAR, STATS>(h, k, stream);
 }
 
 template <int MODE, class GEO>
 static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
     k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
+    // episode counters (ssd_set_stats): their own step instantiations
+    if constexpr (MODE == MODE_STEP || MODE == MODE_STEP_RESET) {
+        if (k.stats) return k.variant_of ? launch_var<MODE, GEO, true, true>(h, k, stream) : launch_var<MODE, GEO, false, true>(h, k, stream);
+    }
     // per-env variants: their own instantiations (a render reads nothing a variant sets, but draws no agent out of play when
     // any variant tags)
     if constexpr (MODE != MODE_RENDER) {
-        if (k.variant_of) return launch_var<MODE, GEO, true>(h, k, stream);
+        if (k.variant_of) return launch_var<MODE, GEO, true, false>(h, k, stream);
     }
-    return launch_var<MODE, GEO, false>(h, k, stream);
+    return launch_var<MODE, GEO, false, false>(h, k, stream);
 }
 
 // The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
@@ -1697,12 +1793,28 @@ int ssd_set_env_variants(ssd_handle* h, const uint8_t* variant_of) {
     return SSD_OK;
 }
 
+int ssd_set_stats(ssd_handle* h, uint32_t* stats, uint32_t* end_stats) {
+    if (!h || (end_stats && !stats)) return SSD_ERR_INVALID;
+    if (stats && h->kp.episode_limit > 65535) return SSD_ERR_INVALID;   // APPLE_T of an episode stays below 2^31
+    h->kp.stats = stats; h->kp.end_stats = end_stats;
+    return SSD_OK;
+}
+
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws, uint8_t* obs, void* stream) {
     KParams k;
     const int rc = fill_common(h, st, draws, k);
     if (rc) return rc;
     k.mask = mask; k.obs = obs;
-    return launch<MODE_RESET>(h, k, stream);
+    const int lrc = launch<MODE_RESET>(h, k, stream);
+    if (lrc || !k.stats) return lrc;
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    const int per_env = SSD_N_STATS * k.NA;
+    const long long total = (long long)k.B * per_env;
+    zero_stats_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(k.stats, mask, total, per_env);
+    ++h->launches;
+    SSD_CUDA(cudaGetLastError());
+    return SSD_OK;
 }
 
 int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
@@ -1759,7 +1871,11 @@ int ssd_step_host(ssd_handle* h, const ssd_state* st, const uint8_t* h_actions, 
     cudaStream_t s = (cudaStream_t)stream;
     const size_t B = (size_t)k.B;
     SSD_CUDA(cudaMemcpyAsync(d_actions, h_actions, B * k.n, cudaMemcpyHostToDevice, s));
-    const int rc = ssd_step(h, st, d_actions, nullptr, d_out, stream);
+    KParams ks;                                               // ssd_step, except that a host step leaves the episode counters alone
+    int rc = fill_step(h, st, d_actions, nullptr, d_out, 0, k.B, ks);
+    if (rc) return rc;
+    ks.stats = ks.end_stats = nullptr;
+    rc = launch<MODE_STEP>(h, ks, stream);
     if (rc) return rc;
     if (h_out->reward) SSD_CUDA(cudaMemcpyAsync(h_out->reward, d_out->reward, B * k.n, cudaMemcpyDeviceToHost, s));
     if (h_out->clean) SSD_CUDA(cudaMemcpyAsync(h_out->clean, d_out->clean, B * k.n, cudaMemcpyDeviceToHost, s));

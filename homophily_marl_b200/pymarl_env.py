@@ -19,6 +19,7 @@ import torch
 
 from . import mapspec
 from .batch_env import SSDBatchEnv
+from .batched_runner import EVENT_FIELDS, SOCIAL_KEYS
 
 
 class MultiAgentEnv(object):
@@ -133,7 +134,15 @@ class _SSDEnv(MultiAgentEnv):
                 raise KeyError(a)                        # agent.py:176,237 action_map lookup
         io, sim = self._io, self.sim
         self._act_host[:] = acts[:self.num_agents]
-        sim.step_host(io)                                # H2D actions, fused step+obs+state kernel, D2H results, sync
+        if sim.stats_buf is None:
+            sim.step_host(io)                            # H2D actions, fused step+obs+state kernel, D2H results, sync
+        else:                                            # episode_stats: ssd_step_host leaves the counters alone, so the same
+            io["d_actions"].copy_(io["actions"], non_blocking=True)      # copies go around ssd_step
+            sim.step(io["d_actions"], want_state=True)
+            for k in ("reward", "clean", "apple_cnt", "done"):
+                io[k].copy_(getattr(sim, k), non_blocking=True)
+            io["obs"].copy_(sim.obs_buf, non_blocking=True)
+            io["state"].copy_(sim.state_buf, non_blocking=True)
         sim.pull_host(io, obs=False, state=False, agent=True)
         reward = io["reward"][0].numpy().astype(float)
         if self.rewards is None:
@@ -150,6 +159,10 @@ class _SSDEnv(MultiAgentEnv):
                 equality_metric = 1 - (np.abs(self.rewards.reshape(1, -1) - self.rewards.reshape(-1, 1)).sum()) / (
                     2 * len(self.rewards) * np.abs(self.rewards).sum())
             info = {"collective_return": collective_return, "equality_metric": equality_metric}
+            if sim.stats_buf is not None:                # episode_stats: one more D2H copy, at episode end only
+                m, tot = sim.social_metrics(), sim.stats()[0].double().sum(1)
+                vals = torch.cat([m[k] for k in SOCIAL_KEYS] + [tot[list(EVENT_FIELDS.values())]]).cpu().tolist()
+                info.update(zip(SOCIAL_KEYS + tuple(EVENT_FIELDS), vals))
         self.clean_num = io["clean"][0].numpy().astype(float)
         density = (int(io["apple_cnt"][0]) & 0xFFFF) / sim.G
         self.apple_den = np.full(self.n_agents, density, dtype=float)

@@ -43,6 +43,16 @@ extern "C" {
 #define SSD_MAX_SPAWN  32
 #define SSD_MAX_VARIANTS 256   /* variant ids are u8 (ssd_set_env_variants) */
 
+/* per-agent episode counters (ssd_set_stats): field indices of stats[B][SSD_N_STATS][agent_stride] */
+#define SSD_N_STATS          7
+#define SSD_STAT_APPLES      0   /* apples the agent consumed (the lowest index on a cell eats)                              */
+#define SSD_STAT_APPLE_T     1   /* sum of t over those consumptions, t = the step's 1-based index in the episode (its `t`)  */
+#define SSD_STAT_FIRES       2   /* FIRE actions taken in play (the ones fire_cost charges)                                  */
+#define SSD_STAT_HITS_DEALT  3   /* rays of the agent's FIRE beams that hit an agent                                         */
+#define SSD_STAT_HITS_TAKEN  4   /* FIRE rays that hit the agent (the one hit_penalty charges); CLEAN never hits             */
+#define SSD_STAT_OUT_STEPS   5   /* steps the agent started out of play (tagging-out timer > 0); 0 without tagging           */
+#define SSD_STAT_CLEANED     6   /* sum of clean_num: waste cells the agent cleaned                                          */
+
 /* cell codes stored in the device grid (one byte per cell) */
 #define SSD_CELL_EMPTY  0
 #define SSD_CELL_WALL   1
@@ -236,6 +246,19 @@ int ssd_set_variants(ssd_handle* h, int32_t n_variants, const ssd_variant* varia
  * NULL (the default) runs every env as variant 0, with no per-env load.  Host-side and serialised like ssd_set_obs_format; a CUDA
  * graph keeps the pointer it was captured with. */
 int ssd_set_env_variants(ssd_handle* h, const uint8_t* variant_of);
+
+/* Per-agent episode counters (DESIGN.md §3 item 16).  stats: caller-owned DEVICE u32 [B][SSD_N_STATS][agent_stride], field-major
+ * (SSD_STAT_*); every counter counts since its env's last reset.  Every later ssd_step, ssd_step_range and ssd_step_autoreset adds
+ * the step's events; every ssd_reset zeroes the counters of the envs it resets (one more kernel launch on the same stream), and so
+ * does the reset half of ssd_step_autoreset, which first copies the finished episode's counters to end_stats (same shape) when
+ * that is set; the end_stats slots of other envs are not written.  ssd_render and ssd_step_host leave the counters alone.  Setting
+ * counters changes no other byte of any buffer.  Hits are counted whatever hit_penalty and tag_timeout are.
+ * Bounds: SSD_STAT_APPLE_T of an episode is at most T(T+1)/2 < 2^31 for T = episode_limit <= 65 535; a caller that steps past
+ * `done` without resetting owns any wrap-around (t above 65 535 enters APPLE_T modulo 2^16).
+ * NULL, NULL (the default) turns counting off.  SSD_ERR_INVALID, before any CUDA call, for a NULL handle, end_stats without
+ * stats, or counters on a handle with episode_limit > 65 535.  Host-side and serialised like ssd_set_obs_format; a CUDA graph
+ * keeps the pointers it was captured with. */
+int ssd_set_stats(ssd_handle* h, uint32_t* stats, uint32_t* end_stats);
 
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */

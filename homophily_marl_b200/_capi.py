@@ -26,7 +26,7 @@ EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_pr
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
-           "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats",
+           "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats", "ssd_set_reward_shaping",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
@@ -47,6 +47,10 @@ class SsdConfig(C.Structure):
 class SsdVariant(C.Structure):
     _fields_ = [("ascii_map", C.c_char_p), ("n_waste_lut", C.c_uint32), ("thr_apple", C.c_void_p), ("thr_waste", C.c_void_p),
                 ("thr_harvest", C.c_uint32 * 4), ("fire_cost", C.c_int32), ("hit_penalty", C.c_int32), ("tag_timeout", C.c_int32)]
+
+
+class SsdShaping(C.Structure):
+    _fields_ = [(k, C.c_float) for k in ("alpha", "beta", "decay", "prosocial")]
 
 
 class SsdLayout(C.Structure):
@@ -115,6 +119,7 @@ def load():
     L.ssd_set_variants.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdVariant)]
     L.ssd_set_env_variants.argtypes = [C.c_void_p, C.c_void_p]
     L.ssd_set_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ssd_set_reward_shaping.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdShaping), C.c_void_p, C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

@@ -49,14 +49,18 @@ class SSDBatchEnv:
         #   dicts ({} = this config); env b runs variant variant_of[b], by default (env_gid_base + b) % len(variants)
         # episode_stats: per-agent episode counters in stats_buf (and, with keep_episode_end, end_stats_buf), the inputs of
         #   social_metrics(); without it nothing is allocated and no kernel counts
+        # reward_shaping: {"alpha", "beta", "decay", "prosocial"} (mapspec.reward_shaping), the inequity-averse / prosocial
+        #   reward every step writes to shaped_buf (trace in shape_trace_buf); a variant dict may carry its own.  Without it (and
+        #   without a variant's) nothing is allocated and no kernel runs
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
                      disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb",
-                     episode_stats=False)
+                     episode_stats=False, reward_shaping=None)
         extra.update(extra_args or {})
         for key in ("obs_format", "state_format"):
             if extra[key] not in OBS_FORMATS:
                 raise ValueError(f"{key} must be one of {sorted(OBS_FORMATS)}, got {extra[key]!r}")
         self.extra_args = extra
+        shaping = None if extra["reward_shaping"] is None else mapspec.reward_shaping(extra["reward_shaping"])
         self.name = name
         self.spec = mapspec.compile_map(name, map, num_agents, view_size, episode_limit,
                                         obs_color=extra["obs_color"], rows=rows, params=params,
@@ -132,6 +136,16 @@ class SSDBatchEnv:
             self.stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32)
             self.end_stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32) if self.keep_episode_end else None
             _capi.check(self.lib.ssd_set_stats(self._h, _ptr(self.stats_buf), _ptr(self.end_stats_buf)))
+        self.shape_trace_buf = self.shaped_buf = self.shaping_params = None
+        if shaping is not None or any(sp.reward_shaping is not None for sp in self.variant_specs):
+            # one parameter set per variant (ssd_set_reward_shaping): a variant's own, else the handle's, else the defaults
+            shaping = shaping or mapspec.reward_shaping({})
+            self.shaping_params = [shaping if sp.reward_shaping is None else sp.reward_shaping for sp in self.variant_specs]
+            self.shape_trace_buf = z((B, lay.agent_stride), torch.float32)
+            self.shaped_buf = z((B, lay.agent_stride), torch.float32)
+            recs = (_capi.SsdShaping * len(self.shaping_params))(*[_capi.SsdShaping(*q) for q in self.shaping_params])
+            _capi.check(self.lib.ssd_set_reward_shaping(self._h, len(recs), recs, _ptr(self.shape_trace_buf),
+                                                        _ptr(self.shaped_buf)))
         self.want_state = bool(want_state)
         self._alloc_state()
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
@@ -323,6 +337,15 @@ class SSDBatchEnv:
     def end_ep_ret(self):
         """[B, n] int32 episode returns written by an auto-reset step for the envs whose episode it ended (keep_episode_end)."""
         return None if self.end_ep_ret_buf is None else self.end_ep_ret_buf[:, :self.n]
+
+    # ------------------------------------------------------------------ shaped rewards
+    def shaped_reward(self):
+        """[B, n] float32 view (no copy) of the shaped reward the last step wrote (extra_args ``reward_shaping``; DESIGN.md §3
+        item 17): ``(w1*r_i + w*mean_j r_j - alpha/(n-1)*D_i) - beta/(n-1)*A_i``, with D_i / A_i the summed disadvantageous /
+        advantageous gaps of the smoothed reward traces ``shape_trace_buf``."""
+        if self.shaped_buf is None:
+            raise ValueError("shaped_reward() needs extra_args reward_shaping (or a variant with its own)")
+        return self.shaped_buf[:, :self.n]
 
     # ------------------------------------------------------------------ episode counters and social metrics
     def stats(self, buf=None):

@@ -148,6 +148,9 @@ class BatchedEpisodeRunner:
                 e.step_range(self._actions_u8, r["lo"], Bg, want_state=True)
             reward = e.reward[sl].float()
             r["ret"] += reward
+            if e.shaped_buf is not None:                      # reward_shaping: the learner gets the shaped reward; the statistics
+                reward = e.shaped_reward()[sl]                # stay extrinsic, plus shaped_return
+                r["sret"] += reward
             post = {"actions": actions, "reward": reward if getattr(self.args, "ind_reward", True) else reward.sum(1, keepdim=True),
                     "terminated": e.done[sl].view(Bg, 1), "clean_num": e.clean[sl].float(),
                     "apple_den": (e.apple_cnt[sl].to(torch.int32) & 0xFFFF).double().view(Bg, 1).expand(Bg, e.n) / e.G}
@@ -198,7 +201,8 @@ class BatchedEpisodeRunner:
             self.mac.init_hidden(batch_size=Bg)
             ranges.append({"sl": sl, "lo": k * Bg, "batch": self.batch if G == 1 else self.batch[sl],
                            "stream": main if G == 1 else self._streams[k], "hidden": self._take_hidden(),
-                           "ret": torch.zeros(Bg, e.n, device=e.device)})
+                           "ret": torch.zeros(Bg, e.n, device=e.device),
+                           "sret": None if e.shaped_buf is None else torch.zeros(Bg, e.n, device=e.device)})
             if G > 1:
                 self._streams[k].wait_stream(main)
         # no host sync in the step loop: every env shares episode_limit and get_done() is constantly False in the reference
@@ -222,7 +226,12 @@ class BatchedEpisodeRunner:
         if e.stats_buf is not None:                           # episode_stats: metrics and event totals ride on the same copy
             m, tot = e.social_metrics(), e.stats().double().sum(2)
             R = torch.cat([R] + [m[k][:, None] for k in SOCIAL_KEYS] + [tot[:, k, None] for k in EVENT_FIELDS.values()], 1)
+        if e.shaped_buf is not None:                          # reward_shaping: the shaped returns ride on the same copy
+            R = torch.cat([R, torch.cat([r["sret"] for r in ranges]).double()], 1)
         R = R.cpu().numpy()
+        shaped = None
+        if e.shaped_buf is not None:
+            R, shaped = R[:, :-e.n], R[:, -e.n:].mean(axis=1)
         R, X = R[:, :e.n], R[:, e.n:]
         coll = R.sum(axis=1)
         denom = 2 * e.n * np.abs(R).sum(axis=1)
@@ -233,6 +242,9 @@ class BatchedEpisodeRunner:
         for j, k in enumerate(SOCIAL_KEYS + tuple(EVENT_FIELDS) if X.shape[1] else ()):
             env_info[k] = float(X[:, j].sum())
             self.last_env_info[k] = X[:, j]
+        if shaped is not None:
+            env_info["shaped_return"] = float(shaped.sum())
+            self.last_env_info["shaped_return"] = shaped
         returns = episode_return.cpu().numpy()
         if len(e.variant_specs) > 1:                          # a sweep: the pooled means alone average the variants away
             vid = np.minimum(e.variant.cpu().numpy().astype(np.int64), len(e.variant_specs) - 1)
@@ -247,6 +259,8 @@ class BatchedEpisodeRunner:
                 a["equality_metric"] += float(eq[m].sum())
                 for j, key in enumerate(SOCIAL_KEYS if X.shape[1] else ()):
                     a[key] = a.get(key, 0.0) + float(X[m, j].sum())
+                if shaped is not None:
+                    a["shaped_return"] = a.get("shaped_return", 0.0) + float(shaped[m].sum())
 
         self._account(env_info, returns, test_mode)
         return self.batch
@@ -282,7 +296,8 @@ class BatchedEpisodeRunner:
         for key in [k for k in stats if k not in skip]:
             log(prefix + key + "_mean", stats[key] / episodes, self.t_env)
         for k, a in sorted(self._vstats.pop(prefix == "test_", {}).items()):
-            for key in ("return", "collective_return", "equality_metric") + tuple(q for q in SOCIAL_KEYS if q in a):
+            extra = tuple(q for q in SOCIAL_KEYS + ("shaped_return",) if q in a)
+            for key in ("return", "collective_return", "equality_metric") + extra:
                 log(f"{prefix}v{k}_{key}_mean", a[key] / a["n"], self.t_env)
         rets.clear()
         stats.clear()

@@ -1350,13 +1350,67 @@ __global__ void incentive_kernel(const long long* __restrict__ a_inc, const floa
 
 // ------------------------------------------------------------------ episode counters of a reset (ssd_reset with ssd_set_stats)
 // Zeroes the SSD_N_STATS x agent_stride counters of every env whose mask byte is non-zero (mask NULL: every env).  A kernel of its
-// own, so that the MODE_RESET instantiations keep their code.
+// own, so that the MODE_RESET instantiations keep their code.  ssd_reset also runs it over the shaping traces (per_env =
+// agent_stride words; 0.0f is the all-zero word).
 __global__ void __launch_bounds__(256) zero_stats_kernel(uint32_t* __restrict__ stats, const uint8_t* __restrict__ mask,
                                                          long long total, int per_env) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     if (mask && mask[i / per_env] == 0) return;
     stats[i] = 0u;
+}
+
+// ------------------------------------------------------------------ shaped rewards (ssd_set_reward_shaping; DESIGN.md §3 item 17)
+// One parameter set as the kernel reads it: a = alpha/(n-1), b = beta/(n-1) and w1 = 1 - w are precomputed on the host in fp32.
+struct ShapeDev { float a, b, decay, w, w1; };
+
+struct ShapeParams {
+    const int8_t* reward;                     // [B][n] the step's rewards
+    const uint8_t* done;                      // [B] auto-reset launches only (NULL otherwise): a done env's trace restarts at 0
+    const uint8_t* variant_of;                // [B] or NULL: every env uses params[0]
+    const ShapeDev* params; int n_params;
+    float* trace; float* shaped;              // [B][NA]
+    int n, NA, env0, env1;
+};
+
+// One warp per env and one lane per agent, as in ssd_kernel.  Every operation is an explicitly rounded fp32 intrinsic, so nothing
+// is contracted into an FMA and the result is bit-exact against a NumPy float32 restatement (tests/shaping_ref.py).  The n-way
+// sums run over n shuffles in ascending j.  A kernel of its own after the step launch, so that no ssd_kernel instantiation
+// changes.
+__global__ void __launch_bounds__(kWarps * 32) shape_rewards_kernel(const __grid_constant__ ShapeParams p) {
+    // Under programmatic dependent launch (small launches, as the step launch before it): wait for the step's outputs, and let
+    // the next step launch of the stream become resident and run its prologue meanwhile (it still waits for this whole grid).
+    // Both are no-ops in a plain launch.
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    const int lane = threadIdx.x & 31;
+    const int env = p.env0 + blockIdx.x * kWarps + (threadIdx.x >> 5);
+    if (env >= p.env1) return;
+    const int pid = p.variant_of ? min((int)__ldcg(p.variant_of + env), p.n_params - 1) : 0;
+    const ShapeDev s = p.params[pid];
+    const bool is_agent = lane < p.n;
+    // mutable buffers are read past L1, as in ssd_kernel: concurrent env ranges may share a line at a range boundary
+    const int ri = is_agent ? (int)__ldcg(p.reward + (size_t)env * p.n + lane) : 0;
+    const size_t at = (size_t)env * p.NA + lane;
+    const float r = (float)ri;
+    const float e = __fadd_rn(__fmul_rn(is_agent ? __ldcg(p.trace + at) : 0.0f, s.decay), r);
+    int sum = 0;
+    float D = 0.0f, A = 0.0f;
+    for (int j = 0; j < p.n; ++j) {
+        const float ej = __shfl_sync(0xffffffffu, e, j);
+        sum += __shfl_sync(0xffffffffu, ri, j);
+        if (j != lane) {
+            D = __fadd_rn(D, fmaxf(__fsub_rn(ej, e), 0.0f));
+            A = __fadd_rn(A, fmaxf(__fsub_rn(e, ej), 0.0f));
+        }
+    }
+    const float c = __fdiv_rn((float)sum, (float)p.n);
+    const float m = __fadd_rn(__fmul_rn(s.w1, r), __fmul_rn(s.w, c));
+    const float u = __fsub_rn(__fsub_rn(m, __fmul_rn(s.a, D)), __fmul_rn(s.b, A));
+    if (is_agent) {
+        p.shaped[at] = u;
+        p.trace[at] = (p.done && __ldcg(p.done + env)) ? 0.0f : e;
+    }
 }
 
 // ------------------------------------------------------------------ index4 -> f32 RGB (ssd_expand_obs, ssd_expand_state)
@@ -1438,6 +1492,9 @@ struct ssd_handle {
     VarDev* d_vars;                                           // variant table: SSD_MAX_VARIANTS records, allocated once when first needed
     VarDev* base;                                             // host copy of the creation config's record (ssd_set_variants(h, 0, ...))
     int tag_any;                                              // some variant of the table has tag_timeout > 0
+    ShapeDev* d_shape;                                        // shaping table: SSD_MAX_VARIANTS records, allocated once when first needed
+    int n_shape;                                              // entries in use; 0 = shaping off
+    float* shape_trace; float* shaped;                        // caller-owned [B][NA] (ssd_set_reward_shaping)
 };
 
 static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws* d, KParams& k) {
@@ -1496,6 +1553,44 @@ static int launch_kernel(ssd_handle* h, const KParams& k, void* stream) {
 // launches gain nothing and pay for the prologue no longer running under the state loads, so they keep the plain launch.
 constexpr int kPdlMaxEnvs = 2048;
 
+static bool use_pdl(const ssd_handle* h, const KParams& k) { return h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs; }
+
+// The shaped rewards of the step launch just queued with `k` (ssd_set_reward_shaping): shape_rewards_kernel on the same stream
+// over the same envs, chained programmatically exactly when the step launch is.  done: the step's done flags for an auto-reset
+// step (the traces of the envs it reset restart at 0), NULL otherwise.  Nothing is launched while shaping is off.
+static int launch_shaping(ssd_handle* h, const KParams& k, const uint8_t* done, void* stream) {
+    if (!h->n_shape) return SSD_OK;
+    const int grid = (k.env1 - k.env0 + kWarps - 1) / kWarps;
+    if (grid <= 0) return SSD_OK;
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    ShapeParams s;
+    s.reward = k.reward; s.done = done; s.variant_of = k.variant_of; s.params = h->d_shape; s.n_params = h->n_shape;
+    s.trace = h->shape_trace; s.shaped = h->shaped;
+    s.n = k.n; s.NA = k.NA; s.env0 = k.env0; s.env1 = k.env1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(kWarps * 32); cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    if (use_pdl(h, k)) { cfg.attrs = attr; cfg.numAttrs = 1; }
+    SSD_CUDA(cudaLaunchKernelEx(&cfg, shape_rewards_kernel, s));
+    ++h->launches;
+    SSD_CUDA(cudaGetLastError());
+    return SSD_OK;
+}
+
+// Zeroes `per_env` u32 words of every env whose mask byte is non-zero (mask NULL: every env): ssd_reset's counter and trace reset.
+static int zero_masked(ssd_handle* h, uint32_t* buf, const uint8_t* mask, int B, int per_env, void* stream) {
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    const long long total = (long long)B * per_env;
+    zero_stats_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(buf, mask, total, per_env);
+    ++h->launches;
+    SSD_CUDA(cudaGetLastError());
+    return SSD_OK;
+}
+
 template <int MODE, class GEO, bool VAR, bool STATS>
 static int launch_var(ssd_handle* h, const KParams& k, void* stream) {
     const bool idx = h->obs_format == SSD_OBS_INDEX4;          // packed colour-index observations: their own instantiations
@@ -1511,7 +1606,7 @@ static int launch_var(ssd_handle* h, const KParams& k, void* stream) {
 template <int MODE, class GEO>
 static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     KParams k = k_in;
-    k.pdl = h->pdl && (k.env1 - k.env0) <= kPdlMaxEnvs;
+    k.pdl = use_pdl(h, k);
     // episode counters (ssd_set_stats): their own step instantiations
     if constexpr (MODE == MODE_STEP || MODE == MODE_STEP_RESET) {
         if (k.stats) return k.variant_of ? launch_var<MODE, GEO, true, true>(h, k, stream) : launch_var<MODE, GEO, false, true>(h, k, stream);
@@ -1711,6 +1806,7 @@ int ssd_destroy(ssd_handle* h) {
     DeviceGuard guard(h->device);
     cudaFree(h->d_map);
     if (h->d_vars) cudaFree(h->d_vars);
+    if (h->d_shape) cudaFree(h->d_shape);
     delete h->base;
     delete h;
     return SSD_OK;
@@ -1800,21 +1896,45 @@ int ssd_set_stats(ssd_handle* h, uint32_t* stats, uint32_t* end_stats) {
     return SSD_OK;
 }
 
+int ssd_set_reward_shaping(ssd_handle* h, int32_t n_params, const ssd_shaping* params, float* trace, float* shaped) {
+    if (!h || n_params < 0 || n_params > SSD_MAX_VARIANTS || (n_params > 0 && !params)) return SSD_ERR_INVALID;
+    if ((trace == nullptr) != (shaped == nullptr) || (trace != nullptr) != (n_params > 0)) return SSD_ERR_INVALID;
+    ShapeDev recs[SSD_MAX_VARIANTS];
+    const int n = h->kp.n;
+    for (int i = 0; i < n_params; ++i) {
+        const ssd_shaping& q = params[i];
+        if (!isfinite(q.alpha) || !isfinite(q.beta) || !isfinite(q.decay) || !isfinite(q.prosocial)) return SSD_ERR_INVALID;
+        if (q.alpha < 0.0f || q.beta < 0.0f || q.decay < 0.0f || q.decay > 1.0f || q.prosocial < 0.0f || q.prosocial > 1.0f)
+            return SSD_ERR_INVALID;
+        const float others = (float)(n - 1);
+        recs[i].a = n > 1 ? q.alpha / others : 0.0f;
+        recs[i].b = n > 1 ? q.beta / others : 0.0f;
+        recs[i].decay = q.decay; recs[i].w = q.prosocial; recs[i].w1 = 1.0f - q.prosocial;
+    }
+    if (n_params > 0) {
+        DeviceGuard guard(h->device);
+        SSD_CUDA(guard.err);
+        if (!h->d_shape) {                                    // allocated once at full size: no launch ever reads a freed table
+            ShapeDev* d = nullptr;
+            SSD_CUDA(cudaMalloc(&d, sizeof(ShapeDev) * SSD_MAX_VARIANTS));
+            h->d_shape = d;
+        }
+        SSD_CUDA(cudaDeviceSynchronize());                    // no launch in flight reads the table while it changes
+        SSD_CUDA(cudaMemcpy(h->d_shape, recs, sizeof(ShapeDev) * n_params, cudaMemcpyHostToDevice));
+    }
+    h->n_shape = n_params; h->shape_trace = trace; h->shaped = shaped;
+    return SSD_OK;
+}
+
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws, uint8_t* obs, void* stream) {
     KParams k;
     const int rc = fill_common(h, st, draws, k);
     if (rc) return rc;
     k.mask = mask; k.obs = obs;
-    const int lrc = launch<MODE_RESET>(h, k, stream);
-    if (lrc || !k.stats) return lrc;
-    DeviceGuard guard(h->device);
-    SSD_CUDA(guard.err);
-    const int per_env = SSD_N_STATS * k.NA;
-    const long long total = (long long)k.B * per_env;
-    zero_stats_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(k.stats, mask, total, per_env);
-    ++h->launches;
-    SSD_CUDA(cudaGetLastError());
-    return SSD_OK;
+    int lrc = launch<MODE_RESET>(h, k, stream);
+    if (!lrc && k.stats) lrc = zero_masked(h, k.stats, mask, k.B, SSD_N_STATS * k.NA, stream);
+    if (!lrc && h->n_shape) lrc = zero_masked(h, reinterpret_cast<uint32_t*>(h->shape_trace), mask, k.B, k.NA, stream);
+    return lrc;
 }
 
 int ssd_step(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
@@ -1840,7 +1960,8 @@ int ssd_step_range(ssd_handle* h, const ssd_state* st, const uint8_t* actions, c
     KParams k;
     const int rc = fill_step(h, st, actions, draws, out, env_begin, env_count, k);
     if (rc) return rc;
-    return launch<MODE_STEP>(h, k, stream);
+    const int lrc = launch<MODE_STEP>(h, k, stream);
+    return lrc ? lrc : launch_shaping(h, k, nullptr, stream);
 }
 
 int ssd_step_autoreset(ssd_handle* h, const ssd_state* st, const uint8_t* actions, const ssd_draws* draws,
@@ -1850,7 +1971,8 @@ int ssd_step_autoreset(ssd_handle* h, const ssd_state* st, const uint8_t* action
     const int rc = fill_step(h, st, actions, draws, out, env_begin, env_count, k);
     if (rc) return rc;
     if (end) { k.end_obs = end->obs; k.end_state = end->state_rgb; k.end_ep_ret = end->ep_ret; }
-    return launch<MODE_STEP_RESET>(h, k, stream);
+    const int lrc = launch<MODE_STEP_RESET>(h, k, stream);
+    return lrc ? lrc : launch_shaping(h, k, k.done, stream);
 }
 
 int ssd_render(ssd_handle* h, const ssd_state* st, uint8_t* obs, uint8_t* state_rgb, void* stream) {
@@ -1876,6 +1998,7 @@ int ssd_step_host(ssd_handle* h, const ssd_state* st, const uint8_t* h_actions, 
     if (rc) return rc;
     ks.stats = ks.end_stats = nullptr;
     rc = launch<MODE_STEP>(h, ks, stream);
+    if (!rc) rc = launch_shaping(h, ks, nullptr, stream);     // the shaped rewards are updated like ssd_step's
     if (rc) return rc;
     if (h_out->reward) SSD_CUDA(cudaMemcpyAsync(h_out->reward, d_out->reward, B * k.n, cudaMemcpyDeviceToHost, s));
     if (h_out->clean) SSD_CUDA(cudaMemcpyAsync(h_out->clean, d_out->clean, B * k.n, cudaMemcpyDeviceToHost, s));

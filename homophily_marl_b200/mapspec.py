@@ -158,6 +158,9 @@ class MapSpec:
     thr_waste: np.ndarray = field(default=None, repr=False)
     thr_harvest: np.ndarray = field(default=None, repr=False)
     lut: np.ndarray = field(default=None, repr=False)
+    # a variant's own shaped-reward parameters (compile_variant key "reward_shaping"): (alpha, beta, decay, prosocial) as
+    # float32 values, or None for the handle's
+    reward_shaping: tuple = None
 
     @property
     def G(self):
@@ -231,7 +234,7 @@ def compile_map(name: str, map_name: str, n_agents: int, view: int, episode_limi
                    lut=color_lut(p.kind, obs_color))
 
 
-VARIANT_KEYS_COMMON = ("rows", "fire_cost", "hit_penalty", "tag_timeout")
+VARIANT_KEYS_COMMON = ("rows", "fire_cost", "hit_penalty", "tag_timeout", "reward_shaping")
 VARIANT_KEYS = {KIND_CLEANUP: VARIANT_KEYS_COMMON + ("threshold_depletion", "threshold_restoration", "waste_spawn_prob",
                                                     "apple_respawn_prob"),
                 KIND_HARVEST: VARIANT_KEYS_COMMON + ("spawn_prob",)}
@@ -241,8 +244,9 @@ def compile_variant(base: MapSpec, overrides: dict) -> MapSpec:
     """One env variant (``ssd_set_variants``): ``base`` (the handle's creation spec) with ``overrides`` applied.  Keys:
     ``rows`` (an ASCII layout of base's exact H x W), ``fire_cost``, ``hit_penalty``, ``tag_timeout``, and the spawn
     dynamics of the kind -- Cleanup ``threshold_depletion``, ``threshold_restoration``, ``waste_spawn_prob``,
-    ``apple_respawn_prob``; Harvest ``spawn_prob`` (4 probabilities).  ``{}`` is the base config.  Everything else (kind,
-    size, view, agents, episode limit, colours) stays the handle's."""
+    ``apple_respawn_prob``; Harvest ``spawn_prob`` (4 probabilities); ``reward_shaping`` (a ``reward_shaping`` dict, see
+    there; absent: the handle's).  ``{}`` is the base config.  Everything else (kind, size, view, agents, episode limit,
+    colours) stays the handle's."""
     ov = dict(overrides or {})
     allowed = VARIANT_KEYS[base.kind]
     other = set(VARIANT_KEYS[KIND_HARVEST if base.kind == KIND_CLEANUP else KIND_CLEANUP]) - set(allowed)
@@ -262,10 +266,34 @@ def compile_variant(base: MapSpec, overrides: dict) -> MapSpec:
             raise ValueError("spawn_prob needs 4 probabilities")
         pk["spawn_prob"] = sp
     params = dataclasses.replace(base.params, **{k: (v if k == "spawn_prob" else float(v)) for k, v in pk.items()})
-    return compile_map("", "", base.n_agents, base.view, base.episode_limit, obs_color=base.obs_color, rows=rows,
+    spec = compile_map("", "", base.n_agents, base.view, base.episode_limit, obs_color=base.obs_color, rows=rows,
                        params=params, fire_cost=int(ov.get("fire_cost", base.fire_cost)),
                        hit_penalty=int(ov.get("hit_penalty", base.hit_penalty)),
                        tag_timeout=int(ov.get("tag_timeout", base.tag_timeout)))
+    if "reward_shaping" in ov:
+        spec.reward_shaping = reward_shaping(ov["reward_shaping"])
+    return spec
+
+
+# Shaped rewards (ssd_set_reward_shaping; DESIGN.md §3 item 17): inequity aversion (Hughes et al., 2018) and prosocial mixing
+# (Peysakhovich & Lerer, 2018).  The default decay is Hughes' gamma * lambda = 0.99 * 0.975, in float32.
+SHAPING_KEYS = ("alpha", "beta", "decay", "prosocial")
+SHAPING_DEFAULTS = {"alpha": 0.0, "beta": 0.0, "decay": float(np.float32(0.99 * 0.975)), "prosocial": 0.0}
+
+
+def reward_shaping(params: dict) -> tuple:
+    """``(alpha, beta, decay, prosocial)`` as float32 values from a ``reward_shaping`` dict: unknown keys are refused, missing
+    ones take ``SHAPING_DEFAULTS``; every value must be finite, alpha and beta >= 0, decay and prosocial in [0, 1]."""
+    unknown = set(params) - set(SHAPING_KEYS)
+    if unknown:
+        raise ValueError(f"unknown reward_shaping keys {sorted(unknown)}; allowed: {list(SHAPING_KEYS)}")
+    with np.errstate(over="ignore"):                        # a value past the float32 range becomes inf and is refused below
+        vals = tuple(float(np.float32(params.get(k, SHAPING_DEFAULTS[k]))) for k in SHAPING_KEYS)
+    alpha, beta, decay, prosocial = vals
+    if not all(math.isfinite(v) for v in vals) or alpha < 0 or beta < 0 or not 0 <= decay <= 1 or not 0 <= prosocial <= 1:
+        raise ValueError("reward_shaping needs finite alpha, beta >= 0 and decay, prosocial in [0, 1], got "
+                         f"{dict(zip(SHAPING_KEYS, vals))}")
+    return vals
 
 
 def dump_maps() -> str:

@@ -118,6 +118,9 @@ class _SSDEnv(MultiAgentEnv):
         self._obs_host = self._io["obs"].numpy().reshape(-1)[: lay.obs_env_stride]
         self._obs_strides = (lay.obs_agent_stride, lay.obs_plane_stride, lay.obs_row_stride, 1)
         self._act_host = self._io["actions"].numpy()[0]   # NumPy view of the pinned action row
+        # reward_shaping: step() returns the shaped rewards (pinned mirror) and the episode's shaped return goes into info
+        self._shaped_host = None if self.sim.shaped_buf is None else torch.zeros(self.sim.shaped_buf.shape).pin_memory()
+        self._shaped_ret = np.zeros(num_agents, dtype=np.float32)
         self.sim.reset()                                # valid state before the first reset() ...
         self.sim.tick_buf.zero_()                       # ... which then replays the same draws (tick 0)
         self.sim.pull_host(self._io)
@@ -134,21 +137,27 @@ class _SSDEnv(MultiAgentEnv):
                 raise KeyError(a)                        # agent.py:176,237 action_map lookup
         io, sim = self._io, self.sim
         self._act_host[:] = acts[:self.num_agents]
-        if sim.stats_buf is None:
+        if sim.stats_buf is None and sim.shaped_buf is None:
             sim.step_host(io)                            # H2D actions, fused step+obs+state kernel, D2H results, sync
         else:                                            # episode_stats: ssd_step_host leaves the counters alone, so the same
-            io["d_actions"].copy_(io["actions"], non_blocking=True)      # copies go around ssd_step
-            sim.step(io["d_actions"], want_state=True)
+            io["d_actions"].copy_(io["actions"], non_blocking=True)      # copies go around ssd_step (reward_shaping: and
+            sim.step(io["d_actions"], want_state=True)                   # one more for the shaped rewards)
             for k in ("reward", "clean", "apple_cnt", "done"):
                 io[k].copy_(getattr(sim, k), non_blocking=True)
             io["obs"].copy_(sim.obs_buf, non_blocking=True)
             io["state"].copy_(sim.state_buf, non_blocking=True)
+            if self._shaped_host is not None:
+                self._shaped_host.copy_(sim.shaped_buf, non_blocking=True)
         sim.pull_host(io, obs=False, state=False, agent=True)
         reward = io["reward"][0].numpy().astype(float)
         if self.rewards is None:
             self.rewards = reward
         else:
             self.rewards += reward
+        if self._shaped_host is not None:                # what the learner sees; the termination metrics stay extrinsic
+            shaped = self._shaped_host[0, :self.num_agents].numpy()
+            self._shaped_ret += shaped
+            reward = shaped.astype(float)
         self._episode_steps += 1
         terminated = bool(io["done"][0])                 # python bool: SURVEY 8b pitfall
         info = {}
@@ -163,6 +172,8 @@ class _SSDEnv(MultiAgentEnv):
                 m, tot = sim.social_metrics(), sim.stats()[0].double().sum(1)
                 vals = torch.cat([m[k] for k in SOCIAL_KEYS] + [tot[list(EVENT_FIELDS.values())]]).cpu().tolist()
                 info.update(zip(SOCIAL_KEYS + tuple(EVENT_FIELDS), vals))
+            if self._shaped_host is not None:            # mean over agents of the episode's shaped return, as the batched runner
+                info["shaped_return"] = float(self._shaped_ret.astype(np.float64).mean())
         self.clean_num = io["clean"][0].numpy().astype(float)
         density = (int(io["apple_cnt"][0]) & 0xFFFF) / sim.G
         self.apple_den = np.full(self.n_agents, density, dtype=float)
@@ -176,6 +187,7 @@ class _SSDEnv(MultiAgentEnv):
         self.sim.pull_host(self._io)
         self._episode_steps = 0
         self.rewards = None
+        self._shaped_ret[:] = 0
         return
 
     # ------------------------------------------------------------------ queries (served from the pinned mirrors)

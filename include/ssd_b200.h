@@ -260,6 +260,33 @@ int ssd_set_env_variants(ssd_handle* h, const uint8_t* variant_of);
  * keeps the pointers it was captured with. */
 int ssd_set_stats(ssd_handle* h, uint32_t* stats, uint32_t* end_stats);
 
+/* One parameter set of the shaped reward (ssd_set_reward_shaping): inequity aversion (Hughes et al., 2018) with disadvantageous
+ * weight alpha >= 0, advantageous weight beta >= 0 and trace decay gamma*lambda in [0, 1], mixed with the mean reward of the env
+ * at weight prosocial in [0, 1] (Peysakhovich & Lerer, 2018).  Every value finite. */
+typedef struct ssd_shaping {
+    float alpha, beta, decay, prosocial;
+} ssd_shaping;
+
+/* Shaped rewards (DESIGN.md §3 item 17).  trace, shaped: caller-owned DEVICE f32 [B][agent_stride].  Every later ssd_step,
+ * ssd_step_range, ssd_step_autoreset and ssd_step_host launches one more kernel on the same stream, over the same envs, that
+ * computes, in fp32 with every operation rounded once in this order (a = alpha/(n-1), b = beta/(n-1), both 0 for n = 1, and
+ * w1 = 1 - prosocial, all precomputed on the host in fp32), for each agent i of the env, r_i = the step's int8 reward:
+ *   e_i <- e_i*decay + r_i;  c = (sum_j r_j)/n;  m_i = w1*r_i + prosocial*c;
+ *   D_i = sum_{j != i} max(e_j - e_i, 0), A_i = sum_{j != i} max(e_i - e_j, 0) (ascending j, updated traces);
+ *   shaped_i = (m_i - a*D_i) - b*A_i.
+ * e is `trace`; every agent's trace is updated, tagged-out agents (reward 0) included.  With alpha = beta = prosocial = 0,
+ * shaped_i == r_i exactly.  Every ssd_reset zeroes the traces of the envs it resets (one more kernel launch on the same stream);
+ * an ssd_step_autoreset step writes the finished step's shaped reward and then zeroes the trace of every env whose episode it
+ * ended.  ssd_render leaves both buffers alone.  Setting shaping changes no other byte of any buffer.
+ * params: n_params = 1 applies params[0] to every env; with per-env variant ids (ssd_set_env_variants) env b uses
+ * params[min(variant_of[b], n_params - 1)], without them params[0].  n_params = 0 with NULL, NULL (the default) turns shaping off.
+ * SSD_ERR_INVALID, before any CUDA call, for a NULL handle, n_params outside 0..SSD_MAX_VARIANTS, NULL params with n_params > 0,
+ * trace without shaped or shaped without trace, buffers without parameters or parameters without buffers, or a parameter that is
+ * not finite or outside its range.  On an error nothing changes.  A configuration call, serialised like ssd_set_obs_format: the
+ * parameter table is allocated once at its full size and overwritten after a device synchronise, so no launch ever reads a freed
+ * table; a CUDA graph keeps the buffer pointers it was captured with. */
+int ssd_set_reward_shaping(ssd_handle* h, int32_t n_params, const ssd_shaping* params, float* trace, float* shaped);
+
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */
 int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd_draws* draws,

@@ -52,13 +52,19 @@ class SSDBatchEnv:
         # reward_shaping: {"alpha", "beta", "decay", "prosocial"} (mapspec.reward_shaping), the inequity-averse / prosocial
         #   reward every step writes to shaped_buf (trace in shape_trace_buf); a variant dict may carry its own.  Without it (and
         #   without a variant's) nothing is allocated and no kernel runs
+        # view_offset: f in 0..view_size, the N x N window centred f cells ahead of the agent along its firing direction, so it
+        #   sees view_size + f cells ahead and view_size - f behind (ssd_set_view_offset; DESIGN.md §3 item 18); 0 = the reference
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
                      disable_fire_action=True, obs_color="simplified", tag_timeout=0, obs_format="rgb", state_format="rgb",
-                     episode_stats=False, reward_shaping=None)
+                     episode_stats=False, reward_shaping=None, view_offset=0)
         extra.update(extra_args or {})
         for key in ("obs_format", "state_format"):
             if extra[key] not in OBS_FORMATS:
                 raise ValueError(f"{key} must be one of {sorted(OBS_FORMATS)}, got {extra[key]!r}")
+        offset = extra["view_offset"]
+        if isinstance(offset, (bool, np.bool_)) or not isinstance(offset, (int, np.integer)) or not 0 <= offset <= int(view_size):
+            raise ValueError(f"view_offset must be an int in 0..view_size ({view_size}), got {offset!r}")
+        self.view_offset = extra["view_offset"] = int(offset)
         self.extra_args = extra
         shaping = None if extra["reward_shaping"] is None else mapspec.reward_shaping(extra["reward_shaping"])
         self.name = name
@@ -102,6 +108,8 @@ class SSDBatchEnv:
         _capi.check(self.lib.ssd_get_layout(self._h, C.byref(lay)))
         self.layout = lay
         assert lay.n_actions == self.n_actions and lay.n_cells == self.G
+        if self.view_offset:
+            _capi.check(self.lib.ssd_set_view_offset(self._h, self.view_offset))
         self.obs_format, self.obs_layout = "rgb", self.get_obs_layout("rgb")
         if extra["obs_format"] != "rgb":
             self._set_format(extra["obs_format"])

@@ -11,7 +11,8 @@
 //     gathered straight from the staged byte grid; large views (Harvest, N = 31) read one run of N
 //     nibbles from a zero-padded nibble-packed index map (or its transpose) held in shared memory.
 //     Either way a lane colours 4 pixels per PRMT through an 8-entry register LUT and writes the
-//     finished row with one 256-bit (st.global.v8.b32, SASS STG.E.ENL2.256) or 128-bit store per plane.
+//     finished row with one 256-bit (st.global.v8.b32, SASS STG.E.ENL2.256) or 128-bit store per plane.  A handle with a
+//     view offset f (ssd_set_view_offset) centres each window f cells ahead of its agent, in kernels of their own (GeoO).
 // The env's grid is staged in shared memory for the whole step.  No tensor cores: nothing here is a
 // contraction.  HBM traffic per env-step is the algorithmic 2G + n(3N^2+11)+3 bytes (+ row padding),
 // ~98% of it observation WRITES.
@@ -66,34 +67,38 @@ struct VarDev {
 };
 
 // ------------------------------------------------------------------ geometry
-// Everything that follows from (kind, H, W, V).  Computed by ONE constexpr function used by the host
-// (ssd_create) and, for the reference's shipped maps, at compile time by the kernels (GeoS), so that index
-// arithmetic folds into immediates; any other geometry runs the same code on runtime values (GeoD).
+// Everything that follows from (kind, H, W, V) and the view offset f.  Computed by ONE constexpr function used by the host
+// (ssd_create, ssd_set_view_offset) and, for the reference's shipped maps, at compile time by the kernels (GeoS), so that index
+// arithmetic folds into immediates; any other geometry runs the same code on runtime values (GeoD), and f > 0 the runtime
+// geometry with the window centre moved f cells ahead (GeoO; DESIGN.md §3 item 18).  A window centred f cells ahead of an agent
+// reaches V + f cells past the agent's own row or column: the padding grows only along the axis the shift runs on.
 struct GeoVals {
     int kind, H, W, V, G, GS, N, RP, PS, AS, LPn, nw8M, nw8T, pitchM, pitchT, PMS;
     int off_map[4];                           // byte offset of the nibble map read by orientation: 0,1 (LEFT/RIGHT) -> MT, 2,3 -> M
     int direct, padF, padB;                   // small views (RP <= 16) are gathered straight from the staged grid: no maps, but
-                                              // V rows of slack before / after the grid so that column runs need no bounds test
+                                              // V + f rows of slack before / after the grid so that column runs need no bounds test
     uint32_t maskM8;                          // valid-nibble mask of the last word of a map row
     int RS4, AS4;                             // SSD_OBS_INDEX4: bytes per row (ceil(N/2) rounded to 4) and per agent (rounded to 16)
 };
 __host__ __device__ constexpr int cround_up(int v, int m) { return (v + m - 1) / m * m; }
-__host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V) {
+__host__ __device__ constexpr GeoVals make_geo(int kind, int H, int W, int V, int offset = 0) {
     GeoVals g{};
     g.kind = kind; g.H = H; g.W = W; g.V = V; g.G = H * W; g.GS = cround_up(H * W, 16);
     g.N = 2 * V + 1; g.RP = cround_up(g.N, 4); g.PS = g.N * g.RP; g.AS = cround_up(3 * g.PS, 16);
-    // nibble-packed padded maps; word pitch kept odd so that lanes gathering consecutive rows hit distinct banks
-    g.LPn = cround_up(V, 8); g.nw8M = (W + 7) / 8; g.nw8T = (H + 7) / 8;
+    // nibble-packed padded maps; word pitch kept odd so that lanes gathering consecutive rows hit distinct banks.  A run
+    // (one window row) lies along a map row of M (UP / DOWN) or of MT (LEFT / RIGHT), which is also the axis the view offset
+    // moves it on: the run padding (LPn in front, the row tail behind) is V + offset nibbles, the V padding rows stay.
+    g.LPn = cround_up(V + offset, 8); g.nw8M = (W + 7) / 8; g.nw8T = (H + 7) / 8;
     g.maskM8 = (W & 7) ? (1u << (4 * (W & 7))) - 1u : 0xffffffffu;
-    int wm = (g.LPn + W + V + 7) / 8; if (wm < g.LPn / 8 + g.nw8M) wm = g.LPn / 8 + g.nw8M; if ((wm & 1) == 0) ++wm;
-    int wt = (g.LPn + H + V + 7) / 8; if (wt < g.LPn / 8 + g.nw8T) wt = g.LPn / 8 + g.nw8T; if ((wt & 1) == 0) ++wt;
+    int wm = (g.LPn + W + V + offset + 7) / 8; if (wm < g.LPn / 8 + g.nw8M) wm = g.LPn / 8 + g.nw8M; if ((wm & 1) == 0) ++wm;
+    int wt = (g.LPn + H + V + offset + 7) / 8; if (wt < g.LPn / 8 + g.nw8T) wt = g.LPn / 8 + g.nw8T; if ((wt & 1) == 0) ++wt;
     g.pitchM = 4 * wm; g.pitchT = 4 * wt;
     const int szM = cround_up((H + 2 * V) * g.pitchM, 16) + 16, szT = cround_up((W + 2 * V) * g.pitchT, 16) + 16;
     g.off_map[0] = 16; g.off_map[1] = 16; g.off_map[2] = 16 + szT; g.off_map[3] = 16 + szT;
     g.PMS = szT + szM + 32;
     g.direct = g.RP <= 16;
-    g.padF = g.direct ? cround_up(V * W + 48, 16) : 16;      // + 32 bytes at the very front for the (class, rank) -> lane table
-    g.padB = g.direct ? cround_up(V * W + 32, 16) : 32;
+    g.padF = g.direct ? cround_up((V + offset) * W + 48, 16) : 16;   // + 32 bytes at the very front for the (class, rank) -> lane table
+    g.padB = g.direct ? cround_up((V + offset) * W + 32, 16) : 32;
     if (g.direct) g.PMS = 0;
     g.RS4 = cround_up((g.N + 1) / 2, 4); g.AS4 = cround_up(g.N * g.RS4, 16);
     return g;
@@ -128,6 +133,7 @@ struct KParams {
     const VarDev* variants;                   // the variant table (n_variants records), read only when variant_of is set
     int n_variants;
     uint32_t* stats; uint32_t* end_stats;     // STATS kernels: per-agent episode counters (ssd_set_stats; DESIGN.md §3 item 16)
+    int view_offset;                          // GeoO kernels: window centre f cells ahead (ssd_set_view_offset; DESIGN.md §3 item 18)
 };
 
 // STATS: one agent's counter deltas of a step, packed in one register so that the step's live registers stay flat.  Bits: 0 ate an
@@ -180,6 +186,7 @@ struct GeoAccess {
     __device__ __forceinline__ int padF() const { return v().padF; }
     __device__ __forceinline__ int padB() const { return v().padB; }
     __device__ __forceinline__ uint32_t maskM8() const { return v().maskM8; }
+    __device__ __forceinline__ static constexpr int view_offset() { return 0; }   // GeoO: KParams::view_offset
 private:
     __device__ __forceinline__ decltype(auto) v() const { return static_cast<const D*>(this)->vals(); }
 };
@@ -207,6 +214,22 @@ struct GeoD : GeoAccess<GeoD> {                               // runtime geometr
     __device__ __forceinline__ int divN(int x) const { return (int)(((uint32_t)x * p.invN20) >> 20); }
     __device__ __forceinline__ int divMW(int x) const { return (int)(((uint32_t)x * p.invMW20) >> 20); }
 };
+
+// The runtime geometry of a handle with a view offset (ssd_set_view_offset).  A class of its own, so that the GeoS and GeoD
+// kernels, whose view_offset() is the constant 0, keep their code: runtime switches inside ssd_kernel move its registers.
+struct GeoO : GeoD {
+    __device__ __forceinline__ explicit GeoO(const KParams& p_) : GeoD(p_) {}
+    __device__ __forceinline__ int view_offset() const { return p.view_offset; }
+};
+
+// The window centre of an agent at (r, c) facing o: f = view_offset() cells along its firing direction ORIENT_VEC[o] (LEFT (-1, 0),
+// RIGHT (+1, 0), UP (0, -1), DOWN (0, +1); map_env.py:28-31).  The agent then sees V + f cells ahead, V - f behind and V to
+// either side, and its own cell is pixel (V, V + f) of its view.  Nothing for GeoS / GeoD.
+template <class GEO>
+__device__ __forceinline__ void window_centre(const GEO& g, int o, int& r, int& c) {
+    const int f = g.view_offset();
+    if (f) { r += o == 0 ? -f : (o == 1 ? f : 0); c += o == 2 ? -f : (o == 3 ? f : 0); }
+}
 
 // ------------------------------------------------------------------ Philox4x32-10
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
@@ -828,8 +851,8 @@ __device__ __forceinline__ void fill_outside(const Warp& w, const GEO& g, const 
 // reads its N cells straight from the staged byte grid -- one unaligned 16-byte run for UP / DOWN (5 aligned words + funnel
 // shifts), N byte loads down a column for LEFT / RIGHT -- packs them to nibbles, replaces the cells outside the map by
 // index 6, reverses the run for DOWN / RIGHT, and colours 4 pixels per PRMT as the map path does.  No padded maps are built.
-// The grid tile has V rows of slack on both sides (zeroed at kernel start), so no load needs a bounds test; agents were
-// written into the staged grid as index 7 by the caller.
+// The grid tile has V + f rows of slack on both sides (zeroed at kernel start; f the view offset), so no load needs a bounds
+// test; agents were written into the staged grid as index 7 by the caller.
 template <bool COLS, bool IDX, class GEO>
 __device__ __forceinline__ void gather_class(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, const uint8_t* rank2lane,
                                              uint8_t* gobs, int lane, uint32_t apack, int n_in_class, unsigned outm) {
@@ -843,7 +866,9 @@ __device__ __forceinline__ void gather_class(const Warp& w, const GEO& g, const 
         const int al = rank2lane[rank];
         const uint32_t ap = w.shfl(apack, al);
         if (!valid) continue;
-        const int ar = (int)(ap & 0xffu), ac = (int)((ap >> 8) & 0xffu), o = (int)(ap >> 16);
+        int ar = (int)(ap & 0xffu), ac = (int)((ap >> 8) & 0xffu);
+        const int o = (int)(ap >> 16);
+        if (!((outm >> al) & 1u)) window_centre(g, o, ar, ac);    // (ar, ac): the window centre, which may lie off the map
         uint32_t b0, b1, b2, b3;                              // element i of the run (ascending map coordinate) in byte i
         int lo, hi;                                           // elements inside the map: [lo, hi)
         if (!COLS) {                                          // UP / DOWN: a run along map row R
@@ -851,7 +876,7 @@ __device__ __forceinline__ void gather_class(const Warp& w, const GEO& g, const 
             const bool rv = (unsigned)R < (unsigned)g.H();
             lo = rv ? max(0, V - ac) : 0;
             hi = rv ? min(N, W + V - ac) : 0;
-            const int start = (rv ? R : 0) * W + ac - V;      // >= -V: inside the front slack
+            const int start = (rv ? R : 0) * W + ac - V;      // >= -(V + f): inside the front slack
             SSD_CHECK(start >= -g.padF() + 32 && start + 20 <= g.GS() + g.padB());
             const uint32_t* wp = reinterpret_cast<const uint32_t*>(sg + (start & ~3));
             const uint32_t sh = (uint32_t)(start & 3) * 8u;
@@ -863,7 +888,7 @@ __device__ __forceinline__ void gather_class(const Warp& w, const GEO& g, const 
             const bool cv = (unsigned)C < (unsigned)W;
             lo = cv ? max(0, V - ar) : 0;
             hi = cv ? min(N, g.H() + V - ar) : 0;
-            const uint8_t* col = sg + (ar - V) * W + (cv ? C : 0);     // rows ar-V .. ar+V: at most V rows into either slack
+            const uint8_t* col = sg + (ar - V) * W + (cv ? C : 0);     // rows ar-V .. ar+V: at most V + f rows into either slack
             SSD_CHECK((ar - V) * W >= -g.padF() + 32 && (ar + V) * W + W <= g.GS() + g.padB());
             uint32_t e[16];
 #pragma unroll
@@ -994,8 +1019,10 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
         // the staged grid as index 7)
         // per agent: which map, first word of its window row 0, row step, funnel shift, direction   (o: 0 LEFT 1 RIGHT 2 UP 3 DOWN)
         const bool colmap = ori < 2, rev = (ori == 1) || (ori == 3);
-        const int rowc = colmap ? c0 : r0;                        // coordinate that selects the map row
-        const int runc = colmap ? r0 : c0;                        // coordinate along the run
+        int wr = r0, wc = c0;                                     // the window centre (an agent out of play: cell (0, 0))
+        if (live) window_centre(g, ori, wr, wc);
+        const int rowc = colmap ? wc : wr;                        // coordinate that selects the map row
+        const int runc = colmap ? wr : wc;                        // coordinate along the run (the one the view offset moves)
         const int pitch = colmap ? g.pitchT() : g.pitchM();
         const bool down = (ori == 0) || (ori == 3);               // window row y walks towards smaller map rows
         const int s = g.LPn() + runc + (rev ? g.V() : -g.V());    // first pixel of the run (highest nibble when descending)
@@ -1035,7 +1062,12 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             const uint32_t api = w.shfl(apack, al), apj = w.shfl(apack, j);
             const bool topj = w.shfl((int)top, j);
             if (!valid || !topj || ((outm >> al) & 1u)) continue;
-            const int a = (int)(apj & 1023) - (int)(api & 1023) + g.V(), b = (int)((apj >> 10) & 1023) - (int)((api >> 10) & 1023) + g.V();
+            int a = (int)(apj & 1023) - (int)(api & 1023) + g.V(), b = (int)((apj >> 10) & 1023) - (int)((api >> 10) & 1023) + g.V();
+            if (g.view_offset()) {                                // the viewer's window centre moves; agent j is painted where it stands
+                int sr = 0, sc = 0;
+                window_centre(g, (int)(api >> 20), sr, sc);
+                a -= sr; b -= sc;
+            }
             if (a < 0 || a >= g.N() || b < 0 || b >= g.N()) continue;
             const int o = api >> 20;
             int y, x;
@@ -1462,6 +1494,20 @@ uint32_t magic20(int d, int max_x) {
     return m;
 }
 
+// The map path addresses its tile with 16-bit byte offsets (render's abase_sh).
+constexpr int kMaxPMS = 60000;
+
+// Dynamic shared memory of a launch: one staging tile per warp.
+size_t tile_bytes(const GeoVals& g) { return (size_t)kWarps * (g.padF + g.GS + g.padB + g.PMS); }
+
+// fits: smem_bytes of dynamic shared memory plus the static colour LUTs fit the device's opt-in limit per block.
+cudaError_t smem_fits(int device, size_t smem_bytes, bool& fits) {
+    int optin = 0;
+    const cudaError_t e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    fits = e == cudaSuccess && smem_bytes + sizeof(ColourLuts) <= (size_t)optin;
+    return e;
+}
+
 // Observation strides of one format (ssd_get_obs_layout; ssd_step_host copies B * env_stride bytes).
 ssd_obs_layout obs_layout(const KParams& k, int32_t format) {
     const GeoVals& g = k.geo;
@@ -1619,10 +1665,12 @@ static int launch_geo(ssd_handle* h, const KParams& k_in, void* stream) {
     return launch_var<MODE, GEO, false, false>(h, k, stream);
 }
 
-// The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.
+// The reference's shipped geometries (constants.py maps x yaml view sizes) get compile-time index arithmetic.  A handle with a
+// view offset runs the offset geometry's kernels, whatever SSD_B200_GENERIC says.
 template <int MODE>
 static int launch(ssd_handle* h, const KParams& k, void* stream) {
     const GeoVals& v = k.geo;
+    if (k.view_offset) return launch_geo<MODE, GeoO>(h, k, stream);
     if (!h->force_generic) {
         if (v.kind == SSD_KIND_HARVEST && v.H == 9 && v.W == 38 && v.V == 15) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 15>>(h, k, stream);
         if (v.kind == SSD_KIND_HARVEST && v.H == 9 && v.W == 38 && v.V == 7) return launch_geo<MODE, GeoS<SSD_KIND_HARVEST, 9, 38, 7>>(h, k, stream);
@@ -1775,8 +1823,8 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     if (k.invN20 == 0 || k.invW20 == 0) { delete v0; delete h; return SSD_ERR_INVALID; }
 
     k.invMW20 = magic20(gv.nw8M, H * gv.nw8M + 32);
-    if (k.invMW20 == 0 || gv.PMS >= 60000) { delete v0; delete h; return SSD_ERR_INVALID; }
-    h->smem_bytes = (size_t)kWarps * (gv.padF + gv.GS + gv.padB + gv.PMS);     // one staging tile per warp
+    if (k.invMW20 == 0 || gv.PMS >= kMaxPMS) { delete v0; delete h; return SSD_ERR_INVALID; }
+    h->smem_bytes = tile_bytes(gv);
     { const char* e = getenv("SSD_B200_GENERIC"); h->force_generic = e && e[0] == '1'; }
     { const char* e = getenv("SSD_B200_PDL"); h->pdl = !(e && e[0] == '0'); }
     h->device = cfg->device;
@@ -1784,9 +1832,9 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out) {
     DeviceGuard guard(cfg->device);
     cudaError_t e = guard.err;
     if (e == cudaSuccess) {                                   // the launch needs smem_bytes dynamic + the static LUTs
-        int optin = 0;
-        e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, cfg->device);
-        if (e == cudaSuccess && h->smem_bytes + sizeof(ColourLuts) > (size_t)optin) { delete v0; delete h; return SSD_ERR_INVALID; }
+        bool fits = false;
+        e = smem_fits(cfg->device, h->smem_bytes, fits);
+        if (e == cudaSuccess && !fits) { delete v0; delete h; return SSD_ERR_INVALID; }
     }
     if (e == cudaSuccess) e = cudaMalloc(&h->d_map, sizeof(MapDev));
     if (e == cudaSuccess) e = cudaMemcpy(h->d_map, hm, sizeof(MapDev), cudaMemcpyHostToDevice);
@@ -1831,6 +1879,23 @@ int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* o) {
 int ssd_set_obs_format(ssd_handle* h, int32_t format) {
     if (!h || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
     h->obs_format = format;
+    return SSD_OK;
+}
+
+int ssd_set_view_offset(ssd_handle* h, int32_t offset) {
+    if (!h || offset < 0 || offset > h->kp.geo.V) return SSD_ERR_INVALID;
+    const GeoVals& g = h->kp.geo;
+    const GeoVals geo = make_geo(g.kind, g.H, g.W, g.V, offset);
+    if (geo.PMS >= kMaxPMS) return SSD_ERR_INVALID;
+    const size_t smem = tile_bytes(geo);
+    DeviceGuard guard(h->device);
+    SSD_CUDA(guard.err);
+    bool fits = false;
+    SSD_CUDA(smem_fits(h->device, smem, fits));
+    if (!fits) return SSD_ERR_INVALID;
+    h->kp.geo = geo;
+    h->kp.view_offset = offset;
+    h->smem_bytes = smem;
     return SSD_OK;
 }
 

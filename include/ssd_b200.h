@@ -227,6 +227,19 @@ int ssd_get_state_layout(const ssd_handle* h, int32_t format, ssd_state_layout* 
  * SSD_ERR_INVALID, before any CUDA call, for a NULL handle or an unknown format. */
 int ssd_set_state_format(ssd_handle* h, int32_t format);
 
+/* Forward-offset observation windows (DESIGN.md §3 item 18).  Every later observation of ssd_reset, ssd_step, ssd_step_range,
+ * ssd_step_autoreset (obs and the episode-end obs), ssd_render and ssd_step_host is the view an agent at (r, c) facing o would
+ * have with offset 0, the default and the reference's view, but with the N x N window centred on (r + f*dr, c + f*dc), where
+ * (dr, dc) is the agent's firing direction (LEFT (-1, 0), RIGHT (+1, 0), UP (0, -1), DOWN (0, +1), as ssd_step's FIRE travels):
+ * the agent sees V + f cells ahead, V - f behind and V to either side, and its own cell is pixel (V, V + f) of its view.  Cells
+ * outside the map, the agent overlay, both colour schemes, tagging-out and the rotation by orientation are as with offset 0, and
+ * so are the observation strides: no buffer is reallocated, and every buffer but the observations is bit-identical to that of a
+ * handle with offset 0.  A handle with f > 0 runs kernels of its own, whatever SSD_B200_GENERIC says.
+ * SSD_ERR_INVALID, before any CUDA call, for a NULL handle or an offset outside 0..view; and SSD_ERR_INVALID when the wider
+ * staging tile does not fit the device's opt-in shared memory (the check ssd_create makes).  On an error nothing changes.
+ * Host-side and serialised like ssd_set_obs_format; a CUDA graph keeps the offset it was captured with. */
+int ssd_set_view_offset(ssd_handle* h, int32_t offset);
+
 /* Sets the handle's variant table to variants[0 .. n_variants) (DESIGN.md §3 item 15), entry 0 included; n_variants = 0 restores
  * the creation config as the only variant.  Env b running variant v is bit-identical, in every buffer and pad byte, to env b of a
  * handle created with v's config alone (same seed and env_gid_base), in every call.  Each entry is validated as ssd_create

@@ -25,6 +25,7 @@ SSD_N_STATS = len(STAT_NAMES)
 EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_prob_to_threshold",
            "ssd_create", "ssd_destroy", "ssd_get_layout", "ssd_get_obs_layout", "ssd_set_obs_format", "ssd_expand_obs",
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state", "ssd_set_view_offset",
+           "ssd_obs_mask_words", "ssd_set_obs_mask",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
            "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats", "ssd_set_reward_shaping",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
@@ -117,6 +118,8 @@ def load():
     L.ssd_set_state_format.argtypes = [C.c_void_p, C.c_int32]
     L.ssd_expand_state.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
     L.ssd_set_view_offset.argtypes = [C.c_void_p, C.c_int32]
+    L.ssd_obs_mask_words.argtypes = [C.c_void_p]
+    L.ssd_set_obs_mask.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.ssd_set_variants.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdVariant)]
     L.ssd_set_env_variants.argtypes = [C.c_void_p, C.c_void_p]
     L.ssd_set_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]

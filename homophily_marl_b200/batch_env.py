@@ -12,6 +12,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 
 import numpy as np
 import torch
@@ -33,6 +34,10 @@ OBS_FORMATS = {"rgb": _capi.SSD_OBS_RGB, "index4": _capi.SSD_OBS_INDEX4}
 
 def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def _addr(t):
+    return None if t is None else t.data_ptr()
 
 
 class SSDBatchEnv:
@@ -111,6 +116,7 @@ class SSDBatchEnv:
         if self.view_offset:
             _capi.check(self.lib.ssd_set_view_offset(self._h, self.view_offset))
         self.obs_format, self.obs_layout = "rgb", self.get_obs_layout("rgb")
+        self.obs_mask_words = int(self.lib.ssd_obs_mask_words(self._h))
         if extra["obs_format"] != "rgb":
             self._set_format(extra["obs_format"])
         self.state_format, self.state_layout = "rgb", self.get_state_layout("rgb")
@@ -136,8 +142,12 @@ class SSDBatchEnv:
         self.apple_cnt = z((B,), torch.int16)
         self.done = z((B,), torch.uint8)
         self.keep_episode_end = bool(keep_episode_end)
-        self.obs_buf = self.new_obs_buffer()
-        self.end_obs_buf = self.new_obs_buffer() if self.keep_episode_end else None
+        # row masks of the tracked observation buffers (new_obs_buffer): data_ptr -> (mask, bytes); obs_buf and end_obs_buf are
+        # plain buffers, which callers may fill themselves
+        self._obs_masks = {}
+        self._mask_pair = None                                 # the pointers ssd_set_obs_mask last received
+        self.obs_buf = self.new_obs_buffer(track=False)
+        self.end_obs_buf = self.new_obs_buffer(track=False) if self.keep_episode_end else None
         self.end_ep_ret_buf = z((B, lay.agent_stride), torch.int32) if self.keep_episode_end else None
         self.stats_buf = self.end_stats_buf = None
         if extra["episode_stats"]:
@@ -197,6 +207,8 @@ class SSDBatchEnv:
     def _set_format(self, fmt):
         _capi.check(self.lib.ssd_set_obs_format(self._h, OBS_FORMATS[fmt]))
         self.obs_format, self.obs_layout = fmt, self.get_obs_layout(fmt)
+        self.obs_mask_words = int(self.lib.ssd_obs_mask_words(self._h))
+        self._mask_pair = None                                 # ssd_set_obs_format cleared the pairing
 
     def set_obs_format(self, fmt):
         """Switches the format every later step / reset / render writes, and reallocates ``obs_buf`` for it.  Host-side: a
@@ -205,9 +217,9 @@ class SSDBatchEnv:
             raise ValueError(f"obs_format must be one of {sorted(OBS_FORMATS)}, got {fmt!r}")
         self._set_format(fmt)
         self.extra_args["obs_format"] = fmt
-        self.obs_buf = self.new_obs_buffer()
+        self.obs_buf = self.new_obs_buffer(track=False)
         if self.keep_episode_end:
-            self.end_obs_buf = self.new_obs_buffer()
+            self.end_obs_buf = self.new_obs_buffer(track=False)
 
     # ------------------------------------------------------------------ state image format
     def get_state_layout(self, fmt):
@@ -277,9 +289,58 @@ class SSDBatchEnv:
         return out
 
     # ------------------------------------------------------------------ buffers / views
-    def new_obs_buffer(self):
-        """Flat u8 [B, env_stride] buffer in the layout of the current observation format."""
-        return torch.zeros((self.B, self.obs_layout.env_stride), dtype=torch.uint8, device=self.device)
+    def new_obs_buffer(self, track=True):
+        """Flat u8 [B, env_stride] zeroed buffer in the layout of the current observation format.
+
+        With ``track`` (the default), and where the kernels can use it (RGB views with 32-byte rows: view size 14 or 15, at most
+        320 rows per env and plane), the env keeps a row mask beside the buffer (ssd_set_obs_mask; DESIGN.md §3 item 19): a
+        write through this env then skips the pixel rows that are zero now and were zero when it last wrote the buffer, and the
+        buffer holds exactly what full stores would leave.  So write into a tracked buffer only through this env's ``reset`` /
+        ``step`` / ``step_range`` / ``render``, or call ``mark_obs_dirty(buf)`` after writing into it yourself.  ``obs_buf``
+        and ``end_obs_buf`` are not tracked."""
+        buf = torch.zeros((self.B, self.obs_layout.env_stride), dtype=torch.uint8, device=self.device)
+        if track and self.obs_mask_words:
+            ptr = buf.data_ptr()
+            self._obs_masks[ptr] = (torch.zeros((self.B, self.obs_mask_words), dtype=torch.int32, device=self.device),
+                                    buf.numel())
+            # the entry dies with the tensor, before its memory can be handed to another tensor
+            weakref.finalize(buf, self._obs_masks.pop, ptr, None)
+        return buf
+
+    def obs_mask(self, buf):
+        """The int32 [B, obs_mask_words] row mask of a tracked buffer (None for an untracked one): bit u % 32 of word
+        3 * (u // 32) + plane covers pixel row u = agent * N + y; a clear bit means the row is all zero in ``buf``."""
+        e = self._obs_masks.get(buf.data_ptr())
+        return None if e is None else e[0]
+
+    def mark_obs_dirty(self, buf):
+        """Sets every bit of the row masks of the tracked buffers that ``buf`` overlaps (on the current stream), so that the next
+        write through this env stores every row: call it after writing into a tracked buffer other than through this env."""
+        self._dirty(buf.data_ptr(), buf.numel() * buf.element_size())
+
+    def _dirty(self, lo, nbytes):
+        for p0, (m, n0) in list(self._obs_masks.items()):
+            if p0 < lo + nbytes and lo < p0 + n0:
+                m.fill_(-1)
+
+    def _launch_mask(self, buf):
+        """The row mask a launch writing observations into ``buf`` maintains, or None (full stores).  A full-store launch
+        into (part of) a tracked buffer first marks that buffer dirty."""
+        if buf is None:
+            return None
+        e = self._obs_masks.get(buf.data_ptr())
+        if e is not None and self.obs_mask_words and buf.numel() * buf.element_size() >= self.B * self.obs_layout.env_stride:
+            return e[0]
+        self._dirty(buf.data_ptr(), self.B * self.obs_layout.env_stride)
+        return None
+
+    def _set_obs_masks(self, obs, end_obs=None):
+        """ssd_set_obs_mask for the next launch (only when the pairing changes)."""
+        m, em = self._launch_mask(obs), self._launch_mask(end_obs)
+        pair = (_addr(obs) if m is not None else None, _addr(m), _addr(end_obs) if em is not None else None, _addr(em))
+        if pair != self._mask_pair:
+            _capi.check(self.lib.ssd_set_obs_mask(self._h, *pair))
+            self._mask_pair = pair
 
     def obs_view(self, buf=None):
         """[B, n, 3, N, N] u8 view (no copy) of an RGB obs buffer; ``view / 256`` equals get_obs()."""
@@ -476,6 +537,7 @@ class SSDBatchEnv:
         out = None if not obs else (self.obs_buf if obs_out is None else obs_out)
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+        self._set_obs_masks(out)
         _capi.check(self.lib.ssd_reset(self._h, C.byref(self._st), _ptr(mask), C.byref(d) if d else None,
                                        _ptr(out), self._stream()))
 
@@ -486,7 +548,9 @@ class SSDBatchEnv:
             # the reference raises KeyError from action_map (agent.py:176,237); the kernel alone would treat the code as a no-op
             raise KeyError(int(actions.max()))
 
-    def _step_out(self, obs_out, want_obs, want_state):
+    def _step_out(self, obs_out, want_obs, want_state, end_obs=None):
+        """The ssd_step_out of a launch; also pairs the row masks of its observation buffers (``end_obs``: the episode-end one)."""
+        self._set_obs_masks((self.obs_buf if obs_out is None else obs_out) if want_obs else None, end_obs)
         return _capi.SsdStepOut(self.reward.data_ptr(), self.clean.data_ptr(), self.apple_cnt.data_ptr(),
                                 self.done.data_ptr(),
                                 (self.obs_buf if obs_out is None else obs_out).data_ptr() if want_obs else None,
@@ -524,7 +588,8 @@ class SSDBatchEnv:
         overlap another group's observation stores."""
         self._check_actions(actions)
         d = self._draws(draws)
-        so = self._step_out(obs_out, want_obs, want_state)
+        end_obs = self.end_obs_buf if (auto_reset and self.keep_episode_end and want_obs) else None
+        so = self._step_out(obs_out, want_obs, want_state, end_obs)
         if auto_reset:
             end = self._episode_end(want_obs, want_state)
             _capi.check(self.lib.ssd_step_autoreset(self._h, C.byref(self._st), _ptr(actions), C.byref(d) if d else None,
@@ -537,6 +602,7 @@ class SSDBatchEnv:
     def render(self, obs_out=None, want_obs=True, want_state=False):
         o = (self.obs_buf if obs_out is None else obs_out) if want_obs else None
         s = self.state_buf if want_state else None
+        self._set_obs_masks(o)
         _capi.check(self.lib.ssd_render(self._h, C.byref(self._st), _ptr(o), _ptr(s), self._stream()))
 
     def make_host_io(self, with_obs=True, with_state=False):

@@ -134,7 +134,18 @@ struct KParams {
     int n_variants;
     uint32_t* stats; uint32_t* end_stats;     // STATS kernels: per-agent episode counters (ssd_set_stats; DESIGN.md §3 item 16)
     int view_offset;                          // GeoO kernels: window centre f cells ahead (ssd_set_view_offset; DESIGN.md §3 item 18)
+    uint32_t* obs_mask; uint32_t* end_obs_mask;   // row masks of obs / end_obs, or NULL: full stores (ssd_set_obs_mask; §3 item 19)
 };
+
+// Row masks of tracked observation buffers (ssd_set_obs_mask; DESIGN.md §3 item 19): one bit per (agent, plane, pixel row) of an
+// env's views, set when the row may hold a non-zero byte.  Row u = agent * N + y of plane pl is bit u & 31 of word
+// 3 * (u >> 5) + pl: word 3 * it + pl is the ballot of plane pl over the 32 rows a warp emits in trip `it` of gather_rows.  Only
+// where one row store covers whole 32-byte sectors of its own (RGB, row stride 32: N = 29, 31) and the words of an env fit one
+// per lane; everywhere else 0 words, and the stores stay full.
+__host__ __device__ constexpr int obs_mask_words(const GeoVals& g, int n) {
+    const int words = 3 * ((n * g.N + 31) / 32);
+    return g.RP == 32 && words <= 32 ? words : 0;
+}
 
 // STATS: one agent's counter deltas of a step, packed in one register so that the step's live registers stay flat.  Bits: 0 ate an
 // apple, 1 fired, 2 started the step out of play, 3-4 FIRE rays of its beam that hit an agent (<= 3), 5-10 rays that hit it
@@ -707,9 +718,12 @@ __device__ __forceinline__ void fetch_row(const Warp& w, const GEO& g, const KPa
     }
 }
 
+// old3 (RGB, OCT_T == 4): bit pl set when plane pl's row must be stored even if it is all zero now (its row-mask bit was set,
+// or the buffer is not tracked).  Returns the planes whose row holds a non-zero byte: the row's new mask bits.
 template <int OCT_T, bool IDX, class GEO>
-__device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const RowUnit<OCT_T>& U, uint32_t lastmask) {
-    if (!U.valid) return;
+__device__ __forceinline__ uint32_t emit_row(const GEO& g, const KParams& p, const RowUnit<OCT_T>& U, uint32_t lastmask, uint32_t old3) {
+    uint32_t nz3 = 0u;
+    if (!U.valid) return nz3;
     const uint32_t sh = U.sh;
     if constexpr (IDX) {                                      // lastmask: valid nibbles of the row's last word
         if constexpr (OCT_T > 0) {
@@ -739,8 +753,22 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
 #pragma unroll
             for (int k = 0; k < 2 * OCT_T; ++k) o[k] = prmt(t0, t1, v[k]);
             o[2 * OCT_T - 1] &= lastmask;
-            if (OCT_T == 4) st_row32(U.dst + pl * g.PS(), o);
-            else st_row16(U.dst + pl * g.PS(), o);
+            if (OCT_T == 4) {                                 // a row that is zero now and was zero before is not stored
+                uint32_t any = 0u;
+#pragma unroll
+                for (int k = 0; k < 8; ++k) any |= o[k];
+                nz3 |= (uint32_t)(any != 0u) << pl;
+                if (any != 0u || ((old3 >> pl) & 1u)) st_row32(U.dst + pl * g.PS(), o);
+#ifdef SSD_BOUNDS_CHECK
+                else {                                        // the mask says this row is zero in memory: check it
+                    const uint32_t* q = reinterpret_cast<const uint32_t*>(U.dst + pl * g.PS());
+                    uint32_t acc = 0u;
+#pragma unroll 1
+                    for (int k = 0; k < 8; ++k) acc |= __ldcg(q + k);
+                    SSD_CHECK(acc == 0u);
+                }
+#endif
+            } else st_row16(U.dst + pl * g.PS(), o);
         }
     } else {
         const int WR = g.RP() >> 2, OCT = (WR + 1) >> 1;
@@ -759,11 +787,30 @@ __device__ __forceinline__ void emit_row(const GEO& g, const KParams& p, const R
             }
         }
     }
+    return nz3;
 }
 
-template <int OCT_T, bool IDX, class GEO>
+// The row-mask words of env `env` in the mask of the observation buffer (`end`: the episode-end one), or NULL when the buffer is
+// not tracked.  Recomputed from the launch parameters where it is used: a pointer held across the render costs the auto-reset
+// kernels spills.
+template <class GEO>
+__device__ __forceinline__ uint32_t* obs_mask_of(const GEO& g, const KParams& p, bool end, int env) {
+    uint32_t* const m = end ? p.end_obs_mask : p.obs_mask;
+    return m ? m + (size_t)env * (3 * ((p.n * g.N() + 31) / 32)) : nullptr;
+}
+
+// RGB, OCT_T == 4: with a row mask (obs_mask_of), lane k loads word k of the env's mask as the previous write left it (all ones
+// for an untracked buffer, so that every row is stored) and writes the new word k back at the end.  One register holds both:
+// trip `it` reads old words 3 it .. 3 it + 2 before its ballots replace them.
+template <int OCT_T, bool IDX, bool MASKS, class GEO>
 __device__ __forceinline__ void gather_rows(const Warp& w, const GEO& g, const KParams& p, const uint8_t* pmap, uint8_t* gobs, int lane,
-                                            uint32_t abase_sh, int astep, unsigned outm) {
+                                            uint32_t abase_sh, int astep, unsigned outm, bool end, int env) {
+    constexpr bool SKIP = OCT_T == 4 && !IDX && MASKS;
+    uint32_t bits = 0xffffffffu;
+    if (SKIP) {
+        const uint32_t* const m = obs_mask_of(g, p, end, env);
+        if (m && lane < 3 * ((p.n * g.N() + 31) / 32)) bits = __ldcg(m + lane);
+    }
     const int WR = g.RP() >> 2;
     const uint32_t lastmask = IDX ? 0xffffffffu >> (4 * (8 * ((WR + 1) >> 1) - g.N())) : 0xffffffffu >> (8 * (4 * WR - g.N()));
     const int units = p.n * g.N(), iters = (units + 31) / 32;
@@ -771,8 +818,25 @@ __device__ __forceinline__ void gather_rows(const Warp& w, const GEO& g, const K
     fetch_row<OCT_T, IDX>(w, g, p, pmap, gobs, lane, 0, units, abase_sh, astep, outm, cur);
     for (int it = 0; it < iters; ++it) {                      // software pipeline: row it+1 is fetched while row it is emitted
         if (it + 1 < iters) fetch_row<OCT_T, IDX>(w, g, p, pmap, gobs, lane, it + 1, units, abase_sh, astep, outm, nxt);
-        emit_row<OCT_T, IDX>(g, p, cur, lastmask);
+        uint32_t old3 = 7u;
+        if (SKIP) {
+            old3 = 0u;
+#pragma unroll
+            for (int pl = 0; pl < 3; ++pl) old3 |= ((w.shfl(bits, 3 * it + pl) >> lane) & 1u) << pl;
+        }
+        const uint32_t nz3 = emit_row<OCT_T, IDX>(g, p, cur, lastmask, old3);
+        if (SKIP) {
+#pragma unroll
+            for (int pl = 0; pl < 3; ++pl) {
+                const unsigned b = w.ballot((nz3 >> pl) & 1u);
+                if (lane == 3 * it + pl) bits = b;
+            }
+        }
         cur = nxt;
+    }
+    if (SKIP) {
+        uint32_t* const m = obs_mask_of(g, p, end, env);
+        if (m && lane < 3 * iters) m[lane] = bits;
     }
 }
 
@@ -956,7 +1020,9 @@ __device__ __forceinline__ void gather_direct(const Warp& w, const GEO& g, const
 
 // live: the lane's agent is on the map; outm: agents out of play (tagged out), whose views are written as zeros.  Their rows go
 // through the same gather at cell (0, 0), masked, so that a warp trip never mixes two kinds of row.
-template <bool IDX, class GEO>
+// MASKS: this kernel keeps the row masks (ssd_set_obs_mask).  The auto-reset kernels, which inline the render twice, have no
+// registers left for them: they store every row, and ssd_step_autoreset sets the masks of their envs to all ones.
+template <bool IDX, bool MASKS, class GEO>
 __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParams& p, const uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s,
                                        int lane, bool is_agent, bool live, int pos, int ori, int env, unsigned same, unsigned outm,
                                        bool end) {
@@ -1038,8 +1104,8 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             build_colmap(w, g, p, M, MT, lane);
             w.sync();
         }
-        if (g.RP() == 32) gather_rows<4, IDX>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
-        else gather_rows<0, IDX>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm);
+        if (g.RP() == 32) gather_rows<4, IDX, MASKS>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm, end, env);
+        else gather_rows<0, IDX, false>(w, g, p, pmap, gobs, lane, abase_sh, astep, outm, end, env);
     }
     if constexpr (IDX) {                                          // pad bytes per agent block (8 for N = 15)
         const int body = g.N() * g.RS4(), tail = g.AS4() - body;
@@ -1076,6 +1142,13 @@ __device__ __forceinline__ void render(const Warp& w, const GEO& g, const KParam
             const uint32_t rgb = lut_s[agent_colour_index(j)];
             uint8_t* d = gobs + al * g.AS() + y * g.RP() + x;
             d[0] = (uint8_t)rgb; d[g.PS()] = (uint8_t)(rgb >> 8); d[2 * g.PS()] = (uint8_t)(rgb >> 16);
+            uint32_t* const m = MASKS && !g.direct() && g.RP() == 32 ? obs_mask_of(g, p, end, env) : nullptr;
+            if (m) {                                              // a painted pixel may land on a row stored as zeros: mark it
+                const int u = al * g.N() + y;                     // (gather_rows stored the words before the w.sync above)
+#pragma unroll
+                for (int pl = 0; pl < 3; ++pl)
+                    if ((rgb >> (8 * pl)) & 0xffu) atomicOr(m + 3 * (u >> 5) + pl, 1u << (u & 31));
+            }
         }
     }
 }
@@ -1113,7 +1186,7 @@ __device__ __forceinline__ void write_back_reset(const Warp& w, const GEO& g, co
 }
 
 // The agent overlay, then render (`end`: into the episode-end buffers).
-template <bool TAG, bool IDX, class GEO>
+template <bool TAG, bool IDX, bool MASKS, class GEO>
 __device__ __forceinline__ void draw(const Warp& w, const GEO& g, const KParams& p, uint8_t* sg, uint8_t* pmap, const uint32_t* lut_s, int lane,
                                      bool is_agent, bool live, int pos, int ori, int env, unsigned same, bool end) {
     // agent overlay: every occupied cell shows an agent (index 7; which agent only matters for the full-colour repaint and
@@ -1124,7 +1197,7 @@ __device__ __forceinline__ void draw(const Warp& w, const GEO& g, const KParams&
     else if (live) sg[pos] = 7;
     w.sync();
     const unsigned outm = TAG ? w.ballot(is_agent && !live) : 0u;
-    render<IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm, end);
+    render<IDX, MASKS>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, outm, end);
 }
 
 // ------------------------------------------------------------------ the kernel
@@ -1340,7 +1413,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
             // them); every env then renders into the step outputs below.
             if (ended) {
                 if (is_agent && p.end_ep_ret) p.end_ep_ret[(size_t)env * p.NA + lane] = ep_ret;
-                if (p.end_obs || p.end_state) draw<TAG, IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, true);
+                if (p.end_obs || p.end_state) draw<TAG, IDX, MODE != MODE_STEP_RESET>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, true);
                 // The base grid is staged again.  Nothing else needs restoring: a render never writes the slack or the "outside"
                 // fill of the maps, and it rebuilds every map cell it reads.
                 w.sync();                                          // the render has read the staged grid
@@ -1352,7 +1425,7 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) ssd_kernel(const __gr
                 live = is_agent; same = 1u << lane;
             }
         }
-        if (p.obs || p.state_rgb) draw<TAG, IDX>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, false);
+        if (p.obs || p.state_rgb) draw<TAG, IDX, MODE != MODE_STEP_RESET>(w, g, p, sg, pmap, lut_s, lane, is_agent, live, pos, ori, env, same, false);
     }
 }
 
@@ -1541,7 +1614,15 @@ struct ssd_handle {
     ShapeDev* d_shape;                                        // shaping table: SSD_MAX_VARIANTS records, allocated once when first needed
     int n_shape;                                              // entries in use; 0 = shaping off
     float* shape_trace; float* shaped;                        // caller-owned [B][NA] (ssd_set_reward_shaping)
+    const uint8_t* mask_obs; uint32_t* mask_obs_bits;         // ssd_set_obs_mask: the buffers the row masks describe, and the masks
+    const uint8_t* mask_end_obs; uint32_t* mask_end_bits;
 };
+
+// The row masks of a launch (ssd_set_obs_mask): a mask is used only by a launch whose buffer is the one it was set with.
+static void apply_obs_masks(const ssd_handle* h, KParams& k) {
+    k.obs_mask = k.obs && k.obs == h->mask_obs ? h->mask_obs_bits : nullptr;
+    k.end_obs_mask = k.end_obs && k.end_obs == h->mask_end_obs ? h->mask_end_bits : nullptr;
+}
 
 static int fill_common(const ssd_handle* h, const ssd_state* st, const ssd_draws* d, KParams& k) {
     if (!h || !st || !st->grid || !st->agent || !st->ep_ret || !st->t || !st->tick || !st->counts) return SSD_ERR_INVALID;
@@ -1879,6 +1960,20 @@ int ssd_get_obs_layout(const ssd_handle* h, int32_t format, ssd_obs_layout* o) {
 int ssd_set_obs_format(ssd_handle* h, int32_t format) {
     if (!h || (format != SSD_OBS_RGB && format != SSD_OBS_INDEX4)) return SSD_ERR_INVALID;
     h->obs_format = format;
+    h->mask_obs = h->mask_end_obs = nullptr; h->mask_obs_bits = h->mask_end_bits = nullptr;   // the masks describe the old format
+    return SSD_OK;
+}
+
+int ssd_obs_mask_words(const ssd_handle* h) {
+    if (!h) return SSD_ERR_INVALID;
+    return h->obs_format == SSD_OBS_RGB ? obs_mask_words(h->kp.geo, h->kp.n) : 0;
+}
+
+int ssd_set_obs_mask(ssd_handle* h, const uint8_t* obs, uint32_t* obs_mask, const uint8_t* end_obs, uint32_t* end_obs_mask) {
+    if (!h || (obs_mask && !obs) || (end_obs_mask && !end_obs)) return SSD_ERR_INVALID;
+    if ((obs_mask || end_obs_mask) && ssd_obs_mask_words(h) <= 0) return SSD_ERR_INVALID;
+    h->mask_obs = obs_mask ? obs : nullptr; h->mask_obs_bits = obs_mask;
+    h->mask_end_obs = end_obs_mask ? end_obs : nullptr; h->mask_end_bits = end_obs_mask;
     return SSD_OK;
 }
 
@@ -1996,6 +2091,7 @@ int ssd_reset(ssd_handle* h, const ssd_state* st, const uint8_t* mask, const ssd
     const int rc = fill_common(h, st, draws, k);
     if (rc) return rc;
     k.mask = mask; k.obs = obs;
+    apply_obs_masks(h, k);
     int lrc = launch<MODE_RESET>(h, k, stream);
     if (!lrc && k.stats) lrc = zero_masked(h, k.stats, mask, k.B, SSD_N_STATS * k.NA, stream);
     if (!lrc && h->n_shape) lrc = zero_masked(h, reinterpret_cast<uint32_t*>(h->shape_trace), mask, k.B, k.NA, stream);
@@ -2017,6 +2113,7 @@ static int fill_step(const ssd_handle* h, const ssd_state* st, const uint8_t* ac
     k.env0 = env_begin; k.env1 = env_begin + env_count;
     k.actions = actions; k.reward = out->reward; k.clean = out->clean; k.apple_cnt = out->apple_cnt; k.done = out->done;
     k.obs = out->obs; k.state_rgb = out->state_rgb;
+    apply_obs_masks(h, k);
     return SSD_OK;
 }
 
@@ -2036,6 +2133,17 @@ int ssd_step_autoreset(ssd_handle* h, const ssd_state* st, const uint8_t* action
     const int rc = fill_step(h, st, actions, draws, out, env_begin, env_count, k);
     if (rc) return rc;
     if (end) { k.end_obs = end->obs; k.end_state = end->state_rgb; k.end_ep_ret = end->ep_ret; }
+    apply_obs_masks(h, k);
+    {   // The auto-reset kernels render twice and have no registers left for the masks: they store every row, so the masks of
+        // the envs they write are set to all ones first (the words of other ranges are not touched).
+        const int words = obs_mask_words(k.geo, k.n);
+        DeviceGuard guard(h->device);
+        SSD_CUDA(guard.err);
+        for (uint32_t* m : { k.obs_mask, k.end_obs_mask })
+            if (m && env_count > 0)
+                SSD_CUDA(cudaMemsetAsync(m + (size_t)env_begin * words, 0xff, (size_t)env_count * words * 4, (cudaStream_t)stream));
+        k.obs_mask = k.end_obs_mask = nullptr;
+    }
     const int lrc = launch<MODE_STEP_RESET>(h, k, stream);
     return lrc ? lrc : launch_shaping(h, k, k.done, stream);
 }
@@ -2046,6 +2154,7 @@ int ssd_render(ssd_handle* h, const ssd_state* st, uint8_t* obs, uint8_t* state_
     if (rc) return rc;
     if (!obs && !state_rgb) return SSD_ERR_INVALID;
     k.obs = obs; k.state_rgb = state_rgb;
+    apply_obs_masks(h, k);
     return launch<MODE_RENDER>(h, k, stream);
 }
 

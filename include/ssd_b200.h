@@ -240,6 +240,27 @@ int ssd_set_state_format(ssd_handle* h, int32_t format);
  * Host-side and serialised like ssd_set_obs_format; a CUDA graph keeps the offset it was captured with. */
 int ssd_set_view_offset(ssd_handle* h, int32_t offset);
 
+/* Row masks of tracked observation buffers (DESIGN.md §3 item 19): the render does not store a pixel row that is all zero now
+ * and was all zero when the buffer was last written, so a mostly-black view costs fewer stored bytes; every buffer still holds
+ * exactly the bytes it would hold with full stores.  A mask is a caller-owned DEVICE u32 [B][ssd_obs_mask_words(h)] array with
+ * one bit per (agent, colour plane, pixel row) of each env's views: row u = agent * N + y of plane pl is bit u % 32 of word
+ * 3 * (u / 32) + pl.  A clear bit promises that the row is all zero in the buffer; a set bit promises nothing.  So a mask of
+ * zeros goes with a zeroed buffer, a mask of ones with any buffer; whoever writes into a tracked buffer other than through the
+ * launches below sets its mask to all ones.
+ * ssd_obs_mask_words: words per env of a mask in the handle's current observation format, or 0 where the stores stay full:
+ * index4, a row stride other than 32 bytes (only N = 29 and 31 qualify), or more than 32 words per env (n * N > 320).  Negative
+ * for a NULL handle.
+ * ssd_set_obs_mask: every later ssd_reset, ssd_step, ssd_step_range, ssd_render and ssd_step_host whose observation buffer IS
+ * `obs` (the same pointer) reads and updates `obs_mask`.  ssd_step_autoreset stores every row, and sets the words of the envs of
+ * its range to all ones in `obs_mask` (buffer `obs`) and `end_obs_mask` (episode-end buffer `end_obs`), one memset each on the
+ * launch stream.  A launch with any other buffer stores every row and touches no mask.  NULL masks (the default) turn
+ * tracking off.  SSD_ERR_INVALID, before any CUDA call, for a NULL handle, a mask without its buffer, or a mask while
+ * ssd_obs_mask_words is 0.  ssd_set_obs_format clears both pairings.  Host-side and serialised like ssd_set_obs_format; a CUDA
+ * graph keeps the pairing it was captured with.  The masks of the checked build's skipped rows are verified: a skipped row that
+ * is not zero in memory is counted by ssd_debug_oob_count. */
+int ssd_obs_mask_words(const ssd_handle* h);
+int ssd_set_obs_mask(ssd_handle* h, const uint8_t* obs, uint32_t* obs_mask, const uint8_t* end_obs, uint32_t* end_obs_mask);
+
 /* Sets the handle's variant table to variants[0 .. n_variants) (DESIGN.md §3 item 15), entry 0 included; n_variants = 0 restores
  * the creation config as the only variant.  Env b running variant v is bit-identical, in every buffer and pad byte, to env b of a
  * handle created with v's config alone (same seed and env_gid_base), in every call.  Each entry is validated as ssd_create

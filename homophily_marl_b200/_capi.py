@@ -27,7 +27,7 @@ EXPORTS = ("ssd_abi_version", "ssd_error_string", "ssd_last_cuda_error", "ssd_pr
            "ssd_get_state_layout", "ssd_set_state_format", "ssd_expand_state", "ssd_set_view_offset",
            "ssd_obs_mask_words", "ssd_set_obs_mask",
            "ssd_reset", "ssd_step", "ssd_step_range", "ssd_step_autoreset", "ssd_render",
-           "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats", "ssd_set_reward_shaping",
+           "ssd_set_variants", "ssd_set_env_variants", "ssd_set_stats", "ssd_set_reward_shaping", "ssd_set_reward_preferences",
            "ssd_step_host", "ssd_incentive", "ssd_launch_count", "ssd_debug_oob_count",
            "ssd_select_actions", "ssd_policy_last_cuda_error",
            "ssd_frontend_create", "ssd_frontend_forward", "ssd_frontend_forward_index4", "ssd_frontend_destroy",
@@ -52,6 +52,10 @@ class SsdVariant(C.Structure):
 
 class SsdShaping(C.Structure):
     _fields_ = [(k, C.c_float) for k in ("alpha", "beta", "decay", "prosocial")]
+
+
+class SsdPreference(C.Structure):
+    _fields_ = [(k, C.c_float) for k in ("alpha", "beta", "decay", "prosocial", "svo_angle", "svo_weight")]
 
 
 class SsdLayout(C.Structure):
@@ -124,6 +128,8 @@ def load():
     L.ssd_set_env_variants.argtypes = [C.c_void_p, C.c_void_p]
     L.ssd_set_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.ssd_set_reward_shaping.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdShaping), C.c_void_p, C.c_void_p]
+    L.ssd_set_reward_preferences.argtypes = [C.c_void_p, C.c_int32, C.POINTER(SsdPreference), C.c_int32, C.c_void_p, C.c_void_p,
+                                             C.c_void_p]
     L.ssd_reset.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.c_void_p, C.c_void_p]
     L.ssd_step.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut), C.c_void_p]
     L.ssd_step_range.argtypes = [C.c_void_p, C.POINTER(SsdState), C.c_void_p, C.POINTER(SsdDraws), C.POINTER(SsdStepOut),

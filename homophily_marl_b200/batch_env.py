@@ -54,9 +54,10 @@ class SSDBatchEnv:
         #   dicts ({} = this config); env b runs variant variant_of[b], by default (env_gid_base + b) % len(variants)
         # episode_stats: per-agent episode counters in stats_buf (and, with keep_episode_end, end_stats_buf), the inputs of
         #   social_metrics(); without it nothing is allocated and no kernel counts
-        # reward_shaping: {"alpha", "beta", "decay", "prosocial"} (mapspec.reward_shaping), the inequity-averse / prosocial
-        #   reward every step writes to shaped_buf (trace in shape_trace_buf); a variant dict may carry its own.  Without it (and
-        #   without a variant's) nothing is allocated and no kernel runs
+        # reward_shaping: {"alpha", "beta", "decay", "prosocial", "svo_angle", "svo_weight"} (mapspec.preference), or a list of
+        #   one such dict per agent: the inequity-averse / prosocial / social-value-orientation reward every step writes to
+        #   shaped_buf (trace in shape_trace_buf); a variant dict may carry its own.  Without it (and without a variant's)
+        #   nothing is allocated and no kernel runs
         # view_offset: f in 0..view_size, the N x N window centred f cells ahead of the agent along its firing direction, so it
         #   sees view_size + f cells ahead and view_size - f behind (ssd_set_view_offset; DESIGN.md §3 item 18); 0 = the reference
         extra = dict(random_spawn_point=False, random_spawn_rotation=0, disable_rotation_action=True,
@@ -71,7 +72,7 @@ class SSDBatchEnv:
             raise ValueError(f"view_offset must be an int in 0..view_size ({view_size}), got {offset!r}")
         self.view_offset = extra["view_offset"] = int(offset)
         self.extra_args = extra
-        shaping = None if extra["reward_shaping"] is None else mapspec.reward_shaping(extra["reward_shaping"])
+        prefs = None if extra["reward_shaping"] is None else mapspec.reward_preferences(extra["reward_shaping"], int(num_agents))
         self.name = name
         self.spec = mapspec.compile_map(name, map, num_agents, view_size, episode_limit,
                                         obs_color=extra["obs_color"], rows=rows, params=params,
@@ -154,21 +155,39 @@ class SSDBatchEnv:
             self.stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32)
             self.end_stats_buf = z((B, _capi.SSD_N_STATS, lay.agent_stride), torch.int32) if self.keep_episode_end else None
             _capi.check(self.lib.ssd_set_stats(self._h, _ptr(self.stats_buf), _ptr(self.end_stats_buf)))
-        self.shape_trace_buf = self.shaped_buf = self.shaping_params = None
-        if shaping is not None or any(sp.reward_shaping is not None for sp in self.variant_specs):
-            # one parameter set per variant (ssd_set_reward_shaping): a variant's own, else the handle's, else the defaults
-            shaping = shaping or mapspec.reward_shaping({})
-            self.shaping_params = [shaping if sp.reward_shaping is None else sp.reward_shaping for sp in self.variant_specs]
-            self.shape_trace_buf = z((B, lay.agent_stride), torch.float32)
-            self.shaped_buf = z((B, lay.agent_stride), torch.float32)
-            recs = (_capi.SsdShaping * len(self.shaping_params))(*[_capi.SsdShaping(*q) for q in self.shaping_params])
-            _capi.check(self.lib.ssd_set_reward_shaping(self._h, len(recs), recs, _ptr(self.shape_trace_buf),
-                                                        _ptr(self.shaped_buf)))
+        self.shape_trace_buf = self.shaped_buf = self.shaping_params = self.preference_sets = self.preference_of = None
+        if prefs is not None or any(sp.preferences is not None for sp in self.variant_specs):
+            self._set_preferences(prefs or mapspec.reward_preferences({}, n))
         self.want_state = bool(want_state)
         self._alloc_state()
         self._st = _capi.SsdState(*[t.data_ptr() for t in (self.grid_buf, self.agent_buf, self.ep_ret_buf,
                                                             self.t_buf, self.tick_buf, self.counts_buf)])
         self._keep = None
+
+    # ------------------------------------------------------------------ shaped rewards
+    def _set_preferences(self, prefs):
+        """Allocates the shaping buffers and sets every agent's preference set: a variant's own, else the handle's ``prefs``.
+        preference_sets are the distinct sets (at most SSD_MAX_VARIANTS), preference_of [n_variants, n] the set of each agent of
+        each variant.  When every variant gives all its agents one set without social value orientation, the call is
+        ssd_set_reward_shaping with one set per variant (shaping_params); otherwise ssd_set_reward_preferences with the roster."""
+        rows = [prefs if sp.preferences is None else sp.preferences for sp in self.variant_specs]
+        sets = list(dict.fromkeys(q for row in rows for q in row))
+        if len(sets) > _capi.SSD_MAX_VARIANTS:
+            raise ValueError(f"reward_shaping needs at most {_capi.SSD_MAX_VARIANTS} distinct preference sets, got {len(sets)}")
+        self.preference_sets = tuple(sets)
+        self.preference_of = np.array([[sets.index(q) for q in row] for row in rows], dtype=np.int64)
+        z = lambda: torch.zeros((self.B, self.layout.agent_stride), dtype=torch.float32, device=self.device)  # noqa: E731
+        self.shape_trace_buf, self.shaped_buf = z(), z()
+        trace, shaped = _ptr(self.shape_trace_buf), _ptr(self.shaped_buf)
+        if all(len(set(row)) == 1 and row[0][4:] == (0.0, 0.0) for row in rows):
+            self.shaping_params = [row[0][:4] for row in rows]
+            recs = (_capi.SsdShaping * len(rows))(*[_capi.SsdShaping(*q) for q in self.shaping_params])
+            _capi.check(self.lib.ssd_set_reward_shaping(self._h, len(recs), recs, trace, shaped))
+        else:
+            recs = (_capi.SsdPreference * len(sets))(*[_capi.SsdPreference(*q) for q in sets])
+            roster = np.ascontiguousarray(self.preference_of, dtype=np.uint8)
+            _capi.check(self.lib.ssd_set_reward_preferences(self._h, len(recs), recs, len(rows), roster.ctypes.data, trace,
+                                                            shaped))
 
     # ------------------------------------------------------------------ per-env variants
     def _set_variants(self, variants, variant_of):
@@ -411,7 +430,9 @@ class SSDBatchEnv:
     def shaped_reward(self):
         """[B, n] float32 view (no copy) of the shaped reward the last step wrote (extra_args ``reward_shaping``; DESIGN.md §3
         item 17): ``(w1*r_i + w*mean_j r_j - alpha/(n-1)*D_i) - beta/(n-1)*A_i``, with D_i / A_i the summed disadvantageous /
-        advantageous gaps of the smoothed reward traces ``shape_trace_buf``."""
+        advantageous gaps of the smoothed reward traces ``shape_trace_buf``, each agent with its own preference set
+        (``preference_sets[preference_of[variant, i]]``), less ``svo_weight * |svo_angle - atan2(others' mean trace, own)|``
+        (item 20)."""
         if self.shaped_buf is None:
             raise ValueError("shaped_reward() needs extra_args reward_shaping (or a variant with its own)")
         return self.shaped_buf[:, :self.n]

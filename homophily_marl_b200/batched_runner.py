@@ -67,6 +67,7 @@ class BatchedEpisodeRunner:
         self._actions_u8 = torch.zeros((e.B, e.n), dtype=torch.uint8, device=e.device)
         self.front = None
         self._vstats = {}                                     # per-variant sums since the last flush, by test_mode
+        self._pstats = {}                                     # per-preference-set sums since the last flush, by test_mode
 
     # ---- reference surface ------------------------------------------------------------------------------
     def setup(self, scheme, groups, preprocess, mac, batch_cls=None):
@@ -229,9 +230,10 @@ class BatchedEpisodeRunner:
         if e.shaped_buf is not None:                          # reward_shaping: the shaped returns ride on the same copy
             R = torch.cat([R, torch.cat([r["sret"] for r in ranges]).double()], 1)
         R = R.cpu().numpy()
-        shaped = None
+        shaped = S = None
         if e.shaped_buf is not None:
-            R, shaped = R[:, :-e.n], R[:, -e.n:].mean(axis=1)
+            R, S = R[:, :-e.n], R[:, -e.n:]
+            shaped = S.mean(axis=1)
         R, X = R[:, :e.n], R[:, e.n:]
         coll = R.sum(axis=1)
         denom = 2 * e.n * np.abs(R).sum(axis=1)
@@ -246,6 +248,7 @@ class BatchedEpisodeRunner:
             env_info["shaped_return"] = float(shaped.sum())
             self.last_env_info["shaped_return"] = shaped
         returns = episode_return.cpu().numpy()
+        vid = None
         if len(e.variant_specs) > 1:                          # a sweep: the pooled means alone average the variants away
             vid = np.minimum(e.variant.cpu().numpy().astype(np.int64), len(e.variant_specs) - 1)
             self.last_env_info["variant"] = vid
@@ -261,6 +264,15 @@ class BatchedEpisodeRunner:
                     a[key] = a.get(key, 0.0) + float(X[m, j].sum())
                 if shaped is not None:
                     a["shaped_return"] = a.get("shaped_return", 0.0) + float(shaped[m].sum())
+        if S is not None and len(e.preference_sets) > 1:      # mixed preferences: means over the (env, agent) pairs of each set
+            sid = e.preference_of[np.zeros(len(R), np.int64) if vid is None else vid]
+            acc = self._pstats.setdefault(bool(test_mode), {})
+            for k in np.unique(sid):
+                m = sid == k
+                a = acc.setdefault(int(k), {"n": 0, "return": 0.0, "shaped_return": 0.0})
+                a["n"] += int(m.sum())
+                a["return"] += float(R[m].sum())
+                a["shaped_return"] += float(S[m].sum())
 
         self._account(env_info, returns, test_mode)
         return self.batch
@@ -299,5 +311,8 @@ class BatchedEpisodeRunner:
             extra = tuple(q for q in SOCIAL_KEYS + ("shaped_return",) if q in a)
             for key in ("return", "collective_return", "equality_metric") + extra:
                 log(f"{prefix}v{k}_{key}_mean", a[key] / a["n"], self.t_env)
+        for k, a in sorted(self._pstats.pop(prefix == "test_", {}).items()):
+            for key in ("return", "shaped_return"):
+                log(f"{prefix}pref{k}_{key}_mean", a[key] / a["n"], self.t_env)
         rets.clear()
         stats.clear()

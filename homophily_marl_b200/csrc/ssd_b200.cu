@@ -1465,23 +1465,48 @@ __global__ void __launch_bounds__(256) zero_stats_kernel(uint32_t* __restrict__ 
     stats[i] = 0u;
 }
 
-// ------------------------------------------------------------------ shaped rewards (ssd_set_reward_shaping; DESIGN.md §3 item 17)
-// One parameter set as the kernel reads it: a = alpha/(n-1), b = beta/(n-1) and w1 = 1 - w are precomputed on the host in fp32.
-struct ShapeDev { float a, b, decay, w, w1; };
+// ------------------------------------------------------------------ shaped rewards (ssd_set_reward_preferences; DESIGN.md §3 items 17, 20)
+// One preference set as the kernel reads it: a = alpha/(n-1), b = beta/(n-1) and w1 = 1 - w are precomputed on the host in fp32;
+// svo = the target reward angle in radians, ws its weight (both 0 for ssd_set_reward_shaping).
+struct ShapeDev { float a, b, decay, w, w1, svo, ws; };
 
 struct ShapeParams {
     const int8_t* reward;                     // [B][n] the step's rewards
     const uint8_t* done;                      // [B] auto-reset launches only (NULL otherwise): a done env's trace restarts at 0
-    const uint8_t* variant_of;                // [B] or NULL: every env uses params[0]
+    const uint8_t* variant_of;                // [B] or NULL: every env uses params[0] (roster row 0)
     const ShapeDev* params; int n_params;
+    const uint8_t* set_of; int n_rows;        // [n_rows][n] each agent's set (a roster), or NULL: every agent takes its env's set
     float* trace; float* shaped;              // [B][NA]
     int n, NA, env0, env1;
 };
 
+// atan2 as one fixed fp32 sequence (include/ssd_b200.h, ssd_set_reward_preferences), so that the restatement
+// (tests/preference_ref.py) matches it bit for bit; atan2f and fast-math are not pinned.  The odd polynomial in q on [0, 1] is
+// a weighted least-squares fit (max error 2.5e-7 rad before fp32 rounding, 5.1e-7 after).
+__device__ __forceinline__ float atan2f_ssd(float y, float x) {
+    const float ax = fabsf(x), ay = fabsf(y);
+    const float mx = fmaxf(ax, ay), mn = fminf(ax, ay);
+    if (mx == 0.0f) return 0.0f;
+    const float q = __fdiv_rn(mn, mx);
+    const float s = __fmul_rn(q, q);
+    float p = 0.006811790633946657f;
+    p = __fadd_rn(__fmul_rn(p, s), -0.0336042121052742f);
+    p = __fadd_rn(__fmul_rn(p, s), 0.07962366193532944f);
+    p = __fadd_rn(__fmul_rn(p, s), -0.1323334127664566f);
+    p = __fadd_rn(__fmul_rn(p, s), 0.19807815551757812f);
+    p = __fadd_rn(__fmul_rn(p, s), -0.3331736922264099f);
+    p = __fadd_rn(__fmul_rn(p, s), 0.9999961256980896f);
+    float t = __fmul_rn(q, p);
+    if (ay > ax) t = __fsub_rn(1.57079637f, t);              // pi/2 and pi rounded to fp32
+    if (x < 0.0f) t = __fsub_rn(3.14159274f, t);
+    if (y < 0.0f) t = -t;
+    return t;
+}
+
 // One warp per env and one lane per agent, as in ssd_kernel.  Every operation is an explicitly rounded fp32 intrinsic, so nothing
-// is contracted into an FMA and the result is bit-exact against a NumPy float32 restatement (tests/shaping_ref.py).  The n-way
-// sums run over n shuffles in ascending j.  A kernel of its own after the step launch, so that no ssd_kernel instantiation
-// changes.
+// is contracted into an FMA and the result is bit-exact against a NumPy float32 restatement (tests/shaping_ref.py,
+// tests/preference_ref.py).  The n-way sums run over n shuffles in ascending j.  Each lane loads its own set.  A kernel of its own
+// after the step launch, so that no ssd_kernel instantiation changes.
 __global__ void __launch_bounds__(kWarps * 32) shape_rewards_kernel(const __grid_constant__ ShapeParams p) {
     // Under programmatic dependent launch (small launches, as the step launch before it): wait for the step's outputs, and let
     // the next step launch of the stream become resident and run its prologue meanwhile (it still waits for this whole grid).
@@ -1491,27 +1516,39 @@ __global__ void __launch_bounds__(kWarps * 32) shape_rewards_kernel(const __grid
     const int lane = threadIdx.x & 31;
     const int env = p.env0 + blockIdx.x * kWarps + (threadIdx.x >> 5);
     if (env >= p.env1) return;
-    const int pid = p.variant_of ? min((int)__ldcg(p.variant_of + env), p.n_params - 1) : 0;
-    const ShapeDev s = p.params[pid];
     const bool is_agent = lane < p.n;
+    int pid;
+    if (p.set_of) {
+        const int row = p.variant_of ? min((int)__ldcg(p.variant_of + env), p.n_rows - 1) : 0;
+        pid = is_agent ? (int)p.set_of[row * p.n + lane] : 0;
+    } else {
+        pid = p.variant_of ? min((int)__ldcg(p.variant_of + env), p.n_params - 1) : 0;
+    }
+    const ShapeDev s = p.params[pid];
     // mutable buffers are read past L1, as in ssd_kernel: concurrent env ranges may share a line at a range boundary
     const int ri = is_agent ? (int)__ldcg(p.reward + (size_t)env * p.n + lane) : 0;
     const size_t at = (size_t)env * p.NA + lane;
     const float r = (float)ri;
     const float e = __fadd_rn(__fmul_rn(is_agent ? __ldcg(p.trace + at) : 0.0f, s.decay), r);
     int sum = 0;
-    float D = 0.0f, A = 0.0f;
+    float D = 0.0f, A = 0.0f, O = 0.0f;
     for (int j = 0; j < p.n; ++j) {
         const float ej = __shfl_sync(0xffffffffu, e, j);
         sum += __shfl_sync(0xffffffffu, ri, j);
         if (j != lane) {
             D = __fadd_rn(D, fmaxf(__fsub_rn(ej, e), 0.0f));
             A = __fadd_rn(A, fmaxf(__fsub_rn(e, ej), 0.0f));
+            O = __fadd_rn(O, ej);
         }
     }
     const float c = __fdiv_rn((float)sum, (float)p.n);
     const float m = __fadd_rn(__fmul_rn(s.w1, r), __fmul_rn(s.w, c));
-    const float u = __fsub_rn(__fsub_rn(m, __fmul_rn(s.a, D)), __fmul_rn(s.b, A));
+    float v = 0.0f;                                           // social value orientation: ws*|th* - angle(others' mean, own)|
+    if (p.n > 1 && s.ws != 0.0f) {
+        const float o = __fdiv_rn(O, (float)(p.n - 1));
+        v = __fmul_rn(s.ws, fabsf(__fsub_rn(s.svo, atan2f_ssd(o, e))));
+    }
+    const float u = __fsub_rn(__fsub_rn(__fsub_rn(m, __fmul_rn(s.a, D)), __fmul_rn(s.b, A)), v);
     if (is_agent) {
         p.shaped[at] = u;
         p.trace[at] = (p.done && __ldcg(p.done + env)) ? 0.0f : e;
@@ -1613,6 +1650,8 @@ struct ssd_handle {
     int tag_any;                                              // some variant of the table has tag_timeout > 0
     ShapeDev* d_shape;                                        // shaping table: SSD_MAX_VARIANTS records, allocated once when first needed
     int n_shape;                                              // entries in use; 0 = shaping off
+    uint8_t* d_roster;                                        // roster: SSD_MAX_VARIANTS x SSD_MAX_AGENTS bytes, allocated once when first needed
+    int n_roster;                                             // roster rows in use; 0 = each agent takes its env's set
     float* shape_trace; float* shaped;                        // caller-owned [B][NA] (ssd_set_reward_shaping)
     const uint8_t* mask_obs; uint32_t* mask_obs_bits;         // ssd_set_obs_mask: the buffers the row masks describe, and the masks
     const uint8_t* mask_end_obs; uint32_t* mask_end_bits;
@@ -1693,6 +1732,7 @@ static int launch_shaping(ssd_handle* h, const KParams& k, const uint8_t* done, 
     SSD_CUDA(guard.err);
     ShapeParams s;
     s.reward = k.reward; s.done = done; s.variant_of = k.variant_of; s.params = h->d_shape; s.n_params = h->n_shape;
+    s.set_of = h->n_roster ? h->d_roster : nullptr; s.n_rows = h->n_roster;
     s.trace = h->shape_trace; s.shaped = h->shaped;
     s.n = k.n; s.NA = k.NA; s.env0 = k.env0; s.env1 = k.env1;
     cudaLaunchConfig_t cfg = {};
@@ -1936,6 +1976,7 @@ int ssd_destroy(ssd_handle* h) {
     cudaFree(h->d_map);
     if (h->d_vars) cudaFree(h->d_vars);
     if (h->d_shape) cudaFree(h->d_shape);
+    if (h->d_roster) cudaFree(h->d_roster);
     delete h->base;
     delete h;
     return SSD_OK;
@@ -2057,32 +2098,57 @@ int ssd_set_stats(ssd_handle* h, uint32_t* stats, uint32_t* end_stats) {
 }
 
 int ssd_set_reward_shaping(ssd_handle* h, int32_t n_params, const ssd_shaping* params, float* trace, float* shaped) {
-    if (!h || n_params < 0 || n_params > SSD_MAX_VARIANTS || (n_params > 0 && !params)) return SSD_ERR_INVALID;
-    if ((trace == nullptr) != (shaped == nullptr) || (trace != nullptr) != (n_params > 0)) return SSD_ERR_INVALID;
-    ShapeDev recs[SSD_MAX_VARIANTS];
+    if (n_params < 0 || n_params > SSD_MAX_VARIANTS || (n_params > 0 && !params)) return SSD_ERR_INVALID;
+    ssd_preference sets[SSD_MAX_VARIANTS];
+    for (int i = 0; i < n_params; ++i)
+        sets[i] = ssd_preference{params[i].alpha, params[i].beta, params[i].decay, params[i].prosocial, 0.0f, 0.0f};
+    return ssd_set_reward_preferences(h, n_params, sets, 0, nullptr, trace, shaped);
+}
+
+int ssd_set_reward_preferences(ssd_handle* h, int32_t n_sets, const ssd_preference* sets, int32_t n_rows, const uint8_t* set_of,
+                               float* trace, float* shaped) {
+    if (!h || n_sets < 0 || n_sets > SSD_MAX_VARIANTS || (n_sets > 0 && !sets)) return SSD_ERR_INVALID;
+    if (n_rows < 0 || n_rows > SSD_MAX_VARIANTS || (n_rows > 0 && !set_of)) return SSD_ERR_INVALID;
+    if ((trace == nullptr) != (shaped == nullptr) || (trace != nullptr) != (n_sets > 0)) return SSD_ERR_INVALID;
     const int n = h->kp.n;
-    for (int i = 0; i < n_params; ++i) {
-        const ssd_shaping& q = params[i];
-        if (!isfinite(q.alpha) || !isfinite(q.beta) || !isfinite(q.decay) || !isfinite(q.prosocial)) return SSD_ERR_INVALID;
-        if (q.alpha < 0.0f || q.beta < 0.0f || q.decay < 0.0f || q.decay > 1.0f || q.prosocial < 0.0f || q.prosocial > 1.0f)
+    for (int i = 0; i < n_rows * n; ++i)
+        if (set_of[i] >= n_sets) return SSD_ERR_INVALID;
+    ShapeDev recs[SSD_MAX_VARIANTS];
+    const float pi = 3.14159274f;                             // pi rounded to fp32, the value of float32(math.radians(180))
+    for (int i = 0; i < n_sets; ++i) {
+        const ssd_preference& q = sets[i];
+        if (!isfinite(q.alpha) || !isfinite(q.beta) || !isfinite(q.decay) || !isfinite(q.prosocial) || !isfinite(q.svo_angle) ||
+            !isfinite(q.svo_weight))
+            return SSD_ERR_INVALID;
+        if (q.alpha < 0.0f || q.beta < 0.0f || q.decay < 0.0f || q.decay > 1.0f || q.prosocial < 0.0f || q.prosocial > 1.0f ||
+            q.svo_angle < -pi || q.svo_angle > pi || q.svo_weight < 0.0f)
             return SSD_ERR_INVALID;
         const float others = (float)(n - 1);
         recs[i].a = n > 1 ? q.alpha / others : 0.0f;
         recs[i].b = n > 1 ? q.beta / others : 0.0f;
         recs[i].decay = q.decay; recs[i].w = q.prosocial; recs[i].w1 = 1.0f - q.prosocial;
+        recs[i].svo = q.svo_angle; recs[i].ws = q.svo_weight;
     }
-    if (n_params > 0) {
+    if (n_sets > 0) {
         DeviceGuard guard(h->device);
         SSD_CUDA(guard.err);
-        if (!h->d_shape) {                                    // allocated once at full size: no launch ever reads a freed table
+        // both tables are allocated once at full size (no launch ever reads a freed table) before either changes, so that a
+        // failed allocation leaves the handle as it was
+        if (!h->d_shape) {
             ShapeDev* d = nullptr;
             SSD_CUDA(cudaMalloc(&d, sizeof(ShapeDev) * SSD_MAX_VARIANTS));
             h->d_shape = d;
         }
-        SSD_CUDA(cudaDeviceSynchronize());                    // no launch in flight reads the table while it changes
-        SSD_CUDA(cudaMemcpy(h->d_shape, recs, sizeof(ShapeDev) * n_params, cudaMemcpyHostToDevice));
+        if (n_rows > 0 && !h->d_roster) {
+            uint8_t* d = nullptr;
+            SSD_CUDA(cudaMalloc(&d, SSD_MAX_VARIANTS * SSD_MAX_AGENTS));
+            h->d_roster = d;
+        }
+        SSD_CUDA(cudaDeviceSynchronize());                    // no launch in flight reads the tables while they change
+        SSD_CUDA(cudaMemcpy(h->d_shape, recs, sizeof(ShapeDev) * n_sets, cudaMemcpyHostToDevice));
+        if (n_rows > 0) SSD_CUDA(cudaMemcpy(h->d_roster, set_of, (size_t)n_rows * n, cudaMemcpyHostToDevice));
     }
-    h->n_shape = n_params; h->shape_trace = trace; h->shaped = shaped;
+    h->n_shape = n_sets; h->n_roster = n_rows; h->shape_trace = trace; h->shaped = shaped;
     return SSD_OK;
 }
 

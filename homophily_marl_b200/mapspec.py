@@ -159,8 +159,11 @@ class MapSpec:
     thr_harvest: np.ndarray = field(default=None, repr=False)
     lut: np.ndarray = field(default=None, repr=False)
     # a variant's own shaped-reward parameters (compile_variant key "reward_shaping"): (alpha, beta, decay, prosocial) as
-    # float32 values, or None for the handle's
+    # float32 values when it gives one dict, or None for the handle's; `preferences` holds every agent's full set
     reward_shaping: tuple = None
+    # a variant's own preference sets (reward_preferences): one (alpha, beta, decay, prosocial, svo_angle in radians,
+    # svo_weight) tuple per agent, or None for the handle's
+    preferences: tuple = None
 
     @property
     def G(self):
@@ -244,8 +247,8 @@ def compile_variant(base: MapSpec, overrides: dict) -> MapSpec:
     """One env variant (``ssd_set_variants``): ``base`` (the handle's creation spec) with ``overrides`` applied.  Keys:
     ``rows`` (an ASCII layout of base's exact H x W), ``fire_cost``, ``hit_penalty``, ``tag_timeout``, and the spawn
     dynamics of the kind -- Cleanup ``threshold_depletion``, ``threshold_restoration``, ``waste_spawn_prob``,
-    ``apple_respawn_prob``; Harvest ``spawn_prob`` (4 probabilities); ``reward_shaping`` (a ``reward_shaping`` dict, see
-    there; absent: the handle's).  ``{}`` is the base config.  Everything else (kind, size, view, agents, episode limit,
+    ``apple_respawn_prob``; Harvest ``spawn_prob`` (4 probabilities); ``reward_shaping`` (a ``reward_shaping`` dict, or a
+    list of one per agent, see ``reward_preferences``; absent: the handle's).  ``{}`` is the base config.  Everything else (kind, size, view, agents, episode limit,
     colours) stays the handle's."""
     ov = dict(overrides or {})
     allowed = VARIANT_KEYS[base.kind]
@@ -271,29 +274,56 @@ def compile_variant(base: MapSpec, overrides: dict) -> MapSpec:
                        hit_penalty=int(ov.get("hit_penalty", base.hit_penalty)),
                        tag_timeout=int(ov.get("tag_timeout", base.tag_timeout)))
     if "reward_shaping" in ov:
-        spec.reward_shaping = reward_shaping(ov["reward_shaping"])
+        spec.preferences = reward_preferences(ov["reward_shaping"], base.n_agents)
+        if isinstance(ov["reward_shaping"], dict):
+            spec.reward_shaping = spec.preferences[0][:4]
     return spec
 
 
 # Shaped rewards (ssd_set_reward_shaping; DESIGN.md §3 item 17): inequity aversion (Hughes et al., 2018) and prosocial mixing
-# (Peysakhovich & Lerer, 2018).  The default decay is Hughes' gamma * lambda = 0.99 * 0.975, in float32.
+# (Peysakhovich & Lerer, 2018).  The default decay is Hughes' gamma * lambda = 0.99 * 0.975, in float32.  Item 20
+# (ssd_set_reward_preferences) adds a social value orientation (McKee et al., 2020): a target reward angle svo_angle, given in
+# degrees (0 individualistic, 45 prosocial, 90 altruistic) and kept in float32 radians, and its weight svo_weight.
 SHAPING_KEYS = ("alpha", "beta", "decay", "prosocial")
 SHAPING_DEFAULTS = {"alpha": 0.0, "beta": 0.0, "decay": float(np.float32(0.99 * 0.975)), "prosocial": 0.0}
+PREFERENCE_KEYS = SHAPING_KEYS + ("svo_angle", "svo_weight")
 
 
-def reward_shaping(params: dict) -> tuple:
-    """``(alpha, beta, decay, prosocial)`` as float32 values from a ``reward_shaping`` dict: unknown keys are refused, missing
-    ones take ``SHAPING_DEFAULTS``; every value must be finite, alpha and beta >= 0, decay and prosocial in [0, 1]."""
-    unknown = set(params) - set(SHAPING_KEYS)
+def preference(params: dict) -> tuple:
+    """``(alpha, beta, decay, prosocial, svo_angle, svo_weight)`` as float32 values from one ``reward_shaping`` dict (svo_angle
+    converted once from degrees to radians): unknown keys are refused, missing ones take ``SHAPING_DEFAULTS`` (svo_angle and
+    svo_weight 0); every value must be finite, alpha, beta and svo_weight >= 0, decay and prosocial in [0, 1], svo_angle in
+    [-180, 180] degrees."""
+    if not isinstance(params, dict):
+        raise ValueError(f"reward_shaping needs a dict of {list(PREFERENCE_KEYS)}, got {params!r}")
+    unknown = set(params) - set(PREFERENCE_KEYS)
     if unknown:
-        raise ValueError(f"unknown reward_shaping keys {sorted(unknown)}; allowed: {list(SHAPING_KEYS)}")
+        raise ValueError(f"unknown reward_shaping keys {sorted(unknown)}; allowed: {list(PREFERENCE_KEYS)}")
     with np.errstate(over="ignore"):                        # a value past the float32 range becomes inf and is refused below
         vals = tuple(float(np.float32(params.get(k, SHAPING_DEFAULTS[k]))) for k in SHAPING_KEYS)
+        deg, weight = float(params.get("svo_angle", 0.0)), float(np.float32(params.get("svo_weight", 0.0)))
     alpha, beta, decay, prosocial = vals
     if not all(math.isfinite(v) for v in vals) or alpha < 0 or beta < 0 or not 0 <= decay <= 1 or not 0 <= prosocial <= 1:
         raise ValueError("reward_shaping needs finite alpha, beta >= 0 and decay, prosocial in [0, 1], got "
                          f"{dict(zip(SHAPING_KEYS, vals))}")
-    return vals
+    if not (math.isfinite(deg) and -180 <= deg <= 180 and math.isfinite(weight) and weight >= 0):
+        raise ValueError(f"reward_shaping needs svo_angle in [-180, 180] degrees and a finite svo_weight >= 0, got {deg}, {weight}")
+    return vals + (float(np.float32(math.radians(deg))), weight)
+
+
+def reward_shaping(params: dict) -> tuple:
+    """``(alpha, beta, decay, prosocial)`` of one ``reward_shaping`` dict, validated as ``preference`` validates it."""
+    return preference(params)[:4]
+
+
+def reward_preferences(value, n_agents: int) -> tuple:
+    """Every agent's preference set (``preference``) from a ``reward_shaping`` value: one dict for every agent, or a list of
+    ``n_agents`` dicts, one per agent."""
+    if isinstance(value, dict):
+        return (preference(value),) * n_agents
+    if not isinstance(value, (list, tuple)) or len(value) != n_agents:
+        raise ValueError(f"reward_shaping needs one dict or a list of {n_agents} dicts (one per agent), got {value!r}")
+    return tuple(preference(d) for d in value)
 
 
 def dump_maps() -> str:

@@ -318,8 +318,39 @@ typedef struct ssd_shaping {
  * trace without shaped or shaped without trace, buffers without parameters or parameters without buffers, or a parameter that is
  * not finite or outside its range.  On an error nothing changes.  A configuration call, serialised like ssd_set_obs_format: the
  * parameter table is allocated once at its full size and overwritten after a device synchronise, so no launch ever reads a freed
- * table; a CUDA graph keeps the buffer pointers it was captured with. */
+ * table; a CUDA graph keeps the buffer pointers it was captured with.
+ * Equivalent to ssd_set_reward_preferences(h, n_params, sets, 0, NULL, trace, shaped) with svo_angle = svo_weight = 0. */
 int ssd_set_reward_shaping(ssd_handle* h, int32_t n_params, const ssd_shaping* params, float* trace, float* shaped);
+
+/* One preference set (ssd_set_reward_preferences): the four values of ssd_shaping plus a social value orientation (McKee et
+ * al., 2020) -- the target reward angle svo_angle in fp32 radians, in [-pi, pi] (pi rounded to fp32; 0 individualistic, pi/4
+ * prosocial, pi/2 altruistic), and its weight svo_weight >= 0.  Every value finite. */
+typedef struct ssd_preference {
+    float alpha, beta, decay, prosocial, svo_angle, svo_weight;
+} ssd_preference;
+
+/* Shaped rewards with a preference set per agent (DESIGN.md §3 item 20; extends ssd_set_reward_shaping, whose buffers, resets,
+ * launches and graph behaviour it keeps).  Agent i of env b uses set s = set_of[row][i] with row = min(variant_of[b], n_rows-1)
+ * (row 0 without per-env variant ids) when a roster is given (n_rows > 0; set_of: HOST u8 [n_rows][n_agents], copied), else
+ * s = min(variant_of[b], n_sets-1) (0 without ids), as ssd_set_reward_shaping.  With a, b, w1 precomputed per set as there, and
+ * th* = svo_angle, ws = svo_weight, each agent computes, in fp32 with every operation rounded once in this order:
+ *   e_i <- e_i*decay_i + r_i;  c = (sum_j r_j)/n;  m_i = w1_i*r_i + prosocial_i*c;
+ *   D_i, A_i as ssd_set_reward_shaping;  o_i = (sum_{j != i} e_j)/(n-1) (ascending j, updated traces);
+ *   v_i = ws_i*|th*_i - atan2f_ssd(o_i, e_i)|  (v_i = +0 when n = 1 or ws_i = 0: the angle is not computed);
+ *   shaped_i = ((m_i - a_i*D_i) - b_i*A_i) - v_i.
+ * atan2f_ssd(y, x) is a fixed fp32 sequence, within 2e-6 rad of the exact angle for finite inputs (DESIGN.md §3 item 20):
+ *   ax = |x|, ay = |y|, mx = max(ax, ay), mn = min(ax, ay); mx == 0 gives 0;  q = mn/mx, s = q*q;
+ *   t = q*(((((( C6*s + C5)*s + C4)*s + C3)*s + C2)*s + C1)*s + C0)  with
+ *   C0 = 0.9999961256980896, C1 = -0.3331736922264099, C2 = 0.19807815551757812, C3 = -0.1323334127664566,
+ *   C4 = 0.07962366193532944, C5 = -0.0336042121052742, C6 = 0.006811790633946657 (each exactly an fp32 value);
+ *   ay > ax: t = pi/2 - t;  x < 0: t = pi - t;  y < 0: t = -t  (pi/2 and pi rounded to fp32).
+ * With every svo_weight 0 and no roster the result is that of ssd_set_reward_shaping bit for bit.
+ * SSD_ERR_INVALID, before any CUDA call and changing nothing, for a NULL handle, n_sets or n_rows outside 0..SSD_MAX_VARIANTS,
+ * NULL sets with n_sets > 0, NULL set_of with n_rows > 0, a roster entry >= n_sets, a field that is not finite or outside its
+ * range, or the buffer mismatches ssd_set_reward_shaping refuses.  The set table and the roster table (SSD_MAX_VARIANTS x
+ * SSD_MAX_AGENTS bytes) are allocated once at full size and overwritten after a device synchronise. */
+int ssd_set_reward_preferences(ssd_handle* h, int32_t n_sets, const ssd_preference* sets, int32_t n_rows, const uint8_t* set_of,
+                               float* trace, float* shaped);
 
 /* MapEnv.reset (map_env.py:986-993 -> _reset 297-326).  mask: [B] bytes, non-zero = reset this
  * env, NULL = all.  When obs != NULL the first observations are rendered too. */
